@@ -39,6 +39,7 @@ sys.path.insert(0, ROOT)
 METRIC = "mesh-sample kNN transfers/sec"
 UNIT = "samples/s"
 CPU_POINT_BUDGET = 64_000_000     # host arm: larger clouds are timed on a same-density patch
+DUMP_BYTES = 64 << 20             # --dump-outputs: larger outputs are written as a seeded row sample
 
 
 def parse_args():
@@ -60,7 +61,15 @@ def parse_args():
     ap.add_argument("--profile-steps", type=int, default=0,
                     help="diagnosis: after the timed region run this many steps under torch.profiler and "
                          "print rank 0's kernel table to stderr (never part of a reported number)")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what the last timed step returned (idx, rgba, normal) as DIR/<name>.npy "
+                         "in float64 / float32, for comparing two builds output for output")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs writes the GPU arm's outputs")
+    return args
 
 
 def algorithmic_bytes_per_sample(k):
@@ -282,7 +291,7 @@ def cpu_leg(pto, w, n, gu, gv, k, steps, warmup):
             "sample": what + "; CGAL-style kd-tree (sliding midpoint, bucket 10) + blend, OpenMP "
                              f"over samples; generated on the host in {gen_s:.1f} s, tree build "
                              f"{build_s:.1f} s, both excluded",
-            "build_s": build_s, "ms_per_step": t * 1e3}
+            "build_s": build_s, "ms_per_step": t * 1e3, "steps": max(1, steps)}
 
 
 def run_reference_arm(args, pkg, world, rank):
@@ -386,6 +395,32 @@ def verify_by_ball(pkg, pto, torch, dist, world, rank, dev, own_pos, own_attrs, 
             raise SystemExit(f"rank {rank}: verification failed (normal) at sample {int(sel[i])}")
         checked += 1
     return checked
+
+
+def dump_outputs(directory, dist, world, rank, out, rows, M, k):
+    """Write the step's outputs as DIR/<name>.npy: idx (float64, -1 where a list is short),
+    rgba and normal (float32), one row per sample, and sample_index (float64), the row of the
+    one global sample array each output row belongs to.  Where M rows would exceed DUMP_BYTES, a
+    fixed, seeded subset of rows is written.  rows: this rank's global sample rows (numpy)."""
+    import numpy as np
+    row_bytes = 8 * k + 4 * 4 + 4 * 3 + 8
+    n_keep = min(M, DUMP_BYTES // row_bytes)
+    keep = np.arange(M) if n_keep == M else \
+        np.random.default_rng(20261020).choice(M, n_keep, replace=False)
+    mask = np.isin(rows, keep)
+    parts = [(rows[mask], {name: t.cpu().numpy()[mask] for name, t in out.items()})]
+    if world > 1:
+        mine, parts = parts[0], [None] * world
+        dist.all_gather_object(parts, mine)
+    if rank != 0:
+        return
+    ids = np.concatenate([p[0] for p in parts])
+    order = np.argsort(ids)
+    os.makedirs(directory, exist_ok=True)
+    np.save(os.path.join(directory, "sample_index.npy"), ids[order].astype(np.float64))
+    for name, dtype in (("idx", np.float64), ("rgba", np.float32), ("normal", np.float32)):
+        a = np.concatenate([p[1][name] for p in parts])[order]
+        np.save(os.path.join(directory, name + ".npy"), a.astype(dtype))
 
 
 def timed_steps(pkg, torch, dist, world, dev, step, flush, steps, warmup):
@@ -545,6 +580,10 @@ def main():
     ms_per_step, ms_per_rank, host_issue_ms, launches = timed_steps(pkg, torch, dist, world, dev, step, flush,
                                                                     args.steps, args.warmup)
     clocks = sampler.stop()
+    if args.dump_outputs:
+        import numpy as np
+        rows = np.arange(M) if world == 1 else perm[rank::world].cpu().numpy()
+        dump_outputs(args.dump_outputs, dist, world, rank, out, rows, M, k)
     if args.profile_steps > 0:
         from torch.profiler import profile, ProfilerActivity
         with profile(activities=[ProfilerActivity.CUDA, ProfilerActivity.CPU]) as prof:
@@ -619,11 +658,10 @@ def main():
         e2e_step()
     if world > 1:
         dist.barrier()
-    e2e_steps = max(3, min(args.steps, 20))
     t0 = time.perf_counter()
-    for _ in range(e2e_steps):
+    for _ in range(args.steps):
         e2e_step()
-    e2e_s = (time.perf_counter() - t0) / e2e_steps
+    e2e_s = (time.perf_counter() - t0) / args.steps
     t = torch.tensor([e2e_s], dtype=torch.float64, device=dev)
     if world > 1:
         dist.all_reduce(t, op=dist.ReduceOp.MAX)
@@ -640,9 +678,9 @@ def main():
         for _ in range(3):
             tree.transfer(qh_np, k, radius=w.radius, want_idx=False, out=o_b)
         t0 = time.perf_counter()
-        for _ in range(e2e_steps):
+        for _ in range(args.steps):
             tree.transfer(qh_np, k, radius=w.radius, want_idx=False, out=o_b)
-        b_s = (time.perf_counter() - t0) / e2e_steps
+        b_s = (time.perf_counter() - t0) / args.steps
         blend_only = {"value": M / b_s, "ms_per_step": b_s * 1e3, "d2h_bytes_per_step": m * 16}
 
     variant_used = pkg.get_option("knn_variant")

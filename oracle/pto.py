@@ -38,16 +38,24 @@ _REF_PATH = os.path.join(_HERE, "_ref", "libref_metric.so")
 _ref = None
 
 
+def reference_src():
+    """The original project's src/ directory, named by the PT_REFERENCE_SRC environment variable
+    (it is not part of this repository), or None where it is not set or holds no Distance.h."""
+    src = os.environ.get("PT_REFERENCE_SRC")
+    return src if src and os.path.exists(os.path.join(src, "Distance.h")) else None
+
+
 def ref_metric():
-    """The reference's OWN src/Point.h + src/Distance.h compiled by `make -C oracle ref`
-    (oracle/ref_shim.cpp), or None where it was never built (/root/reference absent)."""
+    """The reference's OWN src/Point.h + src/Distance.h compiled by `make -C oracle ref REF=<src>`
+    (oracle/ref_shim.cpp), or None where it was never built and no reference_src() is given."""
     global _ref
     if _ref is None:
         if not os.path.exists(_REF_PATH):
-            if os.path.exists("/root/reference/src/Distance.h"):
-                subprocess.run(["make", "-C", _HERE, "-s", "ref"], check=True, stdout=subprocess.DEVNULL)
-            else:
+            src = reference_src()
+            if src is None:
                 return None
+            subprocess.run(["make", "-C", _HERE, "-s", "ref", "REF=" + src], check=True,
+                           stdout=subprocess.DEVNULL)
         R = ctypes.CDLL(_REF_PATH)
         vp, dbl = ctypes.c_void_p, ctypes.c_double
         R.ref_point_layout.argtypes = [vp]

@@ -1,8 +1,8 @@
 /*
  * ref_shim.cpp -- TEST INFRASTRUCTURE: exposes the reference's OWN metric code through a C ABI.
  *
- * It compiles /root/reference/src/Point.h and src/Distance.h from where they lie (the build
- * recipe passes -I to that directory; nothing is copied into this repository) against a minimal
+ * It compiles the reference's src/Point.h and src/Distance.h from where they lie (the build
+ * recipe passes -I$(REF) to that directory; nothing is copied into this repository) against a minimal
  * stand-in for the only two CGAL names Distance.h mentions (src/Distance.h:4,14:
  * CGAL::Dimension_tag, CGAL::Kd_tree_rectangle with min_coord / max_coord).  CGAL's kd-tree search
  * itself is absent from this image, so the neighbour SEARCH stays unpinned; what this pins, bit
@@ -12,7 +12,7 @@
  *   - Distance::new_distance                          src/Distance.h:92-95
  *   - Distance::transformed_distance(d) / inverse     src/Distance.h:97,99
  *   - sizeof(Point) and its field offsets             src/Point.h:1-6
- * Output: oracle/_ref/libref_metric.so (git-ignored; built only where /root/reference exists).
+ * Output: oracle/_ref/libref_metric.so (git-ignored; built only where PT_REFERENCE_SRC is set).
  * Only tests/ may load it.
  */
 #include <cmath>
@@ -29,7 +29,7 @@ template <class FT, class D> struct Kd_tree_rectangle {
 };
 }  // namespace CGAL
 
-#include "Point.h"      // the reference's, via -I/root/reference/src
+#include "Point.h"      // the reference's, via -I$(REF)
 #include "Distance.h"   // the reference's
 
 extern "C" {

@@ -70,3 +70,41 @@ def test_traffic_record_belongs_to_the_shipped_kernel_source():
     rec = bench.ncu_traffic("cfg2", 16, "knn_grid_pair_kernel")
     assert rec is not None and rec["dram_bytes"] > 0
 
+
+
+def test_dump_outputs_writes_the_step_outputs(tmp_path):
+    """--dump-outputs: every output of the step as float64 / float32 .npy in sample order; above
+    the byte budget the same seeded rows on every call."""
+    import numpy as np
+    import torch
+    sys.path.insert(0, ROOT)
+    import importlib
+    bench = importlib.import_module("bench")
+    rng = np.random.default_rng(5)
+    M, k = 1000, 4
+    out = {"idx": torch.from_numpy(rng.integers(-1, 10**6, (M, k), dtype=np.int32)),
+           "rgba": torch.from_numpy(rng.integers(0, 256, (M, 4), dtype=np.uint8)),
+           "normal": torch.from_numpy(rng.standard_normal((M, 3)).astype(np.float32))}
+    bench.dump_outputs(str(tmp_path / "all"), None, 1, 0, out, np.arange(M), M, k)
+    got = {n: np.load(tmp_path / "all" / (n + ".npy")) for n in ("idx", "rgba", "normal", "sample_index")}
+    assert got["idx"].dtype == np.float64 and got["rgba"].dtype == np.float32
+    assert got["normal"].dtype == np.float32 and got["sample_index"].dtype == np.float64
+    assert np.array_equal(got["sample_index"], np.arange(M))
+    for n in ("idx", "rgba", "normal"):
+        assert np.array_equal(got[n], out[n].numpy())
+    # a share of the rows in another order (one rank of several), over a small budget
+    bench.DUMP_BYTES, budget = 100 * (8 * k + 36), bench.DUMP_BYTES
+    try:
+        perm = rng.permutation(M)          # local row i holds global sample perm[i]
+        bench.dump_outputs(str(tmp_path / "a"), None, 1, 0, out, np.arange(M), M, k)
+        bench.dump_outputs(str(tmp_path / "b"), None, 1, 0,
+                           {n: t[torch.from_numpy(perm)] for n, t in out.items()}, perm, M, k)
+    finally:
+        bench.DUMP_BYTES = budget
+    a = {n: np.load(tmp_path / "a" / (n + ".npy")) for n in got}
+    b = {n: np.load(tmp_path / "b" / (n + ".npy")) for n in got}
+    assert len(a["sample_index"]) == 100
+    sel = a["sample_index"].astype(np.int64)
+    for n in got:
+        assert np.array_equal(a[n], b[n])
+    assert np.array_equal(a["idx"], got["idx"][sel])

@@ -34,6 +34,56 @@ def write_mesh(path, V, F):
             f.write("3 %d %d %d\n" % (a, b, c))
 
 
+def read_png_bgra(path):
+    """Decode an 8-bit RGBA, non-interlaced PNG (every chunk CRC checked, all five scanline
+    filters) into B G R A rows, the layout cv::imread(..., IMREAD_UNCHANGED) returns."""
+    import struct
+    import zlib
+    data = open(path, "rb").read()
+    assert data[:8] == b"\x89PNG\r\n\x1a\n", "not a PNG"
+    pos, idat, hdr = 8, b"", None
+    while pos < len(data):
+        n, kind = struct.unpack(">I4s", data[pos:pos + 8])
+        body = data[pos + 8:pos + 8 + n]
+        assert struct.unpack(">I", data[pos + 8 + n:pos + 12 + n])[0] == zlib.crc32(kind + body), kind
+        pos += 12 + n
+        if kind == b"IHDR":
+            hdr = struct.unpack(">IIBBBBB", body)
+        elif kind == b"IDAT":
+            idat += body
+        elif kind == b"IEND":
+            break
+    w, h, depth, ctype, _, _, interlace = hdr
+    assert (depth, ctype, interlace) == (8, 6, 0), hdr
+    raw = zlib.decompress(idat)
+    stride, bpp = 4 * w, 4
+    assert len(raw) == h * (stride + 1)
+    out = np.zeros((h, stride), np.uint8)
+    prev = np.zeros(stride, np.int64)
+    for y in range(h):
+        f, line = raw[y * (stride + 1)], np.frombuffer(raw, np.uint8, stride, y * (stride + 1) + 1)
+        cur = line.astype(np.int64)
+        if f == 2:
+            cur = (cur + prev) & 255
+        elif f in (1, 3, 4):
+            cur = cur.copy()
+            for x in range(stride):
+                a = cur[x - bpp] if x >= bpp else 0
+                c = prev[x - bpp] if x >= bpp else 0
+                if f == 1:
+                    pred = a
+                elif f == 3:
+                    pred = (a + prev[x]) // 2
+                else:
+                    pa, pb, pc = abs(prev[x] - c), abs(a - c), abs(a + prev[x] - 2 * c)
+                    pred = a if pa <= pb and pa <= pc else (prev[x] if pb <= pc else c)
+                cur[x] = (cur[x] + pred) & 255
+        else:
+            assert f == 0, f"scanline filter {f}"
+        out[y], prev = cur, cur
+    return out.reshape(h, w, 4)[..., [2, 1, 0, 3]]
+
+
 def test_usage_and_missing_files(cli, tmp_path):
     r = subprocess.run([cli], capture_output=True, text=True)
     assert r.returncode == 0       # the reference returns 0 on usage (:116-120)
@@ -93,9 +143,8 @@ def test_cli_end_to_end(cli, pkg, pto, tmp_path):
         assert label in r.stdout, label
     # the reference's artefact: texture.png in the working directory (:613), equal to the oracle's
     # restatement of the face loop + post-process on the same inputs (K = 20, :128)
-    import cv2
-    png = cv2.imread(str(tmp_path / "texture.png"), cv2.IMREAD_UNCHANGED)       # BGRA, as cv::Mat
-    assert png is not None and png.shape == (512, 512, 4)
+    png = read_png_bgra(tmp_path / "texture.png")                                # BGRA, as cv::Mat
+    assert png.shape == (512, 512, 4)
     Vm = V.copy()
     Vm["color"] = np.array([10, 20, 30])                  # what write_mesh put in the file
     idx, d2 = pto.knn_bruteforce(P, Vm, 20)

@@ -115,7 +115,7 @@ def test_gpu_d2_is_the_reference_metric(pkg, pto, torch_cuda):
     reference's header) computes for that (sample, neighbour) pair."""
     R = pto.ref_metric()
     if R is None:
-        pytest.skip("oracle/_ref was never built (/root/reference absent at build time)")
+        pytest.skip("needs the reference's own headers: set PT_REFERENCE_SRC to its src/ directory")
     P = pkg.synth.cloud_host(100_000, seed=3, side=50.0)
     V = pkg.synth.samples_host(40, side=50.0)
     for variant in (6, 5, 2, 0):

@@ -73,8 +73,7 @@ def test_texture_from_lists_equals_oracle(pkg, pto, torch_cuda):
 
 def test_cli_with_two_slabs(pkg, pto, torch_cuda, tmp_path):
     """`pointsTransfer -g 2`: the sharded C++ host end to end, same texture.png as the oracle."""
-    from test_cli import CLI, write_cloud, write_mesh
-    cv2 = pytest.importorskip("cv2")
+    from test_cli import CLI, read_png_bgra, write_cloud, write_mesh
     if not os.path.exists(CLI):
         subprocess.run(["make", "-C", os.path.dirname(CLI)], check=True, stdout=subprocess.DEVNULL)
     P = pkg.synth.cloud_host(20_000, 3, side=20.0)
@@ -87,9 +86,9 @@ def test_cli_with_two_slabs(pkg, pto, torch_cuda, tmp_path):
     r = subprocess.run([CLI, "-g", "2", "-R", "512", str(tmp_path / "c.ply"), str(tmp_path / "m.ply")],
                        capture_output=True, text=True, cwd=tmp_path)
     assert r.returncode == 0 and "Draw triangles total time:" in r.stdout, r.stderr
-    png = cv2.imread(str(tmp_path / "texture.png"), cv2.IMREAD_UNCHANGED)
+    png = read_png_bgra(tmp_path / "texture.png")
     Vm = V.copy()
     Vm["color"] = np.array([10, 20, 30])
     idx, _ = pto.knn_bruteforce(P, Vm, 20)
     ref_img, _ = pto.texture(P, Vm, idx, F, 512, pad=True)
-    assert png is not None and np.array_equal(png, ref_img)
+    assert np.array_equal(png, ref_img)

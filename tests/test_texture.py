@@ -2,9 +2,12 @@
 (/root/reference src/pointsTransfer.cpp:462-611, draw_triangle :66-107).
 
 CPU part: the oracle's restatement (oracle/pt_texture_oracle.c) -- its post-process is pinned on
-OpenCV's own dilate / bitwise_not / bitwise_and / add (the calls of :593-611) through the cv2
-wheel; its Delaunay-by-definition is checked against scipy's Qhull Delaunay; the PNG the CLI
-writes is decoded back by cv2.  GPU part: pt_texture_render must equal the oracle bit for bit."""
+OpenCV's own dilate / bitwise_not / bitwise_and / add (the calls of :593-611), stored as golden
+data and, where the cv2 wheel is installed, recomputed; its Delaunay-by-definition is checked
+against scipy's Qhull Delaunay; the PNG the CLI writes is decoded back (test_cli.read_png_bgra,
+and cv2 where installed).  GPU part: pt_texture_render must equal the oracle bit for bit."""
+import os
+
 import numpy as np
 import pytest
 
@@ -17,20 +20,27 @@ def _mesh(pkg, g, side, colour=(200, 90, 30)):
     return V, pkg.synth.grid_faces(g, g)
 
 
-def test_pad_is_opencv_dilate_and_gutter(pto):
-    cv2 = pytest.importorskip("cv2")
-    rng = np.random.default_rng(1)
-    for res, fill in ((256, 0.3), (200, 0.02), (64, 1.0)):
-        img = np.zeros((res, res, 4), np.uint8)
-        m = rng.random((res, res)) < fill
-        img[m, :3] = rng.integers(0, 256, (int(m.sum()), 3))
-        img[m, 3] = 255
-        kern = cv2.getStructuringElement(cv2.MORPH_RECT, (25, 25))      # :595
-        dilated = cv2.dilate(img, kern)                                 # :598
-        bgra = cv2.split(img)                                           # :601
-        alpha_mask = cv2.bitwise_not(cv2.merge([bgra[3]] * 4))          # :603-607
-        padded = cv2.add(img, cv2.bitwise_and(dilated, alpha_mask))     # :609-612
+def _opencv_pad(cv2, img):
+    kern = cv2.getStructuringElement(cv2.MORPH_RECT, (25, 25))      # :595
+    dilated = cv2.dilate(img, kern)                                 # :598
+    bgra = cv2.split(img)                                           # :601
+    alpha_mask = cv2.bitwise_not(cv2.merge([bgra[3]] * 4))          # :603-607
+    return cv2.add(img, cv2.bitwise_and(dilated, alpha_mask))       # :609-612
+
+
+def test_pad_is_opencv_dilate_and_gutter(pto, golden_dir):
+    """Against OpenCV's results on the same images, stored in tests/golden/opencv/pad.npz
+    (tools/make_golden_opencv.py), and against the cv2 wheel itself where it is installed."""
+    try:
+        import cv2
+    except ImportError:
+        cv2 = None
+    z = np.load(os.path.join(golden_dir, "opencv", "pad.npz"))
+    for res in (256, 200, 64):
+        img, padded = z[f"in_{res}"], z[f"padded_{res}"]
         assert np.array_equal(pto.texture_pad(img), padded)
+        if cv2 is not None:
+            assert np.array_equal(_opencv_pad(cv2, img), padded)
 
 
 def test_oracle_texture_covers_the_mesh_and_triangulates(pkg, pto):
@@ -118,11 +128,14 @@ def test_gpu_texture_degenerate_inputs(pkg, pto):
 
 
 def test_png_writer_round_trip(tmp_path):
-    """host/pt_png.h (replaces cv::imwrite, :613): OpenCV decodes the file back to the same B G R A
-    bytes."""
-    import os
+    """host/pt_png.h (replaces cv::imwrite, :613): the file decodes back to the same B G R A bytes,
+    through a strict reader of its own and through OpenCV where it is installed."""
     import subprocess
-    cv2 = pytest.importorskip("cv2")
+    from test_cli import read_png_bgra
+    try:
+        import cv2
+    except ImportError:
+        cv2 = None
     root = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
     host = os.path.join(root, "3d-reconstruction-from-point-cloud_b200", "host")
     src = tmp_path / "t.cpp"
@@ -139,5 +152,7 @@ def test_png_writer_round_trip(tmp_path):
         img[: h // 2] = 0                                     # long zero runs as in a real texture
         (tmp_path / "raw.bin").write_bytes(img.tobytes())
         assert subprocess.run([str(exe), str(tmp_path / "raw.bin"), str(tmp_path / "o.png"), str(w), str(h)]).returncode == 0
-        back = cv2.imread(str(tmp_path / "o.png"), cv2.IMREAD_UNCHANGED)
-        assert back is not None and np.array_equal(back, img)
+        assert np.array_equal(read_png_bgra(tmp_path / "o.png"), img)
+        if cv2 is not None:
+            back = cv2.imread(str(tmp_path / "o.png"), cv2.IMREAD_UNCHANGED)
+            assert back is not None and np.array_equal(back, img)
