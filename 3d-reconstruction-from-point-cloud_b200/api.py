@@ -50,6 +50,7 @@ ABI_SYMBOLS = (
     "pt_halo_merge_device", "pt_ghost_check_device", "pt_route_samples_device",
     "pt_scatter_rows_device", "pt_sharded_build", "pt_sharded_free", "pt_sharded_get_info", "pt_sharded_knn",
     "pt_sharded_transfer", "pt_texture_render_lists", "pt_set_option", "pt_get_option", "pt_debug_stats", "pt_kernel_launch_count",
+    "pt_texture_bake", "pt_bake_texels_device", "pt_bake_compose_device",
 )
 # ... and include/pt_synth.h (bench / test scaffolding, its own library)
 SYNTH_SYMBOLS = ("pt_synth_cloud_device", "pt_synth_samples_device", "pt_synth_pack_points_device",
@@ -81,6 +82,11 @@ class IndexInfo(ctypes.Structure):
 class TextureStats(ctypes.Structure):
     _fields_ = [("triangles", ctypes.c_uint64), ("inside_points", ctypes.c_uint64),
                 ("knn_ms", ctypes.c_float), ("draw_ms", ctypes.c_float), ("pad_ms", ctypes.c_float)]
+
+
+class BakeStats(ctypes.Structure):
+    _fields_ = [("texels", ctypes.c_uint64), ("empty", ctypes.c_uint64), ("raster_ms", ctypes.c_float),
+                ("knn_ms", ctypes.c_float), ("pad_ms", ctypes.c_float)]
 
 
 class ShardedOpts(ctypes.Structure):
@@ -168,6 +174,12 @@ def lib():
     L.pt_texture_render_lists.restype = i32
     L.pt_texture_render_lists.argtypes = [vp, sz, vp, sz, vp, sz, vp, i32, i32, i32, i32, vp,
                                           ctypes.POINTER(TextureStats)]
+    L.pt_texture_bake.restype = i32
+    L.pt_texture_bake.argtypes = [vp, vp, sz, vp, sz, i32, dbl, i32, i32, vp, vp, vp, ctypes.POINTER(BakeStats)]
+    L.pt_bake_texels_device.restype = i32
+    L.pt_bake_texels_device.argtypes = [vp, sz, vp, sz, i32, vp, vp, ctypes.POINTER(sz), i32, vp]
+    L.pt_bake_compose_device.restype = i32
+    L.pt_bake_compose_device.argtypes = [vp, sz, vp, vp, i32, i32, vp, vp, vp, i32, vp]
     L.pt_set_option.restype = i32
     L.pt_set_option.argtypes = [ctypes.c_char_p, i32]
     L.pt_get_option.restype = i32
@@ -396,6 +408,35 @@ class Tree:
         return img, {"triangles": int(st.triangles), "inside_points": int(st.inside_points),
                      "knn_ms": st.knn_ms, "draw_ms": st.draw_ms, "pad_ms": st.pad_ms}
 
+    def bake(self, vertices, faces, k=20, resolution=2048, radius=None, pad=True,
+             want=("bgra", "normal_bgra", "normal")):
+        """Per-texel bake (DESIGN.md section 8): colour and normal maps of the cloud on the mesh's
+        UV atlas.  vertices: Point records (position, U, V), faces: int32 [F,3].  Returns a dict
+        with the requested images -- ``bgra`` uint8 [res,res,4] (B G R 255), ``normal_bgra`` uint8
+        [res,res,4] (object-space normal map, RGB = xyz), ``normal`` float32 [res,res,3] (never
+        padded) -- and ``stats`` (texels, empty, raster_ms, knn_ms, pad_ms)."""
+        v = _as_points(vertices, "vertices")
+        f = np.ascontiguousarray(faces, dtype=np.int32).reshape(-1, 3)
+        unknown = set(want) - {"bgra", "normal_bgra", "normal"}
+        if unknown or not want:
+            raise ValueError(f"want must name some of bgra, normal_bgra, normal (got {want!r})")
+        res = int(resolution)
+        out = {}
+        if "bgra" in want:
+            out["bgra"] = np.empty((res, res, 4), dtype=np.uint8)
+        if "normal_bgra" in want:
+            out["normal_bgra"] = np.empty((res, res, 4), dtype=np.uint8)
+        if "normal" in want:
+            out["normal"] = np.empty((res, res, 3), dtype=np.float32)
+        st = BakeStats()
+        _check(lib().pt_texture_bake(self._h, _np_ptr(v), v.shape[0], _np_ptr(f), f.shape[0], int(k),
+                                     _radius(radius), res, 1 if pad else 0, _np_ptr(out.get("bgra")),
+                                     _np_ptr(out.get("normal_bgra")), _np_ptr(out.get("normal")),
+                                     ctypes.byref(st)), "pt_texture_bake")
+        out["stats"] = {"texels": int(st.texels), "empty": int(st.empty), "raster_ms": st.raster_ms,
+                        "knn_ms": st.knn_ms, "pad_ms": st.pad_ms}
+        return out
+
     def transfer_slab(self, queries_ptr, queries_are_xyz, m, k, radius, boxes6, rank, halo,
                       idx_ptr, rgba_ptr, normal_ptr, d2_ptr=None):
         """pt_transfer_slab on raw host pointers (ints): one slab's pipelined host-buffer step
@@ -565,3 +606,54 @@ def merge_device(lists, n_lists, m, k, idx=None, d2=None, rgba=None, normal=None
         _check(lib().pt_merge_device(_tptr(lists), int(n_lists), int(m), int(k), _tptr(idx),
                                      _tptr(d2), _tptr(rgba), _tptr(normal), _tptr(cand),
                                      lists.device.index, _stream_ptr(stream)), "pt_merge_device")
+
+
+def bake_texels_device(vertices_xyzuv, faces, resolution, texels=None, xyz=None, stream=None):
+    """``pt_bake_texels_device``: the covered texels of the mesh's UV atlas as samples.
+    vertices_xyzuv: float64 [n,5] CUDA tensor (x, y, z, u, v), faces: int32 [F,3] CUDA tensor.
+    Returns (texel ids [m], positions float64 [m,3]) as views into ``texels`` / ``xyz``, which are
+    allocated with room for resolution^2 samples unless given.  Texel ids are row * resolution +
+    col in ascending order, held in an int32 tensor (torch has no uint32 arithmetic; they are
+    < 2^28).  Synchronises ``stream``."""
+    import torch
+    assert vertices_xyzuv.is_cuda and vertices_xyzuv.dtype == torch.float64 and vertices_xyzuv.is_contiguous()
+    assert vertices_xyzuv.dim() == 2 and vertices_xyzuv.shape[1] == 5
+    assert faces.is_cuda and faces.dtype == torch.int32 and faces.is_contiguous() and faces.numel() % 3 == 0
+    dev = vertices_xyzuv.device
+    cap = int(resolution) * int(resolution)
+    if texels is None:
+        texels = torch.empty(cap, dtype=torch.int32, device=dev)
+    if xyz is None:
+        xyz = torch.empty((cap, 3), dtype=torch.float64, device=dev)
+    assert texels.is_cuda and texels.dtype == torch.int32 and texels.is_contiguous() and texels.numel() >= cap
+    assert xyz.is_cuda and xyz.dtype == torch.float64 and xyz.is_contiguous() and xyz.numel() >= 3 * cap
+    count = ctypes.c_size_t(0)
+    with torch.cuda.device(dev):
+        _check(lib().pt_bake_texels_device(_tptr(vertices_xyzuv), vertices_xyzuv.shape[0], _tptr(faces),
+                                           faces.numel() // 3, int(resolution), _tptr(texels), _tptr(xyz),
+                                           ctypes.byref(count), dev.index, _stream_ptr(stream)),
+               "pt_bake_texels_device")
+    m = count.value
+    return texels[:m], xyz.view(-1)[:3 * m].view(m, 3)
+
+
+def bake_compose_device(texels, rgba, normal, resolution, pad=True, bgra=None, normal_bgra=None,
+                        normal_out=None, stream=None):
+    """``pt_bake_compose_device``: the bake's maps from the samples' blend results (``rgba`` uint8
+    [m,4], ``normal`` float32 [m,3] as ``DeviceTree.query`` returns them).  Outputs are
+    pre-allocated CUDA tensors (uint8 [res,res,4], uint8 [res,res,4], float32 [res,res,3]) or
+    None; at least one must be given.  Asynchronous on ``stream``."""
+    import torch
+    m = texels.numel()
+    assert texels.is_cuda and texels.dtype == torch.int32 and texels.is_contiguous()
+    assert rgba.is_cuda and rgba.dtype == torch.uint8 and rgba.is_contiguous() and rgba.numel() == 4 * m
+    assert normal.is_cuda and normal.dtype == torch.float32 and normal.is_contiguous() and normal.numel() == 3 * m
+    n_pix = int(resolution) * int(resolution)
+    for t, dt, cnt in ((bgra, torch.uint8, 4 * n_pix), (normal_bgra, torch.uint8, 4 * n_pix),
+                       (normal_out, torch.float32, 3 * n_pix)):
+        if t is not None:
+            assert t.is_cuda and t.is_contiguous() and t.dtype == dt and t.numel() == cnt
+    with torch.cuda.device(texels.device):
+        _check(lib().pt_bake_compose_device(_tptr(texels), m, _tptr(rgba), _tptr(normal), int(resolution),
+                                            1 if pad else 0, _tptr(bgra), _tptr(normal_bgra), _tptr(normal_out),
+                                            texels.device.index, _stream_ptr(stream)), "pt_bake_compose_device")

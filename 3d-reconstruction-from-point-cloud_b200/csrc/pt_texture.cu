@@ -20,6 +20,10 @@
 // `resolution - j` at j = 0 / column `resolution` (:100-103) and the uninitialised Mat (:402).
 #include <cmath>
 
+#include <cub/device/device_scan.cuh>
+#include <cub/device/device_select.cuh>
+#include <thrust/iterator/counting_iterator.h>
+
 #include "pt_index.cuh"
 
 namespace pt {
@@ -406,6 +410,344 @@ static int texture_render_index(pt_index *ix, const void *vertices, size_t n_ver
                             res, pad, bgra_out, st);
 }
 
+// ---- per-texel bake (DESIGN.md section 8, "Per-texel bake") ---------------------------------------
+// Texel (col, row) of a res x res image (row 0 on top) samples p = (col + 0.5, res - row - 0.5) in
+// UV * res units.  Face f covers it when all barycentrics of p in (U * res, V * res) are >= 0
+// (tx_tri_coords); where faces overlap the highest face index wins.  The sample position is the
+// barycentric mix of the winning face's 3-D corners, fp64, never contracted.
+//
+// Vertices are read through a stride, so both the caller's n x 5 (x, y, z, u, v) rows and the
+// MeshVertex records of tex_unpack_vertices_kernel (x, y, z, u, v first) can be rasterised.
+constexpr int BAKE_TILE = 32;                  // one warp per (face, 32 x 32-texel tile of its box)
+static_assert(sizeof(MeshVertex) % sizeof(double) == 0, "MeshVertex rows are read as doubles");
+
+struct BakeMesh {
+    const double  *v;          // n_vertices rows of `stride` doubles: x, y, z, u, v, ...
+    int            stride;
+    uint32_t       n_vertices;
+    const int32_t *faces;
+    uint32_t       n_faces;
+    int            res;
+};
+
+// corners of face f; false for an out-of-range vertex index (the face covers nothing)
+__device__ __forceinline__ bool bake_corners(const BakeMesh &M, uint32_t f, const double *c[3])
+{
+#pragma unroll
+    for (int j = 0; j < 3; ++j) {
+        const int32_t vi = M.faces[3 * (size_t)f + j];
+        if (vi < 0 || (uint32_t)vi >= M.n_vertices) return false;
+        c[j] = M.v + (size_t)vi * M.stride;
+    }
+    return true;
+}
+
+// UV triangle in UV * res units (the multiplications of tx_draw_triangle)
+__device__ __forceinline__ void bake_uv(const BakeMesh &M, const double *const c[3], V2 t[3])
+{
+#pragma unroll
+    for (int j = 0; j < 3; ++j) { t[j].a = c[j][3] * M.res; t[j].b = c[j][4] * M.res; }
+}
+
+__device__ __forceinline__ V2 bake_texel_point(int res, int col, int row)
+{
+    V2 p;
+    p.a = (double)col + 0.5;
+    p.b = (double)(res - row) - 0.5;
+    return p;
+}
+
+// Texels whose centre lies in the UV triangle's bounding box, widened by one texel so that rounding
+// in the barycentrics can never reach a texel outside it, clipped to the image.  false: none
+// (NaN UVs, or a box outside the image).
+__device__ __forceinline__ bool bake_box(const V2 t[3], int res, int &c0, int &r0, int &nc, int &nr)
+{
+    const double xmin = fmin(t[0].a, fmin(t[1].a, t[2].a)), xmax = fmax(t[0].a, fmax(t[1].a, t[2].a));
+    const double ymin = fmin(t[0].b, fmin(t[1].b, t[2].b)), ymax = fmax(t[0].b, fmax(t[1].b, t[2].b));
+    if (!(xmin <= xmax) || !(ymin <= ymax) || t[0].a != t[0].a || t[1].a != t[1].a || t[2].a != t[2].a ||
+        t[0].b != t[0].b || t[1].b != t[1].b || t[2].b != t[2].b)
+        return false;
+    const double lim = (double)(res - 1);
+    const double cl = fmax(ceil(xmin - 0.5) - 1.0, 0.0), ch = fmin(floor(xmax - 0.5) + 1.0, lim);
+    const double rl = fmax(ceil((double)res - 0.5 - ymax) - 1.0, 0.0), rh = fmin(floor((double)res - 0.5 - ymin) + 1.0, lim);
+    if (!(cl <= ch) || !(rl <= rh)) return false;
+    c0 = (int)cl; r0 = (int)rl;
+    nc = (int)ch - c0 + 1; nr = (int)rh - r0 + 1;
+    return true;
+}
+
+__global__ void __launch_bounds__(256) bake_tile_count_kernel(const BakeMesh M, unsigned long long *tiles)
+{
+    const uint32_t f = blockIdx.x * blockDim.x + threadIdx.x;
+    if (f >= M.n_faces) return;
+    const double *c[3];
+    V2 t[3];
+    int c0, r0, nc, nr;
+    unsigned long long n = 0;
+    if (bake_corners(M, f, c)) {
+        bake_uv(M, c, t);
+        if (bake_box(t, M.res, c0, r0, nc, nr))
+            n = (unsigned long long)((nc + BAKE_TILE - 1) / BAKE_TILE) * (unsigned long long)((nr + BAKE_TILE - 1) / BAKE_TILE);
+    }
+    tiles[f] = n;
+}
+
+// Work item w (< total = first[n_faces - 1] + tiles of the last face, exclusive scan `first`) is tile
+// w - first[f] of face f.  A warp walks its tile column by column (lane = column, coalesced) and
+// claims every covered texel with atomicMax(owner, f + 1): the highest covering face wins whatever
+// the schedule.
+__global__ void __launch_bounds__(256)
+bake_raster_kernel(const BakeMesh M, const unsigned long long *first, const unsigned long long *last_tiles,
+                   uint32_t *owner)
+{
+    const unsigned long long total = first[M.n_faces - 1] + *last_tiles;
+    const unsigned lane = threadIdx.x & 31u;
+    const unsigned long long warps = (unsigned long long)gridDim.x * (blockDim.x >> 5);
+    for (unsigned long long w = ((unsigned long long)blockIdx.x * blockDim.x + threadIdx.x) >> 5; w < total; w += warps) {
+        uint32_t lo = 0, hi = M.n_faces;          // last face with first[f] <= w
+        while (hi - lo > 1) {
+            const uint32_t mid = (lo + hi) >> 1;
+            if (first[mid] <= w) lo = mid; else hi = mid;
+        }
+        const uint32_t f = lo;
+        const double *c[3];
+        bake_corners(M, f, c);                    // a face with tiles has valid corners
+        V2 t[3];
+        bake_uv(M, c, t);
+        int c0, r0, nc, nr;
+        bake_box(t, M.res, c0, r0, nc, nr);
+        const unsigned long long tile = w - first[f];
+        const int tiles_x = (nc + BAKE_TILE - 1) / BAKE_TILE;
+        const int tx = (int)(tile % (unsigned long long)tiles_x), ty = (int)(tile / (unsigned long long)tiles_x);
+        const int col = c0 + tx * BAKE_TILE + (int)lane;
+        if (col >= c0 + nc) continue;
+        const int row_end = min(r0 + (ty + 1) * BAKE_TILE, r0 + nr);
+        for (int row = r0 + ty * BAKE_TILE; row < row_end; ++row) {
+            double bc[3];
+            tx_tri_coords(t[0], t[1], t[2], bake_texel_point(M.res, col, row), bc);
+            if (bc[0] >= 0 && bc[1] >= 0 && bc[2] >= 0)
+                atomicMax(owner + (size_t)row * M.res + col, f + 1u);
+        }
+    }
+}
+
+struct BakeCovered {
+    const uint32_t *owner;
+    __device__ __forceinline__ bool operator()(uint32_t t) const { return owner[t] != 0u; }
+};
+
+// position of sample i (texel texels[i]) on its owner face
+__global__ void __launch_bounds__(256)
+bake_position_kernel(const BakeMesh M, const uint32_t *owner, const uint32_t *texels, uint32_t count, double *xyz)
+{
+    const uint32_t i = blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= count) return;
+    const uint32_t tex = texels[i];
+    const uint32_t f = owner[tex] - 1u;
+    const double *c[3];
+    bake_corners(M, f, c);
+    V2 t[3];
+    bake_uv(M, c, t);
+    double bc[3];
+    tx_tri_coords(t[0], t[1], t[2], bake_texel_point(M.res, (int)(tex % (uint32_t)M.res), (int)(tex / (uint32_t)M.res)), bc);
+#pragma unroll
+    for (int a = 0; a < 3; ++a)
+        xyz[3 * (size_t)i + a] = __dadd_rn(__dadd_rn(__dmul_rn(bc[0], c[0][a]), __dmul_rn(bc[1], c[1][a])),
+                                           __dmul_rn(bc[2], c[2][a]));
+}
+
+// Owner map -> samples in ascending texel order.  M.faces / M.v are device pointers on the current
+// device.  texel_out / xyz_out: room for res * res samples, or both null (count only).  Synchronises
+// `s`; *count_out is the number of covered texels.
+static int bake_texels(const BakeMesh &M, uint32_t *texel_out, double *xyz_out, size_t *count_out, cudaStream_t s)
+{
+    const size_t n_pix = (size_t)M.res * M.res;
+    unsigned long long *d_tiles = nullptr, *d_first = nullptr;
+    uint32_t *d_owner = nullptr, *d_sel = nullptr, *d_count = nullptr;
+    void *d_tmp = nullptr;
+    int rc = PT_OK;
+    auto fail = [&](cudaError_t e) { if (e != cudaSuccess && rc == PT_OK) rc = map_cuda_error(e); return e != cudaSuccess; };
+    *count_out = 0;
+    do {
+        const size_t nf = M.n_faces ? M.n_faces : 1;
+        size_t scan_bytes = 0, select_bytes = 0;
+        thrust::counting_iterator<uint32_t> ids(0);
+        if (fail(cub::DeviceScan::ExclusiveSum(nullptr, scan_bytes, d_tiles, d_first, (int)nf, s))) break;
+        if (fail(cub::DeviceSelect::If(nullptr, select_bytes, ids, d_sel, d_count, (int)n_pix, BakeCovered{d_owner}, s))) break;
+        if (pool_alloc((void **)&d_tiles, sizeof(unsigned long long) * nf, s) ||
+            pool_alloc((void **)&d_first, sizeof(unsigned long long) * nf, s) ||
+            pool_alloc((void **)&d_owner, sizeof(uint32_t) * n_pix, s) || pool_alloc((void **)&d_count, sizeof(uint32_t), s) ||
+            pool_alloc(&d_tmp, scan_bytes > select_bytes ? scan_bytes : select_bytes, s) ||
+            (!texel_out && pool_alloc((void **)&d_sel, sizeof(uint32_t) * n_pix, s))) {
+            rc = PT_ERR_OUT_OF_MEMORY;
+            break;
+        }
+        uint32_t *sel = texel_out ? texel_out : d_sel;
+        if (fail(cudaMemsetAsync(d_owner, 0, sizeof(uint32_t) * n_pix, s))) break;
+        if (M.n_faces) {
+            bake_tile_count_kernel<<<tcdiv(M.n_faces, 256), 256, 0, s>>>(M, d_tiles);
+            count_launch();
+            if (fail(cub::DeviceScan::ExclusiveSum(d_tmp, scan_bytes, d_tiles, d_first, (int)M.n_faces, s))) break;
+            // enough warps to fill the device several times over; each strides over the work list
+            bake_raster_kernel<<<148 * 16, 256, 0, s>>>(M, d_first, d_tiles + (M.n_faces - 1), d_owner);
+            count_launch(2);
+        }
+        if (fail(cub::DeviceSelect::If(d_tmp, select_bytes, ids, sel, d_count, (int)n_pix, BakeCovered{d_owner}, s))) break;
+        count_launch();
+        uint32_t count = 0;
+        if (fail(cudaMemcpyAsync(&count, d_count, sizeof count, cudaMemcpyDeviceToHost, s))) break;
+        if (fail(cudaStreamSynchronize(s))) break;
+        if (xyz_out && count) {
+            bake_position_kernel<<<tcdiv(count, 256), 256, 0, s>>>(M, d_owner, sel, count, xyz_out);
+            count_launch();
+        }
+        if (fail(cudaGetLastError())) break;
+        *count_out = count;
+    } while (0);
+    void *frees[] = {d_tiles, d_first, d_owner, d_sel, d_count, d_tmp};
+    for (void *p : frees) pool_free(p, s);
+    if (fail(cudaStreamSynchronize(s))) *count_out = 0;
+    return rc;
+}
+
+// e(n) = clamp(floor((n + 1) * 127.5 + 0.5), 0, 255), fp64 from the fp32 component
+__device__ __forceinline__ uint32_t bake_encode(float n)
+{
+    const double v = floor(__dadd_rn(__dmul_rn(__dadd_rn((double)n, 1.0), 127.5), 0.5));
+    return (uint32_t)fmin(fmax(v, 0.0), 255.0);
+}
+
+// sample i -> its texel in the three maps; an empty neighbour list (rgba alpha 0) leaves zeros
+__global__ void __launch_bounds__(256)
+bake_compose_kernel(const uint32_t *texels, uint32_t count, const uint8_t *rgba, const float *normal,
+                    uint32_t *bgra, uint32_t *nbgra, float *nf, unsigned long long *empty)
+{
+    const uint32_t i = blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= count) return;
+    const uchar4 c = reinterpret_cast<const uchar4 *>(rgba)[i];
+    if (c.w == 0) {
+        if (empty) atomicAdd(empty, 1ull);
+        return;
+    }
+    const size_t t = texels[i];
+    const float x = normal[3 * (size_t)i], y = normal[3 * (size_t)i + 1], z = normal[3 * (size_t)i + 2];
+    if (bgra) bgra[t] = (uint32_t)c.z | ((uint32_t)c.y << 8) | ((uint32_t)c.x << 16) | 0xff000000u;
+    if (nbgra) nbgra[t] = bake_encode(z) | (bake_encode(y) << 8) | (bake_encode(x) << 16) | 0xff000000u;
+    if (nf) { nf[3 * t] = x; nf[3 * t + 1] = y; nf[3 * t + 2] = z; }
+}
+
+// Zeroes the requested maps, scatters the samples into them and pads the 8-bit ones in place with
+// the texture's dilate + gutter kernels (tex_dilate_v_pad_kernel reads only its own texel of `tex`).
+static int bake_compose(const uint32_t *texels, size_t count, const uint8_t *rgba, const float *normal, int res,
+                        int pad, uint8_t *bgra_out, uint8_t *normal_bgra_out, float *normal_out,
+                        unsigned long long *d_empty, cudaStream_t s)
+{
+    const size_t n_pix = (size_t)res * res;
+    if (bgra_out) PT_CUDA(cudaMemsetAsync(bgra_out, 0, 4 * n_pix, s));
+    if (normal_bgra_out) PT_CUDA(cudaMemsetAsync(normal_bgra_out, 0, 4 * n_pix, s));
+    if (normal_out) PT_CUDA(cudaMemsetAsync(normal_out, 0, sizeof(float) * 3 * n_pix, s));
+    if (count) {
+        bake_compose_kernel<<<tcdiv(count, 256), 256, 0, s>>>(texels, (uint32_t)count, rgba, normal, (uint32_t *)bgra_out,
+                                                              (uint32_t *)normal_bgra_out, normal_out, d_empty);
+        count_launch();
+    }
+    if (pad && (bgra_out || normal_bgra_out)) {
+        uint32_t *d_tmp = nullptr;
+        PT_TRY(pool_alloc((void **)&d_tmp, 4 * n_pix, s));
+        for (uint8_t *img : {bgra_out, normal_bgra_out}) {
+            if (!img) continue;
+            tex_dilate_h_kernel<<<tcdiv(n_pix, 256), 256, 0, s>>>((const uint32_t *)img, res, d_tmp);
+            tex_dilate_v_pad_kernel<<<tcdiv(n_pix, 256), 256, 0, s>>>((const uint32_t *)img, d_tmp, res, (uint32_t *)img);
+            count_launch(2);
+        }
+        pool_free(d_tmp, s);
+    }
+    PT_CUDA(cudaGetLastError());
+    return PT_OK;
+}
+
+static int texture_bake(pt_index *ix, const void *vertices, size_t n_vertices, const int32_t *faces, size_t n_faces,
+                        int k, double radius, int res, int pad, uint8_t *bgra_out, uint8_t *normal_bgra_out,
+                        float *normal_out, pt_bake_stats *st)
+{
+    cudaStream_t s = ix->stream;
+    const size_t n_pix = (size_t)res * res;
+    Raw80t *d_raw = nullptr;
+    MeshVertex *d_mv = nullptr;
+    double *d_xyz = nullptr, *d_q = nullptr;
+    int32_t *d_faces = nullptr;
+    uint32_t *d_texels = nullptr;
+    uint8_t *d_rgba = nullptr, *d_bgra = nullptr, *d_nbgra = nullptr;
+    float *d_normal = nullptr, *d_nf = nullptr;
+    unsigned long long *d_empty = nullptr;
+    cudaEvent_t ev[4] = {};
+    size_t count = 0;
+    int rc = PT_OK;
+    auto fail = [&](cudaError_t e) { if (e != cudaSuccess && rc == PT_OK) rc = map_cuda_error(e); return e != cudaSuccess; };
+    do {
+        for (auto &e : ev) if (fail(cudaEventCreate(&e))) break;
+        if (rc != PT_OK) break;
+        if (pool_alloc((void **)&d_raw, sizeof(Raw80t) * n_vertices, s) || pool_alloc((void **)&d_mv, sizeof(MeshVertex) * n_vertices, s) ||
+            pool_alloc((void **)&d_xyz, sizeof(double) * 3 * n_vertices, s) || pool_alloc((void **)&d_faces, sizeof(int32_t) * 3 * n_faces, s) ||
+            pool_alloc((void **)&d_texels, sizeof(uint32_t) * n_pix, s) || pool_alloc((void **)&d_q, sizeof(double) * 3 * n_pix, s) ||
+            pool_alloc((void **)&d_empty, sizeof(unsigned long long), s) ||
+            (bgra_out && pool_alloc((void **)&d_bgra, 4 * n_pix, s)) || (normal_bgra_out && pool_alloc((void **)&d_nbgra, 4 * n_pix, s)) ||
+            (normal_out && pool_alloc((void **)&d_nf, sizeof(float) * 3 * n_pix, s))) {
+            rc = PT_ERR_OUT_OF_MEMORY;
+            break;
+        }
+        if (fail(cudaEventRecord(ev[0], s))) break;
+        if (fail(cudaMemcpyAsync(d_raw, vertices, sizeof(Raw80t) * n_vertices, cudaMemcpyHostToDevice, s))) break;
+        if (fail(cudaMemcpyAsync(d_faces, faces, sizeof(int32_t) * 3 * n_faces, cudaMemcpyHostToDevice, s))) break;
+        if (fail(cudaMemsetAsync(d_empty, 0, sizeof(unsigned long long), s))) break;
+        if (n_vertices) {
+            tex_unpack_vertices_kernel<<<tcdiv(n_vertices, 256), 256, 0, s>>>(d_raw, (uint32_t)n_vertices, d_mv, d_xyz);
+            count_launch();
+        }
+        const BakeMesh M{reinterpret_cast<const double *>(d_mv), (int)(sizeof(MeshVertex) / sizeof(double)),
+                         (uint32_t)n_vertices, d_faces, (uint32_t)n_faces, res};
+        if ((rc = bake_texels(M, d_texels, d_q, &count, s)) != PT_OK) break;
+        if (fail(cudaEventRecord(ev[1], s))) break;
+        if (pool_alloc((void **)&d_rgba, 4 * (count ? count : 1), s) || pool_alloc((void **)&d_normal, sizeof(float) * 3 * (count ? count : 1), s)) {
+            rc = PT_ERR_OUT_OF_MEMORY;
+            break;
+        }
+        if (count) {
+            QueryParams qp{};
+            qp.pts = ix->pts; qp.attrs = ix->attrs; qp.ids = nullptr; qp.pyr = ix->pyr;
+            qp.n = ix->n; qp.n_leaves = ix->n_leaves; qp.w_levels = ix->w_levels; qp.t_levels = ix->t_levels;
+            qp.pq_cap = opt_queue_cap();
+            qp.queries = d_q; qp.m = (uint32_t)count; qp.k = k;
+            qp.r2 = (!(radius >= 0.0) || std::isinf(radius)) ? INFINITY : radius * radius;
+            qp.rgba_out = d_rgba; qp.normal_out = d_normal;
+            if ((rc = launch_query(ix, qp, s)) != PT_OK) break;
+        }
+        if (fail(cudaEventRecord(ev[2], s))) break;
+        if ((rc = bake_compose(d_texels, count, d_rgba, d_normal, res, pad, d_bgra, d_nbgra, d_nf, d_empty, s)) != PT_OK) break;
+        if (fail(cudaEventRecord(ev[3], s))) break;
+        if (bgra_out && fail(cudaMemcpyAsync(bgra_out, d_bgra, 4 * n_pix, cudaMemcpyDeviceToHost, s))) break;
+        if (normal_bgra_out && fail(cudaMemcpyAsync(normal_bgra_out, d_nbgra, 4 * n_pix, cudaMemcpyDeviceToHost, s))) break;
+        if (normal_out && fail(cudaMemcpyAsync(normal_out, d_nf, sizeof(float) * 3 * n_pix, cudaMemcpyDeviceToHost, s))) break;
+        unsigned long long empty = 0;
+        if (fail(cudaMemcpyAsync(&empty, d_empty, sizeof empty, cudaMemcpyDeviceToHost, s))) break;
+        if (fail(cudaStreamSynchronize(s))) break;
+        if (st) {
+            st->texels = count;
+            st->empty = empty;
+            cudaEventElapsedTime(&st->raster_ms, ev[0], ev[1]);
+            cudaEventElapsedTime(&st->knn_ms, ev[1], ev[2]);
+            cudaEventElapsedTime(&st->pad_ms, ev[2], ev[3]);
+        }
+    } while (0);
+    cudaStreamSynchronize(s);
+    void *frees[] = {d_raw, d_mv, d_xyz, d_faces, d_texels, d_q, d_rgba, d_normal, d_bgra, d_nbgra, d_nf, d_empty};
+    for (void *p : frees) pool_free(p, s);
+    for (auto &e : ev) if (e) cudaEventDestroy(e);
+    cudaStreamSynchronize(s);
+    cudaGetLastError();
+    return rc;
+}
+
 }  // namespace pt
 
 using namespace pt;
@@ -456,4 +798,47 @@ extern "C" int pt_texture_render_lists(const void *points, size_t n, const void 
     if (tmp.stream) cudaStreamDestroy(tmp.stream);
     cudaGetLastError();
     return rc;
+}
+
+extern "C" int pt_bake_texels_device(const double *vertices_xyzuv, size_t n_vertices, const int32_t *faces,
+                                     size_t n_faces, int resolution, uint32_t *texel_out, double *xyz_out,
+                                     size_t *count_out, int device, void *stream)
+{
+    if ((!vertices_xyzuv && n_vertices) || (!faces && n_faces) || !count_out || resolution < 1 || resolution > 16384 ||
+        n_vertices > 0x7ffffff0ull || n_faces >= (1ull << 31) || (!texel_out != !xyz_out))
+        return PT_ERR_INVALID_ARG;
+    *count_out = 0;
+    if (pt_device_count() == 0) return PT_ERR_NO_DEVICE;
+    if (device >= 0) PT_CUDA(cudaSetDevice(device));
+    const BakeMesh M{vertices_xyzuv, 5, (uint32_t)n_vertices, faces, (uint32_t)n_faces, resolution};
+    return bake_texels(M, texel_out, xyz_out, count_out, (cudaStream_t)stream);
+}
+
+extern "C" int pt_bake_compose_device(const uint32_t *texels, size_t count, const uint8_t *rgba, const float *normal,
+                                      int resolution, int pad, uint8_t *bgra_out, uint8_t *normal_bgra_out,
+                                      float *normal_out, int device, void *stream)
+{
+    if ((count && (!texels || !rgba || !normal)) || resolution < 1 || resolution > 16384 ||
+        count > (size_t)resolution * resolution || (!bgra_out && !normal_bgra_out && !normal_out))
+        return PT_ERR_INVALID_ARG;
+    if (pt_device_count() == 0) return PT_ERR_NO_DEVICE;
+    if (device >= 0) PT_CUDA(cudaSetDevice(device));
+    return bake_compose(texels, count, rgba, normal, resolution, pad, bgra_out, normal_bgra_out, normal_out, nullptr,
+                        (cudaStream_t)stream);
+}
+
+extern "C" int pt_texture_bake(pt_index *ix, const void *vertices, size_t n_vertices, const int32_t *faces,
+                               size_t n_faces, int k, double radius, int resolution, int pad, uint8_t *bgra_out,
+                               uint8_t *normal_bgra_out, float *normal_out, pt_bake_stats *stats)
+{
+    if (!ix || (!vertices && n_vertices) || (!faces && n_faces) || (!bgra_out && !normal_bgra_out && !normal_out) ||
+        resolution < 1 || resolution > 16384 || n_vertices > 0x7ffffff0ull || n_faces >= (1ull << 31))
+        return PT_ERR_INVALID_ARG;
+    if (k < 1 || k > PT_MAX_K) return PT_ERR_UNSUPPORTED;
+    if (ix->ids) return PT_ERR_UNSUPPORTED;           // slab indexes answer with global ids
+    if (!ix->attrs && ix->n) return PT_ERR_INVALID_ARG;
+    if (pt_device_count() == 0) return PT_ERR_NO_DEVICE;
+    PT_CUDA(cudaSetDevice(ix->device));
+    return texture_bake(ix, vertices, n_vertices, faces, n_faces, k, radius, resolution, pad, bgra_out, normal_bgra_out,
+                        normal_out, stats);
 }

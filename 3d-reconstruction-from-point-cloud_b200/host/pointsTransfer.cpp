@@ -14,7 +14,9 @@
 // rasteriser stages (:484-615) are out of scope of this build (SURVEY.md section 8 rows N1-N4):
 // instead of texture.png the tool writes `transferred.ply`, the input mesh in the same 11-column
 // ASCII format with the transferred colour and normal per vertex.  Extra options (all default to
-// the reference's behaviour): -k N, -r RADIUS, -o FILE, -d DEVICE.
+// the reference's behaviour): -k N, -r RADIUS, -o FILE, -d DEVICE.  -b FILE / -n FILE also bake the
+// cloud's colour / object-space normal onto every texel of the mesh's UV atlas (pt_texture_bake,
+// same -R, -k, -r) and write them as PNG.
 #include <algorithm>
 #include <charconv>
 #include <chrono>
@@ -244,6 +246,7 @@ static int run(int argc, char **argv)
     int resolution = 8192;  // src/pointsTransfer.cpp:129
     std::string out_name = "texture.png";          // src/pointsTransfer.cpp:613
     std::string ply_name;                          // optional extra: the per-vertex blend as a PLY
+    std::string bake_name, normal_name;            // optional extras: the per-texel colour / normal maps
     for (int i = 1; i < argc; ++i) {
         std::string a = argv[i];
         if (a == "-k" && i + 1 < argc) K = atoi(argv[++i]);
@@ -253,6 +256,8 @@ static int run(int argc, char **argv)
         else if (a == "-R" && i + 1 < argc) resolution = atoi(argv[++i]);
         else if (a == "-d" && i + 1 < argc) device = atoi(argv[++i]);
         else if (a == "-g" && i + 1 < argc) n_gpus = atoi(argv[++i]);
+        else if (a == "-b" && i + 1 < argc) bake_name = argv[++i];
+        else if (a == "-n" && i + 1 < argc) normal_name = argv[++i];
         else pos_args.push_back(a);
     }
     if (pos_args.size() < 2) {
@@ -262,6 +267,11 @@ static int run(int argc, char **argv)
     if (K < 1 || K > PT_MAX_K || resolution < 1 || resolution > 32768 || n_gpus < 1 || n_gpus > 64) {
         // like every error path of the reference: a message, exit code 0
         std::cerr << "-k must be 1.." << PT_MAX_K << ", -R 1..32768 and -g 1..64" << std::endl;
+        return 0;
+    }
+    const bool bake = !bake_name.empty() || !normal_name.empty();
+    if (bake && (n_gpus > 1 || resolution > 16384)) {
+        std::cerr << "-b / -n bake on one GPU (no -g) at -R 1..16384" << std::endl;
         return 0;
     }
     const std::string pc_file_name = pos_args[0], mesh_file_name = pos_args[1];
@@ -367,8 +377,30 @@ static int run(int argc, char **argv)
     std::cout << "Neighbor search total time: " << ts.knn_ms * 1e-3 << " seconds" << std::endl;
     std::cout << "Draw triangles total time: " << (ts.draw_ms + ts.pad_ms) * 1e-3 << " seconds" << std::endl;
 
+    // extra (not in the reference): per-texel colour and normal maps, padded like the texture
+    std::vector<uint8_t> baked, baked_normal;
+    if (bake) {
+        if (!bake_name.empty()) baked.resize((size_t)resolution * resolution * 4);
+        if (!normal_name.empty()) baked_normal.resize((size_t)resolution * resolution * 4);
+        pt_bake_stats bs;
+        rc = pt_texture_bake(index, vertices.data(), m, faces.data(), faces.size() / 3, K, radius, resolution, 1,
+                             baked.empty() ? nullptr : baked.data(), baked_normal.empty() ? nullptr : baked_normal.data(),
+                             nullptr, &bs);
+        if (rc != PT_OK) {
+            std::cerr << "pt_texture_bake failed: " << pt_status_string(rc) << std::endl;
+            pt_index_free(index);
+            return 0;
+        }
+        std::cout << "Bake total time: " << task_timer.time() << " seconds" << std::endl;
+        task_timer.reset();
+    }
+
     if (!ptb::write_png_bgra(out_name.c_str(), texture.data(), resolution, resolution))
         std::cerr << "Cannot write " << out_name << std::endl;
+    if (!baked.empty() && !ptb::write_png_bgra(bake_name.c_str(), baked.data(), resolution, resolution))
+        std::cerr << "Cannot write " << bake_name << std::endl;
+    if (!baked_normal.empty() && !ptb::write_png_bgra(normal_name.c_str(), baked_normal.data(), resolution, resolution))
+        std::cerr << "Cannot write " << normal_name << std::endl;
     if (!ply_name.empty()) {
         // extra (not in the reference): the fused per-vertex colour / normal blend of pt_transfer
         std::vector<uint8_t> rgba(m * 4);

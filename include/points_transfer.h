@@ -15,6 +15,8 @@
  *                       465-479 + the colour blend semantics of :95-103.
  *   pt_texture_render<- the face loop body after the searches and the texture
  *                       post-process, src/pointsTransfer.cpp:484-611 + draw_triangle :66-107.
+ *   pt_texture_bake  <- no reference counterpart: per-texel colour and normal maps on
+ *                       the mesh's UV atlas (the "texel" samples of the transfer).
  *   pt_index_free    <- `tree` going out of scope at src/pointsTransfer.cpp:626.
  *
  * Records are the reference's own 80-byte AoS `struct Point`
@@ -135,6 +137,36 @@ int pt_texture_render(pt_index *index, const void *vertices, size_t n_vertices,
                       const int32_t *faces, size_t n_faces, int k, double radius,
                       int resolution, int pad, uint8_t *bgra_out, pt_texture_stats *stats);
 
+/* Per-texel bake (DESIGN.md section 8, "Per-texel bake"): every texel of the mesh's UV atlas that
+ * a face covers becomes one sample, answered by the k-NN + fused blend of pt_transfer, and the
+ * results are written back as images.  Texel (col, row) of a resolution x resolution image (row 0
+ * on top) samples the UV point ((col + 0.5) / res, (res - row - 0.5) / res): the texel-centre
+ * convention of standard texture sampling, half a texel away from pt_texture_render's lattice.
+ * A face covers a texel when the barycentrics of that point in its UV triangle are all >= 0;
+ * where faces overlap the highest face index wins; degenerate UV triangles and faces with an
+ * out-of-range vertex index cover nothing.  The sample position is the fp64 barycentric mix of
+ * the winning face's 3-D corners.
+ *   bgra_out         blended colour as B G R 255 (cv::Mat CV_8UC4 layout)
+ *   normal_bgra_out  object-space normal map: B G R A = e(z) e(y) e(x) 255 with
+ *                    e(n) = clamp(floor((n + 1) * 127.5 + 0.5), 0, 255), so RGB shows xyz
+ *   normal_out       the blended unit normal, 3 floats per texel
+ * Uncovered texels, and covered texels whose neighbour list is empty (radius-bounded search),
+ * are 0 in all three maps.  pad != 0 runs the two 8-bit maps through the texture's 25 x 25
+ * dilate + gutter; normal_out is never padded.  Host buffers, blocking.  vertices: Point records
+ * (position, U, V are read); faces: 3 int32 per face (n_faces < 2^31).  Any of the three outputs
+ * may be NULL, but not all.  resolution 1..16384. */
+typedef struct pt_bake_stats {
+    uint64_t texels;   /* covered texels = samples answered */
+    uint64_t empty;    /* covered texels whose neighbour list came back empty */
+    float    raster_ms, knn_ms, pad_ms;   /* device time of the stages: upload + raster + compaction,
+                                             k-NN + blend, scatter into the maps + padding */
+} pt_bake_stats;
+int pt_texture_bake(pt_index *index, const void *vertices, size_t n_vertices,
+                    const int32_t *faces, size_t n_faces, int k, double radius,
+                    int resolution, int pad, uint8_t *bgra_out /* res*res*4 */,
+                    uint8_t *normal_bgra_out /* res*res*4 */, float *normal_out /* res*res*3 */,
+                    pt_bake_stats *stats);
+
 /* Device-buffer API: same operations with inputs/outputs already resident in
  * HBM on the index's device (bench `value`, multi-GPU slabs).  `stream` is a
  * cudaStream_t passed as void* (NULL = the CUDA default stream); these calls
@@ -177,6 +209,24 @@ int pt_query_device(pt_index *index, const double *queries_xyz, size_t m, int k,
 int pt_merge_device(const pt_cand *lists, int n_lists, size_t m, int k,
                     int32_t *idx_out, double *d2_out, uint8_t *rgba_out,
                     float *normal_out, pt_cand *cand_out, int device, void *stream);
+
+/* The two device-buffer pieces pt_texture_bake is built from, so the texel samples can go through
+ * pt_query_device or a sharded path.  Run on `device` (-1: the current one).
+ * pt_bake_texels_device: vertices_xyzuv n_vertices x 5 doubles (x, y, z, u, v), faces 3 int32 per
+ * face; the covered texels in ascending texel order (texel id = row * resolution + col) and their
+ * sample positions.  texel_out / xyz_out need room for resolution^2 samples (texel_out uint32,
+ * xyz_out 3 doubles each), or are both NULL to only count.  Synchronises `stream` and returns the
+ * count in *count_out (host). */
+int pt_bake_texels_device(const double *vertices_xyzuv, size_t n_vertices,
+                          const int32_t *faces, size_t n_faces, int resolution,
+                          uint32_t *texel_out, double *xyz_out, size_t *count_out,
+                          int device, void *stream);
+/* pt_bake_compose_device: the maps of pt_texture_bake from count samples (texels as above, rgba
+ * count x 4 and normal count x 3 as pt_query_device returns them).  Outputs as pt_texture_bake's,
+ * in device memory; any may be NULL, but not all.  Asynchronous on `stream`. */
+int pt_bake_compose_device(const uint32_t *texels, size_t count, const uint8_t *rgba,
+                           const float *normal, int resolution, int pad, uint8_t *bgra_out,
+                           uint8_t *normal_bgra_out, float *normal_out, int device, void *stream);
 
 /* Halo exchange helpers for slab-sharded clouds (DESIGN.md section 6).  Fixed-capacity routing,
  * so the exchange needs no host synchronisation: per peer a send block of (cap + 1) rows of 4
