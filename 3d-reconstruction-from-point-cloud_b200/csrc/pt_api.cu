@@ -50,6 +50,8 @@ int opt_grid() { return g_grid.load(); }
 int opt_grid_tma() { return g_grid_tma.load(); }
 static std::atomic<int> g_grid_pair{1};   // grid kernel: two samples per warp when k <= 16
 int opt_grid_pair() { return g_grid_pair.load(); }
+static std::atomic<int> g_grid_span{1};   // two samples per warp: one look-up per parent cell, one copy per span (0: per cell)
+int opt_grid_span() { return g_grid_span.load(); }
 static std::atomic<int> g_grid_min_occ10{40};    // finest table: finest level with >= this / 10 points per occupied cell
 static std::atomic<int> g_grid_lookup_cost{8};   // grid_plan: cost of one bucket look-up, in candidates
 static std::atomic<int> g_grid_admit100{100};    // grid_plan: a block is tried first when rc cells >= this / 100 expected k-th distances
@@ -58,6 +60,8 @@ int opt_grid_min_occ10() { return g_grid_min_occ10.load(); }
 int opt_grid_lookup_cost() { return g_grid_lookup_cost.load(); }
 static std::atomic<int> g_grid_pair_used{0};   // introspection: did the last grid launch run two samples per warp
 void note_grid_pair_used(int used) { g_grid_pair_used.store(used); }
+static std::atomic<int> g_grid_span_used{0};   // introspection: did the last grid launch run knn_grid_span_kernel
+void note_grid_span_used(int used) { g_grid_span_used.store(used); }
 int opt_sort_bits() { return g_sort_bits.load(); }
 size_t opt_pool_keep_bytes()
 {
@@ -101,6 +105,7 @@ int set_option(const char *name, int value)
     if (!strcmp(name, "grid_lookup_cost")) { g_grid_lookup_cost.store(value < 0 ? 0 : value); return PT_OK; }
     if (!strcmp(name, "grid_admit100")) { g_grid_admit100.store(value < 10 ? 10 : value); return PT_OK; }
     if (!strcmp(name, "grid_pair")) { g_grid_pair.store(value < 0 ? 0 : (value > 2 ? 2 : value)); return PT_OK; }
+    if (!strcmp(name, "grid_span")) { g_grid_span.store(value ? 1 : 0); return PT_OK; }
     if (!strcmp(name, "sort_bits")) { g_sort_bits.store(value); return PT_OK; }
     if (!strcmp(name, "pool_keep_mb")) { g_pool_keep_mb.store(value < 0 ? -1 : value); return PT_OK; }
     if (!strcmp(name, "pool_guard")) { g_pool_guard.store(value ? 1 : 0); return PT_OK; }
@@ -123,6 +128,8 @@ int get_option(const char *name, int *value)
     if (!strcmp(name, "grid_admit100")) { *value = g_grid_admit100.load(); return PT_OK; }
     if (!strcmp(name, "grid_pair")) { *value = g_grid_pair.load(); return PT_OK; }
     if (!strcmp(name, "grid_pair_used")) { *value = g_grid_pair_used.load(); return PT_OK; }
+    if (!strcmp(name, "grid_span")) { *value = g_grid_span.load(); return PT_OK; }
+    if (!strcmp(name, "grid_span_used")) { *value = g_grid_span_used.load(); return PT_OK; }
     if (!strcmp(name, "sort_bits")) { *value = g_sort_bits.load(); return PT_OK; }
     if (!strcmp(name, "pool_keep_mb")) { *value = g_pool_keep_mb.load(); return PT_OK; }
     if (!strcmp(name, "pool_guard")) { *value = g_pool_guard.load(); return PT_OK; }
@@ -186,6 +193,7 @@ static void destroy_index(pt_index *ix)
     pool_free(ix->pts, ix->stream);
     pool_free(ix->boxes, ix->stream);
     pool_free(ix->grid_mem, ix->stream);
+    pool_free(ix->attrs_curve, ix->stream);
     pool_free(ix->attrs, ix->stream);         // (attributes and ids too: cudaMalloc / cudaFree of 0.8 GB cost milliseconds)
     pool_free(ix->ids, ix->stream);
     if (ix->stream) cudaStreamSynchronize(ix->stream);
@@ -210,6 +218,7 @@ static void fill_params(const pt_index *ix, QueryParams &qp)
 {
     qp.pts = ix->pts;
     qp.attrs = ix->attrs;
+    qp.attrs_curve = ix->attrs_curve;
     qp.ids = ix->ids;
     qp.pyr = ix->pyr;
     qp.n = ix->n;

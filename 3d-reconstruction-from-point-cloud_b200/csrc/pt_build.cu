@@ -7,7 +7,8 @@
 //       leaf boxes + binary box pyramid ("cell table")    (leaf_box_kernel, pyramid_kernel)
 //
 // HBM layout: pts[n_leaves*32] sorted records; boxes[level][node] 32-byte AABBs, level j
-// node i covering leaves [i*2^j, (i+1)*2^j).  Attributes and ids stay in original order.
+// node i covering leaves [i*2^j, (i+1)*2^j).  Attributes and ids stay in original order; float4
+// clouds with cell tables also keep a sorted-order copy of the attributes (attrs_curve).
 #include <cub/device/device_radix_sort.cuh>
 
 #include <cfloat>
@@ -140,13 +141,15 @@ __global__ void __launch_bounds__(256) morton_kernel(In in, uint32_t n, KeyParam
 // ---- gather into leaves -----------------------------------------------------------------
 template <typename In, typename Out>
 __global__ void __launch_bounds__(256) gather_kernel(In in, const uint32_t *perm, uint32_t n,
-                                                     uint32_t n_pad, Out *out)
+                                                     uint32_t n_pad, Out *out, const pt_attr *attrs,
+                                                     pt_attr *attrs_out)
 {
     uint32_t i = blockIdx.x * blockDim.x + threadIdx.x;
     if (i >= n_pad) return;
     Out o;
     if (i < n) {
         uint32_t src = perm[i];
+        if (attrs_out) attrs_out[i] = attrs[src];   // the attributes in the same (sorted) order
         double x, y, z;
         in.load(src, x, y, z);
         o.x = x; o.y = y; o.z = z;   // exact: F32 storage is only chosen when representable
@@ -665,7 +668,12 @@ static int build_impl(pt_index *ix, In in, uint32_t n)
     size_t n_pad = (size_t)ix->n_leaves * LEAF;
     Out *pts = nullptr;
     PT_TRY(temp_alloc((void **)&pts, sizeof(Out) * n_pad, s));   // pooled: a rebuild reuses the block
-    gather_kernel<In, Out><<<cdiv(n_pad, 256), 256, 0, s>>>(in, vals, n, (uint32_t)n_pad, pts);
+    // attributes in sorted order for knn_grid_span_kernel (float4 records with cell tables only):
+    // the winners of a sample sit in a few adjacent cells, so their records share DRAM lines
+    if (ix->attrs && sizeof(Out) == 16 && kp.order != 2 && opt_grid() != 0 && n >= 64)
+        PT_TRY(temp_alloc((void **)&ix->attrs_curve, sizeof(pt_attr) * (size_t)n, s));
+    gather_kernel<In, Out><<<cdiv(n_pad, 256), 256, 0, s>>>(in, vals, n, (uint32_t)n_pad, pts, ix->attrs,
+                                                            ix->attrs_curve);
     count_launch();
     ix->pts = pts;
     lap("gather");
@@ -719,6 +727,7 @@ static int build_impl(pt_index *ix, In in, uint32_t n)
     pool_trim(ix->device, opt_pool_keep_bytes());   // "pool_keep_mb" of it stays mapped for the next build
     ix->device_bytes = sizeof(Out) * n_pad + sizeof(Box) * total + ix->grid_bytes +
                        (ix->attrs ? sizeof(pt_attr) * (size_t)n : 0) +
+                       (ix->attrs_curve ? sizeof(pt_attr) * (size_t)n : 0) +
                        (ix->ids ? sizeof(int32_t) * (size_t)n : 0);
     return PT_OK;
 }

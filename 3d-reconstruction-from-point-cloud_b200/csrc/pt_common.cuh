@@ -104,6 +104,7 @@ struct GridParams {
 struct QueryParams {
     const void    *pts;        // PointF* or PointD*, n_pad records
     const pt_attr *attrs;      // original (local) order, may be null
+    const pt_attr *attrs_curve; // attrs in the order of pts (attrs_curve[i] = attrs[pts[i].idx]), may be null
     const int32_t *ids;        // local -> global id, may be null
     Pyramid        pyr;
     uint32_t       n;          // points

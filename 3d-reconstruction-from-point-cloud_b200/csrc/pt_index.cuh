@@ -12,6 +12,7 @@ struct pt_index {
     int          t_levels = 0;
     void        *pts = nullptr;      // PointF/PointD [n_leaves*LEAF], Morton order
     pt_attr     *attrs = nullptr;    // [n] original order (may be null)
+    pt_attr     *attrs_curve = nullptr; // [n] attrs in sorted order (float4 records with cell tables only)
     int32_t     *ids = nullptr;      // [n] original order (may be null)
     pt::Box     *boxes = nullptr;    // all pyramid levels, level 0 first
     pt::Pyramid  pyr{};
@@ -126,10 +127,12 @@ int  opt_queue_cap();
 int  opt_grid();
 int  opt_grid_tma();
 int  opt_grid_pair();
+int  opt_grid_span();
 int  opt_grid_min_occ10();
 int  opt_grid_admit100();
 int  opt_grid_lookup_cost();
 void note_grid_pair_used(int used);
+void note_grid_span_used(int used);
 int  opt_sort_bits();
 size_t opt_pool_keep_bytes();
 int  opt_pool_guard();

@@ -3,9 +3,9 @@
 // metric src/Distance.h:6-11, pruning bound src/Distance.h:27-57).
 //
 // Four kernels share the helpers in this file:
-//   variant 6 ("grid",   pt_knn_grid.cuh)  : one warp per sample over the uniform-grid cell
-//     tables, candidate runs staged in shared memory by bulk async copies; the default first
-//     stage -- samples it cannot prove final go to the kernels below;
+//   variant 6 ("grid",   pt_knn_grid.cuh, pt_knn_span.cuh): one warp per sample (two at k <= 16)
+//     over the uniform-grid cell tables, candidate runs staged in shared memory by bulk async
+//     copies; the default first stage -- samples it cannot prove final go to the kernels below;
 //   variant 5 ("scan",   pt_knn_scan.cuh)  : one thread per sample, unsorted top-k slots;
 //   variant 2 ("thread", pt_knn_thread.cuh): one thread per sample, top-k heap;
 //     both walk the box pyramid with pt_knn_traverse.cuh, state in shared-memory columns;
@@ -366,6 +366,7 @@ __global__ void __launch_bounds__(256) empty_result_kernel(const QueryParams P)
 #include "pt_knn_thread.cuh"
 #include "pt_knn_scan.cuh"
 #include "pt_knn_grid.cuh"
+#include "pt_knn_span.cuh"
 namespace pt {
 
 // Launch plan.  Every launch gets its OWN hand-over workspace (two sample lists with their
@@ -388,7 +389,16 @@ static int launch_chain(pt_index *ix, const QueryParams &qp, int variant, cudaSt
     QueryParams q2 = qp;
     const bool grid_first = variant == 6;
     if (rc == PT_OK && variant == 6) {
-        rc = launch_grid<PT>(qp, ix->sm_count, count1, list1, s);
+        // two samples per warp with one look-up per parent cell and one copy per span where the
+        // pair kernel would run (pt_knn_span.cuh); otherwise launch_grid picks
+        const bool span = grid_span_applies<PT>(qp);
+        note_grid_span_used(span ? 1 : 0);
+        if (span) {
+            note_grid_pair_used(0);
+            rc = launch_grid_span(qp, ix->sm_count, count1, list1, s);
+        } else {
+            rc = launch_grid<PT>(qp, ix->sm_count, count1, list1, s);
+        }
         // A short hand-over list is answered by the warp kernel (one warp per sample: a few
         // samples cost ~30 us there, but a whole ~110 us block latency in the scan / thread
         // kernels); a long one by the scan / thread kernel in list mode (min_count).

@@ -346,7 +346,7 @@ static int texture_pipeline(pt_index *ix, POS pos, uint32_t n_points, const pt_a
         if (search) {
             // the neighbour search of every UNIQUE vertex (the reference searches 3 x per face, :474)
             QueryParams qp{};
-            qp.pts = ix->pts; qp.attrs = ix->attrs; qp.ids = nullptr; qp.pyr = ix->pyr;
+            qp.pts = ix->pts; qp.attrs = ix->attrs; qp.attrs_curve = ix->attrs_curve; qp.ids = nullptr; qp.pyr = ix->pyr;
             qp.n = ix->n; qp.n_leaves = ix->n_leaves; qp.w_levels = ix->w_levels; qp.t_levels = ix->t_levels;
             qp.pq_cap = opt_queue_cap();
             qp.queries = d_xyz; qp.m = (uint32_t)n_vertices; qp.k = k;
@@ -714,7 +714,7 @@ static int texture_bake(pt_index *ix, const void *vertices, size_t n_vertices, c
         }
         if (count) {
             QueryParams qp{};
-            qp.pts = ix->pts; qp.attrs = ix->attrs; qp.ids = nullptr; qp.pyr = ix->pyr;
+            qp.pts = ix->pts; qp.attrs = ix->attrs; qp.attrs_curve = ix->attrs_curve; qp.ids = nullptr; qp.pyr = ix->pyr;
             qp.n = ix->n; qp.n_leaves = ix->n_leaves; qp.w_levels = ix->w_levels; qp.t_levels = ix->t_levels;
             qp.pq_cap = opt_queue_cap();
             qp.queries = d_q; qp.m = (uint32_t)count; qp.k = k;

@@ -327,7 +327,10 @@ int pt_texture_render_lists(const void *points, size_t n, const void *vertices, 
  * "grid" (1 build the uniform-grid cell tables [default]), "grid_tma" (1 stage candidate runs
  * with cp.async.bulk [default], 0 per-lane cp.async), "grid_pair" (1 [default]: two samples per
  * warp when k <= 16 and the first attempt's candidates are expected to fit a half-warp; 2: whenever
- * k <= 16; 0: never; the read-only "grid_pair_used" tells what the last launch did),
+ * k <= 16; 0: never; the read-only "grid_pair_used" tells what the last launch did), "grid_span"
+ * (1 [default]: the two-samples-per-warp launch looks up each parent cell once and copies whole
+ * spans of the sorted cloud, reading attributes in sorted order; 0: one look-up and one copy per
+ * cell; the read-only "grid_span_used" tells whether the last grid launch did so),
  * "grid_min_occ10" / "grid_admit100" / "grid_lookup_cost" (search-schedule tuning, see grid_plan:
  * finest table = finest level with >= 4.0 points per occupied cell; a block is tried first when
  * it reaches 1.00 expected k-th-neighbour distances; one bucket look-up costs 8 candidates), "sort_bits" (ordered key bits from the top, 8 per
