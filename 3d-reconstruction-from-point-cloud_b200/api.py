@@ -49,7 +49,7 @@ ABI_SYMBOLS = (
     "pt_merge_device", "pt_halo_route_device", "pt_halo_prepare_device",
     "pt_halo_merge_device", "pt_ghost_check_device", "pt_route_samples_device",
     "pt_scatter_rows_device", "pt_sharded_build", "pt_sharded_free", "pt_sharded_get_info", "pt_sharded_knn",
-    "pt_sharded_transfer", "pt_texture_render_lists", "pt_set_option", "pt_get_option", "pt_debug_stats", "pt_kernel_launch_count",
+    "pt_sharded_transfer", "pt_texture_render_lists", "pt_set_option", "pt_get_option", "pt_debug_stats", "pt_debug_stats_n", "pt_kernel_launch_count",
     "pt_texture_bake", "pt_bake_texels_device", "pt_bake_compose_device",
 )
 # ... and include/pt_synth.h (bench / test scaffolding, its own library)
@@ -231,11 +231,13 @@ def kernel_launch_count():
 
 def debug_stats(reset=True):
     """Work counters of the query kernel (zeros unless the library was built with -DPT_STATS)."""
-    buf = (ctypes.c_uint64 * 16)()
-    _check(lib().pt_debug_stats(buf, 1 if reset else 0), "pt_debug_stats")
     names = ("expansions", "leaves", "pushes", "pops", "compactions", "heap_inserts", "parked",
              "warp_rounds", "overflowed", "samples", "warp_drain_iters", "warp_expand_iters",
-             "grid_attempts", "grid_candidates", "grid_exact_selects", "grid_handed_over")
+             "grid_attempts", "grid_candidates", "grid_exact_selects", "grid_handed_over",
+             "span_lookups", "span_copies", "span_copies_mergeable", "span_warps", "span_warp_busy_ns_sum",
+             "span_warp_busy_ns_max", "span_first_start_ns_inv", "span_last_finish_ns", "span_redo_halves")
+    buf = (ctypes.c_uint64 * len(names))()
+    _check(lib().pt_debug_stats_n(buf, len(names), 1 if reset else 0), "pt_debug_stats_n")
     return {n: int(buf[i]) for i, n in enumerate(names)}
 
 

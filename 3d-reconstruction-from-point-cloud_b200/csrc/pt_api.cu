@@ -52,6 +52,10 @@ static std::atomic<int> g_grid_pair{1};   // grid kernel: two samples per warp w
 int opt_grid_pair() { return g_grid_pair.load(); }
 static std::atomic<int> g_grid_span{1};   // two samples per warp: one look-up per parent cell, one copy per span (0: per cell)
 int opt_grid_span() { return g_grid_span.load(); }
+static std::atomic<int> g_chain_pdl{1};   // hand-over kernels launched as programmatic dependents (0: plain stream order)
+int opt_chain_pdl() { return g_chain_pdl.load(); }
+static std::atomic<int> g_grid_claim{1};   // span kernel: warps claim their next pair with an atomic when each has > 2 pairs (0: static stride)
+int opt_grid_claim() { return g_grid_claim.load(); }
 static std::atomic<int> g_grid_min_occ10{40};    // finest table: finest level with >= this / 10 points per occupied cell
 static std::atomic<int> g_grid_lookup_cost{8};   // grid_plan: cost of one bucket look-up, in candidates
 static std::atomic<int> g_grid_admit100{100};    // grid_plan: a block is tried first when rc cells >= this / 100 expected k-th distances
@@ -106,6 +110,8 @@ int set_option(const char *name, int value)
     if (!strcmp(name, "grid_admit100")) { g_grid_admit100.store(value < 10 ? 10 : value); return PT_OK; }
     if (!strcmp(name, "grid_pair")) { g_grid_pair.store(value < 0 ? 0 : (value > 2 ? 2 : value)); return PT_OK; }
     if (!strcmp(name, "grid_span")) { g_grid_span.store(value ? 1 : 0); return PT_OK; }
+    if (!strcmp(name, "chain_pdl")) { g_chain_pdl.store(value ? 1 : 0); return PT_OK; }
+    if (!strcmp(name, "grid_claim")) { g_grid_claim.store(value ? 1 : 0); return PT_OK; }
     if (!strcmp(name, "sort_bits")) { g_sort_bits.store(value); return PT_OK; }
     if (!strcmp(name, "pool_keep_mb")) { g_pool_keep_mb.store(value < 0 ? -1 : value); return PT_OK; }
     if (!strcmp(name, "pool_guard")) { g_pool_guard.store(value ? 1 : 0); return PT_OK; }
@@ -130,6 +136,8 @@ int get_option(const char *name, int *value)
     if (!strcmp(name, "grid_pair_used")) { *value = g_grid_pair_used.load(); return PT_OK; }
     if (!strcmp(name, "grid_span")) { *value = g_grid_span.load(); return PT_OK; }
     if (!strcmp(name, "grid_span_used")) { *value = g_grid_span_used.load(); return PT_OK; }
+    if (!strcmp(name, "chain_pdl")) { *value = g_chain_pdl.load(); return PT_OK; }
+    if (!strcmp(name, "grid_claim")) { *value = g_grid_claim.load(); return PT_OK; }
     if (!strcmp(name, "sort_bits")) { *value = g_sort_bits.load(); return PT_OK; }
     if (!strcmp(name, "pool_keep_mb")) { *value = g_pool_keep_mb.load(); return PT_OK; }
     if (!strcmp(name, "pool_guard")) { *value = g_pool_guard.load(); return PT_OK; }
@@ -267,6 +275,11 @@ int pt_debug_stats(uint64_t *out16, int reset)
 {
     if (!out16) return PT_ERR_INVALID_ARG;
     return debug_stats(reinterpret_cast<unsigned long long *>(out16), reset);
+}
+int pt_debug_stats_n(uint64_t *out, int n, int reset)
+{
+    if (!out && n > 0) return PT_ERR_INVALID_ARG;
+    return debug_stats_n(reinterpret_cast<unsigned long long *>(out), n, reset);
 }
 
 int pt_index_build(const void *points, size_t n, const pt_build_opts *opts, pt_index **out)

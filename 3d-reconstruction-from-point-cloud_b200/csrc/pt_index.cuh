@@ -128,6 +128,8 @@ int  opt_grid();
 int  opt_grid_tma();
 int  opt_grid_pair();
 int  opt_grid_span();
+int  opt_chain_pdl();
+int  opt_grid_claim();
 int  opt_grid_min_occ10();
 int  opt_grid_admit100();
 int  opt_grid_lookup_cost();
@@ -137,5 +139,6 @@ int  opt_sort_bits();
 size_t opt_pool_keep_bytes();
 int  opt_pool_guard();
 int  debug_stats(unsigned long long *out16, int reset);
+int  debug_stats_n(unsigned long long *out, int n, int reset);
 
 }  // namespace pt

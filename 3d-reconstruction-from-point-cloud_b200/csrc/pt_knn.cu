@@ -18,6 +18,33 @@
 
 namespace pt {
 
+// ---- programmatic dependent launch (the hand-over chain of launch_chain) ---------------------
+// A kernel launched with programmatic stream serialization may start before the kernel ahead of
+// it in the stream has finished; griddepcontrol.wait then blocks until that kernel has completed
+// and its writes are visible (a no-op in a kernel launched the ordinary way).  A kernel lets its
+// dependents launch once all of its blocks have executed launch_dependents or exited.
+__device__ __forceinline__ void pdl_wait() { asm volatile("griddepcontrol.wait;" ::: "memory"); }
+__device__ __forceinline__ void pdl_launch_dependents() { asm volatile("griddepcontrol.launch_dependents;" ::: "memory"); }
+
+// kern<<<grid, block, smem, s>>>(args...), as a programmatic dependent of the kernel before it
+// when `pdl` is set
+template <typename... KArgs, typename... Args>
+static cudaError_t launch_maybe_pdl(bool pdl, void (*kern)(KArgs...), unsigned grid, unsigned block, size_t smem,
+                                    cudaStream_t s, Args... args)
+{
+    cudaLaunchAttribute at[1];
+    at[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
+    at[0].val.programmaticStreamSerializationAllowed = 1;
+    cudaLaunchConfig_t cfg = {};
+    cfg.gridDim = dim3(grid);
+    cfg.blockDim = dim3(block);
+    cfg.dynamicSmemBytes = smem;
+    cfg.stream = s;
+    cfg.attrs = at;
+    cfg.numAttrs = pdl ? 1 : 0;
+    return cudaLaunchKernelEx(&cfg, kern, args...);
+}
+
 // ---- blend (frozen definition, DESIGN.md "blend") --------------------------------------------
 // weights 1/d2 (exact hits: only d2 == 0 neighbours, weight 1); sums accumulated sequentially
 // in neighbour order, fp64, never contracted; colour truncated, normal normalised -> fp32.
@@ -330,6 +357,8 @@ __global__ void __launch_bounds__(WARPS_PER_BLOCK * 32) knn_warp_kernel(const Qu
 }
 
 // Re-runs the samples listed by the thread kernel (queue overflow), grid-stride over the list.
+// Launched as a programmatic dependent: it lets the next kernel of the chain launch at once (its
+// blocks wait for this grid to complete) and waits for the kernel that wrote the list.
 template <typename PT>
 __global__ void __launch_bounds__(WARPS_PER_BLOCK * 32)
 knn_warp_list_kernel(const QueryParams P, const uint32_t *count, const uint32_t *list,
@@ -338,6 +367,8 @@ knn_warp_list_kernel(const QueryParams P, const uint32_t *count, const uint32_t 
     __shared__ float s_lb[WARPS_PER_BLOCK][MAX_W_LEVELS][32];
     const unsigned lane = threadIdx.x & 31;
     const unsigned wib = threadIdx.x >> 5;
+    pdl_launch_dependents();
+    pdl_wait();
     uint32_t n = min(*count, P.m);
     if (stat_out && blockIdx.x == 0 && threadIdx.x == 0) {   // pt_index_info / pt_index_fallback_counts
         stat_out[0] = n;
@@ -382,12 +413,17 @@ static int launch_chain(pt_index *ix, const QueryParams &qp, int variant, cudaSt
 {
     uint32_t *ws = nullptr;
     PT_TRY(pool_alloc((void **)&ws, sizeof(uint32_t) * (8 + 2 * (size_t)qp.m), s));
+    // ws[1]: the span kernel's pair-claim counter, zeroed with the two list counters
     uint32_t *count1 = ws, *count2 = ws + 4, *list1 = ws + 8, *list2 = list1 + qp.m;
     int rc = PT_OK;
     cudaError_t e = cudaMemsetAsync(ws, 0, 8 * sizeof(uint32_t), s);     // both counters at once
     if (e != cudaSuccess) rc = map_cuda_error(e);
     QueryParams q2 = qp;
     const bool grid_first = variant == 6;
+    // Behind a grid kernel the three hand-over kernels are programmatic dependents: each launches
+    // while the kernel ahead of it still runs and waits (griddepcontrol.wait) before it reads a
+    // counter or a list.  Most launches hand nothing over, and the three then only read a counter.
+    const bool pdl = grid_first && opt_chain_pdl() != 0;
     if (rc == PT_OK && variant == 6) {
         // two samples per warp with one look-up per parent cell and one copy per span where the
         // pair kernel would run (pt_knn_span.cuh); otherwise launch_grid picks
@@ -395,7 +431,7 @@ static int launch_chain(pt_index *ix, const QueryParams &qp, int variant, cudaSt
         note_grid_span_used(span ? 1 : 0);
         if (span) {
             note_grid_pair_used(0);
-            rc = launch_grid_span(qp, ix->sm_count, count1, list1, s);
+            rc = launch_grid_span(qp, ix->sm_count, count1, list1, ws + 1, s);
         } else {
             rc = launch_grid<PT>(qp, ix->sm_count, count1, list1, s);
         }
@@ -403,9 +439,11 @@ static int launch_chain(pt_index *ix, const QueryParams &qp, int variant, cudaSt
         // samples cost ~30 us there, but a whole ~110 us block latency in the scan / thread
         // kernels); a long one by the scan / thread kernel in list mode (min_count).
         if (rc == PT_OK) {
-            knn_warp_list_kernel<PT><<<ix->sm_count * 4, WARPS_PER_BLOCK * 32, 0, s>>>(
-                qp, count1, list1, nullptr, nullptr, SHORT_LIST);
+            e = launch_maybe_pdl(pdl, knn_warp_list_kernel<PT>, ix->sm_count * 4, WARPS_PER_BLOCK * 32, 0, s, qp,
+                                 (const uint32_t *)count1, (const uint32_t *)list1, (uint32_t *)nullptr,
+                                 (const uint32_t *)nullptr, SHORT_LIST);
             count_launch();
+            if (e != cudaSuccess) rc = map_cuda_error(e);
         }
         q2.qlist = list1;
         q2.qcount = count1;
@@ -413,12 +451,14 @@ static int launch_chain(pt_index *ix, const QueryParams &qp, int variant, cudaSt
         const bool bounded = qp.r2_per_query != nullptr || qp.r2 < INFINITY;
         variant = (qp.k > 16 || !bounded) ? 5 : 2;
     }
-    if (rc == PT_OK) rc = variant == 5 ? launch_scan<PT>(q2, count2, list2, s) : launch_thread<PT>(q2, count2, list2, s);
+    if (rc == PT_OK)
+        rc = variant == 5 ? launch_scan<PT>(q2, ix->sm_count, pdl, count2, list2, s)
+                          : launch_thread<PT>(q2, ix->sm_count, pdl, count2, list2, s);
     if (rc == PT_OK) {
-        knn_warp_list_kernel<PT><<<ix->sm_count * 4, WARPS_PER_BLOCK * 32, 0, s>>>(
-            qp, count2, list2, ix->fallback_word, grid_first ? count1 : nullptr, 0xffffffffu);
+        e = launch_maybe_pdl(pdl, knn_warp_list_kernel<PT>, ix->sm_count * 4, WARPS_PER_BLOCK * 32, 0, s, qp,
+                             (const uint32_t *)count2, (const uint32_t *)list2, ix->fallback_word,
+                             (const uint32_t *)(grid_first ? count1 : nullptr), 0xffffffffu);
         count_launch();
-        e = cudaGetLastError();
         if (e != cudaSuccess) rc = map_cuda_error(e);
     }
     pool_free(ws, s);

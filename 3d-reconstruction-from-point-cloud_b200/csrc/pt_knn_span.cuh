@@ -149,8 +149,12 @@ __device__ __forceinline__ void span_emit(const QueryParams &P, uint32_t s, bool
         no[sl - 4u] = (len > 0.0 && len < INFINITY) ? __double2float_rn(quo) : 0.0f;
 }
 
+// claim (not null): after its first pair a warp claims its next pair with one atomicAdd (pairs
+// n_warps.. in claiming order) instead of taking every n_warps-th pair, so that the persistent
+// launch ends with the last pair rather than with the warp whose pairs happened to be slowest.
+// Which warp answers a pair never changes the pair's answer.
 __global__ void __launch_bounds__(GRID_WARPS * 32, PT_SPAN_MIN_BLOCKS)
-knn_grid_span_kernel(const QueryParams P, uint32_t *ovf_count, uint32_t *ovf_list)
+knn_grid_span_kernel(const QueryParams P, uint32_t *ovf_count, uint32_t *ovf_list, uint32_t *claim)
 {
     extern __shared__ __align__(128) unsigned char g_smem[];
     const unsigned lane = threadIdx.x & 31, wib = threadIdx.x >> 5;
@@ -163,6 +167,10 @@ knn_grid_span_kernel(const QueryParams P, uint32_t *ovf_count, uint32_t *ovf_lis
     unsigned long long *bars = reinterpret_cast<unsigned long long *>(
         g_smem + sizeof(PointF) * 2 * PAIR_CAP * GRID_WARPS + sizeof(uint2) * 2 * SPAN_MAX * GRID_WARPS);
     const uint32_t bar = smem_u32(bars + wib);
+    // every block is resident from the start (launch_grid_span): the hand-over kernels behind this
+    // one may launch now, they only take the space that finished blocks give up and wait for the
+    // whole grid before they read the list
+    pdl_launch_dependents();
     if (lane == 0) mbar_init(bar, 1);
     __syncwarp();
     uint32_t phase = 0;
@@ -172,14 +180,21 @@ knn_grid_span_kernel(const QueryParams P, uint32_t *ovf_count, uint32_t *ovf_lis
     const PointF *pts = reinterpret_cast<const PointF *>(P.pts);
     uint32_t p = blockIdx.x * GRID_WARPS + wib;
     if (p >= n_pairs) return;
+#ifdef PT_STATS
+    unsigned long long t_start;
+    asm volatile("mov.u64 %0, %%globaltimer;" : "=l"(t_start));
+#endif
     while (p < n_pairs) {
+        // the warp's next pair, claimed now so that the atomic's latency hides behind this pair
+        uint32_t nxt = p + n_warps;
+        if (claim && lane == 0) nxt = n_warps + atomicAdd(claim, 1u);
         // a pair whose second sample does not exist answers the first one twice and emits it once
         const bool valid = 2u * p + (lane >> 4) < P.m;
         const uint32_t s = min(2u * p + (lane >> 4), P.m - 1u);
         const double qx = __ldg(P.queries + 3 * (size_t)s), qy = __ldg(P.queries + 3 * (size_t)s + 1),
                      qz = __ldg(P.queries + 3 * (size_t)s + 2);
-        if (lane == 0 && p + n_warps < n_pairs)      // the next pair's coordinates: towards L2 meanwhile
-            asm volatile("prefetch.global.L2 [%0];" ::"l"(P.queries + 6 * (size_t)(p + n_warps)));
+        if (!claim && lane == 0 && nxt < n_pairs)    // the next pair's coordinates: towards L2 meanwhile
+            asm volatile("prefetch.global.L2 [%0];" ::"l"(P.queries + 6 * (size_t)nxt));
         const double r2 = P.r2_per_query ? __ldg(P.r2_per_query + s) : P.r2;
         const bool dead = valid && !(r2 >= 0.0);
         const bool look = valid && !dead;
@@ -224,6 +239,9 @@ knn_grid_span_kernel(const QueryParams P, uint32_t *ovf_count, uint32_t *ovf_lis
                 oct &= (b0 ? (~m1 & 0xffu) : 0u) | (b1 ? m1 : 0u);
             }
             uint32_t perm = 0;
+#ifdef PT_STATS
+            if (oct) atomicAdd(&g_stats[16], 1ull);
+#endif
             if (oct && grid_parent_lookup(T.buckets, T.cap, pq[0], pq[1], pq[2], pstart, perm, cum)) {
                 const uint32_t occ = perm >> 24, om = oct & occ;
                 if (om && (cum.x & 0xffffu) == 0xffffu) dense = true;
@@ -271,6 +289,18 @@ knn_grid_span_kernel(const QueryParams P, uint32_t *ovf_count, uint32_t *ovf_lis
                 });
             }
             __syncwarp();                           // the span heads are visible to the whole half
+#ifdef PT_STATS
+            if (go) {   // spans whose sorted start is the sorted end of another span of the half
+                uint32_t hits = 0;
+                for (uint32_t a = sl; a < nspan; a += 16u)
+                    for (uint32_t b = 0; b < nspan; ++b) {
+                        const uint32_t nb = (b + 1u < nspan ? heads[b + 1u].x : tot) - heads[b].x;
+                        hits += heads[b].y + nb == heads[a].y ? 1u : 0u;
+                    }
+                if (hits) atomicAdd(&g_stats[18], (unsigned long long)hits);
+                if (sl == 0) atomicAdd(&g_stats[17], (unsigned long long)nspan);
+            }
+#endif
             mbar_wait(bar, phase);
             phase ^= 1u;
         }
@@ -320,6 +350,9 @@ knn_grid_span_kernel(const QueryParams P, uint32_t *ovf_count, uint32_t *ovf_lis
         span_emit(P, s, done, mine, d, li, at, lane, wcand);
         // ---- halves this attempt could not finish: the whole warp, the whole schedule ----------------
         const uint32_t redo = __ballot_sync(0xffffffffu, valid && !done);
+#ifdef PT_STATS
+        if (lane == 0 && redo) atomicAdd(&g_stats[24], (unsigned long long)__popc(redo & 0x10001u));
+#endif
         if (redo & 1u) {
             const double fx = __shfl_sync(0xffffffffu, qx, 0), fy = __shfl_sync(0xffffffffu, qy, 0),
                          fz = __shfl_sync(0xffffffffu, qz, 0);
@@ -330,8 +363,21 @@ knn_grid_span_kernel(const QueryParams P, uint32_t *ovf_count, uint32_t *ovf_lis
                          fz = __shfl_sync(0xffffffffu, qz, 16);
             grid_sample<PointF, true>(P, 2u * p + 1u, fx, fy, fz, lane, wcand, bar, phase, ovf_count, ovf_list);
         }
-        p += n_warps;
+        if (claim && lane == 0 && nxt < n_pairs)
+            asm volatile("prefetch.global.L2 [%0];" ::"l"(P.queries + 6 * (size_t)nxt));
+        p = __shfl_sync(0xffffffffu, nxt, 0);
     }
+#ifdef PT_STATS
+    unsigned long long t_end;
+    asm volatile("mov.u64 %0, %%globaltimer;" : "=l"(t_end));
+    if (lane == 0) {
+        atomicAdd(&g_stats[19], 1ull);
+        atomicAdd(&g_stats[20], t_end - t_start);
+        atomicMax(&g_stats[21], t_end - t_start);
+        atomicMax(&g_stats[22], ~t_start);
+        atomicMax(&g_stats[23], t_end);
+    }
+#endif
 }
 
 // The pair kernel's conditions (launch_grid) plus the curve-ordered attributes wherever the
@@ -346,7 +392,8 @@ static bool grid_span_applies(const QueryParams &qp)
            (qp.attrs_curve != nullptr || qp.attrs == nullptr || !want_attr);
 }
 
-static int launch_grid_span(const QueryParams &qp, int sm_count, uint32_t *count, uint32_t *list, cudaStream_t s)
+static int launch_grid_span(const QueryParams &qp, int sm_count, uint32_t *count, uint32_t *list, uint32_t *claim,
+                            cudaStream_t s)
 {
     const size_t smem = (sizeof(PointF) * 2 * PAIR_CAP + sizeof(uint2) * 2 * SPAN_MAX + 8) * GRID_WARPS;
     if (smem > 48 * 1024)
@@ -356,7 +403,12 @@ static int launch_grid_span(const QueryParams &qp, int sm_count, uint32_t *count
     if (per_sm < 1) per_sm = 1;
     const unsigned want = ((qp.m + 1u) / 2u + GRID_WARPS - 1) / GRID_WARPS;
     const unsigned resident = (unsigned)(sm_count * per_sm);
-    knn_grid_span_kernel<<<want < resident ? want : resident, GRID_WARPS * 32, smem, s>>>(qp, count, list);
+    const unsigned blocks = want < resident ? want : resident;
+    // pairs claimed once a warp has more than two of them (cfg2: 24, cfg5: 120; measured at cfg2
+    // 0.342 -> 0.311 ms, cfg5 7.00 -> 6.49 ms); at cfg1 (1.2 pairs per warp) the static stride is
+    // 1 us faster (DESIGN.md section 4)
+    const bool use_claim = opt_grid_claim() != 0 && (qp.m + 1u) / 2u > 2u * blocks * GRID_WARPS;
+    knn_grid_span_kernel<<<blocks, GRID_WARPS * 32, smem, s>>>(qp, count, list, use_claim ? claim : nullptr);
     count_launch();
     PT_CUDA(cudaGetLastError());
     return PT_OK;

@@ -136,108 +136,111 @@ knn_thread_kernel(const QueryParams P, uint32_t *ovf_count, uint32_t *ovf_list)
     uint32_t *pqk = reinterpret_cast<uint32_t *>(pdi + TPD_CAP * T_THREADS);     // [TPQ_CAP]
     uint32_t *pqw = pqk + TPQ_CAP * T_THREADS;                                    // [TPQ_CAP]
 
-    // list mode (second stage behind the grid kernel, pt_knn_grid.cuh): sample qlist[i], i < *qcount
+    // list mode (second stage behind the grid kernel, pt_knn_grid.cuh): sample qlist[i], i < *qcount,
+    // blocks of T_THREADS list entries grid-stride (the grid is sized to the resident blocks,
+    // launch_thread); the list is read after the kernel that wrote it has completed
+    pdl_wait();
     uint32_t m_eff = P.qlist ? min(*P.qcount, P.m) : P.m;
     if (P.qlist && m_eff < P.qlist_min) m_eff = 0;       // short lists are the warp kernel's
-    if (blockIdx.x * T_THREADS >= m_eff) return;
-    const uint32_t qi = blockIdx.x * T_THREADS + tid;
-    const bool live = qi < m_eff;
-    const uint32_t q = live ? (P.qlist ? P.qlist[qi] : qi) : 0u;
-    bool done = !live || P.t_levels == 0;
-    bool overflow = false;
-
-    double qx = 0, qy = 0, qz = 0, r2 = 0;
-    if (live) {
-        qx = __ldg(P.queries + 3 * (size_t)q);
-        qy = __ldg(P.queries + 3 * (size_t)q + 1);
-        qz = __ldg(P.queries + 3 * (size_t)q + 2);
-        r2 = P.r2_per_query ? __ldg(P.r2_per_query + q) : P.r2;
-    }
-    float bound = __double2float_ru(r2);
-
-#ifdef PT_STATS
-    unsigned st_[16];
-    for (int a = 0; a < 16; ++a) st_[a] = 0;
-#endif
-    int hn = 0;                 // candidates held; the column is a max-heap once hn == k
-    double root_d = INFINITY;   // heap root (current k-th) -- meaningful once hn == k
-    int root_i = IDX_NONE;
-    Traverser<PT, T_THREADS> tr(P, pqk, pqw, qx, qy, qz, !done);
-#ifdef PT_STATS
-    tr.st_ = st_;
-#endif
-
-    for (;;) {
-        const int leaf = tr.next_leaf(bound, hn < k, done);
-        if (__all_sync(0xffffffffu, done)) break;
-
-        // ---- leaf phase: every lane that holds a leaf scans it, 8 points per chunk -------------
-        PT_STAT(1, leaf >= 0 ? 1 : 0);
-        if (tid == 0) PT_STAT(7, 1);
-        const uint32_t base = (uint32_t)(leaf < 0 ? 0 : leaf) * LEAF;
 #pragma unroll 1
-        for (int chunk = 0; chunk < LEAF / PT_T_CHUNK; ++chunk) {
-            int pend = 0;
-            if (leaf >= 0) {
+    for (uint32_t b0 = blockIdx.x * T_THREADS; b0 < m_eff; b0 += gridDim.x * T_THREADS) {
+        const uint32_t qi = b0 + tid;
+        const bool live = qi < m_eff;
+        const uint32_t q = live ? (P.qlist ? P.qlist[qi] : qi) : 0u;
+        bool done = !live || P.t_levels == 0;
+        bool overflow = false;
+
+        double qx = 0, qy = 0, qz = 0, r2 = 0;
+        if (live) {
+            qx = __ldg(P.queries + 3 * (size_t)q);
+            qy = __ldg(P.queries + 3 * (size_t)q + 1);
+            qz = __ldg(P.queries + 3 * (size_t)q + 2);
+            r2 = P.r2_per_query ? __ldg(P.r2_per_query + q) : P.r2;
+        }
+        float bound = __double2float_ru(r2);
+
+#ifdef PT_STATS
+        unsigned st_[16];
+        for (int a = 0; a < 16; ++a) st_[a] = 0;
+#endif
+        int hn = 0;                 // candidates held; the column is a max-heap once hn == k
+        double root_d = INFINITY;   // heap root (current k-th) -- meaningful once hn == k
+        int root_i = IDX_NONE;
+        Traverser<PT, T_THREADS> tr(P, pqk, pqw, qx, qy, qz, !done);
+#ifdef PT_STATS
+        tr.st_ = st_;
+#endif
+
+        for (;;) {
+            const int leaf = tr.next_leaf(bound, hn < k, done);
+            if (__all_sync(0xffffffffu, done)) break;
+
+            // ---- leaf phase: every lane that holds a leaf scans it, 8 points per chunk -------------
+            PT_STAT(1, leaf >= 0 ? 1 : 0);
+            if (tid == 0) PT_STAT(7, 1);
+            const uint32_t base = (uint32_t)(leaf < 0 ? 0 : leaf) * LEAF;
+#pragma unroll 1
+            for (int chunk = 0; chunk < LEAF / PT_T_CHUNK; ++chunk) {
+                int pend = 0;
+                if (leaf >= 0) {
 #pragma unroll
-                for (int p = 0; p < PT_T_CHUNK; ++p) {
-                    const uint32_t pi = base + chunk * PT_T_CHUNK + p;
-                    double px, py, pz;
-                    int pidx;
-                    PointLoad<PT>::load(P.pts, pi, px, py, pz, pidx);
-                    const double d = dist2_exact(qx, qy, qz, px, py, pz);
-                    if (pi < P.n && d <= r2 && (hn < k || key_less(d, pidx, root_d, root_i))) {
-                        pdd[pend * T_THREADS] = d;
-                        pdi[pend * T_THREADS] = pidx;
-                        ++pend;
-                        PT_STAT(6, 1);
+                    for (int p = 0; p < PT_T_CHUNK; ++p) {
+                        const uint32_t pi = base + chunk * PT_T_CHUNK + p;
+                        double px, py, pz;
+                        int pidx;
+                        PointLoad<PT>::load(P.pts, pi, px, py, pz, pidx);
+                        const double d = dist2_exact(qx, qy, qz, px, py, pz);
+                        if (pi < P.n && d <= r2 && (hn < k || key_less(d, pidx, root_d, root_i))) {
+                            pdd[pend * T_THREADS] = d;
+                            pdi[pend * T_THREADS] = pidx;
+                            ++pend;
+                            PT_STAT(6, 1);
+                        }
                     }
                 }
-            }
-            while (__any_sync(0xffffffffu, pend > 0)) {
-                if (tid == 0) PT_STAT(10, 1);
-                if (pend > 0) {
-                    --pend;
-                    const double d = pdd[pend * T_THREADS];
-                    const int pidx = pdi[pend * T_THREADS];
-                    if (hn < k || key_less(d, pidx, root_d, root_i)) PT_STAT(5, 1);
-                    if (hn < k) {
-                        hd[hn * T_THREADS] = d;
-                        hi[hn * T_THREADS] = pidx;
-                        if (++hn == k) {
-                            heapify(hd, hi, k);
+                while (__any_sync(0xffffffffu, pend > 0)) {
+                    if (tid == 0) PT_STAT(10, 1);
+                    if (pend > 0) {
+                        --pend;
+                        const double d = pdd[pend * T_THREADS];
+                        const int pidx = pdi[pend * T_THREADS];
+                        if (hn < k || key_less(d, pidx, root_d, root_i)) PT_STAT(5, 1);
+                        if (hn < k) {
+                            hd[hn * T_THREADS] = d;
+                            hi[hn * T_THREADS] = pidx;
+                            if (++hn == k) {
+                                heapify(hd, hi, k);
+                                root_d = hd[0];
+                                root_i = hi[0];
+                            }
+                        } else if (key_less(d, pidx, root_d, root_i)) {
+                            heap_sift(hd, hi, 0, k, d, pidx);
                             root_d = hd[0];
                             root_i = hi[0];
                         }
-                    } else if (key_less(d, pidx, root_d, root_i)) {
-                        heap_sift(hd, hi, 0, k, d, pidx);
-                        root_d = hd[0];
-                        root_i = hi[0];
                     }
                 }
             }
+            if (hn == k) bound = __double2float_ru(fmin(root_d, r2));
         }
-        if (hn == k) bound = __double2float_ru(fmin(root_d, r2));
-    }
 
-    overflow = tr.proof_failed(bound);
+        overflow = tr.proof_failed(bound);
 #ifdef PT_STATS
-    st_[8] = overflow ? 1 : 0;
-    st_[9] = live ? 1 : 0;
-    for (int a = 0; a < 12; ++a) {
-        unsigned v = st_[a];
-        for (int o = 16; o > 0; o >>= 1) v += __shfl_xor_sync(0xffffffffu, v, o);
-        if (tid == 0 && v) atomicAdd(&g_stats[a], (unsigned long long)v);
-    }
+        st_[8] = overflow ? 1 : 0;
+        st_[9] = live ? 1 : 0;
+        for (int a = 0; a < 12; ++a) {
+            unsigned v = st_[a];
+            for (int o = 16; o > 0; o >>= 1) v += __shfl_xor_sync(0xffffffffu, v, o);
+            if (tid == 0 && v) atomicAdd(&g_stats[a], (unsigned long long)v);
+        }
 #endif
-    if (!live) return;
-    if (overflow) {
-        uint32_t slot = atomicAdd(ovf_count, 1u);
-        ovf_list[slot] = q;
-        return;
+        if (live && overflow) {
+            uint32_t slot = atomicAdd(ovf_count, 1u);
+            ovf_list[slot] = q;
+        } else if (live) {
+            emit_sample<T_THREADS>(P, q, hd, hi, hn);   // sort ascending (d2, index), outputs, blend
+        }
     }
-
-    emit_sample<T_THREADS>(P, q, hd, hi, hn);   // sort ascending (d2, index), outputs, blend
 }
 
 static inline size_t thread_kernel_smem(int k)
@@ -245,28 +248,42 @@ static inline size_t thread_kernel_smem(int k)
     return (size_t)T_THREADS * ((size_t)(k + TPD_CAP) * 12 + (size_t)TPQ_CAP * 8);
 }
 
+// As launch_scan: a list-mode launch gets the resident blocks; `pdl`: a programmatic dependent.
 template <typename PT>
-static int launch_thread(const QueryParams &qp, uint32_t *count, uint32_t *list, cudaStream_t s)
+static int launch_thread(const QueryParams &qp, int sm_count, bool pdl, uint32_t *count, uint32_t *list,
+                         cudaStream_t s)
 {
     const size_t smem = thread_kernel_smem(qp.k) + (size_t)opt_smem_pad();
     if (smem > 48 * 1024)   // only the occupancy probe (smem_pad) ever exceeds the default limit
         PT_CUDA(cudaFuncSetAttribute(knn_thread_kernel<PT>,
                                      cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
     unsigned blocks = (qp.m + T_THREADS - 1) / T_THREADS;
-    knn_thread_kernel<PT><<<blocks, T_THREADS, smem, s>>>(qp, count, list);
+    if (qp.qlist) {
+        // resident blocks per SM, asked once per shared-memory size (it depends on nothing else)
+        static std::atomic<unsigned long long> cached{0};   // smem << 16 | blocks per SM
+        unsigned long long c = cached.load();
+        if (c >> 16 != smem) {
+            int per_sm = 0;
+            PT_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, knn_thread_kernel<PT>, T_THREADS, smem));
+            c = (unsigned long long)smem << 16 | (unsigned long long)max(per_sm, 1);
+            cached.store(c);
+        }
+        blocks = min(blocks, (unsigned)(c & 0xffffu) * (unsigned)sm_count);
+    }
+    PT_CUDA(launch_maybe_pdl(pdl, knn_thread_kernel<PT>, blocks, T_THREADS, smem, s, qp, count, list));
     count_launch();
-    PT_CUDA(cudaGetLastError());
     return PT_OK;
 }
 
-int debug_stats(unsigned long long *out16, int reset)
+int debug_stats_n(unsigned long long *out, int n, int reset)
 {
-    for (int a = 0; a < 16; ++a) out16[a] = 0;
+    if (n < 0) return PT_ERR_INVALID_ARG;
+    for (int a = 0; a < n; ++a) out[a] = 0;
 #ifdef PT_STATS
     PT_CUDA(cudaDeviceSynchronize());
-    PT_CUDA(cudaMemcpyFromSymbol(out16, g_stats, sizeof(unsigned long long) * 16));
+    if (n > 0) PT_CUDA(cudaMemcpyFromSymbol(out, g_stats, sizeof(unsigned long long) * (size_t)min(n, PT_STATS_N)));
     if (reset) {
-        unsigned long long z[16] = {};
+        unsigned long long z[PT_STATS_N] = {};
         PT_CUDA(cudaMemcpyToSymbol(g_stats, z, sizeof z));
     }
 #else
@@ -274,5 +291,7 @@ int debug_stats(unsigned long long *out16, int reset)
 #endif
     return PT_OK;
 }
+
+int debug_stats(unsigned long long *out16, int reset) { return debug_stats_n(out16, 16, reset); }
 
 }  // namespace pt

@@ -21,15 +21,20 @@
 namespace pt {
 
 // -DPT_STATS: per-launch work counters (diagnosis builds only; pt_debug_stats reads them)
+constexpr int PT_STATS_N = 32;   // counter words (pt_debug_stats reads the first 16, pt_debug_stats_n up to all)
 #ifdef PT_STATS
-__device__ unsigned long long g_stats[16];
+__device__ unsigned long long g_stats[PT_STATS_N];
 #define PT_STAT(slot, v) (st_[slot] += (v))
 #else
 #define PT_STAT(slot, v) ((void)0)
 #endif
 // slots: 0 expansions, 1 leaves, 2 pushes, 3 pops, 4 compactions, 5 heap inserts, 6 candidates
 // parked, 7 warp rounds, 8 overflowed samples, 9 samples, 10 drain iterations (warp), 11 expand
-// iterations (warp)
+// iterations (warp); 12-15 grid kernels (pt_knn_grid.cuh); 16-24 knn_grid_span_kernel: 16 parent
+// look-ups, 17 bulk copies, 18 copies that continue another copy of the same half in the sorted
+// cloud (what merging spans across parents would save), 19 warps, 20 / 21 sum / maximum of a
+// warp's busy time (ns), 22 ~earliest warp start, 23 latest warp finish (%globaltimer), 24 halves
+// redone by the whole warp
 
 constexpr int T_LOG = 3;      // 8-wide levels of the box pyramid: binary levels 0, 3, 6, ...
 #ifndef PT_TPQ_CAP

@@ -330,7 +330,11 @@ int pt_texture_render_lists(const void *points, size_t n, const void *vertices, 
  * k <= 16; 0: never; the read-only "grid_pair_used" tells what the last launch did), "grid_span"
  * (1 [default]: the two-samples-per-warp launch looks up each parent cell once and copies whole
  * spans of the sorted cloud, reading attributes in sorted order; 0: one look-up and one copy per
- * cell; the read-only "grid_span_used" tells whether the last grid launch did so),
+ * cell; the read-only "grid_span_used" tells whether the last grid launch did so), "chain_pdl"
+ * (1 [default]: the kernels that answer the samples a grid launch hands over are launched as
+ * programmatic dependents, so their launch overlaps the kernel before them; 0: plain stream order),
+ * "grid_claim" (1 [default]: the span kernel's warps claim their next pair with an atomic when a
+ * launch has more than two pairs per resident warp; 0: every warp takes a fixed stride of pairs),
  * "grid_min_occ10" / "grid_admit100" / "grid_lookup_cost" (search-schedule tuning, see grid_plan:
  * finest table = finest level with >= 4.0 points per occupied cell; a block is tried first when
  * it reaches 1.00 expected k-th-neighbour distances; one bucket look-up costs 8 candidates), "sort_bits" (ordered key bits from the top, 8 per
@@ -348,6 +352,10 @@ int pt_get_option(const char *name, int *value);
 /* Work counters of the query kernel since the last reset (16 words; all zero unless the library
  * was built with -DPT_STATS, a diagnosis build).  Synchronises the device. */
 int pt_debug_stats(uint64_t *out16, int reset);
+/* The same counters, n words of them (up to 32 hold counters, any further words are zero): the
+ * span kernel's look-ups, copies and warp finish times follow the first 16 (see
+ * pt_knn_traverse.cuh).  Synchronises the device. */
+int pt_debug_stats_n(uint64_t *out, int n, int reset);
 /* Number of kernels this library launched since process start (gpu_launches). */
 uint64_t pt_kernel_launch_count(void);
 
