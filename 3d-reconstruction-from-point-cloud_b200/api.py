@@ -51,6 +51,7 @@ ABI_SYMBOLS = (
     "pt_scatter_rows_device", "pt_sharded_build", "pt_sharded_free", "pt_sharded_get_info", "pt_sharded_knn",
     "pt_sharded_transfer", "pt_texture_render_lists", "pt_set_option", "pt_get_option", "pt_debug_stats", "pt_debug_stats_n", "pt_kernel_launch_count",
     "pt_texture_bake", "pt_bake_texels_device", "pt_bake_compose_device",
+    "pt_texture_bake_ex", "pt_bake_samples_device", "pt_bake_frames_device", "pt_bake_compose_tangent_device",
 )
 # ... and include/pt_synth.h (bench / test scaffolding, its own library)
 SYNTH_SYMBOLS = ("pt_synth_cloud_device", "pt_synth_samples_device", "pt_synth_pack_points_device",
@@ -87,6 +88,12 @@ class TextureStats(ctypes.Structure):
 class BakeStats(ctypes.Structure):
     _fields_ = [("texels", ctypes.c_uint64), ("empty", ctypes.c_uint64), ("raster_ms", ctypes.c_float),
                 ("knn_ms", ctypes.c_float), ("pad_ms", ctypes.c_float)]
+
+
+class BakeOutputs(ctypes.Structure):
+    _fields_ = [("bgra", ctypes.c_void_p), ("normal_bgra", ctypes.c_void_p), ("normal", ctypes.c_void_p),
+                ("tangent_bgra", ctypes.c_void_p), ("tangent_normal", ctypes.c_void_p),
+                ("vertex_tangents", ctypes.c_void_p)]
 
 
 class ShardedOpts(ctypes.Structure):
@@ -180,6 +187,15 @@ def lib():
     L.pt_bake_texels_device.argtypes = [vp, sz, vp, sz, i32, vp, vp, ctypes.POINTER(sz), i32, vp]
     L.pt_bake_compose_device.restype = i32
     L.pt_bake_compose_device.argtypes = [vp, sz, vp, vp, i32, i32, vp, vp, vp, i32, vp]
+    L.pt_texture_bake_ex.restype = i32
+    L.pt_texture_bake_ex.argtypes = [vp, vp, sz, vp, sz, i32, dbl, i32, i32, ctypes.POINTER(BakeOutputs),
+                                     ctypes.POINTER(BakeStats)]
+    L.pt_bake_samples_device.restype = i32
+    L.pt_bake_samples_device.argtypes = [vp, sz, vp, sz, i32, vp, vp, vp, ctypes.POINTER(sz), i32, vp]
+    L.pt_bake_frames_device.restype = i32
+    L.pt_bake_frames_device.argtypes = [vp, sz, vp, sz, vp, vp, i32, vp]
+    L.pt_bake_compose_tangent_device.restype = i32
+    L.pt_bake_compose_tangent_device.argtypes = [vp, vp, sz, vp, sz, vp, vp, sz, vp, vp, i32, i32, vp, vp, i32, vp]
     L.pt_set_option.restype = i32
     L.pt_set_option.argtypes = [ctypes.c_char_p, i32]
     L.pt_get_option.restype = i32
@@ -410,31 +426,34 @@ class Tree:
         return img, {"triangles": int(st.triangles), "inside_points": int(st.inside_points),
                      "knn_ms": st.knn_ms, "draw_ms": st.draw_ms, "pad_ms": st.pad_ms}
 
+    _BAKE_OUTPUTS = ("bgra", "normal_bgra", "normal", "tangent_bgra", "tangent_normal", "tangents")
+
     def bake(self, vertices, faces, k=20, resolution=2048, radius=None, pad=True,
              want=("bgra", "normal_bgra", "normal")):
         """Per-texel bake (DESIGN.md section 8): colour and normal maps of the cloud on the mesh's
-        UV atlas.  vertices: Point records (position, U, V), faces: int32 [F,3].  Returns a dict
-        with the requested images -- ``bgra`` uint8 [res,res,4] (B G R 255), ``normal_bgra`` uint8
-        [res,res,4] (object-space normal map, RGB = xyz), ``normal`` float32 [res,res,3] (never
-        padded) -- and ``stats`` (texels, empty, raster_ms, knn_ms, pad_ms)."""
+        UV atlas.  vertices: Point records (position, normal, U, V), faces: int32 [F,3].  Returns a
+        dict with the requested outputs -- ``bgra`` uint8 [res,res,4] (B G R 255), ``normal_bgra``
+        uint8 [res,res,4] (object-space normal map, RGB = xyz), ``normal`` float32 [res,res,3]
+        (never padded), ``tangent_bgra`` uint8 [res,res,4] (tangent-space normal map, glTF / OpenGL
+        convention), ``tangent_normal`` float32 [res,res,3] (never padded), ``tangents`` float32
+        [n_vertices,4] (the per-vertex tangent and handedness the tangent maps are expressed in, glTF
+        TANGENT layout) -- and ``stats`` (texels, empty, raster_ms, knn_ms, pad_ms).  All outputs
+        come from one k-NN pass."""
         v = _as_points(vertices, "vertices")
         f = np.ascontiguousarray(faces, dtype=np.int32).reshape(-1, 3)
-        unknown = set(want) - {"bgra", "normal_bgra", "normal"}
+        unknown = set(want) - set(self._BAKE_OUTPUTS)
         if unknown or not want:
-            raise ValueError(f"want must name some of bgra, normal_bgra, normal (got {want!r})")
+            raise ValueError(f"want must name some of {', '.join(self._BAKE_OUTPUTS)} (got {want!r})")
         res = int(resolution)
-        out = {}
-        if "bgra" in want:
-            out["bgra"] = np.empty((res, res, 4), dtype=np.uint8)
-        if "normal_bgra" in want:
-            out["normal_bgra"] = np.empty((res, res, 4), dtype=np.uint8)
-        if "normal" in want:
-            out["normal"] = np.empty((res, res, 3), dtype=np.float32)
+        shapes = {"bgra": ((res, res, 4), np.uint8), "normal_bgra": ((res, res, 4), np.uint8),
+                  "normal": ((res, res, 3), np.float32), "tangent_bgra": ((res, res, 4), np.uint8),
+                  "tangent_normal": ((res, res, 3), np.float32), "tangents": ((v.shape[0], 4), np.float32)}
+        out = {name: np.empty(*shapes[name]) for name in self._BAKE_OUTPUTS if name in want}
+        o = BakeOutputs(*[out[name].ctypes.data if name in out else None for name in self._BAKE_OUTPUTS])
         st = BakeStats()
-        _check(lib().pt_texture_bake(self._h, _np_ptr(v), v.shape[0], _np_ptr(f), f.shape[0], int(k),
-                                     _radius(radius), res, 1 if pad else 0, _np_ptr(out.get("bgra")),
-                                     _np_ptr(out.get("normal_bgra")), _np_ptr(out.get("normal")),
-                                     ctypes.byref(st)), "pt_texture_bake")
+        _check(lib().pt_texture_bake_ex(self._h, _np_ptr(v), v.shape[0], _np_ptr(f), f.shape[0], int(k),
+                                        _radius(radius), res, 1 if pad else 0, ctypes.byref(o), ctypes.byref(st)),
+               "pt_texture_bake_ex")
         out["stats"] = {"texels": int(st.texels), "empty": int(st.empty), "raster_ms": st.raster_ms,
                         "knn_ms": st.knn_ms, "pad_ms": st.pad_ms}
         return out
@@ -659,3 +678,71 @@ def bake_compose_device(texels, rgba, normal, resolution, pad=True, bgra=None, n
         _check(lib().pt_bake_compose_device(_tptr(texels), m, _tptr(rgba), _tptr(normal), int(resolution),
                                             1 if pad else 0, _tptr(bgra), _tptr(normal_bgra), _tptr(normal_out),
                                             texels.device.index, _stream_ptr(stream)), "pt_bake_compose_device")
+
+
+def bake_samples_device(vertices_xyzuv, faces, resolution, stream=None):
+    """``pt_bake_samples_device``: ``bake_texels_device`` plus the owner face of every sample.
+    Returns (texel ids int32 [m], positions float64 [m,3], faces int32 [m]).  Synchronises
+    ``stream``."""
+    import torch
+    assert vertices_xyzuv.is_cuda and vertices_xyzuv.dtype == torch.float64 and vertices_xyzuv.is_contiguous()
+    assert vertices_xyzuv.dim() == 2 and vertices_xyzuv.shape[1] == 5
+    assert faces.is_cuda and faces.dtype == torch.int32 and faces.is_contiguous() and faces.numel() % 3 == 0
+    dev = vertices_xyzuv.device
+    cap = int(resolution) * int(resolution)
+    texels = torch.empty(cap, dtype=torch.int32, device=dev)
+    xyz = torch.empty((cap, 3), dtype=torch.float64, device=dev)
+    owner = torch.empty(cap, dtype=torch.int32, device=dev)
+    count = ctypes.c_size_t(0)
+    with torch.cuda.device(dev):
+        _check(lib().pt_bake_samples_device(_tptr(vertices_xyzuv), vertices_xyzuv.shape[0], _tptr(faces),
+                                            faces.numel() // 3, int(resolution), _tptr(texels), _tptr(xyz),
+                                            _tptr(owner), ctypes.byref(count), dev.index, _stream_ptr(stream)),
+               "pt_bake_samples_device")
+    m = count.value
+    return texels[:m], xyz.view(-1)[:3 * m].view(m, 3), owner[:m]
+
+
+def bake_frames_device(vertices_xyzuvn, faces, tangents=True, stream=None):
+    """``pt_bake_frames_device``: the tangent bake's vertex frames.  vertices_xyzuvn: float64
+    [n,8] CUDA tensor (x, y, z, u, v, nx, ny, nz), faces: int32 [F,3].  Returns (frames float64
+    [n,8] = N xyz, T xyz, w, 0; tangents float32 [n,4] or None).  Asynchronous on ``stream``."""
+    import torch
+    assert vertices_xyzuvn.is_cuda and vertices_xyzuvn.dtype == torch.float64 and vertices_xyzuvn.is_contiguous()
+    assert vertices_xyzuvn.dim() == 2 and vertices_xyzuvn.shape[1] == 8
+    assert faces.is_cuda and faces.dtype == torch.int32 and faces.is_contiguous() and faces.numel() % 3 == 0
+    dev, n = vertices_xyzuvn.device, vertices_xyzuvn.shape[0]
+    frames = torch.empty((n, 8), dtype=torch.float64, device=dev)
+    tg = torch.empty((n, 4), dtype=torch.float32, device=dev) if tangents else None
+    with torch.cuda.device(dev):
+        _check(lib().pt_bake_frames_device(_tptr(vertices_xyzuvn), n, _tptr(faces), faces.numel() // 3, _tptr(frames),
+                                           _tptr(tg), dev.index, _stream_ptr(stream)), "pt_bake_frames_device")
+    return frames, tg
+
+
+def bake_compose_tangent_device(vertices_xyzuvn, frames, faces, texels, sample_faces, rgba, normal, resolution,
+                                pad=True, tangent_bgra=None, tangent_normal=None, stream=None):
+    """``pt_bake_compose_tangent_device``: the tangent maps from the samples (``texels`` and
+    ``sample_faces`` of ``bake_samples_device``, ``rgba`` / ``normal`` of ``DeviceTree.query``)
+    and the frames of ``bake_frames_device``.  Outputs are pre-allocated CUDA tensors (uint8
+    [res,res,4], float32 [res,res,3]) or None; at least one must be given.  Asynchronous on
+    ``stream``."""
+    import torch
+    m, n = texels.numel(), vertices_xyzuvn.shape[0]
+    assert vertices_xyzuvn.is_cuda and vertices_xyzuvn.dtype == torch.float64 and vertices_xyzuvn.is_contiguous()
+    assert vertices_xyzuvn.dim() == 2 and vertices_xyzuvn.shape[1] == 8
+    assert frames.is_cuda and frames.dtype == torch.float64 and frames.is_contiguous() and frames.numel() == 8 * n
+    assert faces.is_cuda and faces.dtype == torch.int32 and faces.is_contiguous() and faces.numel() % 3 == 0
+    for t, dt, cnt in ((texels, torch.int32, m), (sample_faces, torch.int32, m), (rgba, torch.uint8, 4 * m),
+                       (normal, torch.float32, 3 * m)):
+        assert t.is_cuda and t.is_contiguous() and t.dtype == dt and t.numel() == cnt
+    n_pix = int(resolution) * int(resolution)
+    for t, dt, cnt in ((tangent_bgra, torch.uint8, 4 * n_pix), (tangent_normal, torch.float32, 3 * n_pix)):
+        if t is not None:
+            assert t.is_cuda and t.is_contiguous() and t.dtype == dt and t.numel() == cnt
+    with torch.cuda.device(texels.device):
+        _check(lib().pt_bake_compose_tangent_device(_tptr(vertices_xyzuvn), _tptr(frames), n, _tptr(faces),
+                                                    faces.numel() // 3, _tptr(texels), _tptr(sample_faces), m,
+                                                    _tptr(rgba), _tptr(normal), int(resolution), 1 if pad else 0,
+                                                    _tptr(tangent_bgra), _tptr(tangent_normal), texels.device.index,
+                                                    _stream_ptr(stream)), "pt_bake_compose_tangent_device")

@@ -19,7 +19,9 @@
 // evaluated once per index-sorted quadruple).  Not reproduced: the out-of-bounds row
 // `resolution - j` at j = 0 / column `resolution` (:100-103) and the uninitialised Mat (:402).
 #include <cmath>
+#include <initializer_list>
 
+#include <cub/device/device_radix_sort.cuh>
 #include <cub/device/device_scan.cuh>
 #include <cub/device/device_select.cuh>
 #include <thrust/iterator/counting_iterator.h>
@@ -417,9 +419,8 @@ static int texture_render_index(pt_index *ix, const void *vertices, size_t n_ver
 // barycentric mix of the winning face's 3-D corners, fp64, never contracted.
 //
 // Vertices are read through a stride, so both the caller's n x 5 (x, y, z, u, v) rows and the
-// MeshVertex records of tex_unpack_vertices_kernel (x, y, z, u, v first) can be rasterised.
+// n x 8 rows (x, y, z, u, v, nx, ny, nz) of bake_unpack_vertices_kernel can be rasterised.
 constexpr int BAKE_TILE = 32;                  // one warp per (face, 32 x 32-texel tile of its box)
-static_assert(sizeof(MeshVertex) % sizeof(double) == 0, "MeshVertex rows are read as doubles");
 
 struct BakeMesh {
     const double  *v;          // n_vertices rows of `stride` doubles: x, y, z, u, v, ...
@@ -536,14 +537,16 @@ struct BakeCovered {
     __device__ __forceinline__ bool operator()(uint32_t t) const { return owner[t] != 0u; }
 };
 
-// position of sample i (texel texels[i]) on its owner face
+// position of sample i (texel texels[i]) on its owner face, and the face itself when face_out is set
 __global__ void __launch_bounds__(256)
-bake_position_kernel(const BakeMesh M, const uint32_t *owner, const uint32_t *texels, uint32_t count, double *xyz)
+bake_position_kernel(const BakeMesh M, const uint32_t *owner, const uint32_t *texels, uint32_t count, double *xyz,
+                     int32_t *face_out)
 {
     const uint32_t i = blockIdx.x * blockDim.x + threadIdx.x;
     if (i >= count) return;
     const uint32_t tex = texels[i];
     const uint32_t f = owner[tex] - 1u;
+    if (face_out) face_out[i] = (int32_t)f;
     const double *c[3];
     bake_corners(M, f, c);
     V2 t[3];
@@ -557,9 +560,11 @@ bake_position_kernel(const BakeMesh M, const uint32_t *owner, const uint32_t *te
 }
 
 // Owner map -> samples in ascending texel order.  M.faces / M.v are device pointers on the current
-// device.  texel_out / xyz_out: room for res * res samples, or both null (count only).  Synchronises
-// `s`; *count_out is the number of covered texels.
-static int bake_texels(const BakeMesh &M, uint32_t *texel_out, double *xyz_out, size_t *count_out, cudaStream_t s)
+// device.  texel_out / xyz_out: room for res * res samples, or both null (count only); face_out
+// (owner face per sample, may be null) needs them.  Synchronises `s`; *count_out is the number of
+// covered texels.
+static int bake_texels(const BakeMesh &M, uint32_t *texel_out, double *xyz_out, int32_t *face_out, size_t *count_out,
+                       cudaStream_t s)
 {
     const size_t n_pix = (size_t)M.res * M.res;
     unsigned long long *d_tiles = nullptr, *d_first = nullptr;
@@ -598,7 +603,7 @@ static int bake_texels(const BakeMesh &M, uint32_t *texel_out, double *xyz_out, 
         if (fail(cudaMemcpyAsync(&count, d_count, sizeof count, cudaMemcpyDeviceToHost, s))) break;
         if (fail(cudaStreamSynchronize(s))) break;
         if (xyz_out && count) {
-            bake_position_kernel<<<tcdiv(count, 256), 256, 0, s>>>(M, d_owner, sel, count, xyz_out);
+            bake_position_kernel<<<tcdiv(count, 256), 256, 0, s>>>(M, d_owner, sel, count, xyz_out, face_out);
             count_launch();
         }
         if (fail(cudaGetLastError())) break;
@@ -636,8 +641,27 @@ bake_compose_kernel(const uint32_t *texels, uint32_t count, const uint8_t *rgba,
     if (nf) { nf[3 * t] = x; nf[3 * t + 1] = y; nf[3 * t + 2] = z; }
 }
 
-// Zeroes the requested maps, scatters the samples into them and pads the 8-bit ones in place with
-// the texture's dilate + gutter kernels (tex_dilate_v_pad_kernel reads only its own texel of `tex`).
+// Pads the given 8-bit maps (null entries skipped) in place with the texture's dilate + gutter
+// kernels (tex_dilate_v_pad_kernel reads only its own texel of `tex`).
+static int bake_pad(std::initializer_list<uint8_t *> imgs, int res, cudaStream_t s)
+{
+    const size_t n_pix = (size_t)res * res;
+    bool any = false;
+    for (uint8_t *img : imgs) any |= img != nullptr;
+    if (!any) return PT_OK;
+    uint32_t *d_tmp = nullptr;
+    PT_TRY(pool_alloc((void **)&d_tmp, 4 * n_pix, s));
+    for (uint8_t *img : imgs) {
+        if (!img) continue;
+        tex_dilate_h_kernel<<<tcdiv(n_pix, 256), 256, 0, s>>>((const uint32_t *)img, res, d_tmp);
+        tex_dilate_v_pad_kernel<<<tcdiv(n_pix, 256), 256, 0, s>>>((const uint32_t *)img, d_tmp, res, (uint32_t *)img);
+        count_launch(2);
+    }
+    pool_free(d_tmp, s);
+    return PT_OK;
+}
+
+// Zeroes the requested maps, scatters the samples into them and pads the 8-bit ones in place.
 static int bake_compose(const uint32_t *texels, size_t count, const uint8_t *rgba, const float *normal, int res,
                         int pad, uint8_t *bgra_out, uint8_t *normal_bgra_out, float *normal_out,
                         unsigned long long *d_empty, cudaStream_t s)
@@ -651,34 +675,278 @@ static int bake_compose(const uint32_t *texels, size_t count, const uint8_t *rgb
                                                               (uint32_t *)normal_bgra_out, normal_out, d_empty);
         count_launch();
     }
-    if (pad && (bgra_out || normal_bgra_out)) {
-        uint32_t *d_tmp = nullptr;
-        PT_TRY(pool_alloc((void **)&d_tmp, 4 * n_pix, s));
-        for (uint8_t *img : {bgra_out, normal_bgra_out}) {
-            if (!img) continue;
-            tex_dilate_h_kernel<<<tcdiv(n_pix, 256), 256, 0, s>>>((const uint32_t *)img, res, d_tmp);
-            tex_dilate_v_pad_kernel<<<tcdiv(n_pix, 256), 256, 0, s>>>((const uint32_t *)img, d_tmp, res, (uint32_t *)img);
-            count_launch(2);
-        }
-        pool_free(d_tmp, s);
-    }
+    if (pad) PT_TRY(bake_pad({bgra_out, normal_bgra_out}, res, s));
     PT_CUDA(cudaGetLastError());
     return PT_OK;
 }
 
+// ---- tangent-space bake (DESIGN.md section 8, "Tangent-space bake") -----------------------------
+// Everything below is fp64 with every operation rounded on its own (no contraction, no rsqrt), in
+// the order the definition states, so that tests/bake_tangent_oracle.c equals it bit for bit:
+// a.b = (a.x b.x + a.y b.y) + a.z b.z; "usable" = all components finite and a.a > 0; normalising
+// divides each component by sqrt(a.a).  Mesh rows are 8 doubles: x y z u v nx ny nz.  Frame rows
+// are 8 doubles: N xyz, T xyz, w, 0 -- all zero for a vertex without a frame.
+constexpr int BAKE_ROW = 8;
+
+struct D3 { double x, y, z; };
+
+__device__ __forceinline__ D3 d3_add(D3 a, D3 b) { return {__dadd_rn(a.x, b.x), __dadd_rn(a.y, b.y), __dadd_rn(a.z, b.z)}; }
+__device__ __forceinline__ D3 d3_sub(D3 a, D3 b) { return {__dsub_rn(a.x, b.x), __dsub_rn(a.y, b.y), __dsub_rn(a.z, b.z)}; }
+__device__ __forceinline__ D3 d3_scale(double s, D3 a) { return {__dmul_rn(s, a.x), __dmul_rn(s, a.y), __dmul_rn(s, a.z)}; }
+__device__ __forceinline__ double d3_dot(D3 a, D3 b)
+{
+    return __dadd_rn(__dadd_rn(__dmul_rn(a.x, b.x), __dmul_rn(a.y, b.y)), __dmul_rn(a.z, b.z));
+}
+__device__ __forceinline__ D3 d3_cross(D3 a, D3 b)
+{
+    return {__dsub_rn(__dmul_rn(a.y, b.z), __dmul_rn(a.z, b.y)), __dsub_rn(__dmul_rn(a.z, b.x), __dmul_rn(a.x, b.z)),
+            __dsub_rn(__dmul_rn(a.x, b.y), __dmul_rn(a.y, b.x))};
+}
+__device__ __forceinline__ bool d3_finite(D3 a) { return isfinite(a.x) && isfinite(a.y) && isfinite(a.z); }
+__device__ __forceinline__ bool d3_usable(D3 a) { return d3_finite(a) && d3_dot(a, a) > 0.0; }
+__device__ __forceinline__ D3 d3_normalise(D3 a)
+{
+    const double l = __dsqrt_rn(d3_dot(a, a));
+    return {__ddiv_rn(a.x, l), __ddiv_rn(a.y, l), __ddiv_rn(a.z, l)};
+}
+__device__ __forceinline__ D3 d3_load(const double *p) { return {p[0], p[1], p[2]}; }
+// (b0 a + b1 b) + b2 c, per component
+__device__ __forceinline__ D3 d3_mix(const double bc[3], D3 a, D3 b, D3 c)
+{
+    return d3_add(d3_add(d3_scale(bc[0], a), d3_scale(bc[1], b)), d3_scale(bc[2], c));
+}
+// the unit tangent of unit normal n from t: t - (n.t) n normalised, or the fallback F(n) -- the axis
+// e_i with the smallest |n_i| (lowest i on ties), e_i - n_i n normalised
+__device__ __forceinline__ D3 bake_tangent_dir(D3 n, D3 t)
+{
+    const D3 r = d3_sub(t, d3_scale(d3_dot(n, t), n));
+    if (d3_usable(r)) return d3_normalise(r);
+    const double ax = fabs(n.x), ay = fabs(n.y), az = fabs(n.z);
+    const int i = (ax <= ay && ax <= az) ? 0 : (ay <= az ? 1 : 2);
+    const double ni = i == 0 ? n.x : (i == 1 ? n.y : n.z);
+    const D3 e = {i == 0 ? 1.0 : 0.0, i == 1 ? 1.0 : 0.0, i == 2 ? 1.0 : 0.0};
+    return d3_normalise(d3_sub(e, d3_scale(ni, n)));
+}
+
+struct FaceFrame { D3 t, b, g; };
+
+// T_f, B_f (both 0 when det == 0 or a component is not finite) and G_f = e1 x e2 of a face with
+// valid corners; UV differences in UV units, independent of the resolution
+__device__ __forceinline__ FaceFrame bake_face_frame(const double *const c[3])
+{
+    const D3 xa = d3_load(c[0]);
+    const D3 e1 = d3_sub(d3_load(c[1]), xa), e2 = d3_sub(d3_load(c[2]), xa);
+    const double du1 = __dsub_rn(c[1][3], c[0][3]), dv1 = __dsub_rn(c[1][4], c[0][4]);
+    const double du2 = __dsub_rn(c[2][3], c[0][3]), dv2 = __dsub_rn(c[2][4], c[0][4]);
+    const double det = __dsub_rn(__dmul_rn(du1, dv2), __dmul_rn(du2, dv1));
+    const double r = __ddiv_rn(1.0, det);
+    FaceFrame F;
+    F.t = d3_scale(r, d3_sub(d3_scale(dv2, e1), d3_scale(dv1, e2)));
+    F.b = d3_scale(r, d3_sub(d3_scale(du1, e2), d3_scale(du2, e1)));
+    if (det == 0.0 || !d3_finite(F.t) || !d3_finite(F.b)) F.t = F.b = D3{0.0, 0.0, 0.0};
+    F.g = d3_cross(e1, e2);
+    return F;
+}
+
+// per face: T_f B_f G_f (9 doubles) and its three corner entries (vertex id, corner id 3f + j); a
+// face with an out-of-range index pushes the key n_vertices, which sorts behind every vertex
+__global__ void __launch_bounds__(256)
+bake_face_frame_kernel(const BakeMesh M, double *face_tbg, uint32_t *corner_vertex, uint32_t *corner_id)
+{
+    const uint32_t f = blockIdx.x * blockDim.x + threadIdx.x;
+    if (f >= M.n_faces) return;
+    const double *c[3];
+    const bool ok = bake_corners(M, f, c);
+    FaceFrame F = {};
+    if (ok) F = bake_face_frame(c);
+    double *o = face_tbg + 9 * (size_t)f;
+    o[0] = F.t.x; o[1] = F.t.y; o[2] = F.t.z;
+    o[3] = F.b.x; o[4] = F.b.y; o[5] = F.b.z;
+    o[6] = F.g.x; o[7] = F.g.y; o[8] = F.g.z;
+#pragma unroll
+    for (int j = 0; j < 3; ++j) {
+        corner_vertex[3 * (size_t)f + j] = ok ? (uint32_t)M.faces[3 * (size_t)f + j] : M.n_vertices;
+        corner_id[3 * (size_t)f + j] = 3u * f + (uint32_t)j;
+    }
+}
+
+__device__ __forceinline__ uint32_t bake_lower_bound(const uint32_t *a, uint32_t n, uint32_t key)
+{
+    uint32_t lo = 0, hi = n;
+    while (lo < hi) {
+        const uint32_t mid = lo + ((hi - lo) >> 1);
+        if (a[mid] < key) lo = mid + 1; else hi = mid;
+    }
+    return lo;
+}
+
+// One thread per vertex: the sums over its corners in ascending corner id (= face order, then
+// a, b, c: the sort is stable), then N, T and w.  No atomics, so the sums are the oracle's.
+__global__ void __launch_bounds__(256)
+bake_vertex_frame_kernel(const BakeMesh M, const double *face_tbg, const uint32_t *sorted_vertex,
+                         const uint32_t *sorted_corner, uint32_t n_corners, double *frames, float *tangents)
+{
+    const uint32_t v = blockIdx.x * blockDim.x + threadIdx.x;
+    if (v >= M.n_vertices) return;
+    const uint32_t lo = bake_lower_bound(sorted_vertex, n_corners, v);
+    const uint32_t hi = bake_lower_bound(sorted_vertex, n_corners, v + 1u);
+    D3 T = {0.0, 0.0, 0.0}, B = T, G = T;
+    for (uint32_t i = lo; i < hi; ++i) {
+        const double *fr = face_tbg + 9 * (size_t)(sorted_corner[i] / 3u);
+        T = d3_add(T, d3_load(fr));
+        B = d3_add(B, d3_load(fr + 3));
+        G = d3_add(G, d3_load(fr + 6));
+    }
+    const D3 nv = d3_load(M.v + (size_t)v * M.stride + 5);
+    double out[BAKE_ROW] = {0.0, 0.0, 0.0, 0.0, 0.0, 0.0, 0.0, 0.0};
+    if (d3_usable(nv) || d3_usable(G)) {
+        const D3 N = d3_normalise(d3_usable(nv) ? nv : G);
+        const D3 Th = bake_tangent_dir(N, T);
+        const double w = d3_dot(d3_cross(N, Th), B) < 0.0 ? -1.0 : 1.0;
+        out[0] = N.x; out[1] = N.y; out[2] = N.z;
+        out[3] = Th.x; out[4] = Th.y; out[5] = Th.z;
+        out[6] = w;
+    }
+#pragma unroll
+    for (int j = 0; j < BAKE_ROW; ++j) frames[(size_t)v * BAKE_ROW + j] = out[j];
+    if (tangents)
+#pragma unroll
+        for (int j = 0; j < 4; ++j) tangents[4 * (size_t)v + j] = (float)out[3 + j];
+}
+
+// Vertex frames of a mesh of rows of 8 doubles into frames (n_vertices x 8) and, when set,
+// tangents (n_vertices x float4).  Needs 3 * n_faces <= INT_MAX (the sort's item count).
+// Asynchronous on s.
+static int bake_frames(const BakeMesh &M, double *frames, float *tangents, cudaStream_t s)
+{
+    if (!M.n_vertices) return PT_OK;
+    const size_t n_corners = 3 * (size_t)M.n_faces;
+    const size_t nc = n_corners ? n_corners : 1;
+    double *d_tbg = nullptr;
+    uint32_t *d_key = nullptr, *d_val = nullptr, *d_key_s = nullptr, *d_val_s = nullptr;
+    void *d_tmp = nullptr;
+    int rc = PT_OK;
+    auto fail = [&](cudaError_t e) { if (e != cudaSuccess && rc == PT_OK) rc = map_cuda_error(e); return e != cudaSuccess; };
+    do {
+        // keys are vertex ids <= n_vertices (the sentinel): sort only the bits they use
+        const int end_bit = 32 - __builtin_clz(M.n_vertices);
+        size_t sort_bytes = 0;
+        if (fail(cub::DeviceRadixSort::SortPairs(nullptr, sort_bytes, d_key, d_key_s, d_val, d_val_s, (int)nc, 0, end_bit, s)))
+            break;
+        if (pool_alloc((void **)&d_tbg, sizeof(double) * 9 * (M.n_faces ? M.n_faces : 1), s) ||
+            pool_alloc((void **)&d_key, sizeof(uint32_t) * nc, s) || pool_alloc((void **)&d_val, sizeof(uint32_t) * nc, s) ||
+            pool_alloc((void **)&d_key_s, sizeof(uint32_t) * nc, s) || pool_alloc((void **)&d_val_s, sizeof(uint32_t) * nc, s) ||
+            pool_alloc(&d_tmp, sort_bytes ? sort_bytes : 1, s)) {
+            rc = PT_ERR_OUT_OF_MEMORY;
+            break;
+        }
+        if (M.n_faces) {
+            bake_face_frame_kernel<<<tcdiv(M.n_faces, 256), 256, 0, s>>>(M, d_tbg, d_key, d_val);
+            count_launch();
+            if (fail(cub::DeviceRadixSort::SortPairs(d_tmp, sort_bytes, d_key, d_key_s, d_val, d_val_s, (int)n_corners, 0,
+                                                     end_bit, s)))
+                break;
+            count_launch();
+        }
+        bake_vertex_frame_kernel<<<tcdiv(M.n_vertices, 256), 256, 0, s>>>(M, d_tbg, d_key_s, d_val_s, (uint32_t)n_corners,
+                                                                        frames, tangents);
+        count_launch();
+        fail(cudaGetLastError());
+    } while (0);
+    void *frees[] = {d_tbg, d_key, d_val, d_key_s, d_val_s, d_tmp};
+    for (void *p : frees) pool_free(p, s);
+    return rc;
+}
+
+// One thread per sample: the owner face's barycentrics of the texel centre (as the texel stage
+// computes them), the mixed vertex frames made orthonormal, the handedness of the owner face's B_f,
+// and the blended cloud normal in that basis.  An empty neighbour list (alpha 0) or an unusable
+// mixed normal leaves the texel 0.
+__global__ void __launch_bounds__(256)
+bake_tangent_compose_kernel(const BakeMesh M, const double *frames, const uint32_t *texels, const int32_t *sample_faces,
+                            uint32_t count, const uint8_t *rgba, const float *normal, uint32_t *tbgra, float *tnf,
+                            unsigned long long *empty)
+{
+    const uint32_t i = blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= count) return;
+    if (rgba[4 * (size_t)i + 3] == 0) {
+        if (empty) atomicAdd(empty, 1ull);
+        return;
+    }
+    const int32_t f = sample_faces[i];
+    const uint32_t tex = texels[i];
+    const double *c[3];
+    if (f < 0 || (uint32_t)f >= M.n_faces || tex >= (uint32_t)M.res * (uint32_t)M.res || !bake_corners(M, (uint32_t)f, c))
+        return;
+    V2 t[3];
+    bake_uv(M, c, t);
+    double bc[3];
+    tx_tri_coords(t[0], t[1], t[2], bake_texel_point(M.res, (int)(tex % (uint32_t)M.res), (int)(tex / (uint32_t)M.res)), bc);
+    const double *fr[3];
+#pragma unroll
+    for (int j = 0; j < 3; ++j) fr[j] = frames + (size_t)M.faces[3 * (size_t)f + j] * BAKE_ROW;
+    const D3 n = d3_mix(bc, d3_load(fr[0]), d3_load(fr[1]), d3_load(fr[2]));
+    if (!d3_usable(n)) return;
+    const D3 tm = d3_mix(bc, d3_load(fr[0] + 3), d3_load(fr[1] + 3), d3_load(fr[2] + 3));
+    const D3 N = d3_normalise(n);
+    const D3 T = bake_tangent_dir(N, tm);
+    const D3 x = d3_cross(N, T);
+    const double w = d3_dot(x, bake_face_frame(c).b) < 0.0 ? -1.0 : 1.0;
+    const D3 B = d3_scale(w, x);
+    const D3 m = {(double)normal[3 * (size_t)i], (double)normal[3 * (size_t)i + 1], (double)normal[3 * (size_t)i + 2]};
+    const float sx = (float)d3_dot(m, T), sy = (float)d3_dot(m, B), sz = (float)d3_dot(m, N);
+    if (tbgra) tbgra[tex] = bake_encode(sz) | (bake_encode(sy) << 8) | (bake_encode(sx) << 16) | 0xff000000u;
+    if (tnf) { tnf[3 * (size_t)tex] = sx; tnf[3 * (size_t)tex + 1] = sy; tnf[3 * (size_t)tex + 2] = sz; }
+}
+
+// Zeroes the requested tangent maps, composes the samples into them and pads the 8-bit one.
+static int bake_compose_tangent(const BakeMesh &M, const double *frames, const uint32_t *texels,
+                                const int32_t *sample_faces, size_t count, const uint8_t *rgba, const float *normal,
+                                int pad, uint8_t *tbgra_out, float *tnormal_out, unsigned long long *d_empty,
+                                cudaStream_t s)
+{
+    const size_t n_pix = (size_t)M.res * M.res;
+    if (tbgra_out) PT_CUDA(cudaMemsetAsync(tbgra_out, 0, 4 * n_pix, s));
+    if (tnormal_out) PT_CUDA(cudaMemsetAsync(tnormal_out, 0, sizeof(float) * 3 * n_pix, s));
+    if (count) {
+        bake_tangent_compose_kernel<<<tcdiv(count, 256), 256, 0, s>>>(M, frames, texels, sample_faces, (uint32_t)count, rgba,
+                                                                     normal, (uint32_t *)tbgra_out, tnormal_out, d_empty);
+        count_launch();
+    }
+    if (pad) PT_TRY(bake_pad({tbgra_out}, M.res, s));
+    PT_CUDA(cudaGetLastError());
+    return PT_OK;
+}
+
+// 80-byte Point records -> rows of 8 doubles (x y z u v nx ny nz), what the raster and the frames read
+__global__ void __launch_bounds__(256) bake_unpack_vertices_kernel(const Raw80t *raw, uint32_t n, double *rows)
+{
+    const uint32_t i = blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= n) return;
+    const Raw80t r = raw[i];
+    double *o = rows + (size_t)i * BAKE_ROW;
+    o[0] = r.ver[0]; o[1] = r.ver[1]; o[2] = r.ver[2];
+    o[3] = r.U; o[4] = r.V;
+    o[5] = r.normal[0]; o[6] = r.normal[1]; o[7] = r.normal[2];
+}
+
+static bool bake_wants_tangent_maps(const pt_bake_outputs &o) { return o.tangent_bgra || o.tangent_normal; }
+static bool bake_wants_frames(const pt_bake_outputs &o) { return bake_wants_tangent_maps(o) || o.vertex_tangents; }
+static bool bake_wants_object_maps(const pt_bake_outputs &o) { return o.bgra || o.normal_bgra || o.normal; }
+
 static int texture_bake(pt_index *ix, const void *vertices, size_t n_vertices, const int32_t *faces, size_t n_faces,
-                        int k, double radius, int res, int pad, uint8_t *bgra_out, uint8_t *normal_bgra_out,
-                        float *normal_out, pt_bake_stats *st)
+                        int k, double radius, int res, int pad, const pt_bake_outputs &o, pt_bake_stats *st)
 {
     cudaStream_t s = ix->stream;
     const size_t n_pix = (size_t)res * res;
+    const bool maps = bake_wants_object_maps(o) || bake_wants_tangent_maps(o);
+    const bool tmaps = bake_wants_tangent_maps(o), frames = bake_wants_frames(o);
     Raw80t *d_raw = nullptr;
-    MeshVertex *d_mv = nullptr;
-    double *d_xyz = nullptr, *d_q = nullptr;
-    int32_t *d_faces = nullptr;
+    double *d_rows = nullptr, *d_q = nullptr, *d_frames = nullptr;
+    int32_t *d_faces = nullptr, *d_sface = nullptr;
     uint32_t *d_texels = nullptr;
-    uint8_t *d_rgba = nullptr, *d_bgra = nullptr, *d_nbgra = nullptr;
-    float *d_normal = nullptr, *d_nf = nullptr;
+    uint8_t *d_rgba = nullptr, *d_bgra = nullptr, *d_nbgra = nullptr, *d_tbgra = nullptr;
+    float *d_normal = nullptr, *d_nf = nullptr, *d_tnf = nullptr, *d_vt = nullptr;
     unsigned long long *d_empty = nullptr;
     cudaEvent_t ev[4] = {};
     size_t count = 0;
@@ -687,12 +955,20 @@ static int texture_bake(pt_index *ix, const void *vertices, size_t n_vertices, c
     do {
         for (auto &e : ev) if (fail(cudaEventCreate(&e))) break;
         if (rc != PT_OK) break;
-        if (pool_alloc((void **)&d_raw, sizeof(Raw80t) * n_vertices, s) || pool_alloc((void **)&d_mv, sizeof(MeshVertex) * n_vertices, s) ||
-            pool_alloc((void **)&d_xyz, sizeof(double) * 3 * n_vertices, s) || pool_alloc((void **)&d_faces, sizeof(int32_t) * 3 * n_faces, s) ||
-            pool_alloc((void **)&d_texels, sizeof(uint32_t) * n_pix, s) || pool_alloc((void **)&d_q, sizeof(double) * 3 * n_pix, s) ||
+        if (pool_alloc((void **)&d_raw, sizeof(Raw80t) * n_vertices, s) ||
+            pool_alloc((void **)&d_rows, sizeof(double) * BAKE_ROW * n_vertices, s) ||
+            pool_alloc((void **)&d_faces, sizeof(int32_t) * 3 * n_faces, s) ||
             pool_alloc((void **)&d_empty, sizeof(unsigned long long), s) ||
-            (bgra_out && pool_alloc((void **)&d_bgra, 4 * n_pix, s)) || (normal_bgra_out && pool_alloc((void **)&d_nbgra, 4 * n_pix, s)) ||
-            (normal_out && pool_alloc((void **)&d_nf, sizeof(float) * 3 * n_pix, s))) {
+            (maps && (pool_alloc((void **)&d_texels, sizeof(uint32_t) * n_pix, s) ||
+                      pool_alloc((void **)&d_q, sizeof(double) * 3 * n_pix, s))) ||
+            (tmaps && pool_alloc((void **)&d_sface, sizeof(int32_t) * n_pix, s)) ||
+            (frames && pool_alloc((void **)&d_frames, sizeof(double) * BAKE_ROW * n_vertices, s)) ||
+            (o.bgra && pool_alloc((void **)&d_bgra, 4 * n_pix, s)) ||
+            (o.normal_bgra && pool_alloc((void **)&d_nbgra, 4 * n_pix, s)) ||
+            (o.normal && pool_alloc((void **)&d_nf, sizeof(float) * 3 * n_pix, s)) ||
+            (o.tangent_bgra && pool_alloc((void **)&d_tbgra, 4 * n_pix, s)) ||
+            (o.tangent_normal && pool_alloc((void **)&d_tnf, sizeof(float) * 3 * n_pix, s)) ||
+            (o.vertex_tangents && pool_alloc((void **)&d_vt, sizeof(float) * 4 * n_vertices, s))) {
             rc = PT_ERR_OUT_OF_MEMORY;
             break;
         }
@@ -701,12 +977,12 @@ static int texture_bake(pt_index *ix, const void *vertices, size_t n_vertices, c
         if (fail(cudaMemcpyAsync(d_faces, faces, sizeof(int32_t) * 3 * n_faces, cudaMemcpyHostToDevice, s))) break;
         if (fail(cudaMemsetAsync(d_empty, 0, sizeof(unsigned long long), s))) break;
         if (n_vertices) {
-            tex_unpack_vertices_kernel<<<tcdiv(n_vertices, 256), 256, 0, s>>>(d_raw, (uint32_t)n_vertices, d_mv, d_xyz);
+            bake_unpack_vertices_kernel<<<tcdiv(n_vertices, 256), 256, 0, s>>>(d_raw, (uint32_t)n_vertices, d_rows);
             count_launch();
         }
-        const BakeMesh M{reinterpret_cast<const double *>(d_mv), (int)(sizeof(MeshVertex) / sizeof(double)),
-                         (uint32_t)n_vertices, d_faces, (uint32_t)n_faces, res};
-        if ((rc = bake_texels(M, d_texels, d_q, &count, s)) != PT_OK) break;
+        const BakeMesh M{d_rows, BAKE_ROW, (uint32_t)n_vertices, d_faces, (uint32_t)n_faces, res};
+        if (maps && (rc = bake_texels(M, d_texels, d_q, d_sface, &count, s)) != PT_OK) break;
+        if (frames && (rc = bake_frames(M, d_frames, d_vt, s)) != PT_OK) break;
         if (fail(cudaEventRecord(ev[1], s))) break;
         if (pool_alloc((void **)&d_rgba, 4 * (count ? count : 1), s) || pool_alloc((void **)&d_normal, sizeof(float) * 3 * (count ? count : 1), s)) {
             rc = PT_ERR_OUT_OF_MEMORY;
@@ -723,11 +999,24 @@ static int texture_bake(pt_index *ix, const void *vertices, size_t n_vertices, c
             if ((rc = launch_query(ix, qp, s)) != PT_OK) break;
         }
         if (fail(cudaEventRecord(ev[2], s))) break;
-        if ((rc = bake_compose(d_texels, count, d_rgba, d_normal, res, pad, d_bgra, d_nbgra, d_nf, d_empty, s)) != PT_OK) break;
+        if (bake_wants_object_maps(o) &&
+            (rc = bake_compose(d_texels, count, d_rgba, d_normal, res, pad, d_bgra, d_nbgra, d_nf, d_empty, s)) != PT_OK)
+            break;
+        // the empty lists are counted by whichever composition runs
+        if (tmaps && (rc = bake_compose_tangent(M, d_frames, d_texels, d_sface, count, d_rgba, d_normal, pad, d_tbgra,
+                                                d_tnf, bake_wants_object_maps(o) ? nullptr : d_empty, s)) != PT_OK)
+            break;
         if (fail(cudaEventRecord(ev[3], s))) break;
-        if (bgra_out && fail(cudaMemcpyAsync(bgra_out, d_bgra, 4 * n_pix, cudaMemcpyDeviceToHost, s))) break;
-        if (normal_bgra_out && fail(cudaMemcpyAsync(normal_bgra_out, d_nbgra, 4 * n_pix, cudaMemcpyDeviceToHost, s))) break;
-        if (normal_out && fail(cudaMemcpyAsync(normal_out, d_nf, sizeof(float) * 3 * n_pix, cudaMemcpyDeviceToHost, s))) break;
+        if (o.bgra && fail(cudaMemcpyAsync(o.bgra, d_bgra, 4 * n_pix, cudaMemcpyDeviceToHost, s))) break;
+        if (o.normal_bgra && fail(cudaMemcpyAsync(o.normal_bgra, d_nbgra, 4 * n_pix, cudaMemcpyDeviceToHost, s))) break;
+        if (o.normal && fail(cudaMemcpyAsync(o.normal, d_nf, sizeof(float) * 3 * n_pix, cudaMemcpyDeviceToHost, s))) break;
+        if (o.tangent_bgra && fail(cudaMemcpyAsync(o.tangent_bgra, d_tbgra, 4 * n_pix, cudaMemcpyDeviceToHost, s))) break;
+        if (o.tangent_normal &&
+            fail(cudaMemcpyAsync(o.tangent_normal, d_tnf, sizeof(float) * 3 * n_pix, cudaMemcpyDeviceToHost, s)))
+            break;
+        if (o.vertex_tangents && n_vertices &&
+            fail(cudaMemcpyAsync(o.vertex_tangents, d_vt, sizeof(float) * 4 * n_vertices, cudaMemcpyDeviceToHost, s)))
+            break;
         unsigned long long empty = 0;
         if (fail(cudaMemcpyAsync(&empty, d_empty, sizeof empty, cudaMemcpyDeviceToHost, s))) break;
         if (fail(cudaStreamSynchronize(s))) break;
@@ -740,7 +1029,8 @@ static int texture_bake(pt_index *ix, const void *vertices, size_t n_vertices, c
         }
     } while (0);
     cudaStreamSynchronize(s);
-    void *frees[] = {d_raw, d_mv, d_xyz, d_faces, d_texels, d_q, d_rgba, d_normal, d_bgra, d_nbgra, d_nf, d_empty};
+    void *frees[] = {d_raw, d_rows, d_faces, d_texels, d_q, d_sface, d_frames, d_rgba, d_normal, d_bgra, d_nbgra, d_nf,
+                     d_tbgra, d_tnf, d_vt, d_empty};
     for (void *p : frees) pool_free(p, s);
     for (auto &e : ev) if (e) cudaEventDestroy(e);
     cudaStreamSynchronize(s);
@@ -800,18 +1090,60 @@ extern "C" int pt_texture_render_lists(const void *points, size_t n, const void 
     return rc;
 }
 
-extern "C" int pt_bake_texels_device(const double *vertices_xyzuv, size_t n_vertices, const int32_t *faces,
-                                     size_t n_faces, int resolution, uint32_t *texel_out, double *xyz_out,
-                                     size_t *count_out, int device, void *stream)
+extern "C" int pt_bake_samples_device(const double *vertices_xyzuv, size_t n_vertices, const int32_t *faces,
+                                      size_t n_faces, int resolution, uint32_t *texel_out, double *xyz_out,
+                                      int32_t *face_out, size_t *count_out, int device, void *stream)
 {
     if ((!vertices_xyzuv && n_vertices) || (!faces && n_faces) || !count_out || resolution < 1 || resolution > 16384 ||
-        n_vertices > 0x7ffffff0ull || n_faces >= (1ull << 31) || (!texel_out != !xyz_out))
+        n_vertices > 0x7ffffff0ull || n_faces >= (1ull << 31) || (!texel_out != !xyz_out) || (face_out && !texel_out))
         return PT_ERR_INVALID_ARG;
     *count_out = 0;
     if (pt_device_count() == 0) return PT_ERR_NO_DEVICE;
     if (device >= 0) PT_CUDA(cudaSetDevice(device));
     const BakeMesh M{vertices_xyzuv, 5, (uint32_t)n_vertices, faces, (uint32_t)n_faces, resolution};
-    return bake_texels(M, texel_out, xyz_out, count_out, (cudaStream_t)stream);
+    return bake_texels(M, texel_out, xyz_out, face_out, count_out, (cudaStream_t)stream);
+}
+
+extern "C" int pt_bake_texels_device(const double *vertices_xyzuv, size_t n_vertices, const int32_t *faces,
+                                     size_t n_faces, int resolution, uint32_t *texel_out, double *xyz_out,
+                                     size_t *count_out, int device, void *stream)
+{
+    return pt_bake_samples_device(vertices_xyzuv, n_vertices, faces, n_faces, resolution, texel_out, xyz_out, nullptr,
+                                  count_out, device, stream);
+}
+
+// the corner list of the frames is sorted with an int item count
+static bool bake_corners_fit(size_t n_faces) { return n_faces <= (size_t)INT32_MAX / 3; }
+
+extern "C" int pt_bake_frames_device(const double *vertices_xyzuvn, size_t n_vertices, const int32_t *faces,
+                                     size_t n_faces, double *frames_out, float *tangents_out, int device, void *stream)
+{
+    if ((!vertices_xyzuvn && n_vertices) || (!faces && n_faces) || (!frames_out && n_vertices) ||
+        n_vertices > 0x7ffffff0ull)
+        return PT_ERR_INVALID_ARG;
+    if (!bake_corners_fit(n_faces)) return PT_ERR_UNSUPPORTED;
+    if (pt_device_count() == 0) return PT_ERR_NO_DEVICE;
+    if (device >= 0) PT_CUDA(cudaSetDevice(device));
+    const BakeMesh M{vertices_xyzuvn, BAKE_ROW, (uint32_t)n_vertices, faces, (uint32_t)n_faces, 1};
+    return bake_frames(M, frames_out, tangents_out, (cudaStream_t)stream);
+}
+
+extern "C" int pt_bake_compose_tangent_device(const double *vertices_xyzuvn, const double *frames, size_t n_vertices,
+                                              const int32_t *faces, size_t n_faces, const uint32_t *texels,
+                                              const int32_t *sample_faces, size_t count, const uint8_t *rgba,
+                                              const float *normal, int resolution, int pad, uint8_t *tangent_bgra_out,
+                                              float *tangent_normal_out, int device, void *stream)
+{
+    if ((n_vertices && (!vertices_xyzuvn || !frames)) || (!faces && n_faces) ||
+        (count && (!texels || !sample_faces || !rgba || !normal)) || resolution < 1 || resolution > 16384 ||
+        count > (size_t)resolution * resolution || n_vertices > 0x7ffffff0ull || n_faces >= (1ull << 31) ||
+        (!tangent_bgra_out && !tangent_normal_out))
+        return PT_ERR_INVALID_ARG;
+    if (pt_device_count() == 0) return PT_ERR_NO_DEVICE;
+    if (device >= 0) PT_CUDA(cudaSetDevice(device));
+    const BakeMesh M{vertices_xyzuvn, BAKE_ROW, (uint32_t)n_vertices, faces, (uint32_t)n_faces, resolution};
+    return bake_compose_tangent(M, frames, texels, sample_faces, count, rgba, normal, pad, tangent_bgra_out,
+                                tangent_normal_out, nullptr, (cudaStream_t)stream);
 }
 
 extern "C" int pt_bake_compose_device(const uint32_t *texels, size_t count, const uint8_t *rgba, const float *normal,
@@ -827,18 +1159,27 @@ extern "C" int pt_bake_compose_device(const uint32_t *texels, size_t count, cons
                         (cudaStream_t)stream);
 }
 
-extern "C" int pt_texture_bake(pt_index *ix, const void *vertices, size_t n_vertices, const int32_t *faces,
-                               size_t n_faces, int k, double radius, int resolution, int pad, uint8_t *bgra_out,
-                               uint8_t *normal_bgra_out, float *normal_out, pt_bake_stats *stats)
+extern "C" int pt_texture_bake_ex(pt_index *ix, const void *vertices, size_t n_vertices, const int32_t *faces,
+                                  size_t n_faces, int k, double radius, int resolution, int pad,
+                                  const pt_bake_outputs *out, pt_bake_stats *stats)
 {
-    if (!ix || (!vertices && n_vertices) || (!faces && n_faces) || (!bgra_out && !normal_bgra_out && !normal_out) ||
-        resolution < 1 || resolution > 16384 || n_vertices > 0x7ffffff0ull || n_faces >= (1ull << 31))
+    if (!ix || (!vertices && n_vertices) || (!faces && n_faces) || !out ||
+        (!bake_wants_object_maps(*out) && !bake_wants_frames(*out)) || resolution < 1 || resolution > 16384 ||
+        n_vertices > 0x7ffffff0ull || n_faces >= (1ull << 31))
         return PT_ERR_INVALID_ARG;
     if (k < 1 || k > PT_MAX_K) return PT_ERR_UNSUPPORTED;
+    if (bake_wants_frames(*out) && !bake_corners_fit(n_faces)) return PT_ERR_UNSUPPORTED;
     if (ix->ids) return PT_ERR_UNSUPPORTED;           // slab indexes answer with global ids
     if (!ix->attrs && ix->n) return PT_ERR_INVALID_ARG;
     if (pt_device_count() == 0) return PT_ERR_NO_DEVICE;
     PT_CUDA(cudaSetDevice(ix->device));
-    return texture_bake(ix, vertices, n_vertices, faces, n_faces, k, radius, resolution, pad, bgra_out, normal_bgra_out,
-                        normal_out, stats);
+    return texture_bake(ix, vertices, n_vertices, faces, n_faces, k, radius, resolution, pad, *out, stats);
+}
+
+extern "C" int pt_texture_bake(pt_index *ix, const void *vertices, size_t n_vertices, const int32_t *faces,
+                               size_t n_faces, int k, double radius, int resolution, int pad, uint8_t *bgra_out,
+                               uint8_t *normal_bgra_out, float *normal_out, pt_bake_stats *stats)
+{
+    const pt_bake_outputs out = {bgra_out, normal_bgra_out, normal_out, nullptr, nullptr, nullptr};
+    return pt_texture_bake_ex(ix, vertices, n_vertices, faces, n_faces, k, radius, resolution, pad, &out, stats);
 }

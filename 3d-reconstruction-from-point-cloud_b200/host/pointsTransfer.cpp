@@ -15,8 +15,10 @@
 // instead of texture.png the tool writes `transferred.ply`, the input mesh in the same 11-column
 // ASCII format with the transferred colour and normal per vertex.  Extra options (all default to
 // the reference's behaviour): -k N, -r RADIUS, -o FILE, -d DEVICE.  -b FILE / -n FILE also bake the
-// cloud's colour / object-space normal onto every texel of the mesh's UV atlas (pt_texture_bake,
-// same -R, -k, -r) and write them as PNG.
+// cloud's colour / object-space normal onto every texel of the mesh's UV atlas (pt_texture_bake_ex,
+// same -R, -k, -r) and write them as PNG; -t FILE writes the tangent-space normal map as PNG and
+// -T FILE the input mesh as PLY with the per-vertex tangents (tx ty tz tw) that map is expressed
+// in.  All of them come from one bake.
 #include <algorithm>
 #include <charconv>
 #include <chrono>
@@ -247,6 +249,7 @@ static int run(int argc, char **argv)
     std::string out_name = "texture.png";          // src/pointsTransfer.cpp:613
     std::string ply_name;                          // optional extra: the per-vertex blend as a PLY
     std::string bake_name, normal_name;            // optional extras: the per-texel colour / normal maps
+    std::string tangent_name, tangent_ply_name;    // ... the tangent-space normal map, the mesh with tangents
     for (int i = 1; i < argc; ++i) {
         std::string a = argv[i];
         if (a == "-k" && i + 1 < argc) K = atoi(argv[++i]);
@@ -258,6 +261,8 @@ static int run(int argc, char **argv)
         else if (a == "-g" && i + 1 < argc) n_gpus = atoi(argv[++i]);
         else if (a == "-b" && i + 1 < argc) bake_name = argv[++i];
         else if (a == "-n" && i + 1 < argc) normal_name = argv[++i];
+        else if (a == "-t" && i + 1 < argc) tangent_name = argv[++i];
+        else if (a == "-T" && i + 1 < argc) tangent_ply_name = argv[++i];
         else pos_args.push_back(a);
     }
     if (pos_args.size() < 2) {
@@ -269,9 +274,9 @@ static int run(int argc, char **argv)
         std::cerr << "-k must be 1.." << PT_MAX_K << ", -R 1..32768 and -g 1..64" << std::endl;
         return 0;
     }
-    const bool bake = !bake_name.empty() || !normal_name.empty();
+    const bool bake = !bake_name.empty() || !normal_name.empty() || !tangent_name.empty() || !tangent_ply_name.empty();
     if (bake && (n_gpus > 1 || resolution > 16384)) {
-        std::cerr << "-b / -n bake on one GPU (no -g) at -R 1..16384" << std::endl;
+        std::cerr << "-b / -n / -t / -T bake on one GPU (no -g) at -R 1..16384" << std::endl;
         return 0;
     }
     const std::string pc_file_name = pos_args[0], mesh_file_name = pos_args[1];
@@ -377,17 +382,27 @@ static int run(int argc, char **argv)
     std::cout << "Neighbor search total time: " << ts.knn_ms * 1e-3 << " seconds" << std::endl;
     std::cout << "Draw triangles total time: " << (ts.draw_ms + ts.pad_ms) * 1e-3 << " seconds" << std::endl;
 
-    // extra (not in the reference): per-texel colour and normal maps, padded like the texture
-    std::vector<uint8_t> baked, baked_normal;
+    // extra (not in the reference): per-texel colour, normal and tangent-space normal maps, padded
+    // like the texture, and the per-vertex tangents
+    std::vector<uint8_t> baked, baked_normal, baked_tangent;
+    std::vector<float> vertex_tangents;
     if (bake) {
-        if (!bake_name.empty()) baked.resize((size_t)resolution * resolution * 4);
-        if (!normal_name.empty()) baked_normal.resize((size_t)resolution * resolution * 4);
+        const size_t n_bytes = (size_t)resolution * resolution * 4;
+        if (!bake_name.empty()) baked.resize(n_bytes);
+        if (!normal_name.empty()) baked_normal.resize(n_bytes);
+        if (!tangent_name.empty()) baked_tangent.resize(n_bytes);
+        if (!tangent_ply_name.empty()) vertex_tangents.resize(4 * m);
+        pt_bake_outputs bo;
+        memset(&bo, 0, sizeof bo);
+        bo.bgra = baked.empty() ? nullptr : baked.data();
+        bo.normal_bgra = baked_normal.empty() ? nullptr : baked_normal.data();
+        bo.tangent_bgra = baked_tangent.empty() ? nullptr : baked_tangent.data();
+        bo.vertex_tangents = tangent_ply_name.empty() ? nullptr : vertex_tangents.data();
         pt_bake_stats bs;
-        rc = pt_texture_bake(index, vertices.data(), m, faces.data(), faces.size() / 3, K, radius, resolution, 1,
-                             baked.empty() ? nullptr : baked.data(), baked_normal.empty() ? nullptr : baked_normal.data(),
-                             nullptr, &bs);
+        rc = pt_texture_bake_ex(index, vertices.data(), m, faces.data(), faces.size() / 3, K, radius, resolution, 1,
+                                &bo, &bs);
         if (rc != PT_OK) {
-            std::cerr << "pt_texture_bake failed: " << pt_status_string(rc) << std::endl;
+            std::cerr << "pt_texture_bake_ex failed: " << pt_status_string(rc) << std::endl;
             pt_index_free(index);
             return 0;
         }
@@ -401,6 +416,32 @@ static int run(int argc, char **argv)
         std::cerr << "Cannot write " << bake_name << std::endl;
     if (!baked_normal.empty() && !ptb::write_png_bgra(normal_name.c_str(), baked_normal.data(), resolution, resolution))
         std::cerr << "Cannot write " << normal_name << std::endl;
+    if (!baked_tangent.empty() && !ptb::write_png_bgra(tangent_name.c_str(), baked_tangent.data(), resolution, resolution))
+        std::cerr << "Cannot write " << tangent_name << std::endl;
+    if (!tangent_ply_name.empty()) {
+        // the input mesh with the tangent frame of the tangent-space map: tx ty tz tw per vertex
+        // (%.9g round-trips the fp32 values)
+        std::ofstream out(tangent_ply_name);
+        out << "ply\nformat ascii 1.0\nelement vertex " << m << "\n"
+            << "property double x\nproperty double y\nproperty double z\n"
+            << "property double nx\nproperty double ny\nproperty double nz\n"
+            << "property double s\nproperty double t\n"
+            << "property uchar red\nproperty uchar green\nproperty uchar blue\n"
+            << "property float tx\nproperty float ty\nproperty float tz\nproperty float tw\n"
+            << "element face " << faces.size() / 3 << "\nproperty list uchar int vertex_indices\nend_header\n";
+        char line[640];
+        for (size_t i = 0; i < m; ++i) {
+            const Point &v = vertices[i];
+            const float *t = vertex_tangents.data() + 4 * i;
+            snprintf(line, sizeof line, "%.17g %.17g %.17g %.17g %.17g %.17g %.17g %.17g %d %d %d %.9g %.9g %.9g %.9g\n",
+                     v.ver[0], v.ver[1], v.ver[2], v.normal[0], v.normal[1], v.normal[2], v.U, v.V, v.color[0],
+                     v.color[1], v.color[2], t[0], t[1], t[2], t[3]);
+            out << line;
+        }
+        for (size_t f = 0; f + 2 < faces.size(); f += 3)
+            out << "3 " << faces[f] << ' ' << faces[f + 1] << ' ' << faces[f + 2] << '\n';
+        if (!out) std::cerr << "Cannot write " << tangent_ply_name << std::endl;
+    }
     if (!ply_name.empty()) {
         // extra (not in the reference): the fused per-vertex colour / normal blend of pt_transfer
         std::vector<uint8_t> rgba(m * 4);

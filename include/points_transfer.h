@@ -16,7 +16,9 @@
  *   pt_texture_render<- the face loop body after the searches and the texture
  *                       post-process, src/pointsTransfer.cpp:484-611 + draw_triangle :66-107.
  *   pt_texture_bake  <- no reference counterpart: per-texel colour and normal maps on
- *                       the mesh's UV atlas (the "texel" samples of the transfer).
+ *                       the mesh's UV atlas (the "texel" samples of the transfer);
+ *                       pt_texture_bake_ex adds tangent-space normal maps and the
+ *                       per-vertex tangents they are expressed in.
  *   pt_index_free    <- `tree` going out of scope at src/pointsTransfer.cpp:626.
  *
  * Records are the reference's own 80-byte AoS `struct Point`
@@ -167,6 +169,37 @@ int pt_texture_bake(pt_index *index, const void *vertices, size_t n_vertices,
                     uint8_t *normal_bgra_out /* res*res*4 */, float *normal_out /* res*res*3 */,
                     pt_bake_stats *stats);
 
+/* Tangent-space bake (DESIGN.md section 8, "Tangent-space bake").  pt_texture_bake_ex runs one
+ * texel raster and one k-NN pass for every requested output:
+ *   bgra, normal_bgra, normal  as pt_texture_bake (res*res*4, res*res*4, res*res*3)
+ *   tangent_bgra     tangent-space normal map, B G R A = e(z) e(y) e(x) 255 (res*res*4 bytes),
+ *                    padded like the other 8-bit maps when pad != 0
+ *   tangent_normal   the blended normal in the texel's tangent frame, 3 floats per texel (res*res*3),
+ *                    never padded
+ *   vertex_tangents  per vertex (T.x, T.y, T.z, w) in fp32, the glTF TANGENT layout: the unit
+ *                    tangent and the handedness w = +-1 with bitangent = w * (N x T); (0, 0, 0, 0)
+ *                    for a vertex without a frame (n_vertices*4 floats)
+ * Any output may be NULL, but not all; all are host buffers.  The convention is glTF's / OpenGL's:
+ * +X along +U, +Y along +V (up in the image: row 0 is the top row), +Z out of the surface.  Frames
+ * come from the mesh's per-vertex normals (Point.normal; the summed face normals where a normal is
+ * zero or not finite) and its UVs; a UV seam is a duplicated vertex, so frames split there.
+ * Faces with an out-of-range vertex index are skipped.  The tangent outputs need
+ * 3 * n_faces <= INT32_MAX, otherwise PT_ERR_UNSUPPORTED before any input is read.  With only
+ * vertex_tangents requested nothing is rasterised or searched (stats texels = empty = 0).  The
+ * frames are part of raster_ms, the tangent composition part of pad_ms. */
+typedef struct pt_bake_outputs {
+    uint8_t *bgra;             /* res*res*4 */
+    uint8_t *normal_bgra;      /* res*res*4 */
+    float   *normal;           /* res*res*3 */
+    uint8_t *tangent_bgra;     /* res*res*4 */
+    float   *tangent_normal;   /* res*res*3 */
+    float   *vertex_tangents;  /* n_vertices*4 */
+} pt_bake_outputs;
+int pt_texture_bake_ex(pt_index *index, const void *vertices, size_t n_vertices,
+                       const int32_t *faces, size_t n_faces, int k, double radius,
+                       int resolution, int pad, const pt_bake_outputs *out,
+                       pt_bake_stats *stats);
+
 /* Device-buffer API: same operations with inputs/outputs already resident in
  * HBM on the index's device (bench `value`, multi-GPU slabs).  `stream` is a
  * cudaStream_t passed as void* (NULL = the CUDA default stream); these calls
@@ -221,12 +254,37 @@ int pt_bake_texels_device(const double *vertices_xyzuv, size_t n_vertices,
                           const int32_t *faces, size_t n_faces, int resolution,
                           uint32_t *texel_out, double *xyz_out, size_t *count_out,
                           int device, void *stream);
+/* pt_bake_samples_device: pt_bake_texels_device plus the owner face of every sample in face_out
+ * (room for resolution^2 int32, may be NULL; needs texel_out). */
+int pt_bake_samples_device(const double *vertices_xyzuv, size_t n_vertices,
+                           const int32_t *faces, size_t n_faces, int resolution,
+                           uint32_t *texel_out, double *xyz_out, int32_t *face_out,
+                           size_t *count_out, int device, void *stream);
 /* pt_bake_compose_device: the maps of pt_texture_bake from count samples (texels as above, rgba
  * count x 4 and normal count x 3 as pt_query_device returns them).  Outputs as pt_texture_bake's,
  * in device memory; any may be NULL, but not all.  Asynchronous on `stream`. */
 int pt_bake_compose_device(const uint32_t *texels, size_t count, const uint8_t *rgba,
                            const float *normal, int resolution, int pad, uint8_t *bgra_out,
                            uint8_t *normal_bgra_out, float *normal_out, int device, void *stream);
+/* The device pieces of the tangent bake.  vertices_xyzuvn: n_vertices x 8 doubles
+ * (x, y, z, u, v, nx, ny, nz); the texel calls above read rows of 5 (the first five columns).
+ * pt_bake_frames_device: the vertex frames into frames_out (n_vertices x 8 doubles:
+ * N xyz, T xyz, w, 0; all zero for a vertex without a frame) and, when tangents_out is not NULL,
+ * the exported fp32 tangents (n_vertices x 4).  3 * n_faces <= INT32_MAX, otherwise
+ * PT_ERR_UNSUPPORTED.  Asynchronous on `stream`. */
+int pt_bake_frames_device(const double *vertices_xyzuvn, size_t n_vertices,
+                          const int32_t *faces, size_t n_faces, double *frames_out,
+                          float *tangents_out, int device, void *stream);
+/* pt_bake_compose_tangent_device: the two tangent maps of pt_texture_bake_ex from count samples
+ * (texels and sample_faces of pt_bake_samples_device, rgba / normal of pt_query_device on their
+ * positions, frames of pt_bake_frames_device).  Outputs in device memory, either may be NULL but
+ * not both; tangent_bgra_out is padded when pad != 0.  Asynchronous on `stream`. */
+int pt_bake_compose_tangent_device(const double *vertices_xyzuvn, const double *frames,
+                                   size_t n_vertices, const int32_t *faces, size_t n_faces,
+                                   const uint32_t *texels, const int32_t *sample_faces,
+                                   size_t count, const uint8_t *rgba, const float *normal,
+                                   int resolution, int pad, uint8_t *tangent_bgra_out,
+                                   float *tangent_normal_out, int device, void *stream);
 
 /* Halo exchange helpers for slab-sharded clouds (DESIGN.md section 6).  Fixed-capacity routing,
  * so the exchange needs no host synchronisation: per peer a send block of (cap + 1) rows of 4
