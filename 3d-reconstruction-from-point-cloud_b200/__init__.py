@@ -7,7 +7,8 @@ directory name is not a Python identifier) or through ``__graft_entry__.package(
 from .api import (  # noqa: F401
     ABI_SYMBOLS, SYNTH_SYMBOLS, ATTR_DTYPE, CAND_DTYPE, COORD_AUTO, COORD_F32, COORD_F64, LIB_PATH,
     POINT_DTYPE, PT_MAX_K, DeviceTree, Distance, K_neighbor_search, PointsTransferError, ShardedTree, Tree, texture_from_lists,
-    bake_compose_device, bake_compose_tangent_device, bake_frames_device, bake_samples_device, bake_texels_device,
+    bake_compose_device, bake_compose_height_device, bake_compose_tangent_device, bake_frames_device,
+    bake_samples_device, bake_texels_device,
     device_count, get_option, kernel_launch_count, lib, synth_lib,
     make_points, merge_device, set_option,
     status_string, version,

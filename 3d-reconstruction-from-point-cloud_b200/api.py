@@ -52,6 +52,7 @@ ABI_SYMBOLS = (
     "pt_sharded_transfer", "pt_texture_render_lists", "pt_set_option", "pt_get_option", "pt_debug_stats", "pt_debug_stats_n", "pt_kernel_launch_count",
     "pt_texture_bake", "pt_bake_texels_device", "pt_bake_compose_device",
     "pt_texture_bake_ex", "pt_bake_samples_device", "pt_bake_frames_device", "pt_bake_compose_tangent_device",
+    "pt_texture_bake_height", "pt_bake_compose_height_device",
 )
 # ... and include/pt_synth.h (bench / test scaffolding, its own library)
 SYNTH_SYMBOLS = ("pt_synth_cloud_device", "pt_synth_samples_device", "pt_synth_pack_points_device",
@@ -94,6 +95,11 @@ class BakeOutputs(ctypes.Structure):
     _fields_ = [("bgra", ctypes.c_void_p), ("normal_bgra", ctypes.c_void_p), ("normal", ctypes.c_void_p),
                 ("tangent_bgra", ctypes.c_void_p), ("tangent_normal", ctypes.c_void_p),
                 ("vertex_tangents", ctypes.c_void_p)]
+
+
+class BakeHeight(ctypes.Structure):
+    _fields_ = [("height", ctypes.c_void_p), ("height_u16", ctypes.c_void_p), ("range", ctypes.c_double * 2),
+                ("range_used", ctypes.c_double * 2), ("texels", ctypes.c_uint64)]
 
 
 class ShardedOpts(ctypes.Structure):
@@ -196,6 +202,12 @@ def lib():
     L.pt_bake_frames_device.argtypes = [vp, sz, vp, sz, vp, vp, i32, vp]
     L.pt_bake_compose_tangent_device.restype = i32
     L.pt_bake_compose_tangent_device.argtypes = [vp, vp, sz, vp, sz, vp, vp, sz, vp, vp, i32, i32, vp, vp, i32, vp]
+    L.pt_texture_bake_height.restype = i32
+    L.pt_texture_bake_height.argtypes = [vp, vp, sz, vp, sz, i32, dbl, i32, i32, ctypes.POINTER(BakeOutputs),
+                                         ctypes.POINTER(BakeHeight), ctypes.POINTER(BakeStats)]
+    L.pt_bake_compose_height_device.restype = i32
+    L.pt_bake_compose_height_device.argtypes = [vp, vp, sz, vp, sz, vp, vp, vp, sz, vp, i32, vp, sz, i32, i32, vp, vp,
+                                                vp, vp, i32, vp]
     L.pt_set_option.restype = i32
     L.pt_set_option.argtypes = [ctypes.c_char_p, i32]
     L.pt_get_option.restype = i32
@@ -427,9 +439,10 @@ class Tree:
                      "knn_ms": st.knn_ms, "draw_ms": st.draw_ms, "pad_ms": st.pad_ms}
 
     _BAKE_OUTPUTS = ("bgra", "normal_bgra", "normal", "tangent_bgra", "tangent_normal", "tangents")
+    _HEIGHT_OUTPUTS = ("height", "height_u16")
 
     def bake(self, vertices, faces, k=20, resolution=2048, radius=None, pad=True,
-             want=("bgra", "normal_bgra", "normal")):
+             want=("bgra", "normal_bgra", "normal"), height_range=None):
         """Per-texel bake (DESIGN.md section 8): colour and normal maps of the cloud on the mesh's
         UV atlas.  vertices: Point records (position, normal, U, V), faces: int32 [F,3].  Returns a
         dict with the requested outputs -- ``bgra`` uint8 [res,res,4] (B G R 255), ``normal_bgra``
@@ -437,25 +450,41 @@ class Tree:
         (never padded), ``tangent_bgra`` uint8 [res,res,4] (tangent-space normal map, glTF / OpenGL
         convention), ``tangent_normal`` float32 [res,res,3] (never padded), ``tangents`` float32
         [n_vertices,4] (the per-vertex tangent and handedness the tangent maps are expressed in, glTF
-        TANGENT layout) -- and ``stats`` (texels, empty, raster_ms, knn_ms, pad_ms).  All outputs
-        come from one k-NN pass."""
+        TANGENT layout), ``height`` float32 [res,res] (the cloud's signed height above the mesh along
+        the interpolated mesh normal, NaN without a value, never padded), ``height_u16`` uint16
+        [res,res] (its 16-bit code over ``height_range`` = (lo, hi) when finite with lo < hi, else
+        over the heights' min and max; decode with lo + E * (hi - lo) / 65535) -- and ``stats``
+        (texels, empty, raster_ms, knn_ms, pad_ms).  With a height output the result also carries
+        ``height_range`` (the (lo, hi) used) and ``stats["height_texels"]`` (texels with a value).
+        All outputs come from one k-NN pass."""
         v = _as_points(vertices, "vertices")
         f = np.ascontiguousarray(faces, dtype=np.int32).reshape(-1, 3)
-        unknown = set(want) - set(self._BAKE_OUTPUTS)
+        names = self._BAKE_OUTPUTS + self._HEIGHT_OUTPUTS
+        unknown = set(want) - set(names)
         if unknown or not want:
-            raise ValueError(f"want must name some of {', '.join(self._BAKE_OUTPUTS)} (got {want!r})")
+            raise ValueError(f"want must name some of {', '.join(names)} (got {want!r})")
         res = int(resolution)
         shapes = {"bgra": ((res, res, 4), np.uint8), "normal_bgra": ((res, res, 4), np.uint8),
                   "normal": ((res, res, 3), np.float32), "tangent_bgra": ((res, res, 4), np.uint8),
-                  "tangent_normal": ((res, res, 3), np.float32), "tangents": ((v.shape[0], 4), np.float32)}
-        out = {name: np.empty(*shapes[name]) for name in self._BAKE_OUTPUTS if name in want}
+                  "tangent_normal": ((res, res, 3), np.float32), "tangents": ((v.shape[0], 4), np.float32),
+                  "height": ((res, res), np.float32), "height_u16": ((res, res), np.uint16)}
+        out = {name: np.empty(*shapes[name]) for name in names if name in want}
         o = BakeOutputs(*[out[name].ctypes.data if name in out else None for name in self._BAKE_OUTPUTS])
+        hb = None
+        if any(name in out for name in self._HEIGHT_OUTPUTS):
+            lo, hi = (float("nan"), float("nan")) if height_range is None else map(float, height_range)
+            hb = BakeHeight(*[out[name].ctypes.data if name in out else None for name in self._HEIGHT_OUTPUTS],
+                            (ctypes.c_double * 2)(lo, hi))
         st = BakeStats()
-        _check(lib().pt_texture_bake_ex(self._h, _np_ptr(v), v.shape[0], _np_ptr(f), f.shape[0], int(k),
-                                        _radius(radius), res, 1 if pad else 0, ctypes.byref(o), ctypes.byref(st)),
-               "pt_texture_bake_ex")
+        _check(lib().pt_texture_bake_height(self._h, _np_ptr(v), v.shape[0], _np_ptr(f), f.shape[0], int(k),
+                                            _radius(radius), res, 1 if pad else 0, ctypes.byref(o),
+                                            None if hb is None else ctypes.byref(hb), ctypes.byref(st)),
+               "pt_texture_bake_height")
         out["stats"] = {"texels": int(st.texels), "empty": int(st.empty), "raster_ms": st.raster_ms,
                         "knn_ms": st.knn_ms, "pad_ms": st.pad_ms}
+        if hb is not None:
+            out["height_range"] = (hb.range_used[0], hb.range_used[1])
+            out["stats"]["height_texels"] = int(hb.texels)
         return out
 
     def transfer_slab(self, queries_ptr, queries_are_xyz, m, k, radius, boxes6, rank, halo,
@@ -746,3 +775,40 @@ def bake_compose_tangent_device(vertices_xyzuvn, frames, faces, texels, sample_f
                                                     _tptr(rgba), _tptr(normal), int(resolution), 1 if pad else 0,
                                                     _tptr(tangent_bgra), _tptr(tangent_normal), texels.device.index,
                                                     _stream_ptr(stream)), "pt_bake_compose_tangent_device")
+
+
+def bake_compose_height_device(vertices_xyzuvn, frames, faces, texels, sample_faces, sample_xyz, idx, k, cloud_xyz,
+                               resolution, pad=True, height_range=None, height=None, height_u16=None, range_out=None,
+                               stream=None):
+    """``pt_bake_compose_height_device``: the height maps from the samples (``texels``,
+    ``sample_faces`` and ``sample_xyz`` of ``bake_samples_device``), their neighbour lists ``idx``
+    (int32 [m,k] of ``DeviceTree.query``), the frames of ``bake_frames_device`` and the cloud's
+    positions ``cloud_xyz`` (float64 [n,3], original order).  Outputs are pre-allocated CUDA tensors
+    (float32 [res,res], uint16 [res,res], float64 [2] for the range used) or None; at least one map
+    must be given.  ``height_range`` = (lo, hi) fixes the code range when finite with lo < hi.
+    Asynchronous on ``stream``."""
+    import torch
+    m, n = texels.numel(), vertices_xyzuvn.shape[0]
+    assert vertices_xyzuvn.is_cuda and vertices_xyzuvn.dtype == torch.float64 and vertices_xyzuvn.is_contiguous()
+    assert vertices_xyzuvn.dim() == 2 and vertices_xyzuvn.shape[1] == 8
+    assert frames.is_cuda and frames.dtype == torch.float64 and frames.is_contiguous() and frames.numel() == 8 * n
+    assert faces.is_cuda and faces.dtype == torch.int32 and faces.is_contiguous() and faces.numel() % 3 == 0
+    for t, dt, cnt in ((texels, torch.int32, m), (sample_faces, torch.int32, m), (sample_xyz, torch.float64, 3 * m),
+                       (idx, torch.int32, m * int(k))):
+        assert t.is_cuda and t.is_contiguous() and t.dtype == dt and t.numel() == cnt
+    assert cloud_xyz.is_cuda and cloud_xyz.dtype == torch.float64 and cloud_xyz.is_contiguous()
+    assert cloud_xyz.numel() % 3 == 0
+    n_pix = int(resolution) * int(resolution)
+    for t, dt, cnt in ((height, torch.float32, n_pix), (height_u16, torch.uint16, n_pix), (range_out, torch.float64, 2)):
+        if t is not None:
+            assert t.is_cuda and t.is_contiguous() and t.dtype == dt and t.numel() == cnt
+    rng = None if height_range is None else (ctypes.c_double * 2)(*map(float, height_range))
+    with torch.cuda.device(texels.device):
+        _check(lib().pt_bake_compose_height_device(_tptr(vertices_xyzuvn), _tptr(frames), n, _tptr(faces),
+                                                   faces.numel() // 3, _tptr(texels), _tptr(sample_faces),
+                                                   _tptr(sample_xyz), m, _tptr(idx), int(k), _tptr(cloud_xyz),
+                                                   cloud_xyz.numel() // 3, int(resolution), 1 if pad else 0,
+                                                   None if rng is None else ctypes.cast(rng, ctypes.c_void_p),
+                                                   _tptr(height), _tptr(height_u16), _tptr(range_out),
+                                                   texels.device.index, _stream_ptr(stream)),
+               "pt_bake_compose_height_device")

@@ -138,6 +138,16 @@ __device__ __forceinline__ double dist2_exact(double qx, double qy, double qz, d
     return __dadd_rn(__dadd_rn(__dmul_rn(dx, dx), __dmul_rn(dy, dy)), __dmul_rn(dz, dz));
 }
 
+// Weight of neighbour j in the blend (DESIGN.md "blend"), shared by the blend and the height bake.
+// mode 0: 1/d2; 1 (the nearest is an exact hit): exact hits only; 2 (the mode 0 / 1 sum is not in
+// (0, inf)): the nearest only.
+__device__ __forceinline__ double blend_weight(int mode, double d2, int j)
+{
+    if (mode == 0) return __ddiv_rn(1.0, d2);
+    if (mode == 1) return d2 == 0.0 ? 1.0 : 0.0;
+    return j == 0 ? 1.0 : 0.0;
+}
+
 // Ordering key (d2, index): lowest index wins ties.
 __device__ __forceinline__ bool key_less(double da, int ia, double db, int ib)
 {

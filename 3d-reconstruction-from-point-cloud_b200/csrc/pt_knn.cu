@@ -93,13 +93,6 @@ struct BlendAcc {
     }
 };
 
-__device__ __forceinline__ double blend_weight(int mode, double d2, int j)
-{
-    if (mode == 0) return __ddiv_rn(1.0, d2);
-    if (mode == 1) return d2 == 0.0 ? 1.0 : 0.0;
-    return j == 0 ? 1.0 : 0.0;
-}
-
 __device__ __forceinline__ void store_empty_blend(uint8_t *rgba_out, float *normal_out)
 {
     if (rgba_out) *reinterpret_cast<uchar4 *>(rgba_out) = make_uchar4(0, 0, 0, 0);

@@ -18,8 +18,10 @@
 // triple is a face iff no other point is strictly inside its circumcircle; the in-circle sign is
 // evaluated once per index-sorted quadruple).  Not reproduced: the out-of-bounds row
 // `resolution - j` at j = 0 / column `resolution` (:100-103) and the uninitialised Mat (:402).
+#include <algorithm>
 #include <cmath>
 #include <initializer_list>
+#include <vector>
 
 #include <cub/device/device_radix_sort.cuh>
 #include <cub/device/device_scan.cuh>
@@ -397,16 +399,24 @@ static int texture_pipeline(pt_index *ix, POS pos, uint32_t n_points, const pt_a
     return rc;
 }
 
+// original index -> position in the sorted cloud, built once per index
+template <typename PT>
+static int index_inverse_perm(pt_index *ix)
+{
+    if (!ix->inv_perm && ix->n) {
+        PT_TRY(dev_alloc((void **)&ix->inv_perm, sizeof(uint32_t) * (size_t)ix->n));
+        tex_inverse_perm_kernel<PT><<<tcdiv(ix->n, 256), 256, 0, ix->stream>>>((const PT *)ix->pts, ix->n, ix->inv_perm);
+        count_launch();
+    }
+    return PT_OK;
+}
+
 template <typename PT>
 static int texture_render_index(pt_index *ix, const void *vertices, size_t n_vertices, const int32_t *faces,
                                 size_t n_faces, int k, double radius, int res, int pad, uint8_t *bgra_out,
                                 pt_texture_stats *st)
 {
-    if (!ix->inv_perm && ix->n) {            // original index -> position in the sorted cloud, built once
-        PT_TRY(dev_alloc((void **)&ix->inv_perm, sizeof(uint32_t) * (size_t)ix->n));
-        tex_inverse_perm_kernel<PT><<<tcdiv(ix->n, 256), 256, 0, ix->stream>>>((const PT *)ix->pts, ix->n, ix->inv_perm);
-        count_launch();
-    }
+    PT_TRY(index_inverse_perm<PT>(ix));
     PosSorted<PT> pos{(const PT *)ix->pts, ix->inv_perm};
     return texture_pipeline(ix, pos, ix->n, ix->attrs, true, nullptr, vertices, n_vertices, faces, n_faces, k, radius,
                             res, pad, bgra_out, st);
@@ -930,25 +940,316 @@ __global__ void __launch_bounds__(256) bake_unpack_vertices_kernel(const Raw80t 
     o[5] = r.normal[0]; o[6] = r.normal[1]; o[7] = r.normal[2];
 }
 
+// ---- height bake (DESIGN.md section 8, "Height bake") ---------------------------------------------
+// h = (sum_j w_j ((p_j - x) . N)) / W over the sample's neighbour list: the blend's weights, the
+// texel's unit mesh normal N of the tangent bake, sums sequential in neighbour order from +0.0.
+// NaN (always the quiet NaN 0x7fc00000) is "no value".  Samples per launch of the query + height
+// kernel in the bake: the neighbour lists of one chunk are 4 k bytes per sample.
+constexpr uint32_t HEIGHT_CHUNK = 1u << 22;
+constexpr uint32_t HEIGHT_NAN = 0x7fc00000u;
+
+// the texel's unit mesh normal, exactly as bake_tangent_compose_kernel computes it; false when the
+// sample is malformed or the mixed normal is not usable
+__device__ __forceinline__ bool bake_texel_normal(const BakeMesh &M, const double *frames, uint32_t tex, int32_t f, D3 &N)
+{
+    const double *c[3];
+    if (f < 0 || (uint32_t)f >= M.n_faces || tex >= (uint32_t)M.res * (uint32_t)M.res || !bake_corners(M, (uint32_t)f, c))
+        return false;
+    V2 t[3];
+    bake_uv(M, c, t);
+    double bc[3];
+    tx_tri_coords(t[0], t[1], t[2], bake_texel_point(M.res, (int)(tex % (uint32_t)M.res), (int)(tex / (uint32_t)M.res)), bc);
+    const double *fr[3];
+#pragma unroll
+    for (int j = 0; j < 3; ++j) fr[j] = frames + (size_t)M.faces[3 * (size_t)f + j] * BAKE_ROW;
+    const D3 n = d3_mix(bc, d3_load(fr[0]), d3_load(fr[1]), d3_load(fr[2]));
+    if (!d3_usable(n)) return false;
+    N = d3_normalise(n);
+    return true;
+}
+
+__device__ __forceinline__ double shfl_d(double v, int src) { return __shfl_sync(0xffffffffu, v, src); }
+
+// A warp takes 32 consecutive samples.  First each lane computes the normal of one of them; then
+// the warp walks them in `width` rounds, a group of `width` (the power of two >= k) lanes per
+// sample: lane j of a group gathers neighbour j through the position source (independent random
+// reads, in parallel), computes d2 in the metric's operation order and w_j (p_j - x).N, and the
+// group adds the terms in neighbour order through shuffles.  Every lane runs the same loops, so
+// the shuffles see the full warp.
+template <typename POS>
+__global__ void __launch_bounds__(256)
+bake_height_kernel(const BakeMesh M, const double *frames, const uint32_t *texels, const int32_t *sample_faces,
+                   const double *xyz, uint32_t count, const int32_t *idx, int k, int width, const POS pos,
+                   uint32_t n_points, float *height)
+{
+    const unsigned lane = threadIdx.x & 31u;
+    const uint32_t base = (uint32_t)(((size_t)blockIdx.x * blockDim.x + threadIdx.x) >> 5) * 32u;
+    if (base >= count) return;                                    // warp-uniform
+    D3 myN = {0.0, 0.0, 0.0}, myX = myN;
+    bool myOk = false;
+    if (base + lane < count) {
+        const uint32_t i = base + lane;
+        myOk = bake_texel_normal(M, frames, texels[i], sample_faces[i], myN);
+        myX = d3_load(xyz + 3 * (size_t)i);
+    }
+    const unsigned per_round = 32u / (unsigned)width;
+    const unsigned g = lane / (unsigned)width, j = lane % (unsigned)width, g0 = g * (unsigned)width;
+    for (unsigned r = 0; r < (unsigned)width; ++r) {
+        const unsigned src = r * per_round + g;                    // < 32
+        const D3 N = {shfl_d(myN.x, src), shfl_d(myN.y, src), shfl_d(myN.z, src)};
+        const D3 x = {shfl_d(myX.x, src), shfl_d(myX.y, src), shfl_d(myX.z, src)};
+        const bool ok = __shfl_sync(0xffffffffu, (int)myOk, src) != 0;
+        const uint32_t s = base + src;
+        bool has = false;
+        double d2 = 0.0, o = 0.0;
+        if (ok && s < count && (int)j < k) {
+            const int id = idx[(size_t)s * k + j];
+            if (id >= 0 && (uint32_t)id < n_points) {
+                double p[3];
+                pos.get(id, p);
+                const D3 pj = {p[0], p[1], p[2]};
+                d2 = dist2_exact(x.x, x.y, x.z, pj.x, pj.y, pj.z);
+                o = d3_dot(d3_sub(pj, x), N);
+                has = true;
+            }
+        }
+        // the list is its leading run of valid entries
+        const unsigned seg = (__ballot_sync(0xffffffffu, has) >> g0) & (width == 32 ? 0xffffffffu : ((1u << width) - 1u));
+        const int cnt = __ffsll(~(unsigned long long)seg) - 1;
+        int mode = shfl_d(d2, g0) == 0.0 ? 1 : 0;
+        double W = 0.0, S = 0.0;
+        bool done = cnt == 0;
+        for (int pass = 0; pass < 2; ++pass) {
+            if (!__any_sync(0xffffffffu, !done)) break;
+            const double w = blend_weight(mode, d2, (int)j);
+            const double wo = __dmul_rn(w, o);
+            double w_sum = 0.0, s_sum = 0.0;
+            for (int jj = 0; jj < k; ++jj) {
+                const double wj = shfl_d(w, (int)g0 + jj), woj = shfl_d(wo, (int)g0 + jj);
+                if (jj < cnt) {
+                    w_sum = __dadd_rn(w_sum, wj);
+                    s_sum = __dadd_rn(s_sum, woj);
+                }
+            }
+            if (!done) {
+                W = w_sum;
+                S = s_sum;
+                done = W > 0.0 && W < INFINITY;
+            }
+            mode = 2;
+        }
+        if (j == 0 && cnt > 0 && s < count) {
+            const float h = __double2float_rn(__ddiv_rn(S, W));
+            height[texels[s]] = h != h ? __uint_as_float(HEIGHT_NAN) : h;
+        }
+    }
+}
+
+__global__ void __launch_bounds__(256) bake_height_fill_kernel(float *h, size_t n)
+{
+    for (size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += (size_t)gridDim.x * blockDim.x)
+        h[i] = __uint_as_float(HEIGHT_NAN);
+}
+
+// float -> uint32 with the same order (-0 below +0)
+__device__ __forceinline__ uint32_t height_key(float h)
+{
+    const uint32_t u = __float_as_uint(h);
+    return (u & 0x80000000u) ? ~u : (u | 0x80000000u);
+}
+__device__ __forceinline__ float height_unkey(uint32_t k)
+{
+    return __uint_as_float((k & 0x80000000u) ? (k & 0x7fffffffu) : ~k);
+}
+
+// mm[0] = min key, mm[1] = max key of the non-NaN heights (start 0xffffffff / 0), *valued (may be null)
+// += their count
+__global__ void __launch_bounds__(256)
+bake_height_minmax_kernel(const float *h, size_t n, uint32_t *mm, unsigned long long *valued)
+{
+    uint32_t lo = 0xffffffffu, hi = 0u;
+    unsigned long long c = 0;
+    for (size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += (size_t)gridDim.x * blockDim.x) {
+        const float v = h[i];
+        if (v != v) continue;
+        const uint32_t key = height_key(v);
+        lo = min(lo, key);
+        hi = max(hi, key);
+        ++c;
+    }
+    for (int off = 16; off; off >>= 1) {
+        lo = min(lo, __shfl_xor_sync(0xffffffffu, lo, off));
+        hi = max(hi, __shfl_xor_sync(0xffffffffu, hi, off));
+        c += __shfl_xor_sync(0xffffffffu, c, off);
+    }
+    if ((threadIdx.x & 31u) == 0 && c) {
+        atomicMin(mm, lo);
+        atomicMax(mm + 1, hi);
+        if (valued) atomicAdd(valued, c);
+    }
+}
+
+// the code range: the caller's when `fixed`, else the heights' min and max, (0, 0) without any
+__global__ void bake_height_range_kernel(const uint32_t *mm, int fixed, double lo, double hi, double *range)
+{
+    if (!fixed) {
+        const bool any = mm[0] <= mm[1];
+        lo = any ? (double)height_unkey(mm[0]) : 0.0;
+        hi = any ? (double)height_unkey(mm[1]) : 0.0;
+    }
+    range[0] = lo;
+    range[1] = hi;
+}
+
+// E(h) = clamp(floor((h - lo) * s + 0.5), 0, 65535), s = 65535 / (hi - lo); 0 for every h when hi == lo
+__device__ __forceinline__ uint32_t height_encode(float h, double lo, double hi)
+{
+    if (hi == lo) return 0u;
+    const double s = __ddiv_rn(65535.0, __dsub_rn(hi, lo));
+    const double e = floor(__dadd_rn(__dmul_rn(__dsub_rn((double)h, lo), s), 0.5));
+    return (uint32_t)fmin(fmax(e, 0.0), 65535.0);
+}
+
+// Per texel: code16 = E(h), 0 without a value; or, for the padding, word = E(h) + 1, 0 without a value.
+__global__ void __launch_bounds__(256)
+bake_height_encode_kernel(const float *h, size_t n, const double *range, uint16_t *code16, uint32_t *word)
+{
+    const size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= n) return;
+    const float v = h[i];
+    const uint32_t e = v != v ? 0u : height_encode(v, range[0], range[1]) + 1u;
+    if (code16) code16[i] = (uint16_t)(e ? e - 1u : 0u);
+    if (word) word[i] = e;
+}
+
+// The texture's 25 x 25 window on words (E + 1 or 0): the 8-bit pair takes byte-wise maxima, which
+// would mix the two bytes of a code.  A texel without a value takes the window's largest code.
+__global__ void __launch_bounds__(256) bake_height_dilate_h_kernel(const uint32_t *word, int res, uint32_t *tmp)
+{
+    const size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= (size_t)res * res) return;
+    const int y = (int)(i / res), x = (int)(i % res);
+    uint32_t m = 0;
+    for (int dx = -12; dx <= 12; ++dx) {
+        const int xx = x + dx;
+        if (xx >= 0 && xx < res) m = max(m, word[(size_t)y * res + xx]);
+    }
+    tmp[i] = m;
+}
+__global__ void __launch_bounds__(256)
+bake_height_dilate_v_pad_kernel(const uint32_t *word, const uint32_t *tmp, int res, uint16_t *code16)
+{
+    const size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= (size_t)res * res) return;
+    const int y = (int)(i / res), x = (int)(i % res);
+    uint32_t m = 0;
+    for (int dy = -12; dy <= 12; ++dy) {
+        const int yy = y + dy;
+        if (yy >= 0 && yy < res) m = max(m, tmp[(size_t)yy * res + x]);
+    }
+    const uint32_t t = word[i] ? word[i] : m;
+    code16[i] = (uint16_t)(t ? t - 1u : 0u);
+}
+
+static int bake_height_width(int k)
+{
+    int w = 1;
+    while (w < k) w <<= 1;
+    return w;
+}
+
+template <typename POS>
+static int launch_height(const BakeMesh &M, const double *frames, const uint32_t *texels, const int32_t *sample_faces,
+                         const double *xyz, size_t count, const int32_t *idx, int k, const POS &pos,
+                         uint32_t n_points, float *height, cudaStream_t s)
+{
+    if (!count) return PT_OK;
+    bake_height_kernel<POS><<<tcdiv(count, 256), 256, 0, s>>>(M, frames, texels, sample_faces, xyz, (uint32_t)count, idx, k,
+                                                              bake_height_width(k), pos, n_points, height);
+    count_launch();
+    PT_CUDA(cudaGetLastError());
+    return PT_OK;
+}
+
+static bool height_range_fixed(const double *r)
+{
+    return r && std::isfinite(r[0]) && std::isfinite(r[1]) && r[0] < r[1];
+}
+
+// From the float map: the code range into range_out (device, 2 doubles), the number of valued texels
+// into *d_valued (device, added to; may be null) and, when code16 is set, the 16-bit map, padded when pad != 0.
+static int bake_height_finish(const float *height, int res, int pad, const double *range_in, double *range_out,
+                              uint16_t *code16, unsigned long long *d_valued, cudaStream_t s)
+{
+    const size_t n_pix = (size_t)res * res;
+    uint32_t *d_mm = nullptr, *d_word = nullptr, *d_tmp = nullptr;
+    int rc = PT_OK;
+    auto fail = [&](cudaError_t e) { if (e != cudaSuccess && rc == PT_OK) rc = map_cuda_error(e); return e != cudaSuccess; };
+    do {
+        const bool padded = code16 && pad;
+        if (pool_alloc((void **)&d_mm, 2 * sizeof(uint32_t), s) ||
+            (padded && (pool_alloc((void **)&d_word, 4 * n_pix, s) || pool_alloc((void **)&d_tmp, 4 * n_pix, s)))) {
+            rc = PT_ERR_OUT_OF_MEMORY;
+            break;
+        }
+        if (fail(cudaMemsetAsync(d_mm, 0xff, sizeof(uint32_t), s)) || fail(cudaMemsetAsync(d_mm + 1, 0, sizeof(uint32_t), s)))
+            break;
+        bake_height_minmax_kernel<<<148 * 8, 256, 0, s>>>(height, n_pix, d_mm, d_valued);
+        const bool fixed = height_range_fixed(range_in);
+        bake_height_range_kernel<<<1, 1, 0, s>>>(d_mm, fixed ? 1 : 0, fixed ? range_in[0] : 0.0, fixed ? range_in[1] : 0.0,
+                                                 range_out);
+        count_launch(2);
+        if (code16) {
+            bake_height_encode_kernel<<<tcdiv(n_pix, 256), 256, 0, s>>>(height, n_pix, range_out, padded ? nullptr : code16,
+                                                                        d_word);
+            count_launch();
+            if (padded) {
+                bake_height_dilate_h_kernel<<<tcdiv(n_pix, 256), 256, 0, s>>>(d_word, res, d_tmp);
+                bake_height_dilate_v_pad_kernel<<<tcdiv(n_pix, 256), 256, 0, s>>>(d_word, d_tmp, res, code16);
+                count_launch(2);
+            }
+        }
+        fail(cudaGetLastError());
+    } while (0);
+    void *frees[] = {d_mm, d_word, d_tmp};
+    for (void *p : frees) pool_free(p, s);
+    return rc;
+}
+
 static bool bake_wants_tangent_maps(const pt_bake_outputs &o) { return o.tangent_bgra || o.tangent_normal; }
 static bool bake_wants_frames(const pt_bake_outputs &o) { return bake_wants_tangent_maps(o) || o.vertex_tangents; }
 static bool bake_wants_object_maps(const pt_bake_outputs &o) { return o.bgra || o.normal_bgra || o.normal; }
+static bool bake_wants_height(const pt_bake_height *h) { return h && (h->height || h->height_u16); }
+
+template <typename PT>
+static int launch_height_index(pt_index *ix, const BakeMesh &M, const double *frames, const uint32_t *texels,
+                               const int32_t *sample_faces, const double *xyz, size_t count, const int32_t *idx, int k,
+                               float *height, cudaStream_t s)
+{
+    PT_TRY(index_inverse_perm<PT>(ix));
+    const PosSorted<PT> pos{(const PT *)ix->pts, ix->inv_perm};
+    return launch_height(M, frames, texels, sample_faces, xyz, count, idx, k, pos, ix->n, height, s);
+}
 
 static int texture_bake(pt_index *ix, const void *vertices, size_t n_vertices, const int32_t *faces, size_t n_faces,
-                        int k, double radius, int res, int pad, const pt_bake_outputs &o, pt_bake_stats *st)
+                        int k, double radius, int res, int pad, const pt_bake_outputs &o, pt_bake_height *hb,
+                        pt_bake_stats *st)
 {
     cudaStream_t s = ix->stream;
     const size_t n_pix = (size_t)res * res;
-    const bool maps = bake_wants_object_maps(o) || bake_wants_tangent_maps(o);
-    const bool tmaps = bake_wants_tangent_maps(o), frames = bake_wants_frames(o);
+    const bool heights = bake_wants_height(hb);
+    const bool maps = bake_wants_object_maps(o) || bake_wants_tangent_maps(o) || heights;
+    const bool tmaps = bake_wants_tangent_maps(o), frames = bake_wants_frames(o) || heights;
     Raw80t *d_raw = nullptr;
-    double *d_rows = nullptr, *d_q = nullptr, *d_frames = nullptr;
-    int32_t *d_faces = nullptr, *d_sface = nullptr;
+    double *d_rows = nullptr, *d_q = nullptr, *d_frames = nullptr, *d_range = nullptr;
+    int32_t *d_faces = nullptr, *d_sface = nullptr, *d_idx = nullptr;
     uint32_t *d_texels = nullptr;
     uint8_t *d_rgba = nullptr, *d_bgra = nullptr, *d_nbgra = nullptr, *d_tbgra = nullptr;
-    float *d_normal = nullptr, *d_nf = nullptr, *d_tnf = nullptr, *d_vt = nullptr;
+    float *d_normal = nullptr, *d_nf = nullptr, *d_tnf = nullptr, *d_vt = nullptr, *d_height = nullptr;
+    uint16_t *d_h16 = nullptr;
     unsigned long long *d_empty = nullptr;
     cudaEvent_t ev[4] = {};
+    std::vector<cudaEvent_t> marks;                // around each query chunk when heights are baked
     size_t count = 0;
     int rc = PT_OK;
     auto fail = [&](cudaError_t e) { if (e != cudaSuccess && rc == PT_OK) rc = map_cuda_error(e); return e != cudaSuccess; };
@@ -958,10 +1259,13 @@ static int texture_bake(pt_index *ix, const void *vertices, size_t n_vertices, c
         if (pool_alloc((void **)&d_raw, sizeof(Raw80t) * n_vertices, s) ||
             pool_alloc((void **)&d_rows, sizeof(double) * BAKE_ROW * n_vertices, s) ||
             pool_alloc((void **)&d_faces, sizeof(int32_t) * 3 * n_faces, s) ||
-            pool_alloc((void **)&d_empty, sizeof(unsigned long long), s) ||
+            pool_alloc((void **)&d_empty, sizeof(unsigned long long) * (heights ? 2 : 1), s) ||
             (maps && (pool_alloc((void **)&d_texels, sizeof(uint32_t) * n_pix, s) ||
                       pool_alloc((void **)&d_q, sizeof(double) * 3 * n_pix, s))) ||
-            (tmaps && pool_alloc((void **)&d_sface, sizeof(int32_t) * n_pix, s)) ||
+            ((tmaps || heights) && pool_alloc((void **)&d_sface, sizeof(int32_t) * n_pix, s)) ||
+            (heights && (pool_alloc((void **)&d_height, sizeof(float) * n_pix, s) ||
+                         pool_alloc((void **)&d_range, 2 * sizeof(double), s))) ||
+            (heights && hb->height_u16 && pool_alloc((void **)&d_h16, sizeof(uint16_t) * n_pix, s)) ||
             (frames && pool_alloc((void **)&d_frames, sizeof(double) * BAKE_ROW * n_vertices, s)) ||
             (o.bgra && pool_alloc((void **)&d_bgra, 4 * n_pix, s)) ||
             (o.normal_bgra && pool_alloc((void **)&d_nbgra, 4 * n_pix, s)) ||
@@ -984,20 +1288,43 @@ static int texture_bake(pt_index *ix, const void *vertices, size_t n_vertices, c
         if (maps && (rc = bake_texels(M, d_texels, d_q, d_sface, &count, s)) != PT_OK) break;
         if (frames && (rc = bake_frames(M, d_frames, d_vt, s)) != PT_OK) break;
         if (fail(cudaEventRecord(ev[1], s))) break;
-        if (pool_alloc((void **)&d_rgba, 4 * (count ? count : 1), s) || pool_alloc((void **)&d_normal, sizeof(float) * 3 * (count ? count : 1), s)) {
+        // heights need the neighbour lists: the query and the height kernel then run in chunks, so
+        // the lists take at most HEIGHT_CHUNK * k * 4 bytes
+        const size_t chunk = heights ? HEIGHT_CHUNK : (count ? count : 1);
+        if (pool_alloc((void **)&d_rgba, 4 * (count ? count : 1), s) || pool_alloc((void **)&d_normal, sizeof(float) * 3 * (count ? count : 1), s) ||
+            (heights && pool_alloc((void **)&d_idx, sizeof(int32_t) * k * std::min(chunk, count ? count : 1), s))) {
             rc = PT_ERR_OUT_OF_MEMORY;
             break;
         }
-        if (count) {
+        if (heights) {
+            bake_height_fill_kernel<<<148 * 8, 256, 0, s>>>(d_height, n_pix);
+            count_launch();
+        }
+        for (size_t c0 = 0; c0 < count; c0 += chunk) {
+            const size_t cm = std::min(chunk, count - c0);
+            if (heights) {
+                marks.emplace_back();
+                if (fail(cudaEventCreate(&marks.back())) || fail(cudaEventRecord(marks.back(), s))) break;
+            }
             QueryParams qp{};
             qp.pts = ix->pts; qp.attrs = ix->attrs; qp.attrs_curve = ix->attrs_curve; qp.ids = nullptr; qp.pyr = ix->pyr;
             qp.n = ix->n; qp.n_leaves = ix->n_leaves; qp.w_levels = ix->w_levels; qp.t_levels = ix->t_levels;
             qp.pq_cap = opt_queue_cap();
-            qp.queries = d_q; qp.m = (uint32_t)count; qp.k = k;
+            qp.queries = d_q + 3 * c0; qp.m = (uint32_t)cm; qp.k = k;
             qp.r2 = (!(radius >= 0.0) || std::isinf(radius)) ? INFINITY : radius * radius;
-            qp.rgba_out = d_rgba; qp.normal_out = d_normal;
+            qp.rgba_out = d_rgba + 4 * c0; qp.normal_out = d_normal + 3 * c0;
+            qp.idx_out = d_idx;
             if ((rc = launch_query(ix, qp, s)) != PT_OK) break;
+            if (!heights) continue;
+            marks.emplace_back();
+            if (fail(cudaEventCreate(&marks.back())) || fail(cudaEventRecord(marks.back(), s))) break;
+            rc = ix->coord_f64 ? launch_height_index<PointD>(ix, M, d_frames, d_texels + c0, d_sface + c0, d_q + 3 * c0, cm,
+                                                             d_idx, k, d_height, s)
+                               : launch_height_index<PointF>(ix, M, d_frames, d_texels + c0, d_sface + c0, d_q + 3 * c0, cm,
+                                                             d_idx, k, d_height, s);
+            if (rc != PT_OK) break;
         }
+        if (rc != PT_OK) break;
         if (fail(cudaEventRecord(ev[2], s))) break;
         if (bake_wants_object_maps(o) &&
             (rc = bake_compose(d_texels, count, d_rgba, d_normal, res, pad, d_bgra, d_nbgra, d_nf, d_empty, s)) != PT_OK)
@@ -1006,6 +1333,10 @@ static int texture_bake(pt_index *ix, const void *vertices, size_t n_vertices, c
         if (tmaps && (rc = bake_compose_tangent(M, d_frames, d_texels, d_sface, count, d_rgba, d_normal, pad, d_tbgra,
                                                 d_tnf, bake_wants_object_maps(o) ? nullptr : d_empty, s)) != PT_OK)
             break;
+        if (heights) {
+            if (fail(cudaMemsetAsync(d_empty + 1, 0, sizeof(unsigned long long), s))) break;
+            if ((rc = bake_height_finish(d_height, res, pad, hb->range, d_range, d_h16, d_empty + 1, s)) != PT_OK) break;
+        }
         if (fail(cudaEventRecord(ev[3], s))) break;
         if (o.bgra && fail(cudaMemcpyAsync(o.bgra, d_bgra, 4 * n_pix, cudaMemcpyDeviceToHost, s))) break;
         if (o.normal_bgra && fail(cudaMemcpyAsync(o.normal_bgra, d_nbgra, 4 * n_pix, cudaMemcpyDeviceToHost, s))) break;
@@ -1017,22 +1348,40 @@ static int texture_bake(pt_index *ix, const void *vertices, size_t n_vertices, c
         if (o.vertex_tangents && n_vertices &&
             fail(cudaMemcpyAsync(o.vertex_tangents, d_vt, sizeof(float) * 4 * n_vertices, cudaMemcpyDeviceToHost, s)))
             break;
-        unsigned long long empty = 0;
-        if (fail(cudaMemcpyAsync(&empty, d_empty, sizeof empty, cudaMemcpyDeviceToHost, s))) break;
+        if (heights) {
+            if (hb->height && fail(cudaMemcpyAsync(hb->height, d_height, sizeof(float) * n_pix, cudaMemcpyDeviceToHost, s)))
+                break;
+            if (hb->height_u16 &&
+                fail(cudaMemcpyAsync(hb->height_u16, d_h16, sizeof(uint16_t) * n_pix, cudaMemcpyDeviceToHost, s)))
+                break;
+            if (fail(cudaMemcpyAsync(hb->range_used, d_range, 2 * sizeof(double), cudaMemcpyDeviceToHost, s))) break;
+        }
+        unsigned long long empty[2] = {0, 0};
+        if (fail(cudaMemcpyAsync(empty, d_empty, sizeof(unsigned long long) * (heights ? 2 : 1), cudaMemcpyDeviceToHost, s)))
+            break;
         if (fail(cudaStreamSynchronize(s))) break;
+        if (heights) hb->texels = empty[1];
         if (st) {
             st->texels = count;
-            st->empty = empty;
+            st->empty = empty[0];
             cudaEventElapsedTime(&st->raster_ms, ev[0], ev[1]);
             cudaEventElapsedTime(&st->knn_ms, ev[1], ev[2]);
             cudaEventElapsedTime(&st->pad_ms, ev[2], ev[3]);
+            if (heights) {                         // the height kernels between the query chunks count as pad_ms
+                float knn = 0.0f, t = 0.0f;
+                for (size_t c = 0; c + 1 < marks.size(); c += 2)
+                    if (cudaEventElapsedTime(&t, marks[c], marks[c + 1]) == cudaSuccess) knn += t;
+                st->pad_ms += st->knn_ms - knn;
+                st->knn_ms = knn;
+            }
         }
     } while (0);
     cudaStreamSynchronize(s);
     void *frees[] = {d_raw, d_rows, d_faces, d_texels, d_q, d_sface, d_frames, d_rgba, d_normal, d_bgra, d_nbgra, d_nf,
-                     d_tbgra, d_tnf, d_vt, d_empty};
+                     d_tbgra, d_tnf, d_vt, d_empty, d_idx, d_height, d_range, d_h16};
     for (void *p : frees) pool_free(p, s);
     for (auto &e : ev) if (e) cudaEventDestroy(e);
+    for (auto &e : marks) if (e) cudaEventDestroy(e);
     cudaStreamSynchronize(s);
     cudaGetLastError();
     return rc;
@@ -1159,21 +1508,70 @@ extern "C" int pt_bake_compose_device(const uint32_t *texels, size_t count, cons
                         (cudaStream_t)stream);
 }
 
-extern "C" int pt_texture_bake_ex(pt_index *ix, const void *vertices, size_t n_vertices, const int32_t *faces,
-                                  size_t n_faces, int k, double radius, int resolution, int pad,
-                                  const pt_bake_outputs *out, pt_bake_stats *stats)
+extern "C" int pt_texture_bake_height(pt_index *ix, const void *vertices, size_t n_vertices, const int32_t *faces,
+                                      size_t n_faces, int k, double radius, int resolution, int pad,
+                                      const pt_bake_outputs *out, pt_bake_height *height, pt_bake_stats *stats)
 {
-    if (!ix || (!vertices && n_vertices) || (!faces && n_faces) || !out ||
-        (!bake_wants_object_maps(*out) && !bake_wants_frames(*out)) || resolution < 1 || resolution > 16384 ||
+    const pt_bake_outputs none = {nullptr, nullptr, nullptr, nullptr, nullptr, nullptr};
+    const pt_bake_outputs &o = out ? *out : none;
+    const bool heights = bake_wants_height(height);
+    if (!ix || (!vertices && n_vertices) || (!faces && n_faces) || (height && !heights) ||
+        (!bake_wants_object_maps(o) && !bake_wants_frames(o) && !heights) || resolution < 1 || resolution > 16384 ||
         n_vertices > 0x7ffffff0ull || n_faces >= (1ull << 31))
         return PT_ERR_INVALID_ARG;
     if (k < 1 || k > PT_MAX_K) return PT_ERR_UNSUPPORTED;
-    if (bake_wants_frames(*out) && !bake_corners_fit(n_faces)) return PT_ERR_UNSUPPORTED;
+    if ((bake_wants_frames(o) || heights) && !bake_corners_fit(n_faces)) return PT_ERR_UNSUPPORTED;
     if (ix->ids) return PT_ERR_UNSUPPORTED;           // slab indexes answer with global ids
     if (!ix->attrs && ix->n) return PT_ERR_INVALID_ARG;
     if (pt_device_count() == 0) return PT_ERR_NO_DEVICE;
     PT_CUDA(cudaSetDevice(ix->device));
-    return texture_bake(ix, vertices, n_vertices, faces, n_faces, k, radius, resolution, pad, *out, stats);
+    return texture_bake(ix, vertices, n_vertices, faces, n_faces, k, radius, resolution, pad, o, height, stats);
+}
+
+extern "C" int pt_texture_bake_ex(pt_index *ix, const void *vertices, size_t n_vertices, const int32_t *faces,
+                                  size_t n_faces, int k, double radius, int resolution, int pad,
+                                  const pt_bake_outputs *out, pt_bake_stats *stats)
+{
+    if (!out) return PT_ERR_INVALID_ARG;
+    return pt_texture_bake_height(ix, vertices, n_vertices, faces, n_faces, k, radius, resolution, pad, out, nullptr,
+                                  stats);
+}
+
+extern "C" int pt_bake_compose_height_device(const double *vertices_xyzuvn, const double *frames, size_t n_vertices,
+                                             const int32_t *faces, size_t n_faces, const uint32_t *texels,
+                                             const int32_t *sample_faces, const double *sample_xyz, size_t count,
+                                             const int32_t *idx, int k, const double *cloud_xyz, size_t n_points,
+                                             int resolution, int pad, const double *range_in, float *height_out,
+                                             uint16_t *height_u16_out, double *range_out, int device, void *stream)
+{
+    if ((n_vertices && (!vertices_xyzuvn || !frames)) || (!faces && n_faces) ||
+        (count && (!texels || !sample_faces || !sample_xyz || !idx)) || (!cloud_xyz && n_points) || resolution < 1 ||
+        resolution > 16384 || count > (size_t)resolution * resolution || n_vertices > 0x7ffffff0ull ||
+        n_faces >= (1ull << 31) || n_points > (size_t)INT32_MAX || (!height_out && !height_u16_out))
+        return PT_ERR_INVALID_ARG;
+    if (k < 1 || k > PT_MAX_K || !bake_corners_fit(n_faces)) return PT_ERR_UNSUPPORTED;
+    if (pt_device_count() == 0) return PT_ERR_NO_DEVICE;
+    if (device >= 0) PT_CUDA(cudaSetDevice(device));
+    cudaStream_t s = (cudaStream_t)stream;
+    const size_t n_pix = (size_t)resolution * resolution;
+    const BakeMesh M{vertices_xyzuvn, BAKE_ROW, (uint32_t)n_vertices, faces, (uint32_t)n_faces, resolution};
+    float *h = height_out;
+    double *range = range_out;
+    int rc = PT_OK;
+    do {
+        if ((!h && (rc = pool_alloc((void **)&h, sizeof(float) * n_pix, s)) != PT_OK) ||
+            (!range && (rc = pool_alloc((void **)&range, 2 * sizeof(double), s)) != PT_OK))
+            break;
+        bake_height_fill_kernel<<<148 * 8, 256, 0, s>>>(h, n_pix);
+        count_launch();
+        if ((rc = launch_height(M, frames, texels, sample_faces, sample_xyz, count, idx, k, PosPlain{cloud_xyz},
+                                (uint32_t)n_points, h, s)) != PT_OK)
+            break;
+        rc = bake_height_finish(h, resolution, pad, range_in, range, height_u16_out, nullptr, s);
+    } while (0);
+    if (h != height_out) pool_free(h, s);
+    if (range != range_out) pool_free(range, s);
+    return rc;
 }
 
 extern "C" int pt_texture_bake(pt_index *ix, const void *vertices, size_t n_vertices, const int32_t *faces,

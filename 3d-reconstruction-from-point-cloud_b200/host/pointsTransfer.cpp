@@ -15,10 +15,11 @@
 // instead of texture.png the tool writes `transferred.ply`, the input mesh in the same 11-column
 // ASCII format with the transferred colour and normal per vertex.  Extra options (all default to
 // the reference's behaviour): -k N, -r RADIUS, -o FILE, -d DEVICE.  -b FILE / -n FILE also bake the
-// cloud's colour / object-space normal onto every texel of the mesh's UV atlas (pt_texture_bake_ex,
+// cloud's colour / object-space normal onto every texel of the mesh's UV atlas (pt_texture_bake_height,
 // same -R, -k, -r) and write them as PNG; -t FILE writes the tangent-space normal map as PNG and
 // -T FILE the input mesh as PLY with the per-vertex tangents (tx ty tz tw) that map is expressed
-// in.  All of them come from one bake.
+// in, -H FILE the height map as a 16-bit greyscale PNG over the heights' own range (printed as
+// "Height range: lo hi").  All of them come from one bake.
 #include <algorithm>
 #include <charconv>
 #include <chrono>
@@ -250,6 +251,7 @@ static int run(int argc, char **argv)
     std::string ply_name;                          // optional extra: the per-vertex blend as a PLY
     std::string bake_name, normal_name;            // optional extras: the per-texel colour / normal maps
     std::string tangent_name, tangent_ply_name;    // ... the tangent-space normal map, the mesh with tangents
+    std::string height_name;                       // ... the height map
     for (int i = 1; i < argc; ++i) {
         std::string a = argv[i];
         if (a == "-k" && i + 1 < argc) K = atoi(argv[++i]);
@@ -263,6 +265,7 @@ static int run(int argc, char **argv)
         else if (a == "-n" && i + 1 < argc) normal_name = argv[++i];
         else if (a == "-t" && i + 1 < argc) tangent_name = argv[++i];
         else if (a == "-T" && i + 1 < argc) tangent_ply_name = argv[++i];
+        else if (a == "-H" && i + 1 < argc) height_name = argv[++i];
         else pos_args.push_back(a);
     }
     if (pos_args.size() < 2) {
@@ -274,9 +277,10 @@ static int run(int argc, char **argv)
         std::cerr << "-k must be 1.." << PT_MAX_K << ", -R 1..32768 and -g 1..64" << std::endl;
         return 0;
     }
-    const bool bake = !bake_name.empty() || !normal_name.empty() || !tangent_name.empty() || !tangent_ply_name.empty();
+    const bool bake = !bake_name.empty() || !normal_name.empty() || !tangent_name.empty() || !tangent_ply_name.empty() ||
+                      !height_name.empty();
     if (bake && (n_gpus > 1 || resolution > 16384)) {
-        std::cerr << "-b / -n / -t / -T bake on one GPU (no -g) at -R 1..16384" << std::endl;
+        std::cerr << "-b / -n / -t / -T / -H bake on one GPU (no -g) at -R 1..16384" << std::endl;
         return 0;
     }
     const std::string pc_file_name = pos_args[0], mesh_file_name = pos_args[1];
@@ -382,10 +386,11 @@ static int run(int argc, char **argv)
     std::cout << "Neighbor search total time: " << ts.knn_ms * 1e-3 << " seconds" << std::endl;
     std::cout << "Draw triangles total time: " << (ts.draw_ms + ts.pad_ms) * 1e-3 << " seconds" << std::endl;
 
-    // extra (not in the reference): per-texel colour, normal and tangent-space normal maps, padded
-    // like the texture, and the per-vertex tangents
+    // extra (not in the reference): per-texel colour, normal and tangent-space normal maps and the
+    // 16-bit height map, padded like the texture, and the per-vertex tangents
     std::vector<uint8_t> baked, baked_normal, baked_tangent;
     std::vector<float> vertex_tangents;
+    std::vector<uint16_t> baked_height;
     if (bake) {
         const size_t n_bytes = (size_t)resolution * resolution * 4;
         if (!bake_name.empty()) baked.resize(n_bytes);
@@ -398,13 +403,24 @@ static int run(int argc, char **argv)
         bo.normal_bgra = baked_normal.empty() ? nullptr : baked_normal.data();
         bo.tangent_bgra = baked_tangent.empty() ? nullptr : baked_tangent.data();
         bo.vertex_tangents = tangent_ply_name.empty() ? nullptr : vertex_tangents.data();
+        pt_bake_height hb;
+        memset(&hb, 0, sizeof hb);                 // range (0, 0): the heights' own min and max
+        if (!height_name.empty()) {
+            baked_height.resize((size_t)resolution * resolution);
+            hb.height_u16 = baked_height.data();
+        }
         pt_bake_stats bs;
-        rc = pt_texture_bake_ex(index, vertices.data(), m, faces.data(), faces.size() / 3, K, radius, resolution, 1,
-                                &bo, &bs);
+        rc = pt_texture_bake_height(index, vertices.data(), m, faces.data(), faces.size() / 3, K, radius, resolution, 1,
+                                    &bo, height_name.empty() ? nullptr : &hb, &bs);
         if (rc != PT_OK) {
-            std::cerr << "pt_texture_bake_ex failed: " << pt_status_string(rc) << std::endl;
+            std::cerr << "pt_texture_bake_height failed: " << pt_status_string(rc) << std::endl;
             pt_index_free(index);
             return 0;
+        }
+        if (!height_name.empty()) {
+            char line[96];
+            snprintf(line, sizeof line, "Height range: %.9g %.9g", hb.range_used[0], hb.range_used[1]);
+            std::cout << line << std::endl;
         }
         std::cout << "Bake total time: " << task_timer.time() << " seconds" << std::endl;
         task_timer.reset();
@@ -418,6 +434,8 @@ static int run(int argc, char **argv)
         std::cerr << "Cannot write " << normal_name << std::endl;
     if (!baked_tangent.empty() && !ptb::write_png_bgra(tangent_name.c_str(), baked_tangent.data(), resolution, resolution))
         std::cerr << "Cannot write " << tangent_name << std::endl;
+    if (!baked_height.empty() && !ptb::write_png_gray16(height_name.c_str(), baked_height.data(), resolution, resolution))
+        std::cerr << "Cannot write " << height_name << std::endl;
     if (!tangent_ply_name.empty()) {
         // the input mesh with the tangent frame of the tangent-space map: tx ty tz tw per vertex
         // (%.9g round-trips the fp32 values)

@@ -18,7 +18,8 @@
  *   pt_texture_bake  <- no reference counterpart: per-texel colour and normal maps on
  *                       the mesh's UV atlas (the "texel" samples of the transfer);
  *                       pt_texture_bake_ex adds tangent-space normal maps and the
- *                       per-vertex tangents they are expressed in.
+ *                       per-vertex tangents they are expressed in, pt_texture_bake_height
+ *                       height (displacement) maps.
  *   pt_index_free    <- `tree` going out of scope at src/pointsTransfer.cpp:626.
  *
  * Records are the reference's own 80-byte AoS `struct Point`
@@ -200,6 +201,39 @@ int pt_texture_bake_ex(pt_index *index, const void *vertices, size_t n_vertices,
                        int resolution, int pad, const pt_bake_outputs *out,
                        pt_bake_stats *stats);
 
+/* Height bake (DESIGN.md section 8, "Height bake"): the cloud's signed height above the mesh along
+ * the interpolated mesh normal N (the +Z of the tangent maps, the direction renderers displace
+ * along).  Per covered texel with sample position x and neighbours p_j (the k-NN list, blend
+ * weights w_j, W = sum w_j): h = (float)((sum_j w_j (p_j - x).N) / W), positive where the cloud
+ * lies outside the mesh.
+ *   height      h per texel (res*res floats), NaN where there is no value (uncovered texel,
+ *               empty neighbour list, unusable mesh normal); never padded
+ *   height_u16  E(h) = clamp(floor((h - lo) * 65535 / (hi - lo) + 0.5), 0, 65535), 0 without a
+ *               value and for every texel when hi == lo (res*res uint16); padded like the 8-bit
+ *               maps when pad != 0, a texel without a value taking the largest code in its
+ *               25 x 25 window.  Decode with h = lo + E * (hi - lo) / 65535.
+ *   range       in: a finite lo < hi fixes the code range; otherwise it is the min and max of the
+ *               valued heights ((0, 0) without any)
+ *   range_used  out: the (lo, hi) the codes use
+ *   texels      out: texels with a value
+ * Either map may be NULL, but not both. */
+typedef struct pt_bake_height {
+    float    *height;        /* res*res, NaN = no value, never padded (may be NULL) */
+    uint16_t *height_u16;    /* res*res, padded when pad != 0 (may be NULL) */
+    double    range[2];      /* in: lo < hi, finite => fixed code range; else automatic */
+    double    range_used[2]; /* out */
+    uint64_t  texels;        /* out: texels with a value */
+} pt_bake_height;
+/* One texel raster and one k-NN pass for the outputs of `out` and `height`; either may be NULL, but
+ * not both.  pt_texture_bake_ex(..., out, stats) is this call with height = NULL.  With heights the
+ * neighbour lists are kept, so the search runs in chunks of at most 2^22 samples (4 k bytes of
+ * lists each); the outputs do not depend on it.  The height stage needs 3 * n_faces <= INT32_MAX,
+ * otherwise PT_ERR_UNSUPPORTED before any input is read; its time is part of pad_ms. */
+int pt_texture_bake_height(pt_index *index, const void *vertices, size_t n_vertices,
+                           const int32_t *faces, size_t n_faces, int k, double radius,
+                           int resolution, int pad, const pt_bake_outputs *out /* may be NULL */,
+                           pt_bake_height *height /* may be NULL, not both */, pt_bake_stats *stats);
+
 /* Device-buffer API: same operations with inputs/outputs already resident in
  * HBM on the index's device (bench `value`, multi-GPU slabs).  `stream` is a
  * cudaStream_t passed as void* (NULL = the CUDA default stream); these calls
@@ -285,6 +319,23 @@ int pt_bake_compose_tangent_device(const double *vertices_xyzuvn, const double *
                                    size_t count, const uint8_t *rgba, const float *normal,
                                    int resolution, int pad, uint8_t *tangent_bgra_out,
                                    float *tangent_normal_out, int device, void *stream);
+/* pt_bake_compose_height_device: the height maps of pt_texture_bake_height from count samples
+ * (texels, sample_faces and sample_xyz of pt_bake_samples_device, frames of pt_bake_frames_device)
+ * and their neighbour lists idx (count x k, original point ids ascending by (d2, id), -1 or any id
+ * outside 0..n_points-1 ends a list, as pt_query_device returns them).  cloud_xyz: n_points x 3
+ * doubles in original order.  range_in (host, 2 doubles, may be NULL: automatic) as
+ * pt_bake_height.range; range_out (device, 2 doubles, may be NULL) receives the range used.
+ * height_out (res*res floats) and height_u16_out (res*res uint16, padded when pad != 0) are device
+ * buffers, either may be NULL but not both.  3 * n_faces <= INT32_MAX, otherwise
+ * PT_ERR_UNSUPPORTED.  Asynchronous on `stream`. */
+int pt_bake_compose_height_device(const double *vertices_xyzuvn, const double *frames,
+                                  size_t n_vertices, const int32_t *faces, size_t n_faces,
+                                  const uint32_t *texels, const int32_t *sample_faces,
+                                  const double *sample_xyz, size_t count, const int32_t *idx, int k,
+                                  const double *cloud_xyz, size_t n_points, int resolution, int pad,
+                                  const double *range_in, float *height_out,
+                                  uint16_t *height_u16_out, double *range_out, int device,
+                                  void *stream);
 
 /* Halo exchange helpers for slab-sharded clouds (DESIGN.md section 6).  Fixed-capacity routing,
  * so the exchange needs no host synchronisation: per peer a send block of (cap + 1) rows of 4
