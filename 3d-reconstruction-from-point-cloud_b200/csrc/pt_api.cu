@@ -216,13 +216,13 @@ static void destroy_index(pt_index *ix)
     delete ix;
 }
 
-static double radius_to_r2(double radius)
+double radius_to_r2(double radius)
 {
     if (!(radius >= 0.0) || std::isinf(radius)) return INFINITY;
     return radius * radius;  // Distance::transformed_distance(d), src/Distance.h:97
 }
 
-static void fill_params(const pt_index *ix, QueryParams &qp)
+void fill_params(const pt_index *ix, QueryParams &qp)
 {
     qp.pts = ix->pts;
     qp.attrs = ix->attrs;

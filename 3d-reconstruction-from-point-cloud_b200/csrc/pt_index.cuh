@@ -78,6 +78,10 @@ int ingest_points_aos(pt_index *ix, const void *points, size_t n, int coord_mode
 int unpack_queries_aos(const void *raw80_dev, size_t m, double *xyz_dev, cudaStream_t s);
 
 int launch_query(pt_index *ix, const QueryParams &qp, cudaStream_t s);
+// the index's part of the query parameters (pt_api.cu); the caller adds the samples, k, r2, outputs
+void fill_params(const pt_index *ix, QueryParams &qp);
+// squared radius bound: +inf for a negative, NaN or infinite radius
+double radius_to_r2(double radius);
 // Stream-ordered allocation from the library's PRIVATE memory pool of the current device (the
 // application's default pool is never touched); release with pool_free.  dev_alloc / dev_free:
 // cudaMalloc / cudaFree for the long-lived buffers.  Both carry guard words under "pool_guard".

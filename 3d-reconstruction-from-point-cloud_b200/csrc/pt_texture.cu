@@ -276,8 +276,33 @@ tex_resolve_kernel(const unsigned long long *canvas, size_t n_pix, uint32_t *tex
     if (i < n_pix) tex[i] = (uint32_t)(canvas[i] & 0xffffffffull);     // never written: 0 (alpha 0)
 }
 
-// :593-611 as two separable 25-tap byte-wise maxima (OpenCV ignores the border) + the combine
-__global__ void __launch_bounds__(256) tex_dilate_h_kernel(const uint32_t *tex, int res, uint32_t *tmp)
+// The 25 x 25 padding window as two separable 25-tap maxima (OpenCV ignores the border), then the
+// combine of each texel's own value with its window's maximum.  PAD gives both:
+//   PadBgra    :593-611 on BGRA texels: byte-wise maxima, padded = texture + (dilated & ~alpha)
+//   PadHeight  height words (E + 1, or 0 without a value): word maxima, since byte-wise ones would
+//              mix the two bytes of a code; a texel without a value takes the window's largest code
+struct PadBgra {
+    using Out = uint32_t;
+    __device__ __forceinline__ static uint32_t max(uint32_t a, uint32_t b) { return __vmaxu4(a, b); }
+    __device__ __forceinline__ static Out combine(uint32_t t, uint32_t m)
+    {
+        const uint32_t alpha = t >> 24;
+        const uint32_t not_alpha = (alpha ^ 0xffu) * 0x01010101u;  // ~alpha replicated to the 4 channels
+        return __vaddus4(t, m & not_alpha);
+    }
+};
+struct PadHeight {
+    using Out = uint16_t;
+    __device__ __forceinline__ static uint32_t max(uint32_t a, uint32_t b) { return ::max(a, b); }
+    __device__ __forceinline__ static Out combine(uint32_t w, uint32_t m)
+    {
+        const uint32_t t = w ? w : m;
+        return (uint16_t)(t ? t - 1u : 0u);
+    }
+};
+
+template <typename PAD>
+__global__ void __launch_bounds__(256) pad_window_h_kernel(const uint32_t *img, int res, uint32_t *tmp)
 {
     const size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
     if (i >= (size_t)res * res) return;
@@ -285,12 +310,14 @@ __global__ void __launch_bounds__(256) tex_dilate_h_kernel(const uint32_t *tex, 
     uint32_t m = 0;
     for (int dx = -12; dx <= 12; ++dx) {
         const int xx = x + dx;
-        if (xx >= 0 && xx < res) m = __vmaxu4(m, tex[(size_t)y * res + xx]);
+        if (xx >= 0 && xx < res) m = PAD::max(m, img[(size_t)y * res + xx]);
     }
     tmp[i] = m;
 }
+// reads only its own texel of img, so out may be img
+template <typename PAD>
 __global__ void __launch_bounds__(256)
-tex_dilate_v_pad_kernel(const uint32_t *tex, const uint32_t *tmp, int res, uint32_t *out)
+pad_window_v_kernel(const uint32_t *img, const uint32_t *tmp, int res, typename PAD::Out *out)
 {
     const size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
     if (i >= (size_t)res * res) return;
@@ -298,15 +325,36 @@ tex_dilate_v_pad_kernel(const uint32_t *tex, const uint32_t *tmp, int res, uint3
     uint32_t m = 0;
     for (int dy = -12; dy <= 12; ++dy) {
         const int yy = y + dy;
-        if (yy >= 0 && yy < res) m = __vmaxu4(m, tmp[(size_t)yy * res + x]);
+        if (yy >= 0 && yy < res) m = PAD::max(m, tmp[(size_t)yy * res + x]);
     }
-    const uint32_t t = tex[i];
-    const uint32_t alpha = t >> 24;
-    const uint32_t not_alpha = (alpha ^ 0xffu) * 0x01010101u;      // ~alpha replicated to the 4 channels
-    out[i] = __vaddus4(t, m & not_alpha);
+    out[i] = PAD::combine(img[i], m);
 }
 
 static inline unsigned tcdiv(size_t a, size_t b) { return (unsigned)((a + b - 1) / b); }
+
+// tmp: res * res words of scratch
+template <typename PAD>
+static void launch_pad_window(const uint32_t *img, uint32_t *tmp, int res, typename PAD::Out *out, cudaStream_t s)
+{
+    const size_t n_pix = (size_t)res * res;
+    pad_window_h_kernel<PAD><<<tcdiv(n_pix, 256), 256, 0, s>>>(img, res, tmp);
+    pad_window_v_kernel<PAD><<<tcdiv(n_pix, 256), 256, 0, s>>>(img, tmp, res, out);
+    count_launch(2);
+}
+
+// Pads the given 8-bit maps (null entries skipped) in place.
+static int bake_pad(std::initializer_list<uint8_t *> imgs, int res, cudaStream_t s)
+{
+    bool any = false;
+    for (uint8_t *img : imgs) any |= img != nullptr;
+    if (!any) return PT_OK;
+    uint32_t *d_tmp = nullptr;
+    PT_TRY(pool_alloc((void **)&d_tmp, 4 * (size_t)res * res, s));
+    for (uint8_t *img : imgs)
+        if (img) launch_pad_window<PadBgra>((const uint32_t *)img, d_tmp, res, (uint32_t *)img, s);
+    pool_free(d_tmp, s);
+    return PT_OK;
+}
 
 // Mesh upload + (optionally) the neighbour search + face kernel + post-process.  `ix` gives the
 // stream, the query kernels (when d_idx_given is null) and the attribute array.
@@ -323,7 +371,7 @@ static int texture_pipeline(pt_index *ix, POS pos, uint32_t n_points, const pt_a
     double *d_xyz = nullptr;
     int32_t *d_idx = nullptr, *d_faces = nullptr;
     unsigned long long *d_canvas = nullptr, *d_stats = nullptr;
-    uint32_t *d_tex = nullptr, *d_tmp = nullptr, *d_out = nullptr;
+    uint32_t *d_tex = nullptr;
     cudaEvent_t ev[4] = {};
     int rc = PT_OK;
     auto fail = [&](cudaError_t e) { if (e != cudaSuccess && rc == PT_OK) rc = map_cuda_error(e); return e != cudaSuccess; };
@@ -333,8 +381,7 @@ static int texture_pipeline(pt_index *ix, POS pos, uint32_t n_points, const pt_a
         if (pool_alloc((void **)&d_raw, sizeof(Raw80t) * n_vertices, s) || pool_alloc((void **)&d_mv, sizeof(MeshVertex) * n_vertices, s) ||
             pool_alloc((void **)&d_xyz, sizeof(double) * 3 * n_vertices, s) || pool_alloc((void **)&d_idx, sizeof(int32_t) * n_vertices * k, s) ||
             pool_alloc((void **)&d_faces, sizeof(int32_t) * 3 * n_faces, s) || pool_alloc((void **)&d_canvas, sizeof(unsigned long long) * n_pix, s) ||
-            pool_alloc((void **)&d_stats, 16, s) || pool_alloc((void **)&d_tex, 4 * n_pix, s) ||
-            (pad && (pool_alloc((void **)&d_tmp, 4 * n_pix, s) || pool_alloc((void **)&d_out, 4 * n_pix, s)))) {
+            pool_alloc((void **)&d_stats, 16, s) || pool_alloc((void **)&d_tex, 4 * n_pix, s)) {
             rc = PT_ERR_OUT_OF_MEMORY;
             break;
         }
@@ -350,11 +397,9 @@ static int texture_pipeline(pt_index *ix, POS pos, uint32_t n_points, const pt_a
         if (search) {
             // the neighbour search of every UNIQUE vertex (the reference searches 3 x per face, :474)
             QueryParams qp{};
-            qp.pts = ix->pts; qp.attrs = ix->attrs; qp.attrs_curve = ix->attrs_curve; qp.ids = nullptr; qp.pyr = ix->pyr;
-            qp.n = ix->n; qp.n_leaves = ix->n_leaves; qp.w_levels = ix->w_levels; qp.t_levels = ix->t_levels;
-            qp.pq_cap = opt_queue_cap();
+            fill_params(ix, qp);
             qp.queries = d_xyz; qp.m = (uint32_t)n_vertices; qp.k = k;
-            qp.r2 = (!(radius >= 0.0) || std::isinf(radius)) ? INFINITY : radius * radius;
+            qp.r2 = radius_to_r2(radius);
             qp.idx_out = d_idx;
             if ((rc = launch_query(ix, qp, s)) != PT_OK) break;
         } else if (n_vertices) {
@@ -370,16 +415,10 @@ static int texture_pipeline(pt_index *ix, POS pos, uint32_t n_points, const pt_a
         tex_resolve_kernel<<<tcdiv(n_pix, 256), 256, 0, s>>>(d_canvas, n_pix, d_tex);
         count_launch();
         if (fail(cudaEventRecord(ev[2], s))) break;
-        const uint32_t *result = d_tex;
-        if (pad) {
-            tex_dilate_h_kernel<<<tcdiv(n_pix, 256), 256, 0, s>>>(d_tex, res, d_tmp);
-            tex_dilate_v_pad_kernel<<<tcdiv(n_pix, 256), 256, 0, s>>>(d_tex, d_tmp, res, d_out);
-            count_launch(2);
-            result = d_out;
-        }
+        if (pad && (rc = bake_pad({(uint8_t *)d_tex}, res, s)) != PT_OK) break;
         if (fail(cudaEventRecord(ev[3], s))) break;
         if (fail(cudaGetLastError())) break;
-        if (fail(cudaMemcpyAsync(bgra_out, result, 4 * n_pix, cudaMemcpyDeviceToHost, s))) break;
+        if (fail(cudaMemcpyAsync(bgra_out, d_tex, 4 * n_pix, cudaMemcpyDeviceToHost, s))) break;
         unsigned long long h_stats[2] = {0, 0};
         if (fail(cudaMemcpyAsync(h_stats, d_stats, 16, cudaMemcpyDeviceToHost, s))) break;
         if (fail(cudaStreamSynchronize(s))) break;
@@ -392,7 +431,7 @@ static int texture_pipeline(pt_index *ix, POS pos, uint32_t n_points, const pt_a
         }
     } while (0);
     cudaStreamSynchronize(s);
-    void *frees[] = {d_raw, d_mv, d_xyz, d_idx, d_faces, d_canvas, d_stats, d_tex, d_tmp, d_out};
+    void *frees[] = {d_raw, d_mv, d_xyz, d_idx, d_faces, d_canvas, d_stats, d_tex};
     for (void *p : frees) pool_free(p, s);
     for (auto &e : ev) if (e) cudaEventDestroy(e);
     cudaGetLastError();
@@ -466,6 +505,14 @@ __device__ __forceinline__ V2 bake_texel_point(int res, int col, int row)
     p.a = (double)col + 0.5;
     p.b = (double)(res - row) - 0.5;
     return p;
+}
+
+// barycentrics of texel tex's centre on the face with corners c, as the texel stage computes them
+__device__ __forceinline__ void bake_texel_bary(const BakeMesh &M, const double *const c[3], uint32_t tex, double bc[3])
+{
+    V2 t[3];
+    bake_uv(M, c, t);
+    tx_tri_coords(t[0], t[1], t[2], bake_texel_point(M.res, (int)(tex % (uint32_t)M.res), (int)(tex / (uint32_t)M.res)), bc);
 }
 
 // Texels whose centre lies in the UV triangle's bounding box, widened by one texel so that rounding
@@ -559,10 +606,8 @@ bake_position_kernel(const BakeMesh M, const uint32_t *owner, const uint32_t *te
     if (face_out) face_out[i] = (int32_t)f;
     const double *c[3];
     bake_corners(M, f, c);
-    V2 t[3];
-    bake_uv(M, c, t);
     double bc[3];
-    tx_tri_coords(t[0], t[1], t[2], bake_texel_point(M.res, (int)(tex % (uint32_t)M.res), (int)(tex / (uint32_t)M.res)), bc);
+    bake_texel_bary(M, c, tex, bc);
 #pragma unroll
     for (int a = 0; a < 3; ++a)
         xyz[3 * (size_t)i + a] = __dadd_rn(__dadd_rn(__dmul_rn(bc[0], c[0][a]), __dmul_rn(bc[1], c[1][a])),
@@ -651,26 +696,6 @@ bake_compose_kernel(const uint32_t *texels, uint32_t count, const uint8_t *rgba,
     if (nf) { nf[3 * t] = x; nf[3 * t + 1] = y; nf[3 * t + 2] = z; }
 }
 
-// Pads the given 8-bit maps (null entries skipped) in place with the texture's dilate + gutter
-// kernels (tex_dilate_v_pad_kernel reads only its own texel of `tex`).
-static int bake_pad(std::initializer_list<uint8_t *> imgs, int res, cudaStream_t s)
-{
-    const size_t n_pix = (size_t)res * res;
-    bool any = false;
-    for (uint8_t *img : imgs) any |= img != nullptr;
-    if (!any) return PT_OK;
-    uint32_t *d_tmp = nullptr;
-    PT_TRY(pool_alloc((void **)&d_tmp, 4 * n_pix, s));
-    for (uint8_t *img : imgs) {
-        if (!img) continue;
-        tex_dilate_h_kernel<<<tcdiv(n_pix, 256), 256, 0, s>>>((const uint32_t *)img, res, d_tmp);
-        tex_dilate_v_pad_kernel<<<tcdiv(n_pix, 256), 256, 0, s>>>((const uint32_t *)img, d_tmp, res, (uint32_t *)img);
-        count_launch(2);
-    }
-    pool_free(d_tmp, s);
-    return PT_OK;
-}
-
 // Zeroes the requested maps, scatters the samples into them and pads the 8-bit ones in place.
 static int bake_compose(const uint32_t *texels, size_t count, const uint8_t *rgba, const float *normal, int res,
                         int pad, uint8_t *bgra_out, uint8_t *normal_bgra_out, float *normal_out,
@@ -692,7 +717,7 @@ static int bake_compose(const uint32_t *texels, size_t count, const uint8_t *rgb
 
 // ---- tangent-space bake (DESIGN.md section 8, "Tangent-space bake") -----------------------------
 // Everything below is fp64 with every operation rounded on its own (no contraction, no rsqrt), in
-// the order the definition states, so that tests/bake_tangent_oracle.c equals it bit for bit:
+// the order the definition states, so that oracle/pt_bake_oracle.c equals it bit for bit:
 // a.b = (a.x b.x + a.y b.y) + a.z b.z; "usable" = all components finite and a.a > 0; normalising
 // divides each component by sqrt(a.a).  Mesh rows are 8 doubles: x y z u v nx ny nz.  Frame rows
 // are 8 doubles: N xyz, T xyz, w, 0 -- all zero for a vertex without a frame.
@@ -868,10 +893,33 @@ static int bake_frames(const BakeMesh &M, double *frames, float *tangents, cudaS
     return rc;
 }
 
-// One thread per sample: the owner face's barycentrics of the texel centre (as the texel stage
-// computes them), the mixed vertex frames made orthonormal, the handedness of the owner face's B_f,
-// and the blended cloud normal in that basis.  An empty neighbour list (alpha 0) or an unusable
-// mixed normal leaves the texel 0.
+// What a sample of the tangent and height bakes needs of its texel: the owner face's corners, the
+// barycentrics of the texel centre, the corners' vertex frame rows and the unit mesh normal N (the
+// mixed N rows, normalised).  false when the sample is malformed or the mixed normal is not usable.
+struct TexelFrame {
+    const double *c[3];
+    double        bc[3];
+    const double *fr[3];
+    D3            N;
+};
+
+__device__ __forceinline__ bool bake_texel_frame(const BakeMesh &M, const double *frames, uint32_t tex, int32_t f,
+                                                 TexelFrame &X)
+{
+    if (f < 0 || (uint32_t)f >= M.n_faces || tex >= (uint32_t)M.res * (uint32_t)M.res || !bake_corners(M, (uint32_t)f, X.c))
+        return false;
+    bake_texel_bary(M, X.c, tex, X.bc);
+#pragma unroll
+    for (int j = 0; j < 3; ++j) X.fr[j] = frames + (size_t)M.faces[3 * (size_t)f + j] * BAKE_ROW;
+    const D3 n = d3_mix(X.bc, d3_load(X.fr[0]), d3_load(X.fr[1]), d3_load(X.fr[2]));
+    if (!d3_usable(n)) return false;
+    X.N = d3_normalise(n);
+    return true;
+}
+
+// One thread per sample: the texel's frame, its mixed tangent made orthonormal to N, the handedness
+// of the owner face's B_f, and the blended cloud normal in that basis.  An empty neighbour list
+// (alpha 0) or an unusable mixed normal leaves the texel 0.
 __global__ void __launch_bounds__(256)
 bake_tangent_compose_kernel(const BakeMesh M, const double *frames, const uint32_t *texels, const int32_t *sample_faces,
                             uint32_t count, const uint8_t *rgba, const float *normal, uint32_t *tbgra, float *tnf,
@@ -883,25 +931,14 @@ bake_tangent_compose_kernel(const BakeMesh M, const double *frames, const uint32
         if (empty) atomicAdd(empty, 1ull);
         return;
     }
-    const int32_t f = sample_faces[i];
     const uint32_t tex = texels[i];
-    const double *c[3];
-    if (f < 0 || (uint32_t)f >= M.n_faces || tex >= (uint32_t)M.res * (uint32_t)M.res || !bake_corners(M, (uint32_t)f, c))
-        return;
-    V2 t[3];
-    bake_uv(M, c, t);
-    double bc[3];
-    tx_tri_coords(t[0], t[1], t[2], bake_texel_point(M.res, (int)(tex % (uint32_t)M.res), (int)(tex / (uint32_t)M.res)), bc);
-    const double *fr[3];
-#pragma unroll
-    for (int j = 0; j < 3; ++j) fr[j] = frames + (size_t)M.faces[3 * (size_t)f + j] * BAKE_ROW;
-    const D3 n = d3_mix(bc, d3_load(fr[0]), d3_load(fr[1]), d3_load(fr[2]));
-    if (!d3_usable(n)) return;
-    const D3 tm = d3_mix(bc, d3_load(fr[0] + 3), d3_load(fr[1] + 3), d3_load(fr[2] + 3));
-    const D3 N = d3_normalise(n);
+    TexelFrame X;
+    if (!bake_texel_frame(M, frames, tex, sample_faces[i], X)) return;
+    const D3 tm = d3_mix(X.bc, d3_load(X.fr[0] + 3), d3_load(X.fr[1] + 3), d3_load(X.fr[2] + 3));
+    const D3 N = X.N;
     const D3 T = bake_tangent_dir(N, tm);
     const D3 x = d3_cross(N, T);
-    const double w = d3_dot(x, bake_face_frame(c).b) < 0.0 ? -1.0 : 1.0;
+    const double w = d3_dot(x, bake_face_frame(X.c).b) < 0.0 ? -1.0 : 1.0;
     const D3 B = d3_scale(w, x);
     const D3 m = {(double)normal[3 * (size_t)i], (double)normal[3 * (size_t)i + 1], (double)normal[3 * (size_t)i + 2]};
     const float sx = (float)d3_dot(m, T), sy = (float)d3_dot(m, B), sz = (float)d3_dot(m, N);
@@ -948,26 +985,6 @@ __global__ void __launch_bounds__(256) bake_unpack_vertices_kernel(const Raw80t 
 constexpr uint32_t HEIGHT_CHUNK = 1u << 22;
 constexpr uint32_t HEIGHT_NAN = 0x7fc00000u;
 
-// the texel's unit mesh normal, exactly as bake_tangent_compose_kernel computes it; false when the
-// sample is malformed or the mixed normal is not usable
-__device__ __forceinline__ bool bake_texel_normal(const BakeMesh &M, const double *frames, uint32_t tex, int32_t f, D3 &N)
-{
-    const double *c[3];
-    if (f < 0 || (uint32_t)f >= M.n_faces || tex >= (uint32_t)M.res * (uint32_t)M.res || !bake_corners(M, (uint32_t)f, c))
-        return false;
-    V2 t[3];
-    bake_uv(M, c, t);
-    double bc[3];
-    tx_tri_coords(t[0], t[1], t[2], bake_texel_point(M.res, (int)(tex % (uint32_t)M.res), (int)(tex / (uint32_t)M.res)), bc);
-    const double *fr[3];
-#pragma unroll
-    for (int j = 0; j < 3; ++j) fr[j] = frames + (size_t)M.faces[3 * (size_t)f + j] * BAKE_ROW;
-    const D3 n = d3_mix(bc, d3_load(fr[0]), d3_load(fr[1]), d3_load(fr[2]));
-    if (!d3_usable(n)) return false;
-    N = d3_normalise(n);
-    return true;
-}
-
 __device__ __forceinline__ double shfl_d(double v, int src) { return __shfl_sync(0xffffffffu, v, src); }
 
 // A warp takes 32 consecutive samples.  First each lane computes the normal of one of them; then
@@ -989,7 +1006,9 @@ bake_height_kernel(const BakeMesh M, const double *frames, const uint32_t *texel
     bool myOk = false;
     if (base + lane < count) {
         const uint32_t i = base + lane;
-        myOk = bake_texel_normal(M, frames, texels[i], sample_faces[i], myN);
+        TexelFrame X;
+        myOk = bake_texel_frame(M, frames, texels[i], sample_faces[i], X);
+        if (myOk) myN = X.N;
         myX = d3_load(xyz + 3 * (size_t)i);
     }
     const unsigned per_round = 32u / (unsigned)width;
@@ -1122,35 +1141,6 @@ bake_height_encode_kernel(const float *h, size_t n, const double *range, uint16_
     if (word) word[i] = e;
 }
 
-// The texture's 25 x 25 window on words (E + 1 or 0): the 8-bit pair takes byte-wise maxima, which
-// would mix the two bytes of a code.  A texel without a value takes the window's largest code.
-__global__ void __launch_bounds__(256) bake_height_dilate_h_kernel(const uint32_t *word, int res, uint32_t *tmp)
-{
-    const size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
-    if (i >= (size_t)res * res) return;
-    const int y = (int)(i / res), x = (int)(i % res);
-    uint32_t m = 0;
-    for (int dx = -12; dx <= 12; ++dx) {
-        const int xx = x + dx;
-        if (xx >= 0 && xx < res) m = max(m, word[(size_t)y * res + xx]);
-    }
-    tmp[i] = m;
-}
-__global__ void __launch_bounds__(256)
-bake_height_dilate_v_pad_kernel(const uint32_t *word, const uint32_t *tmp, int res, uint16_t *code16)
-{
-    const size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
-    if (i >= (size_t)res * res) return;
-    const int y = (int)(i / res), x = (int)(i % res);
-    uint32_t m = 0;
-    for (int dy = -12; dy <= 12; ++dy) {
-        const int yy = y + dy;
-        if (yy >= 0 && yy < res) m = max(m, tmp[(size_t)yy * res + x]);
-    }
-    const uint32_t t = word[i] ? word[i] : m;
-    code16[i] = (uint16_t)(t ? t - 1u : 0u);
-}
-
 static int bake_height_width(int k)
 {
     int w = 1;
@@ -1203,11 +1193,7 @@ static int bake_height_finish(const float *height, int res, int pad, const doubl
             bake_height_encode_kernel<<<tcdiv(n_pix, 256), 256, 0, s>>>(height, n_pix, range_out, padded ? nullptr : code16,
                                                                         d_word);
             count_launch();
-            if (padded) {
-                bake_height_dilate_h_kernel<<<tcdiv(n_pix, 256), 256, 0, s>>>(d_word, res, d_tmp);
-                bake_height_dilate_v_pad_kernel<<<tcdiv(n_pix, 256), 256, 0, s>>>(d_word, d_tmp, res, code16);
-                count_launch(2);
-            }
+            if (padded) launch_pad_window<PadHeight>(d_word, d_tmp, res, code16, s);
         }
         fail(cudaGetLastError());
     } while (0);
@@ -1300,18 +1286,17 @@ static int texture_bake(pt_index *ix, const void *vertices, size_t n_vertices, c
             bake_height_fill_kernel<<<148 * 8, 256, 0, s>>>(d_height, n_pix);
             count_launch();
         }
+        QueryParams qp{};
+        fill_params(ix, qp);
+        qp.k = k;
+        qp.r2 = radius_to_r2(radius);
         for (size_t c0 = 0; c0 < count; c0 += chunk) {
             const size_t cm = std::min(chunk, count - c0);
             if (heights) {
                 marks.emplace_back();
                 if (fail(cudaEventCreate(&marks.back())) || fail(cudaEventRecord(marks.back(), s))) break;
             }
-            QueryParams qp{};
-            qp.pts = ix->pts; qp.attrs = ix->attrs; qp.attrs_curve = ix->attrs_curve; qp.ids = nullptr; qp.pyr = ix->pyr;
-            qp.n = ix->n; qp.n_leaves = ix->n_leaves; qp.w_levels = ix->w_levels; qp.t_levels = ix->t_levels;
-            qp.pq_cap = opt_queue_cap();
-            qp.queries = d_q + 3 * c0; qp.m = (uint32_t)cm; qp.k = k;
-            qp.r2 = (!(radius >= 0.0) || std::isinf(radius)) ? INFINITY : radius * radius;
+            qp.queries = d_q + 3 * c0; qp.m = (uint32_t)cm;
             qp.rgba_out = d_rgba + 4 * c0; qp.normal_out = d_normal + 3 * c0;
             qp.idx_out = d_idx;
             if ((rc = launch_query(ix, qp, s)) != PT_OK) break;

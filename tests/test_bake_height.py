@@ -1,7 +1,7 @@
 """Height bake (DESIGN.md section 8, "Height bake"): the cloud's signed height above the mesh along the
 interpolated mesh normal, as a float map and a padded 16-bit code map.
 
-CPU part: the oracle (tests/bake_height_oracle.c via tests/bake_height_oracle.py) against an
+CPU part: the oracle (oracle/pt_bake_oracle.c via oracle/pto_bake.py) against an
 independent numpy statement of the frozen definition, the 16-bit padding against a direct 25 x 25
 window, known answers on a flat quad, the exact symmetries, and the CLI's refusals.  GPU part:
 pt_texture_bake_height, the device piece and the CLI must equal the oracle bit for bit; the other
@@ -15,8 +15,7 @@ import zlib
 import numpy as np
 import pytest
 
-import bake_height_oracle as hgo
-import bake_tangent_oracle as tgo
+from oracle import pto_bake
 from test_bake import awkward_mesh, grid_mesh, lattice_case
 from test_bake_tangent import (ALL_OUTPUTS, _bary, _dot, _normalise, _scale, _usable, tilted_normals, turn,
                                turn_case, variant_mesh)
@@ -112,18 +111,18 @@ def cloud_around(pto, V, n, seed, exact_hits=None):
 
 
 def oracle_vs_numpy(pto, P, V, F, k, res, radius=-1.0, frames=None, ranges=((-1.0, 2.0), None, (3.0, 3.0))):
-    texels, xyz, owner = tgo.bake_samples(V, F, res)
+    texels, xyz, owner = pto_bake.bake_samples(V, F, res)
     if frames is None:
-        frames, _ = tgo.bake_frames(V, F)
-    idx, d2 = hgo.neighbours(P, xyz, k, radius)
-    h = hgo.bake_height(V, frames, F, texels, owner, xyz, P, idx, d2, res)
+        frames, _ = pto_bake.bake_frames(V, F)
+    idx, d2 = pto_bake.neighbours(P, xyz, k, radius)
+    h = pto_bake.bake_height(V, frames, F, texels, owner, xyz, P, idx, d2, res)
     assert_heights(h, numpy_height(V, frames, F, texels, owner, xyz, P, idx, d2, res))
     for rng_in in ranges:
-        codes, used, valued = hgo.encode(h, rng_in)
+        codes, used, valued = pto_bake.bake_height_encode(h, rng_in)
         ref_codes, ref_used, ref_valued = numpy_encode(h, rng_in)
         assert np.array_equal(codes, ref_codes) and valued == ref_valued
         assert np.array_equal(np.array(used).view(np.uint64), np.array(ref_used).view(np.uint64))
-        assert np.array_equal(hgo.pad(h, codes), direct_pad(h, codes))
+        assert np.array_equal(pto_bake.bake_height_pad(h, codes), direct_pad(h, codes))
     return h, (texels, owner, xyz), (idx, d2)
 
 
@@ -132,7 +131,7 @@ def oracle_vs_numpy(pto, P, V, F, k, res, radius=-1.0, frames=None, ranges=((-1.
 @pytest.mark.parametrize("seed,res,k", [(1, 40, 6), (2, 57, 1), (3, 64, 32)])
 def test_oracle_equals_numpy_definition(pto, variant, seed, res, k):
     V, F = variant_mesh(pto, seed, variant)
-    texels, xyz, _ = tgo.bake_samples(V, F, res)
+    texels, xyz, _ = pto_bake.bake_samples(V, F, res)
     P = cloud_around(pto, V, 3000, seed, exact_hits=xyz[::7])
     h, _, (idx, d2) = oracle_vs_numpy(pto, P, V, F, k, res)
     assert (d2[:, 0] == 0).any() and np.isfinite(h).sum() > len(texels) // 2
@@ -144,12 +143,12 @@ def test_oracle_equals_numpy_definition(pto, variant, seed, res, k):
 
 def test_oracle_unusable_normals_and_degenerate_frames(pto):
     V, F = awkward_mesh(pto, 4)
-    frames, _ = tgo.bake_frames(V, F)
+    frames, _ = pto_bake.bake_frames(V, F)
     frames = frames.copy()
     frames[::3, 0:3] = 0.0                                        # zero normals
     frames[1::5, 0:3] = np.nan                                    # NaN normals
     res = 48
-    texels, xyz, _ = tgo.bake_samples(V, F, res)
+    texels, xyz, _ = pto_bake.bake_samples(V, F, res)
     P = cloud_around(pto, V, 2000, 4)
     h, _, _ = oracle_vs_numpy(pto, P, V, F, 5, res, frames=frames)
     assert np.isnan(h.reshape(-1)[texels]).any() and np.isfinite(h).any()
@@ -166,9 +165,9 @@ def test_oracle_no_value_at_all(pto):
     P, V, F, res = lattice_case(pto, res=32)
     h, _, _ = oracle_vs_numpy(pto, P, V, F, 4, res, radius=1e-6)
     assert np.isnan(h).all()
-    codes, used, valued = hgo.encode(h)
+    codes, used, valued = pto_bake.bake_height_encode(h)
     assert used == (0.0, 0.0) and valued == 0 and not codes.any()
-    assert not hgo.pad(h, codes).any()
+    assert not pto_bake.bake_height_pad(h, codes).any()
 
 
 def test_pad_equals_direct_window(pto):
@@ -177,8 +176,8 @@ def test_pad_equals_direct_window(pto):
     h = rng.normal(0, 3, (res, res)).astype(np.float32)
     h[rng.random((res, res)) < 0.7] = np.nan
     h[40:75, 10:60] = np.nan                                      # a hole wider than the window
-    codes, _, _ = hgo.encode(h)
-    padded = hgo.pad(h, codes)
+    codes, _, _ = pto_bake.bake_height_encode(h)
+    padded = pto_bake.bake_height_pad(h, codes)
     assert np.array_equal(padded, direct_pad(h, codes))
     assert (padded[~np.isnan(h)] == codes[~np.isnan(h)]).all() and (padded[55:60, 30:40] == 0).all()
 
@@ -199,7 +198,7 @@ def flat_quad(pto, z, normal=(0.0, 0.0, 1.0)):
 def test_known_answers_flat_quad(pto, z):
     P, V, F = flat_quad(pto, z)
     res = 40
-    out = hgo.bake(P, V, F, 6, res, pad_codes=False, height_range=(-2.0, 0.25))
+    out = pto_bake.bake_heights(P, V, F, 6, res, pad_codes=False, height_range=(-2.0, 0.25))
     texels = out["samples"][0]
     h = out["height"].reshape(-1)
     assert out["texels"] == len(texels) > res * res // 2
@@ -209,14 +208,14 @@ def test_known_answers_flat_quad(pto, z):
     assert (h[uncovered].view(np.uint32) == NAN_BITS).all()
     assert (out["height_u16"].reshape(-1)[texels] == (65535 if z > 0 else 0)).all()
     assert not out["height_u16"].reshape(-1)[uncovered].any()
-    auto = hgo.bake(P, V, F, 6, res)                              # automatic range (z, z): every code 0
+    auto = pto_bake.bake_heights(P, V, F, 6, res)                 # automatic range (z, z): every code 0
     assert auto["height_range"] == (z, z) and not auto["height_u16"].any()
 
 
 def test_quarter_turn_invariance(pto):
     P, V, F = turn_case(pto)
-    a = hgo.bake(P, V, F, 8, 96)
-    b = hgo.bake(turn(P), turn(V), F, 8, 96)
+    a = pto_bake.bake_heights(P, V, F, 8, 96)
+    b = pto_bake.bake_heights(turn(P), turn(V), F, 8, 96)
     assert_heights(a["height"], b["height"])
     assert np.array_equal(a["height_u16"], b["height_u16"]) and a["height_range"] == b["height_range"]
     assert a["texels"] > 96 * 96 // 2
@@ -227,7 +226,7 @@ def test_negated_normals_negate_heights(pto):
     Vn = V.copy()
     Vn["normal"] = -V["normal"]
     assert _usable(V["normal"].astype(np.float64)).all()
-    a, b = hgo.bake(P, V, F, 8, 96)["height"], hgo.bake(P, Vn, F, 8, 96)["height"]
+    a, b = pto_bake.bake_heights(P, V, F, 8, 96)["height"], pto_bake.bake_heights(P, Vn, F, 8, 96)["height"]
     has = ~np.isnan(a)
     assert np.array_equal(has, ~np.isnan(b)) and has.sum() > 96 * 96 // 2
     assert np.array_equal(np.negative(a[has]).view(np.uint32), b[has].view(np.uint32))
@@ -269,7 +268,7 @@ def _need_gpu():
 def check_height(pkg, pto, P, V, F, k, res, pad=True, radius=None, coord_mode=0, height_range=None):
     with pkg.Tree(P, coord_mode=coord_mode) as tree:
         got = tree.bake(V, F, k=k, resolution=res, radius=radius, pad=pad, want=HEIGHTS, height_range=height_range)
-    ref = hgo.bake(P, V, F, k, res, radius=-1.0 if radius is None else radius, pad_codes=pad,
+    ref = pto_bake.bake_heights(P, V, F, k, res, radius=-1.0 if radius is None else radius, pad_codes=pad,
                    height_range=height_range)
     assert_heights(got["height"], ref["height"])
     assert np.array_equal(got["height_u16"], ref["height_u16"])
@@ -345,15 +344,15 @@ def test_gpu_bake_height_two_chunks(pkg, pto):
     with pkg.Tree(P) as tree:
         got = tree.bake(V, F, k=k, resolution=res, pad=False, want=HEIGHTS)
     assert got["stats"]["texels"] == res * res > 2 * 2**22
-    texels, xyz, owner = tgo.bake_samples(V, F, res)
+    texels, xyz, owner = pto_bake.bake_samples(V, F, res)
     pick = np.sort(np.random.default_rng(11).choice(len(texels), 50_000, replace=False))
-    frames, _ = tgo.bake_frames(V, F)
-    idx, d2 = hgo.neighbours(P, xyz[pick], k)
-    ref = hgo.bake_height(V, frames, F, texels[pick], owner[pick], xyz[pick], P, idx, d2, res)
+    frames, _ = pto_bake.bake_frames(V, F)
+    idx, d2 = pto_bake.neighbours(P, xyz[pick], k)
+    ref = pto_bake.bake_height(V, frames, F, texels[pick], owner[pick], xyz[pick], P, idx, d2, res)
     assert np.array_equal(got["height"].reshape(-1)[texels[pick]].view(np.uint32),
                           ref.reshape(-1)[texels[pick]].view(np.uint32))
     h = got["height"]
-    codes, used, valued = hgo.encode(h)
+    codes, used, valued = pto_bake.bake_height_encode(h)
     assert used == got["height_range"] == (float(np.nanmin(h)), float(np.nanmax(h)))
     assert valued == got["stats"]["height_texels"] == res * res
     assert np.array_equal(codes, got["height_u16"])
@@ -474,7 +473,7 @@ def test_gpu_cli_height_bake(pkg, pto, tmp_path):
     assert r.returncode == 0, r.stderr
     Vm = V.copy()
     Vm["normal"] = [0, 0, 1]
-    ref = hgo.bake(P, Vm, F, 20, 256)
+    ref = pto_bake.bake_heights(P, Vm, F, 20, 256)
     assert np.array_equal(read_png_gray16(tmp_path / "height.png"), ref["height_u16"])
     line = next(ln for ln in r.stdout.splitlines() if ln.startswith("Height range:"))
     assert line == "Height range: %.9g %.9g" % ref["height_range"]

@@ -1,7 +1,7 @@
 """Tangent-space bake (DESIGN.md section 8, "Tangent-space bake"): tangent-space normal maps and the
 per-vertex tangents they are expressed in.
 
-CPU part: the oracle (tests/bake_tangent_oracle.c via tests/bake_tangent_oracle.py) against an independent numpy
+CPU part: the oracle (oracle/pt_bake_oracle.c via oracle/pto_bake.py) against an independent numpy
 statement of the frozen definition, known answers on a flat quad, the exact invariance under a
 quarter turn about z, and the CLI's refusals.  GPU part: pt_texture_bake_ex, the device pieces and
 the CLI must equal the oracle bit for bit."""
@@ -12,7 +12,6 @@ import subprocess
 import numpy as np
 import pytest
 
-import bake_tangent_oracle as tgo
 from oracle import pto_bake
 from test_bake import awkward_mesh, grid_mesh, lattice_case
 from test_cli import read_png_bgra, write_cloud, write_mesh
@@ -203,15 +202,15 @@ VARIANTS = ("zero", "random", "nan", "mirrored", "coincident")
 @pytest.mark.parametrize("seed,res", [(1, 40), (2, 57), (3, 64)])
 def test_oracle_equals_numpy_definition(pto, variant, seed, res):
     V, F = variant_mesh(pto, seed, variant)
-    frames, tangents = tgo.bake_frames(V, F)
+    frames, tangents = pto_bake.bake_frames(V, F)
     ref_frames, ref_tangents = numpy_frames(V, F)
     assert_same(frames, ref_frames, "frames")
     assert_same(tangents, ref_tangents, "tangents")
-    texels, _, owner = tgo.bake_samples(V, F, res)
+    texels, _, owner = pto_bake.bake_samples(V, F, res)
     ref_t, ref_owner = numpy_owner(V, F, res)
     assert np.array_equal(texels, ref_t) and np.array_equal(owner, ref_owner)
     rgba, m = sample_blend(np.random.default_rng(seed), len(texels))
-    tb, tn = tgo.bake_compose_tangent(V, frames, F, texels, owner, rgba, m, res, pad=False)
+    tb, tn = pto_bake.bake_compose_tangent(V, frames, F, texels, owner, rgba, m, res, pad=False)
     ref_tb, ref_tn = numpy_compose_tangent(V, ref_frames, F, texels, owner, rgba, m, res)
     assert_same(tb, ref_tb, "tangent_bgra")
     assert_same(tn, ref_tn, "tangent_normal")
@@ -253,7 +252,7 @@ def test_known_answers_flat_quad(pto, case):
     uv_map, expect, tangent = KNOWN[case]
     P, V, F = flat_quad_case(pto, uv_map)
     res = 48
-    out = tgo.bake_tangent(P, V, F, 4, res, pad=False)
+    out = pto_bake.bake_tangent(P, V, F, 4, res, pad=False)
     assert np.array_equal(out["tangents"], np.tile(np.float32(tangent), (4, 1)))
     texels, m = out["samples"][0], out["m"]
     assert out["texels"] == len(texels) > res * res // 2 and out["empty"] == 0
@@ -298,8 +297,8 @@ def turn_case(pto, n_points=6000, g=9):
 
 def test_quarter_turn_invariance(pto):
     P, V, F = turn_case(pto)
-    a = tgo.bake_tangent(P, V, F, 8, 96)
-    b = tgo.bake_tangent(turn(P), turn(V), F, 8, 96)
+    a = pto_bake.bake_tangent(P, V, F, 8, 96)
+    b = pto_bake.bake_tangent(turn(P), turn(V), F, 8, 96)
     # no vertex and no texel took the fallback: every T is the projection of the summed T_f
     T_f, _, _, _ = numpy_face_frames(V, F)
     assert _usable(T_f).all()
@@ -348,7 +347,7 @@ def _need_gpu():
 def check_bake_ex(pkg, pto, P, V, F, k, res, pad=True, radius=None, coord_mode=0):
     with pkg.Tree(P, coord_mode=coord_mode) as tree:
         got = tree.bake(V, F, k=k, resolution=res, radius=radius, pad=pad, want=ALL_OUTPUTS)
-    ref = tgo.bake_tangent(P, V, F, k, res, radius=-1.0 if radius is None else radius, pad=pad)
+    ref = pto_bake.bake_tangent(P, V, F, k, res, radius=-1.0 if radius is None else radius, pad=pad)
     assert (got["stats"]["texels"], got["stats"]["empty"]) == (ref["texels"], ref["empty"])
     for key in ALL_OUTPUTS:
         assert_same(got[key], ref[key], key)
@@ -430,7 +429,7 @@ def test_gpu_bake_ex_tangent_outputs_alone(pkg, pto):
     P, V, F, res = lattice_case(pto, res=128)
     V = V.copy()
     V["normal"] = tilted_normals(np.random.default_rng(4), len(V))
-    ref = tgo.bake_tangent(P, V, F, 8, res, radius=0.3)
+    ref = pto_bake.bake_tangent(P, V, F, 8, res, radius=0.3)
     with pkg.Tree(P) as tree:
         got = tree.bake(V, F, k=8, resolution=res, radius=0.3, want=("tangent_bgra", "tangent_normal"))
         only = tree.bake(V, F, k=8, resolution=res, want=("tangents",))
@@ -456,11 +455,11 @@ def test_gpu_bake_tangent_device_pieces(pkg, pto):
     texels, xyz, owner = pkg.bake_samples_device(xyzuv, faces, res)
     texels0, xyz0 = pkg.bake_texels_device(xyzuv, faces, res)
     assert torch.equal(texels, texels0) and torch.equal(xyz.view(torch.int64), xyz0.view(torch.int64))
-    ref_t, ref_xyz, ref_owner = tgo.bake_samples(V, F, res)
+    ref_t, ref_xyz, ref_owner = pto_bake.bake_samples(V, F, res)
     assert np.array_equal(texels.cpu().numpy().astype(np.uint32), ref_t)
     assert np.array_equal(owner.cpu().numpy(), ref_owner)
     frames, tangents = pkg.bake_frames_device(xyzuvn, faces)
-    ref_frames, ref_tangents = tgo.bake_frames(V, F)
+    ref_frames, ref_tangents = pto_bake.bake_frames(V, F)
     assert_same(frames.cpu().numpy(), ref_frames, "frames")
     assert_same(tangents.cpu().numpy(), ref_tangents, "tangents")
     pos = torch.from_numpy(np.c_[P["ver"], np.zeros(len(P))].astype(np.float32)).cuda()
@@ -564,7 +563,7 @@ def test_gpu_cli_tangent_bake(pkg, pto, tmp_path):
     Vm = V.copy()
     Vm["normal"] = [0, 0, 1]
     Vm["color"] = np.array([10, 20, 30])                  # what write_mesh put in the file
-    ref = tgo.bake_tangent(P, Vm, F, 20, 256)
+    ref = pto_bake.bake_tangent(P, Vm, F, 20, 256)
     assert np.array_equal(read_png_bgra(tmp_path / "tangent.png"), ref["tangent_bgra"])
     rows, tangents = read_tangent_ply(tmp_path / "tangents.ply")
     assert np.array_equal(tangents, ref["tangents"])
