@@ -52,7 +52,7 @@ ABI_SYMBOLS = (
     "pt_sharded_transfer", "pt_texture_render_lists", "pt_set_option", "pt_get_option", "pt_debug_stats", "pt_debug_stats_n", "pt_kernel_launch_count",
     "pt_texture_bake", "pt_bake_texels_device", "pt_bake_compose_device",
     "pt_texture_bake_ex", "pt_bake_samples_device", "pt_bake_frames_device", "pt_bake_compose_tangent_device",
-    "pt_texture_bake_height", "pt_bake_compose_height_device",
+    "pt_texture_bake_height", "pt_bake_compose_height_device", "pt_sharded_bake",
 )
 # ... and include/pt_synth.h (bench / test scaffolding, its own library)
 SYNTH_SYMBOLS = ("pt_synth_cloud_device", "pt_synth_samples_device", "pt_synth_pack_points_device",
@@ -205,6 +205,9 @@ def lib():
     L.pt_texture_bake_height.restype = i32
     L.pt_texture_bake_height.argtypes = [vp, vp, sz, vp, sz, i32, dbl, i32, i32, ctypes.POINTER(BakeOutputs),
                                          ctypes.POINTER(BakeHeight), ctypes.POINTER(BakeStats)]
+    L.pt_sharded_bake.restype = i32
+    L.pt_sharded_bake.argtypes = [vp, vp, sz, vp, sz, i32, dbl, i32, i32, ctypes.POINTER(BakeOutputs),
+                                  ctypes.POINTER(BakeHeight), ctypes.POINTER(BakeStats)]
     L.pt_bake_compose_height_device.restype = i32
     L.pt_bake_compose_height_device.argtypes = [vp, vp, sz, vp, sz, vp, vp, vp, sz, vp, i32, vp, sz, i32, i32, vp, vp,
                                                 vp, vp, i32, vp]
@@ -438,9 +441,6 @@ class Tree:
         return img, {"triangles": int(st.triangles), "inside_points": int(st.inside_points),
                      "knn_ms": st.knn_ms, "draw_ms": st.draw_ms, "pad_ms": st.pad_ms}
 
-    _BAKE_OUTPUTS = ("bgra", "normal_bgra", "normal", "tangent_bgra", "tangent_normal", "tangents")
-    _HEIGHT_OUTPUTS = ("height", "height_u16")
-
     def bake(self, vertices, faces, k=20, resolution=2048, radius=None, pad=True,
              want=("bgra", "normal_bgra", "normal"), height_range=None):
         """Per-texel bake (DESIGN.md section 8): colour and normal maps of the cloud on the mesh's
@@ -457,35 +457,8 @@ class Tree:
         (texels, empty, raster_ms, knn_ms, pad_ms).  With a height output the result also carries
         ``height_range`` (the (lo, hi) used) and ``stats["height_texels"]`` (texels with a value).
         All outputs come from one k-NN pass."""
-        v = _as_points(vertices, "vertices")
-        f = np.ascontiguousarray(faces, dtype=np.int32).reshape(-1, 3)
-        names = self._BAKE_OUTPUTS + self._HEIGHT_OUTPUTS
-        unknown = set(want) - set(names)
-        if unknown or not want:
-            raise ValueError(f"want must name some of {', '.join(names)} (got {want!r})")
-        res = int(resolution)
-        shapes = {"bgra": ((res, res, 4), np.uint8), "normal_bgra": ((res, res, 4), np.uint8),
-                  "normal": ((res, res, 3), np.float32), "tangent_bgra": ((res, res, 4), np.uint8),
-                  "tangent_normal": ((res, res, 3), np.float32), "tangents": ((v.shape[0], 4), np.float32),
-                  "height": ((res, res), np.float32), "height_u16": ((res, res), np.uint16)}
-        out = {name: np.empty(*shapes[name]) for name in names if name in want}
-        o = BakeOutputs(*[out[name].ctypes.data if name in out else None for name in self._BAKE_OUTPUTS])
-        hb = None
-        if any(name in out for name in self._HEIGHT_OUTPUTS):
-            lo, hi = (float("nan"), float("nan")) if height_range is None else map(float, height_range)
-            hb = BakeHeight(*[out[name].ctypes.data if name in out else None for name in self._HEIGHT_OUTPUTS],
-                            (ctypes.c_double * 2)(lo, hi))
-        st = BakeStats()
-        _check(lib().pt_texture_bake_height(self._h, _np_ptr(v), v.shape[0], _np_ptr(f), f.shape[0], int(k),
-                                            _radius(radius), res, 1 if pad else 0, ctypes.byref(o),
-                                            None if hb is None else ctypes.byref(hb), ctypes.byref(st)),
-               "pt_texture_bake_height")
-        out["stats"] = {"texels": int(st.texels), "empty": int(st.empty), "raster_ms": st.raster_ms,
-                        "knn_ms": st.knn_ms, "pad_ms": st.pad_ms}
-        if hb is not None:
-            out["height_range"] = (hb.range_used[0], hb.range_used[1])
-            out["stats"]["height_texels"] = int(hb.texels)
-        return out
+        return _bake(lib().pt_texture_bake_height, "pt_texture_bake_height", self._h, vertices, faces, k, resolution,
+                     radius, pad, want, height_range)
 
     def transfer_slab(self, queries_ptr, queries_are_xyz, m, k, radius, boxes6, rank, halo,
                       idx_ptr, rgba_ptr, normal_ptr, d2_ptr=None):
@@ -499,6 +472,42 @@ class Tree:
                                       int(rank), float(halo), idx_ptr, d2_ptr, rgba_ptr,
                                       normal_ptr, ctypes.byref(need)), "pt_transfer_slab")
         return need.value == 0
+
+
+_BAKE_OUTPUTS = ("bgra", "normal_bgra", "normal", "tangent_bgra", "tangent_normal", "tangents")
+_HEIGHT_OUTPUTS = ("height", "height_u16")
+
+
+def _bake(fn, name, handle, vertices, faces, k, resolution, radius, pad, want, height_range):
+    """Arguments, output arrays and result dict of ``Tree.bake`` and ``ShardedTree.bake``: ``fn`` is
+    ``pt_texture_bake_height`` or ``pt_sharded_bake``, which take the same arguments after the handle."""
+    v = _as_points(vertices, "vertices")
+    f = np.ascontiguousarray(faces, dtype=np.int32).reshape(-1, 3)
+    names = _BAKE_OUTPUTS + _HEIGHT_OUTPUTS
+    unknown = set(want) - set(names)
+    if unknown or not want:
+        raise ValueError(f"want must name some of {', '.join(names)} (got {want!r})")
+    res = int(resolution)
+    shapes = {"bgra": ((res, res, 4), np.uint8), "normal_bgra": ((res, res, 4), np.uint8),
+              "normal": ((res, res, 3), np.float32), "tangent_bgra": ((res, res, 4), np.uint8),
+              "tangent_normal": ((res, res, 3), np.float32), "tangents": ((v.shape[0], 4), np.float32),
+              "height": ((res, res), np.float32), "height_u16": ((res, res), np.uint16)}
+    out = {n: np.empty(*shapes[n]) for n in names if n in want}
+    o = BakeOutputs(*[out[n].ctypes.data if n in out else None for n in _BAKE_OUTPUTS])
+    hb = None
+    if any(n in out for n in _HEIGHT_OUTPUTS):
+        lo, hi = (float("nan"), float("nan")) if height_range is None else map(float, height_range)
+        hb = BakeHeight(*[out[n].ctypes.data if n in out else None for n in _HEIGHT_OUTPUTS],
+                        (ctypes.c_double * 2)(lo, hi))
+    st = BakeStats()
+    _check(fn(handle, _np_ptr(v), v.shape[0], _np_ptr(f), f.shape[0], int(k), _radius(radius), res, 1 if pad else 0,
+              ctypes.byref(o), None if hb is None else ctypes.byref(hb), ctypes.byref(st)), name)
+    out["stats"] = {"texels": int(st.texels), "empty": int(st.empty), "raster_ms": st.raster_ms,
+                    "knn_ms": st.knn_ms, "pad_ms": st.pad_ms}
+    if hb is not None:
+        out["height_range"] = (hb.range_used[0], hb.range_used[1])
+        out["stats"]["height_texels"] = int(hb.texels)
+    return out
 
 
 class ShardedTree:
@@ -542,6 +551,15 @@ class ShardedTree:
                                          _np_ptr(out.get("d2")), _np_ptr(out["rgba"]), _np_ptr(out["normal"])),
                "pt_sharded_transfer")
         return out
+
+    def bake(self, vertices, faces, k=20, resolution=2048, radius=None, pad=True,
+             want=("bgra", "normal_bgra", "normal"), height_range=None):
+        """``Tree.bake`` on the sharded cloud (``pt_sharded_bake``): same arguments and result, every
+        output byte-identical to ``Tree.bake`` on one index of the same cloud.  The raster, frames and
+        composition run on slab 0's device and each slab answers the texels in its x-range on its
+        own device; ``stats["knn_ms"]`` is the host wall time of that part."""
+        return _bake(lib().pt_sharded_bake, "pt_sharded_bake", self._h, vertices, faces, k, resolution, radius, pad,
+                     want, height_range)
 
     def close(self):
         if getattr(self, "_h", None) and self._h.value:

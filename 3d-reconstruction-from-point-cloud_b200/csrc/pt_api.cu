@@ -92,6 +92,8 @@ static std::atomic<int> g_queue_cap{1 << 20};   // tests: shrink the per-sample 
 int opt_queue_cap() { return g_queue_cap.load(); }
 static std::atomic<int> g_smem_pad{0};   // diagnosis: extra dynamic smem per query block (occupancy probe)
 int opt_smem_pad() { return g_smem_pad.load(); }
+static std::atomic<int> g_sharded_copy{0};   // tests: the sharded bake copies the rows of slabs on its home device too
+int opt_sharded_copy() { return g_sharded_copy.load(); }
 
 int set_option(const char *name, int value)
 {
@@ -118,6 +120,7 @@ int set_option(const char *name, int value)
     if (!strcmp(name, "smem_pad")) { g_smem_pad.store(value < 0 ? 0 : value); return PT_OK; }
     if (!strcmp(name, "queue_cap")) { g_queue_cap.store(value < 2 ? 2 : value); return PT_OK; }
     if (!strcmp(name, "host_chunks")) { g_host_chunks.store(value < 1 ? 1 : (value > 64 ? 64 : value)); return PT_OK; }
+    if (!strcmp(name, "sharded_copy")) { g_sharded_copy.store(value ? 1 : 0); return PT_OK; }
     if (!strcmp(name, "verbose")) { g_verbose.store(value ? 1 : 0); return PT_OK; }
     return PT_ERR_INVALID_ARG;
 }
@@ -145,6 +148,7 @@ int get_option(const char *name, int *value)
     if (!strcmp(name, "smem_pad")) { *value = g_smem_pad.load(); return PT_OK; }
     if (!strcmp(name, "queue_cap")) { *value = g_queue_cap.load(); return PT_OK; }
     if (!strcmp(name, "host_chunks")) { *value = g_host_chunks.load(); return PT_OK; }
+    if (!strcmp(name, "sharded_copy")) { *value = g_sharded_copy.load(); return PT_OK; }
     if (!strcmp(name, "verbose")) { *value = verbose() ? 1 : 0; return PT_OK; }
     return PT_ERR_INVALID_ARG;
 }

@@ -133,6 +133,7 @@ int  opt_grid_tma();
 int  opt_grid_pair();
 int  opt_grid_span();
 int  opt_chain_pdl();
+int  opt_sharded_copy();
 int  opt_grid_claim();
 int  opt_grid_min_occ10();
 int  opt_grid_admit100();

@@ -13,12 +13,18 @@
 //             zone towards another slab (exactness argument: DESIGN.md section 6).  If some
 //             slab reports needs_exchange the halo is widened (x4, at least the bounding-box estimate), the slabs are rebuilt and the
 //             call is repeated, so the result is always exact; `rebuilds` counts that.
+//   bake    : the per-texel bake of pt_texture_bake_height on the sharded cloud (DESIGN.md section
+//             8, "Sharded bake"): raster, frames, composition and padding on slab 0's device (the
+//             home device, pt_bake.cuh pieces); the samples are partitioned by slab there, each
+//             slab answers its rows on its own device (k-NN + blend + ghost check + heights from
+//             its own records) and the results are scattered back into sample order.
 //
 // The reference has no multi-GPU path (its query loop is src/pointsTransfer.cpp:465-479); the
 // torch.distributed / NCCL form of the same sharding (one process per GPU, unsorted samples
 // routed over all_to_all) is sharded.py.  Devices may repeat in the device list: several slabs
 // then share one GPU, which is how the single-GPU test box exercises this file.
 #include <algorithm>
+#include <chrono>
 #include <cmath>
 #include <cstring>
 #include <new>
@@ -26,6 +32,7 @@
 #include <vector>
 
 #include "points_transfer.h"
+#include "pt_bake.cuh"
 
 namespace {
 
@@ -207,6 +214,226 @@ int sharded_query(pt_sharded *S, const void *queries, size_t m, int k, double ra
     return PT_ERR_UNSUPPORTED;
 }
 
+// Sample rows in slab order on the home device (struct of arrays, so a slab's rows are one range
+// of each), or one slab's rows on its own device.
+struct BakeRows {
+    double *xyz = nullptr;
+    uint32_t *texel = nullptr;
+    int32_t *face = nullptr;      // heights only
+    uint8_t *rgba = nullptr;
+    float *normal = nullptr;
+    float *height = nullptr;      // heights only
+    double *mesh = nullptr;       // heights on another device: mesh rows | frames (n_vertices x 8 each)
+    int32_t *faces = nullptr;     //   and faces
+};
+
+// Buffers that a peer copy reads or writes are cudaMalloc memory (`peer`: dev_alloc), since the
+// library's memory pools grant no access to other devices; the others come from the pool on s.
+int rows_alloc(BakeRows &B, size_t m, bool heights, size_t mesh_rows, size_t n_faces, bool peer, cudaStream_t s)
+{
+    auto dev_alloc = [&](void **p, size_t bytes) { return peer ? pt::dev_alloc(p, bytes) : pt::pool_alloc(p, bytes, s); };
+    if (dev_alloc((void **)&B.xyz, sizeof(double) * 3 * m) || dev_alloc((void **)&B.texel, sizeof(uint32_t) * m) ||
+        dev_alloc((void **)&B.rgba, 4 * m) || dev_alloc((void **)&B.normal, sizeof(float) * 3 * m) ||
+        (heights && (dev_alloc((void **)&B.face, sizeof(int32_t) * m) || dev_alloc((void **)&B.height, sizeof(float) * m))) ||
+        (mesh_rows && (dev_alloc((void **)&B.mesh, sizeof(double) * 2 * pt::BAKE_ROW * mesh_rows) ||
+                       dev_alloc((void **)&B.faces, sizeof(int32_t) * 3 * n_faces))))
+        return PT_ERR_OUT_OF_MEMORY;
+    return PT_OK;
+}
+
+void rows_free(BakeRows &B, bool peer, cudaStream_t s)
+{
+    void *frees[] = {B.xyz, B.texel, B.face, B.rgba, B.normal, B.height, B.mesh, B.faces};
+    for (void *p : frees) {
+        if (peer) pt::dev_free(p);
+        else pt::pool_free(p, s);
+    }
+    B = BakeRows{};
+}
+
+// One slab's step 3 of the bake, on the slab's own stream and host thread: its rows (home device,
+// from row `first`) to its device, k-NN + blend + ghost check + heights there, the per-row results
+// back into the home rows.  `copy`: the slab works on copies of its rows (it is on another device,
+// or the test option asks for it), else on the home rows in place.  *needs = 1 when the ghost check
+// flags the step.
+int slab_bake(pt_sharded *S, int r, int home, const pt::BakeJob &J, const BakeRows &rows, size_t first, size_t m,
+              bool copy, int k, double radius, int *needs)
+{
+    using namespace pt;
+    const Slab &sl = S->slabs[r];
+    pt_index *ix = sl.index;
+    if (!ix) return PT_ERR_INVALID_ARG;
+    PT_CUDA(cudaSetDevice(sl.device));
+    cudaStream_t s = ix->stream;
+    const bool heights = J.heights;
+    const size_t R = S->slabs.size(), nv = J.n_vertices, nf = J.M.n_faces;
+    BakeRows d, mine;
+    double *boxes = nullptr;
+    uint32_t *flag = nullptr;
+    uint32_t h_flag = 0;
+    int rc = PT_OK;
+    auto fail = [&](cudaError_t e) { if (e != cudaSuccess && rc == PT_OK) rc = map_cuda_error(e); return e != cudaSuccess; };
+    auto put = [&](void *dst, int dst_dev, const void *src, int src_dev, size_t bytes) {
+        return fail(dst_dev == src_dev ? cudaMemcpyAsync(dst, src, bytes, cudaMemcpyDeviceToDevice, s)
+                                       : cudaMemcpyPeerAsync(dst, dst_dev, src, src_dev, bytes, s));
+    };
+    do {
+        if (pool_alloc((void **)&boxes, sizeof(double) * 6 * R, s) || pool_alloc((void **)&flag, sizeof(uint32_t), s)) {
+            rc = PT_ERR_OUT_OF_MEMORY;
+            break;
+        }
+        if (!copy) {
+            d.xyz = rows.xyz + 3 * first; d.texel = rows.texel + first; d.rgba = rows.rgba + 4 * first;
+            d.normal = rows.normal + 3 * first;
+            if (heights) { d.face = rows.face + first; d.height = rows.height + first; }
+        } else {
+            if ((rc = rows_alloc(mine, m, heights, heights ? nv : 0, nf, true, s)) != PT_OK) break;
+            d = mine;
+            const int dv = sl.device;
+            if (put(d.xyz, dv, rows.xyz + 3 * first, home, sizeof(double) * 3 * m) ||
+                put(d.texel, dv, rows.texel + first, home, sizeof(uint32_t) * m))
+                break;
+            if (heights && (put(d.face, dv, rows.face + first, home, sizeof(int32_t) * m) ||
+                            put(d.mesh, dv, rows.mesh, home, sizeof(double) * 2 * BAKE_ROW * nv) ||
+                            put(d.faces, dv, rows.faces, home, sizeof(int32_t) * 3 * nf)))
+                break;
+        }
+        if (fail(cudaMemcpyAsync(boxes, S->boxes.data(), sizeof(double) * 6 * R, cudaMemcpyHostToDevice, s)) ||
+            fail(cudaMemsetAsync(flag, 0, sizeof(uint32_t), s)))
+            break;
+        // a slab whose index holds the whole cloud answers every sample exactly: no check
+        const bool whole = sl.n_own + sl.n_ghost == S->n;
+        const BakeGhost ghost{boxes, (int)R, r, S->halo, flag};
+        const BakeMesh M = copy ? BakeMesh{d.mesh, BAKE_ROW, (uint32_t)nv, d.faces, (uint32_t)nf, J.res} : J.M;
+        const double *frames = copy ? d.mesh + BAKE_ROW * nv : J.d_frames;
+        if ((rc = bake_answer_rows(ix, M, frames, d.xyz, d.texel, d.face, m, k, radius, whole ? nullptr : &ghost, d.rgba,
+                                   d.normal, d.height, true, nullptr, s)) != PT_OK)
+            break;
+        if (copy && (put(rows.rgba + 4 * first, home, d.rgba, sl.device, 4 * m) ||
+                     put(rows.normal + 3 * first, home, d.normal, sl.device, sizeof(float) * 3 * m) ||
+                     (heights && put(rows.height + first, home, d.height, sl.device, sizeof(float) * m))))
+            break;
+        if (fail(cudaMemcpyAsync(&h_flag, flag, sizeof h_flag, cudaMemcpyDeviceToHost, s))) break;
+        if (fail(cudaStreamSynchronize(s))) break;
+        *needs = whole ? 0 : (h_flag ? 1 : 0);
+    } while (0);
+    cudaStreamSynchronize(s);
+    pool_free(boxes, s);
+    pool_free(flag, s);
+    cudaStreamSynchronize(s);
+    rows_free(mine, true, s);
+    return rc;
+}
+
+// Steps 2-4 of the sharded bake: route the samples, answer them slab by slab until no ghost zone is
+// too narrow (widening the halo and rebuilding as sharded_query does), scatter the results into
+// J's sample order.  On the home device, current on entry.
+int sharded_answer(pt_sharded *S, int home, pt::BakeJob &J, int k, double radius)
+{
+    using namespace pt;
+    const int R = (int)S->slabs.size();
+    const size_t count = J.count, nv = J.n_vertices, nf = J.M.n_faces;
+    cudaStream_t s = J.s;
+    std::vector<char> copy(R, 0);
+    bool any_copy = false;
+    for (int r = 0; r < R; ++r) {
+        copy[r] = S->slabs[r].device != home || opt_sharded_copy();
+        any_copy |= copy[r] != 0;
+    }
+    BakeRows rows;
+    int32_t *sel = nullptr;
+    std::vector<size_t> starts(R + 1, 0);
+    int rc = PT_OK;
+    auto fail = [&](cudaError_t e) { if (e != cudaSuccess && rc == PT_OK) rc = map_cuda_error(e); return e != cudaSuccess; };
+    do {
+        const bool mesh = any_copy && J.heights;
+        if (pool_alloc((void **)&sel, sizeof(int32_t) * count, s) ||
+            (rc = rows_alloc(rows, count, J.heights, mesh ? nv : 0, nf, any_copy, s)) != PT_OK) {
+            rc = PT_ERR_OUT_OF_MEMORY;
+            break;
+        }
+        // the height kernel of a slab on another device reads the mesh rows, frames and faces there
+        if (mesh && (fail(cudaMemcpyAsync(rows.mesh, J.d_rows, sizeof(double) * BAKE_ROW * nv, cudaMemcpyDeviceToDevice, s)) ||
+                     fail(cudaMemcpyAsync(rows.mesh + BAKE_ROW * nv, J.d_frames, sizeof(double) * BAKE_ROW * nv,
+                                          cudaMemcpyDeviceToDevice, s)) ||
+                     fail(cudaMemcpyAsync(rows.faces, J.d_faces, sizeof(int32_t) * 3 * nf, cudaMemcpyDeviceToDevice, s))))
+            break;
+        // samples with a NaN component are routed nowhere: their lists are empty (alpha 0, no height)
+        if (fail(cudaMemsetAsync(J.d_rgba, 0, 4 * count, s)) || fail(cudaMemsetAsync(J.d_normal, 0, sizeof(float) * 3 * count, s)))
+            break;
+        if ((rc = bake_partition(J.d_q, J.d_texels, J.heights ? J.d_sface : nullptr, count, S->cuts.data() + 1, R, sel,
+                                 rows.xyz, rows.texel, rows.face, starts.data(), s)) != PT_OK)
+            break;
+        bool done = false;
+        for (int attempt = 0; attempt < 8 && !done; ++attempt) {
+            std::vector<int> status(R, PT_OK), needs(R, 0);
+            std::vector<std::thread> th;
+            auto work = [&](int r) {
+                const size_t m = starts[r + 1] - starts[r];
+                if (m == 0) return;
+                try {
+                    status[r] = slab_bake(S, r, home, J, rows, starts[r], m, copy[r] != 0, k, radius, &needs[r]);
+                } catch (...) { status[r] = PT_ERR_OUT_OF_MEMORY; }
+            };
+            for (int r = 0; r < R; ++r) {
+                try { th.emplace_back(work, r); } catch (...) { work(r); }
+            }
+            for (auto &t : th) t.join();
+            bool again = false;
+            for (int r = 0; r < R; ++r) {
+                if (status[r] != PT_OK && rc == PT_OK) rc = status[r];
+                again |= needs[r] != 0;
+            }
+            if (rc != PT_OK) break;
+            if (!again) { done = true; break; }
+            // some k-th-neighbour ball may leave a ghost zone: widen it and answer the rows again
+            S->halo = std::max(4.0 * S->halo, S->halo_auto);
+            ++S->rebuilds;
+            if ((rc = build_slabs(S)) != PT_OK) break;
+        }
+        if (rc != PT_OK) break;
+        if (!done) { rc = PT_ERR_UNSUPPORTED; break; }
+        if (fail(cudaSetDevice(home))) break;
+        const uint32_t routed = (uint32_t)starts[R];
+        if ((rc = launch_scatter_rows(rows.rgba, sel, routed, 4, J.d_rgba, s)) != PT_OK ||
+            (rc = launch_scatter_rows(rows.normal, sel, routed, 12, J.d_normal, s)) != PT_OK)
+            break;
+        // a row's height goes straight to its texel of the image
+        if (J.heights && (rc = launch_scatter_rows(rows.height, (const int32_t *)rows.texel, routed, 4, J.d_height, s)) != PT_OK)
+            break;
+        fail(cudaStreamSynchronize(s));
+    } while (0);
+    cudaSetDevice(home);
+    cudaStreamSynchronize(s);
+    pool_free(sel, s);
+    cudaStreamSynchronize(s);
+    rows_free(rows, any_copy, s);
+    return rc;
+}
+
+int sharded_bake(pt_sharded *S, const void *vertices, size_t n_vertices, const int32_t *faces, size_t n_faces, int k,
+                 double radius, int res, int pad, const pt_bake_outputs &o, pt_bake_height *hb, pt_bake_stats *st)
+{
+    using namespace pt;
+    const int home = S->slabs[0].device;
+    PT_CUDA(cudaSetDevice(home));
+    cudaStream_t s = nullptr;
+    PT_CUDA(cudaStreamCreateWithFlags(&s, cudaStreamNonBlocking));
+    BakeJob J;
+    float knn_ms = 0.0f;
+    int rc = bake_prepare(J, s, vertices, n_vertices, faces, n_faces, res, o, hb);
+    if (rc == PT_OK && J.count) {
+        const auto t0 = std::chrono::steady_clock::now();
+        rc = sharded_answer(S, home, J, k, radius);
+        knn_ms = std::chrono::duration<float, std::milli>(std::chrono::steady_clock::now() - t0).count();
+    }
+    if (rc == PT_OK) rc = bake_finish(J, pad, o, hb, st);
+    if (rc == PT_OK && st) st->knn_ms = knn_ms;
+    bake_release(J);
+    cudaStreamDestroy(s);
+    return rc;
+}
+
 }  // namespace
 
 extern "C" {
@@ -298,6 +525,21 @@ int pt_sharded_transfer(pt_sharded *S, const void *queries, size_t m, int k, dou
     if ((!rgba_out && !normal_out) && m) return PT_ERR_INVALID_ARG;
     try {
         return sharded_query(S, queries, m, k, radius, idx_out, d2_out, rgba_out, normal_out);
+    } catch (...) { return PT_ERR_OUT_OF_MEMORY; }
+}
+
+int pt_sharded_bake(pt_sharded *S, const void *vertices, size_t n_vertices, const int32_t *faces, size_t n_faces,
+                    int k, double radius, int resolution, int pad, const pt_bake_outputs *out, pt_bake_height *height,
+                    pt_bake_stats *stats)
+{
+    const pt_bake_outputs none = {nullptr, nullptr, nullptr, nullptr, nullptr, nullptr};
+    const pt_bake_outputs &o = out ? *out : none;
+    if (!S) return PT_ERR_INVALID_ARG;
+    const int rc = pt::bake_check_args(vertices, n_vertices, faces, n_faces, k, resolution, o, height);
+    if (rc != PT_OK) return rc;
+    if (pt_device_count() == 0) return PT_ERR_NO_DEVICE;
+    try {
+        return sharded_bake(S, vertices, n_vertices, faces, n_faces, k, radius, resolution, pad, o, height, stats);
     } catch (...) { return PT_ERR_OUT_OF_MEMORY; }
 }
 

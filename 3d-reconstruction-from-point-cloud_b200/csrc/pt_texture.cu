@@ -28,7 +28,7 @@
 #include <cub/device/device_select.cuh>
 #include <thrust/iterator/counting_iterator.h>
 
-#include "pt_index.cuh"
+#include "pt_bake.cuh"
 
 namespace pt {
 
@@ -471,15 +471,6 @@ static int texture_render_index(pt_index *ix, const void *vertices, size_t n_ver
 // n x 8 rows (x, y, z, u, v, nx, ny, nz) of bake_unpack_vertices_kernel can be rasterised.
 constexpr int BAKE_TILE = 32;                  // one warp per (face, 32 x 32-texel tile of its box)
 
-struct BakeMesh {
-    const double  *v;          // n_vertices rows of `stride` doubles: x, y, z, u, v, ...
-    int            stride;
-    uint32_t       n_vertices;
-    const int32_t *faces;
-    uint32_t       n_faces;
-    int            res;
-};
-
 // corners of face f; false for an out-of-range vertex index (the face covers nothing)
 __device__ __forceinline__ bool bake_corners(const BakeMesh &M, uint32_t f, const double *c[3])
 {
@@ -721,8 +712,6 @@ static int bake_compose(const uint32_t *texels, size_t count, const uint8_t *rgb
 // a.b = (a.x b.x + a.y b.y) + a.z b.z; "usable" = all components finite and a.a > 0; normalising
 // divides each component by sqrt(a.a).  Mesh rows are 8 doubles: x y z u v nx ny nz.  Frame rows
 // are 8 doubles: N xyz, T xyz, w, 0 -- all zero for a vertex without a frame.
-constexpr int BAKE_ROW = 8;
-
 struct D3 { double x, y, z; };
 
 __device__ __forceinline__ D3 d3_add(D3 a, D3 b) { return {__dadd_rn(a.x, b.x), __dadd_rn(a.y, b.y), __dadd_rn(a.z, b.z)}; }
@@ -980,9 +969,7 @@ __global__ void __launch_bounds__(256) bake_unpack_vertices_kernel(const Raw80t 
 // ---- height bake (DESIGN.md section 8, "Height bake") ---------------------------------------------
 // h = (sum_j w_j ((p_j - x) . N)) / W over the sample's neighbour list: the blend's weights, the
 // texel's unit mesh normal N of the tangent bake, sums sequential in neighbour order from +0.0.
-// NaN (always the quiet NaN 0x7fc00000) is "no value".  Samples per launch of the query + height
-// kernel in the bake: the neighbour lists of one chunk are 4 k bytes per sample.
-constexpr uint32_t HEIGHT_CHUNK = 1u << 22;
+// NaN (always the quiet NaN 0x7fc00000) is "no value".
 constexpr uint32_t HEIGHT_NAN = 0x7fc00000u;
 
 __device__ __forceinline__ double shfl_d(double v, int src) { return __shfl_sync(0xffffffffu, v, src); }
@@ -992,8 +979,9 @@ __device__ __forceinline__ double shfl_d(double v, int src) { return __shfl_sync
 // sample: lane j of a group gathers neighbour j through the position source (independent random
 // reads, in parallel), computes d2 in the metric's operation order and w_j (p_j - x).N, and the
 // group adds the terms in neighbour order through shuffles.  Every lane runs the same loops, so
-// the shuffles see the full warp.
-template <typename POS>
+// the shuffles see the full warp.  The height of sample s goes to height[texels[s]] (the image), or
+// with BY_SAMPLE to height[s] (a slab's rows, scattered into the image on the bake's home device).
+template <typename POS, bool BY_SAMPLE>
 __global__ void __launch_bounds__(256)
 bake_height_kernel(const BakeMesh M, const double *frames, const uint32_t *texels, const int32_t *sample_faces,
                    const double *xyz, uint32_t count, const int32_t *idx, int k, int width, const POS pos,
@@ -1059,7 +1047,7 @@ bake_height_kernel(const BakeMesh M, const double *frames, const uint32_t *texel
         }
         if (j == 0 && cnt > 0 && s < count) {
             const float h = __double2float_rn(__ddiv_rn(S, W));
-            height[texels[s]] = h != h ? __uint_as_float(HEIGHT_NAN) : h;
+            height[BY_SAMPLE ? s : texels[s]] = h != h ? __uint_as_float(HEIGHT_NAN) : h;
         }
     }
 }
@@ -1148,14 +1136,14 @@ static int bake_height_width(int k)
     return w;
 }
 
-template <typename POS>
+template <bool BY_SAMPLE, typename POS>
 static int launch_height(const BakeMesh &M, const double *frames, const uint32_t *texels, const int32_t *sample_faces,
                          const double *xyz, size_t count, const int32_t *idx, int k, const POS &pos,
                          uint32_t n_points, float *height, cudaStream_t s)
 {
     if (!count) return PT_OK;
-    bake_height_kernel<POS><<<tcdiv(count, 256), 256, 0, s>>>(M, frames, texels, sample_faces, xyz, (uint32_t)count, idx, k,
-                                                              bake_height_width(k), pos, n_points, height);
+    bake_height_kernel<POS, BY_SAMPLE><<<tcdiv(count, 256), 256, 0, s>>>(M, frames, texels, sample_faces, xyz, (uint32_t)count,
+                                                                         idx, k, bake_height_width(k), pos, n_points, height);
     count_launch();
     PT_CUDA(cudaGetLastError());
     return PT_OK;
@@ -1210,165 +1198,321 @@ static bool bake_wants_height(const pt_bake_height *h) { return h && (h->height 
 template <typename PT>
 static int launch_height_index(pt_index *ix, const BakeMesh &M, const double *frames, const uint32_t *texels,
                                const int32_t *sample_faces, const double *xyz, size_t count, const int32_t *idx, int k,
-                               float *height, cudaStream_t s)
+                               float *height, bool by_sample, cudaStream_t s)
 {
     PT_TRY(index_inverse_perm<PT>(ix));
     const PosSorted<PT> pos{(const PT *)ix->pts, ix->inv_perm};
-    return launch_height(M, frames, texels, sample_faces, xyz, count, idx, k, pos, ix->n, height, s);
+    return by_sample ? launch_height<true>(M, frames, texels, sample_faces, xyz, count, idx, k, pos, ix->n, height, s)
+                     : launch_height<false>(M, frames, texels, sample_faces, xyz, count, idx, k, pos, ix->n, height, s);
+}
+
+// the corner list of the frames is sorted with an int item count
+static bool bake_corners_fit(size_t n_faces) { return n_faces <= (size_t)INT32_MAX / 3; }
+
+int bake_check_args(const void *vertices, size_t n_vertices, const int32_t *faces, size_t n_faces, int k,
+                    int resolution, const pt_bake_outputs &o, const pt_bake_height *height)
+{
+    const bool heights = bake_wants_height(height);
+    if ((!vertices && n_vertices) || (!faces && n_faces) || (height && !heights) ||
+        (!bake_wants_object_maps(o) && !bake_wants_frames(o) && !heights) || resolution < 1 || resolution > 16384 ||
+        n_vertices > 0x7ffffff0ull || n_faces >= (1ull << 31))
+        return PT_ERR_INVALID_ARG;
+    if (k < 1 || k > PT_MAX_K) return PT_ERR_UNSUPPORTED;
+    if ((bake_wants_frames(o) || heights) && !bake_corners_fit(n_faces)) return PT_ERR_UNSUPPORTED;
+    return PT_OK;
+}
+
+int bake_prepare(BakeJob &J, cudaStream_t s, const void *vertices, size_t n_vertices, const int32_t *faces,
+                 size_t n_faces, int res, const pt_bake_outputs &o, const pt_bake_height *hb)
+{
+    J.s = s;
+    J.res = res;
+    J.n_vertices = n_vertices;
+    J.heights = bake_wants_height(hb);
+    const size_t n_pix = (size_t)res * res;
+    const bool heights = J.heights;
+    const bool maps = bake_wants_object_maps(o) || bake_wants_tangent_maps(o) || heights;
+    const bool tmaps = bake_wants_tangent_maps(o), frames = bake_wants_frames(o) || heights;
+    for (auto &e : J.ev) PT_CUDA(cudaEventCreate(&e));
+    if (pool_alloc(&J.d_raw, sizeof(Raw80t) * n_vertices, s) ||
+        pool_alloc((void **)&J.d_rows, sizeof(double) * BAKE_ROW * n_vertices, s) ||
+        pool_alloc((void **)&J.d_faces, sizeof(int32_t) * 3 * n_faces, s) ||
+        pool_alloc((void **)&J.d_empty, sizeof(unsigned long long) * (heights ? 2 : 1), s) ||
+        (maps && (pool_alloc((void **)&J.d_texels, sizeof(uint32_t) * n_pix, s) ||
+                  pool_alloc((void **)&J.d_q, sizeof(double) * 3 * n_pix, s))) ||
+        ((tmaps || heights) && pool_alloc((void **)&J.d_sface, sizeof(int32_t) * n_pix, s)) ||
+        (heights && (pool_alloc((void **)&J.d_height, sizeof(float) * n_pix, s) ||
+                     pool_alloc((void **)&J.d_range, 2 * sizeof(double), s))) ||
+        (heights && hb->height_u16 && pool_alloc((void **)&J.d_h16, sizeof(uint16_t) * n_pix, s)) ||
+        (frames && pool_alloc((void **)&J.d_frames, sizeof(double) * BAKE_ROW * n_vertices, s)) ||
+        (o.bgra && pool_alloc((void **)&J.d_bgra, 4 * n_pix, s)) ||
+        (o.normal_bgra && pool_alloc((void **)&J.d_nbgra, 4 * n_pix, s)) ||
+        (o.normal && pool_alloc((void **)&J.d_nf, sizeof(float) * 3 * n_pix, s)) ||
+        (o.tangent_bgra && pool_alloc((void **)&J.d_tbgra, 4 * n_pix, s)) ||
+        (o.tangent_normal && pool_alloc((void **)&J.d_tnf, sizeof(float) * 3 * n_pix, s)) ||
+        (o.vertex_tangents && pool_alloc((void **)&J.d_vt, sizeof(float) * 4 * n_vertices, s)))
+        return PT_ERR_OUT_OF_MEMORY;
+    PT_CUDA(cudaEventRecord(J.ev[0], s));
+    PT_CUDA(cudaMemcpyAsync(J.d_raw, vertices, sizeof(Raw80t) * n_vertices, cudaMemcpyHostToDevice, s));
+    PT_CUDA(cudaMemcpyAsync(J.d_faces, faces, sizeof(int32_t) * 3 * n_faces, cudaMemcpyHostToDevice, s));
+    PT_CUDA(cudaMemsetAsync(J.d_empty, 0, sizeof(unsigned long long), s));
+    if (n_vertices) {
+        bake_unpack_vertices_kernel<<<tcdiv(n_vertices, 256), 256, 0, s>>>((const Raw80t *)J.d_raw, (uint32_t)n_vertices,
+                                                                         J.d_rows);
+        count_launch();
+    }
+    J.M = BakeMesh{J.d_rows, BAKE_ROW, (uint32_t)n_vertices, J.d_faces, (uint32_t)n_faces, res};
+    if (maps) PT_TRY(bake_texels(J.M, J.d_texels, J.d_q, J.d_sface, &J.count, s));
+    if (frames) PT_TRY(bake_frames(J.M, J.d_frames, J.d_vt, s));
+    PT_CUDA(cudaEventRecord(J.ev[1], s));
+    const size_t count = J.count ? J.count : 1;
+    if (pool_alloc((void **)&J.d_rgba, 4 * count, s) || pool_alloc((void **)&J.d_normal, sizeof(float) * 3 * count, s))
+        return PT_ERR_OUT_OF_MEMORY;
+    if (heights) {
+        bake_height_fill_kernel<<<148 * 8, 256, 0, s>>>(J.d_height, n_pix);
+        count_launch();
+    }
+    return PT_OK;
+}
+
+int bake_answer_rows(pt_index *ix, const BakeMesh &M, const double *frames, const double *xyz,
+                     const uint32_t *texels, const int32_t *sample_faces, size_t m, int k, double radius,
+                     const BakeGhost *ghost, uint8_t *rgba, float *normal, float *height, bool by_sample,
+                     std::vector<cudaEvent_t> *marks, cudaStream_t s)
+{
+    if (m == 0) return PT_OK;
+    // the lists (heights) and the distances (ghost check) of one chunk take at most
+    // HEIGHT_CHUNK * k * 4 and HEIGHT_CHUNK * k * 8 bytes
+    const bool heights = height != nullptr;
+    const size_t chunk = heights || ghost ? std::min((size_t)HEIGHT_CHUNK, m) : m;
+    int32_t *d_idx = nullptr;
+    double *d_d2 = nullptr;
+    int rc = PT_OK;
+    auto fail = [&](cudaError_t e) { if (e != cudaSuccess && rc == PT_OK) rc = map_cuda_error(e); return e != cudaSuccess; };
+    auto mark = [&]() {
+        if (!marks) return false;
+        marks->emplace_back();
+        return fail(cudaEventCreate(&marks->back())) || fail(cudaEventRecord(marks->back(), s));
+    };
+    do {
+        if ((heights && pool_alloc((void **)&d_idx, sizeof(int32_t) * k * chunk, s)) ||
+            (ghost && pool_alloc((void **)&d_d2, sizeof(double) * k * chunk, s))) {
+            rc = PT_ERR_OUT_OF_MEMORY;
+            break;
+        }
+        if (heights && by_sample) {
+            bake_height_fill_kernel<<<148 * 8, 256, 0, s>>>(height, m);
+            count_launch();
+        }
+        QueryParams qp{};
+        fill_params(ix, qp);
+        qp.ids = nullptr;          // the index's own ids: the height kernel reads its records by them
+        qp.k = k;
+        qp.r2 = radius_to_r2(radius);
+        for (size_t c0 = 0; c0 < m; c0 += chunk) {
+            const size_t cm = std::min(chunk, m - c0);
+            if (heights && mark()) break;
+            qp.queries = xyz + 3 * c0; qp.m = (uint32_t)cm;
+            qp.rgba_out = rgba + 4 * c0; qp.normal_out = normal + 3 * c0;
+            qp.idx_out = d_idx; qp.d2_out = d_d2;
+            if ((rc = launch_query(ix, qp, s)) != PT_OK) break;
+            if (ghost && (rc = launch_ghost_check(xyz + 3 * c0, d_d2, (uint32_t)cm, k, qp.r2, ghost->boxes, ghost->n_ranks,
+                                                  ghost->self, ghost->halo, ghost->flag, s)) != PT_OK)
+                break;
+            if (!heights) continue;
+            if (mark()) break;
+            float *h = by_sample ? height + c0 : height;
+            rc = ix->coord_f64 ? launch_height_index<PointD>(ix, M, frames, texels + c0, sample_faces + c0, xyz + 3 * c0, cm,
+                                                             d_idx, k, h, by_sample, s)
+                               : launch_height_index<PointF>(ix, M, frames, texels + c0, sample_faces + c0, xyz + 3 * c0, cm,
+                                                             d_idx, k, h, by_sample, s);
+            if (rc != PT_OK) break;
+        }
+        fail(cudaGetLastError());
+    } while (0);
+    pool_free(d_idx, s);
+    pool_free(d_d2, s);
+    return rc;
+}
+
+// ---- sharded bake: samples -> slabs (DESIGN.md section 8, "Sharded bake") ----------------------------
+struct BakeCuts { int n; double c[BAKE_MAX_SLABS - 1]; };      // the interior x-cuts, ascending
+constexpr int PARTITION_WARPS = 8;
+
+// The number of cuts c with !(x < c), which is the host's upper_bound for every x (+-inf included);
+// n_slabs = C.n + 1 for a sample with a NaN component.  Unrolled so the cuts stay in parameter space.
+__device__ __forceinline__ int bake_slab_of(const BakeCuts &C, double x, double y, double z)
+{
+    if (x != x || y != y || z != z) return C.n + 1;
+    int r = 0;
+#pragma unroll
+    for (int j = 0; j < BAKE_MAX_SLABS - 1; ++j) r += (j < C.n && !(x < C.c[j])) ? 1 : 0;
+    return r;
+}
+
+// Block b counts its samples per slab into counts[r * gridDim.x + b] (!SCATTER); with SCATTER, base
+// holds the exclusive scan of those counts and every routed sample i lands in row base[r][b] + the
+// samples of its slab before it in the block: a stable partition.  Block 0 also writes the slabs'
+// first rows into starts[0 .. n_slabs].
+template <bool SCATTER>
+__global__ void __launch_bounds__(PARTITION_WARPS * 32)
+bake_partition_kernel(const double *xyz, const uint32_t *texels, const int32_t *faces, uint32_t count, const BakeCuts C,
+                      uint32_t *counts, const uint32_t *base, int32_t *sel, double *pxyz, uint32_t *ptex, int32_t *pface,
+                      uint32_t *starts)
+{
+    __shared__ uint32_t s_warp[PARTITION_WARPS][BAKE_MAX_SLABS + 1];
+    const int n_slabs = C.n + 1;
+    for (int t = threadIdx.x; t < PARTITION_WARPS * (BAKE_MAX_SLABS + 1); t += blockDim.x) (&s_warp[0][0])[t] = 0u;
+    __syncthreads();
+    const uint32_t i = blockIdx.x * blockDim.x + threadIdx.x;
+    const unsigned lane = threadIdx.x & 31u, warp = threadIdx.x >> 5;
+    double x = 0.0, y = 0.0, z = 0.0;
+    int r = n_slabs;                                  // past the slabs: not routed
+    if (i < count) {
+        x = xyz[3 * (size_t)i]; y = xyz[3 * (size_t)i + 1]; z = xyz[3 * (size_t)i + 2];
+        r = bake_slab_of(C, x, y, z);
+    }
+    const unsigned peers = __match_any_sync(0xffffffffu, r);
+    if ((int)lane == __ffs(peers) - 1) s_warp[warp][r] = (uint32_t)__popc(peers);
+    __syncthreads();
+    if (!SCATTER) {
+        for (int b = threadIdx.x; b < n_slabs; b += blockDim.x) {
+            uint32_t c = 0;
+            for (int w = 0; w < PARTITION_WARPS; ++w) c += s_warp[w][b];
+            counts[(size_t)b * gridDim.x + blockIdx.x] = c;
+        }
+        return;
+    }
+    if (blockIdx.x == 0)
+        for (int b = threadIdx.x; b <= n_slabs; b += blockDim.x) starts[b] = base[(size_t)b * gridDim.x];
+    if (r >= n_slabs) return;
+    uint32_t row = base[(size_t)r * gridDim.x + blockIdx.x] + (uint32_t)__popc(peers & ((1u << lane) - 1u));
+    for (unsigned w = 0; w < warp; ++w) row += s_warp[w][r];
+    sel[row] = (int32_t)i;
+    pxyz[3 * (size_t)row] = x; pxyz[3 * (size_t)row + 1] = y; pxyz[3 * (size_t)row + 2] = z;
+    ptex[row] = texels[i];
+    if (pface) pface[row] = faces[i];
+}
+
+int bake_partition(const double *xyz, const uint32_t *texels, const int32_t *faces, size_t count,
+                   const double *cuts, int n_slabs, int32_t *sel, double *pxyz, uint32_t *ptex, int32_t *pface,
+                   size_t *starts, cudaStream_t s)
+{
+    if (n_slabs < 1 || n_slabs > BAKE_MAX_SLABS || count > 0xffffffffull) return PT_ERR_INVALID_ARG;
+    for (int r = 0; r <= n_slabs; ++r) starts[r] = 0;
+    if (count == 0) return PT_OK;
+    BakeCuts C{};
+    C.n = n_slabs - 1;
+    for (int j = 0; j < C.n; ++j) C.c[j] = cuts[j];
+    const unsigned threads = PARTITION_WARPS * 32, blocks = tcdiv(count, threads);
+    const size_t cells = (size_t)n_slabs * blocks + 1;      // + 1: the scan's total
+    uint32_t *d_counts = nullptr, *d_base = nullptr, *d_starts = nullptr;
+    void *d_tmp = nullptr;
+    size_t scan_bytes = 0;
+    int rc = PT_OK;
+    auto fail = [&](cudaError_t e) { if (e != cudaSuccess && rc == PT_OK) rc = map_cuda_error(e); return e != cudaSuccess; };
+    do {
+        if (cells > (size_t)INT32_MAX) { rc = PT_ERR_UNSUPPORTED; break; }
+        if (fail(cub::DeviceScan::ExclusiveSum(nullptr, scan_bytes, d_counts, d_base, (int)cells, s))) break;
+        if (pool_alloc((void **)&d_counts, sizeof(uint32_t) * cells, s) || pool_alloc((void **)&d_base, sizeof(uint32_t) * cells, s) ||
+            pool_alloc((void **)&d_starts, sizeof(uint32_t) * (n_slabs + 1), s) || pool_alloc(&d_tmp, scan_bytes ? scan_bytes : 1, s)) {
+            rc = PT_ERR_OUT_OF_MEMORY;
+            break;
+        }
+        if (fail(cudaMemsetAsync(d_counts + cells - 1, 0, sizeof(uint32_t), s))) break;
+        bake_partition_kernel<false><<<blocks, threads, 0, s>>>(xyz, texels, faces, (uint32_t)count, C, d_counts, nullptr,
+                                                                nullptr, nullptr, nullptr, nullptr, nullptr);
+        count_launch();
+        if (fail(cub::DeviceScan::ExclusiveSum(d_tmp, scan_bytes, d_counts, d_base, (int)cells, s))) break;
+        count_launch();
+        bake_partition_kernel<true><<<blocks, threads, 0, s>>>(xyz, texels, faces, (uint32_t)count, C, nullptr, d_base, sel,
+                                                               pxyz, ptex, pface, d_starts);
+        count_launch();
+        std::vector<uint32_t> h(n_slabs + 1);
+        if (fail(cudaMemcpyAsync(h.data(), d_starts, sizeof(uint32_t) * (n_slabs + 1), cudaMemcpyDeviceToHost, s))) break;
+        if (fail(cudaStreamSynchronize(s))) break;
+        for (int r = 0; r <= n_slabs; ++r) starts[r] = h[r];
+    } while (0);
+    void *frees[] = {d_counts, d_base, d_starts, d_tmp};
+    for (void *p : frees) pool_free(p, s);
+    return rc;
+}
+
+int bake_finish(BakeJob &J, int pad, const pt_bake_outputs &o, pt_bake_height *hb, pt_bake_stats *st)
+{
+    cudaStream_t s = J.s;
+    const size_t n_pix = (size_t)J.res * J.res, count = J.count;
+    const bool heights = J.heights, tmaps = bake_wants_tangent_maps(o);
+    PT_CUDA(cudaEventRecord(J.ev[2], s));
+    if (bake_wants_object_maps(o))
+        PT_TRY(bake_compose(J.d_texels, count, J.d_rgba, J.d_normal, J.res, pad, J.d_bgra, J.d_nbgra, J.d_nf, J.d_empty, s));
+    // the empty lists are counted by whichever composition runs
+    if (tmaps)
+        PT_TRY(bake_compose_tangent(J.M, J.d_frames, J.d_texels, J.d_sface, count, J.d_rgba, J.d_normal, pad, J.d_tbgra,
+                                    J.d_tnf, bake_wants_object_maps(o) ? nullptr : J.d_empty, s));
+    if (heights) {
+        PT_CUDA(cudaMemsetAsync(J.d_empty + 1, 0, sizeof(unsigned long long), s));
+        PT_TRY(bake_height_finish(J.d_height, J.res, pad, hb->range, J.d_range, J.d_h16, J.d_empty + 1, s));
+    }
+    PT_CUDA(cudaEventRecord(J.ev[3], s));
+    if (o.bgra) PT_CUDA(cudaMemcpyAsync(o.bgra, J.d_bgra, 4 * n_pix, cudaMemcpyDeviceToHost, s));
+    if (o.normal_bgra) PT_CUDA(cudaMemcpyAsync(o.normal_bgra, J.d_nbgra, 4 * n_pix, cudaMemcpyDeviceToHost, s));
+    if (o.normal) PT_CUDA(cudaMemcpyAsync(o.normal, J.d_nf, sizeof(float) * 3 * n_pix, cudaMemcpyDeviceToHost, s));
+    if (o.tangent_bgra) PT_CUDA(cudaMemcpyAsync(o.tangent_bgra, J.d_tbgra, 4 * n_pix, cudaMemcpyDeviceToHost, s));
+    if (o.tangent_normal) PT_CUDA(cudaMemcpyAsync(o.tangent_normal, J.d_tnf, sizeof(float) * 3 * n_pix, cudaMemcpyDeviceToHost, s));
+    if (o.vertex_tangents && J.n_vertices)
+        PT_CUDA(cudaMemcpyAsync(o.vertex_tangents, J.d_vt, sizeof(float) * 4 * J.n_vertices, cudaMemcpyDeviceToHost, s));
+    if (heights) {
+        if (hb->height) PT_CUDA(cudaMemcpyAsync(hb->height, J.d_height, sizeof(float) * n_pix, cudaMemcpyDeviceToHost, s));
+        if (hb->height_u16) PT_CUDA(cudaMemcpyAsync(hb->height_u16, J.d_h16, sizeof(uint16_t) * n_pix, cudaMemcpyDeviceToHost, s));
+        PT_CUDA(cudaMemcpyAsync(hb->range_used, J.d_range, 2 * sizeof(double), cudaMemcpyDeviceToHost, s));
+    }
+    unsigned long long empty[2] = {0, 0};
+    PT_CUDA(cudaMemcpyAsync(empty, J.d_empty, sizeof(unsigned long long) * (heights ? 2 : 1), cudaMemcpyDeviceToHost, s));
+    PT_CUDA(cudaStreamSynchronize(s));
+    if (heights) hb->texels = empty[1];
+    if (st) {
+        st->texels = count;
+        st->empty = empty[0];
+        cudaEventElapsedTime(&st->raster_ms, J.ev[0], J.ev[1]);
+        cudaEventElapsedTime(&st->knn_ms, J.ev[1], J.ev[2]);
+        cudaEventElapsedTime(&st->pad_ms, J.ev[2], J.ev[3]);
+        if (!J.marks.empty()) {                // the height kernels between the query chunks count as pad_ms
+            float knn = 0.0f, t = 0.0f;
+            for (size_t c = 0; c + 1 < J.marks.size(); c += 2)
+                if (cudaEventElapsedTime(&t, J.marks[c], J.marks[c + 1]) == cudaSuccess) knn += t;
+            st->pad_ms += st->knn_ms - knn;
+            st->knn_ms = knn;
+        }
+    }
+    return PT_OK;
+}
+
+void bake_release(BakeJob &J)
+{
+    cudaStream_t s = J.s;
+    if (s) cudaStreamSynchronize(s);
+    void *frees[] = {J.d_raw, J.d_rows, J.d_faces, J.d_texels, J.d_q, J.d_sface, J.d_frames, J.d_rgba, J.d_normal, J.d_bgra,
+                     J.d_nbgra, J.d_nf, J.d_tbgra, J.d_tnf, J.d_vt, J.d_empty, J.d_height, J.d_range, J.d_h16};
+    for (void *p : frees) pool_free(p, s);
+    for (auto &e : J.ev) if (e) cudaEventDestroy(e);
+    for (auto &e : J.marks) if (e) cudaEventDestroy(e);
+    J = BakeJob{};
+    if (s) cudaStreamSynchronize(s);
+    cudaGetLastError();
 }
 
 static int texture_bake(pt_index *ix, const void *vertices, size_t n_vertices, const int32_t *faces, size_t n_faces,
                         int k, double radius, int res, int pad, const pt_bake_outputs &o, pt_bake_height *hb,
                         pt_bake_stats *st)
 {
-    cudaStream_t s = ix->stream;
-    const size_t n_pix = (size_t)res * res;
-    const bool heights = bake_wants_height(hb);
-    const bool maps = bake_wants_object_maps(o) || bake_wants_tangent_maps(o) || heights;
-    const bool tmaps = bake_wants_tangent_maps(o), frames = bake_wants_frames(o) || heights;
-    Raw80t *d_raw = nullptr;
-    double *d_rows = nullptr, *d_q = nullptr, *d_frames = nullptr, *d_range = nullptr;
-    int32_t *d_faces = nullptr, *d_sface = nullptr, *d_idx = nullptr;
-    uint32_t *d_texels = nullptr;
-    uint8_t *d_rgba = nullptr, *d_bgra = nullptr, *d_nbgra = nullptr, *d_tbgra = nullptr;
-    float *d_normal = nullptr, *d_nf = nullptr, *d_tnf = nullptr, *d_vt = nullptr, *d_height = nullptr;
-    uint16_t *d_h16 = nullptr;
-    unsigned long long *d_empty = nullptr;
-    cudaEvent_t ev[4] = {};
-    std::vector<cudaEvent_t> marks;                // around each query chunk when heights are baked
-    size_t count = 0;
-    int rc = PT_OK;
-    auto fail = [&](cudaError_t e) { if (e != cudaSuccess && rc == PT_OK) rc = map_cuda_error(e); return e != cudaSuccess; };
-    do {
-        for (auto &e : ev) if (fail(cudaEventCreate(&e))) break;
-        if (rc != PT_OK) break;
-        if (pool_alloc((void **)&d_raw, sizeof(Raw80t) * n_vertices, s) ||
-            pool_alloc((void **)&d_rows, sizeof(double) * BAKE_ROW * n_vertices, s) ||
-            pool_alloc((void **)&d_faces, sizeof(int32_t) * 3 * n_faces, s) ||
-            pool_alloc((void **)&d_empty, sizeof(unsigned long long) * (heights ? 2 : 1), s) ||
-            (maps && (pool_alloc((void **)&d_texels, sizeof(uint32_t) * n_pix, s) ||
-                      pool_alloc((void **)&d_q, sizeof(double) * 3 * n_pix, s))) ||
-            ((tmaps || heights) && pool_alloc((void **)&d_sface, sizeof(int32_t) * n_pix, s)) ||
-            (heights && (pool_alloc((void **)&d_height, sizeof(float) * n_pix, s) ||
-                         pool_alloc((void **)&d_range, 2 * sizeof(double), s))) ||
-            (heights && hb->height_u16 && pool_alloc((void **)&d_h16, sizeof(uint16_t) * n_pix, s)) ||
-            (frames && pool_alloc((void **)&d_frames, sizeof(double) * BAKE_ROW * n_vertices, s)) ||
-            (o.bgra && pool_alloc((void **)&d_bgra, 4 * n_pix, s)) ||
-            (o.normal_bgra && pool_alloc((void **)&d_nbgra, 4 * n_pix, s)) ||
-            (o.normal && pool_alloc((void **)&d_nf, sizeof(float) * 3 * n_pix, s)) ||
-            (o.tangent_bgra && pool_alloc((void **)&d_tbgra, 4 * n_pix, s)) ||
-            (o.tangent_normal && pool_alloc((void **)&d_tnf, sizeof(float) * 3 * n_pix, s)) ||
-            (o.vertex_tangents && pool_alloc((void **)&d_vt, sizeof(float) * 4 * n_vertices, s))) {
-            rc = PT_ERR_OUT_OF_MEMORY;
-            break;
-        }
-        if (fail(cudaEventRecord(ev[0], s))) break;
-        if (fail(cudaMemcpyAsync(d_raw, vertices, sizeof(Raw80t) * n_vertices, cudaMemcpyHostToDevice, s))) break;
-        if (fail(cudaMemcpyAsync(d_faces, faces, sizeof(int32_t) * 3 * n_faces, cudaMemcpyHostToDevice, s))) break;
-        if (fail(cudaMemsetAsync(d_empty, 0, sizeof(unsigned long long), s))) break;
-        if (n_vertices) {
-            bake_unpack_vertices_kernel<<<tcdiv(n_vertices, 256), 256, 0, s>>>(d_raw, (uint32_t)n_vertices, d_rows);
-            count_launch();
-        }
-        const BakeMesh M{d_rows, BAKE_ROW, (uint32_t)n_vertices, d_faces, (uint32_t)n_faces, res};
-        if (maps && (rc = bake_texels(M, d_texels, d_q, d_sface, &count, s)) != PT_OK) break;
-        if (frames && (rc = bake_frames(M, d_frames, d_vt, s)) != PT_OK) break;
-        if (fail(cudaEventRecord(ev[1], s))) break;
-        // heights need the neighbour lists: the query and the height kernel then run in chunks, so
-        // the lists take at most HEIGHT_CHUNK * k * 4 bytes
-        const size_t chunk = heights ? HEIGHT_CHUNK : (count ? count : 1);
-        if (pool_alloc((void **)&d_rgba, 4 * (count ? count : 1), s) || pool_alloc((void **)&d_normal, sizeof(float) * 3 * (count ? count : 1), s) ||
-            (heights && pool_alloc((void **)&d_idx, sizeof(int32_t) * k * std::min(chunk, count ? count : 1), s))) {
-            rc = PT_ERR_OUT_OF_MEMORY;
-            break;
-        }
-        if (heights) {
-            bake_height_fill_kernel<<<148 * 8, 256, 0, s>>>(d_height, n_pix);
-            count_launch();
-        }
-        QueryParams qp{};
-        fill_params(ix, qp);
-        qp.k = k;
-        qp.r2 = radius_to_r2(radius);
-        for (size_t c0 = 0; c0 < count; c0 += chunk) {
-            const size_t cm = std::min(chunk, count - c0);
-            if (heights) {
-                marks.emplace_back();
-                if (fail(cudaEventCreate(&marks.back())) || fail(cudaEventRecord(marks.back(), s))) break;
-            }
-            qp.queries = d_q + 3 * c0; qp.m = (uint32_t)cm;
-            qp.rgba_out = d_rgba + 4 * c0; qp.normal_out = d_normal + 3 * c0;
-            qp.idx_out = d_idx;
-            if ((rc = launch_query(ix, qp, s)) != PT_OK) break;
-            if (!heights) continue;
-            marks.emplace_back();
-            if (fail(cudaEventCreate(&marks.back())) || fail(cudaEventRecord(marks.back(), s))) break;
-            rc = ix->coord_f64 ? launch_height_index<PointD>(ix, M, d_frames, d_texels + c0, d_sface + c0, d_q + 3 * c0, cm,
-                                                             d_idx, k, d_height, s)
-                               : launch_height_index<PointF>(ix, M, d_frames, d_texels + c0, d_sface + c0, d_q + 3 * c0, cm,
-                                                             d_idx, k, d_height, s);
-            if (rc != PT_OK) break;
-        }
-        if (rc != PT_OK) break;
-        if (fail(cudaEventRecord(ev[2], s))) break;
-        if (bake_wants_object_maps(o) &&
-            (rc = bake_compose(d_texels, count, d_rgba, d_normal, res, pad, d_bgra, d_nbgra, d_nf, d_empty, s)) != PT_OK)
-            break;
-        // the empty lists are counted by whichever composition runs
-        if (tmaps && (rc = bake_compose_tangent(M, d_frames, d_texels, d_sface, count, d_rgba, d_normal, pad, d_tbgra,
-                                                d_tnf, bake_wants_object_maps(o) ? nullptr : d_empty, s)) != PT_OK)
-            break;
-        if (heights) {
-            if (fail(cudaMemsetAsync(d_empty + 1, 0, sizeof(unsigned long long), s))) break;
-            if ((rc = bake_height_finish(d_height, res, pad, hb->range, d_range, d_h16, d_empty + 1, s)) != PT_OK) break;
-        }
-        if (fail(cudaEventRecord(ev[3], s))) break;
-        if (o.bgra && fail(cudaMemcpyAsync(o.bgra, d_bgra, 4 * n_pix, cudaMemcpyDeviceToHost, s))) break;
-        if (o.normal_bgra && fail(cudaMemcpyAsync(o.normal_bgra, d_nbgra, 4 * n_pix, cudaMemcpyDeviceToHost, s))) break;
-        if (o.normal && fail(cudaMemcpyAsync(o.normal, d_nf, sizeof(float) * 3 * n_pix, cudaMemcpyDeviceToHost, s))) break;
-        if (o.tangent_bgra && fail(cudaMemcpyAsync(o.tangent_bgra, d_tbgra, 4 * n_pix, cudaMemcpyDeviceToHost, s))) break;
-        if (o.tangent_normal &&
-            fail(cudaMemcpyAsync(o.tangent_normal, d_tnf, sizeof(float) * 3 * n_pix, cudaMemcpyDeviceToHost, s)))
-            break;
-        if (o.vertex_tangents && n_vertices &&
-            fail(cudaMemcpyAsync(o.vertex_tangents, d_vt, sizeof(float) * 4 * n_vertices, cudaMemcpyDeviceToHost, s)))
-            break;
-        if (heights) {
-            if (hb->height && fail(cudaMemcpyAsync(hb->height, d_height, sizeof(float) * n_pix, cudaMemcpyDeviceToHost, s)))
-                break;
-            if (hb->height_u16 &&
-                fail(cudaMemcpyAsync(hb->height_u16, d_h16, sizeof(uint16_t) * n_pix, cudaMemcpyDeviceToHost, s)))
-                break;
-            if (fail(cudaMemcpyAsync(hb->range_used, d_range, 2 * sizeof(double), cudaMemcpyDeviceToHost, s))) break;
-        }
-        unsigned long long empty[2] = {0, 0};
-        if (fail(cudaMemcpyAsync(empty, d_empty, sizeof(unsigned long long) * (heights ? 2 : 1), cudaMemcpyDeviceToHost, s)))
-            break;
-        if (fail(cudaStreamSynchronize(s))) break;
-        if (heights) hb->texels = empty[1];
-        if (st) {
-            st->texels = count;
-            st->empty = empty[0];
-            cudaEventElapsedTime(&st->raster_ms, ev[0], ev[1]);
-            cudaEventElapsedTime(&st->knn_ms, ev[1], ev[2]);
-            cudaEventElapsedTime(&st->pad_ms, ev[2], ev[3]);
-            if (heights) {                         // the height kernels between the query chunks count as pad_ms
-                float knn = 0.0f, t = 0.0f;
-                for (size_t c = 0; c + 1 < marks.size(); c += 2)
-                    if (cudaEventElapsedTime(&t, marks[c], marks[c + 1]) == cudaSuccess) knn += t;
-                st->pad_ms += st->knn_ms - knn;
-                st->knn_ms = knn;
-            }
-        }
-    } while (0);
-    cudaStreamSynchronize(s);
-    void *frees[] = {d_raw, d_rows, d_faces, d_texels, d_q, d_sface, d_frames, d_rgba, d_normal, d_bgra, d_nbgra, d_nf,
-                     d_tbgra, d_tnf, d_vt, d_empty, d_idx, d_height, d_range, d_h16};
-    for (void *p : frees) pool_free(p, s);
-    for (auto &e : ev) if (e) cudaEventDestroy(e);
-    for (auto &e : marks) if (e) cudaEventDestroy(e);
-    cudaStreamSynchronize(s);
-    cudaGetLastError();
+    BakeJob J;
+    int rc = bake_prepare(J, ix->stream, vertices, n_vertices, faces, n_faces, res, o, hb);
+    if (rc == PT_OK)
+        rc = bake_answer_rows(ix, J.M, J.d_frames, J.d_q, J.d_texels, J.d_sface, J.count, k, radius, nullptr, J.d_rgba,
+                              J.d_normal, J.d_height, false, J.heights ? &J.marks : nullptr, J.s);
+    if (rc == PT_OK) rc = bake_finish(J, pad, o, hb, st);
+    bake_release(J);
     return rc;
 }
 
@@ -1446,9 +1590,6 @@ extern "C" int pt_bake_texels_device(const double *vertices_xyzuv, size_t n_vert
                                   count_out, device, stream);
 }
 
-// the corner list of the frames is sorted with an int item count
-static bool bake_corners_fit(size_t n_faces) { return n_faces <= (size_t)INT32_MAX / 3; }
-
 extern "C" int pt_bake_frames_device(const double *vertices_xyzuvn, size_t n_vertices, const int32_t *faces,
                                      size_t n_faces, double *frames_out, float *tangents_out, int device, void *stream)
 {
@@ -1499,13 +1640,9 @@ extern "C" int pt_texture_bake_height(pt_index *ix, const void *vertices, size_t
 {
     const pt_bake_outputs none = {nullptr, nullptr, nullptr, nullptr, nullptr, nullptr};
     const pt_bake_outputs &o = out ? *out : none;
-    const bool heights = bake_wants_height(height);
-    if (!ix || (!vertices && n_vertices) || (!faces && n_faces) || (height && !heights) ||
-        (!bake_wants_object_maps(o) && !bake_wants_frames(o) && !heights) || resolution < 1 || resolution > 16384 ||
-        n_vertices > 0x7ffffff0ull || n_faces >= (1ull << 31))
-        return PT_ERR_INVALID_ARG;
-    if (k < 1 || k > PT_MAX_K) return PT_ERR_UNSUPPORTED;
-    if ((bake_wants_frames(o) || heights) && !bake_corners_fit(n_faces)) return PT_ERR_UNSUPPORTED;
+    if (!ix) return PT_ERR_INVALID_ARG;
+    const int rc = bake_check_args(vertices, n_vertices, faces, n_faces, k, resolution, o, height);
+    if (rc != PT_OK) return rc;
     if (ix->ids) return PT_ERR_UNSUPPORTED;           // slab indexes answer with global ids
     if (!ix->attrs && ix->n) return PT_ERR_INVALID_ARG;
     if (pt_device_count() == 0) return PT_ERR_NO_DEVICE;
@@ -1549,8 +1686,8 @@ extern "C" int pt_bake_compose_height_device(const double *vertices_xyzuvn, cons
             break;
         bake_height_fill_kernel<<<148 * 8, 256, 0, s>>>(h, n_pix);
         count_launch();
-        if ((rc = launch_height(M, frames, texels, sample_faces, sample_xyz, count, idx, k, PosPlain{cloud_xyz},
-                                (uint32_t)n_points, h, s)) != PT_OK)
+        if ((rc = launch_height<false>(M, frames, texels, sample_faces, sample_xyz, count, idx, k, PosPlain{cloud_xyz},
+                                       (uint32_t)n_points, h, s)) != PT_OK)
             break;
         rc = bake_height_finish(h, resolution, pad, range_in, range, height_u16_out, nullptr, s);
     } while (0);

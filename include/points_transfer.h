@@ -420,6 +420,24 @@ int pt_sharded_knn(pt_sharded *sharded, const void *queries, size_t m, int k, do
                    int32_t *idx_out, double *d2_out);
 int pt_sharded_transfer(pt_sharded *sharded, const void *queries, size_t m, int k, double radius,
                         int32_t *idx_out, double *d2_out, uint8_t *rgba_out, float *normal_out);
+/* pt_texture_bake_height on the sharded cloud (DESIGN.md section 8, "Sharded bake"): same arguments,
+ * argument rules, error codes and output layouts, and every output -- maps, vertex_tangents, height
+ * (NaN bits included), height_u16, range_used, height->texels, stats->texels, stats->empty -- is
+ * byte-identical to pt_texture_bake_height on one pt_index built from the same cloud, for any slab
+ * count and device list.  Slab 0's device (the home device) rasterises the texels, builds the frames
+ * and composes, encodes and pads the maps; every slab answers the samples in its x-range on its own
+ * device, heights included, from its own records.  A ghost zone found too narrow widens the halo and
+ * rebuilds the slabs as pt_sharded_transfer does (counted in `rebuilds`).  Stats:
+ *   raster_ms  device time on the home device: upload, raster, compaction, frames
+ *   knn_ms     host wall time of routing the samples, the copies between devices, the slabs'
+ *              queries, ghost checks and heights, and the scatter back into sample order, ending
+ *              in a synchronise
+ *   pad_ms     device time on the home device: composition, tangent maps, height range and
+ *              encoding, padding */
+int pt_sharded_bake(pt_sharded *sharded, const void *vertices, size_t n_vertices,
+                    const int32_t *faces, size_t n_faces, int k, double radius,
+                    int resolution, int pad, const pt_bake_outputs *out /* may be NULL */,
+                    pt_bake_height *height /* may be NULL, not both */, pt_bake_stats *stats);
 
 /* pt_texture_render for neighbour lists that were computed elsewhere (e.g. pt_sharded_knn): the
  * cloud's positions and colours are uploaded to `device` in original order, idx[n_vertices * k]
