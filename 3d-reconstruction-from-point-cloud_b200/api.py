@@ -53,6 +53,7 @@ ABI_SYMBOLS = (
     "pt_texture_bake", "pt_bake_texels_device", "pt_bake_compose_device",
     "pt_texture_bake_ex", "pt_bake_samples_device", "pt_bake_frames_device", "pt_bake_compose_tangent_device",
     "pt_texture_bake_height", "pt_bake_compose_height_device", "pt_sharded_bake",
+    "pt_index_estimate_normals", "pt_estimate_normals_device",
 )
 # ... and include/pt_synth.h (bench / test scaffolding, its own library)
 SYNTH_SYMBOLS = ("pt_synth_cloud_device", "pt_synth_samples_device", "pt_synth_pack_points_device",
@@ -100,6 +101,10 @@ class BakeOutputs(ctypes.Structure):
 class BakeHeight(ctypes.Structure):
     _fields_ = [("height", ctypes.c_void_p), ("height_u16", ctypes.c_void_p), ("range", ctypes.c_double * 2),
                 ("range_used", ctypes.c_double * 2), ("texels", ctypes.c_uint64)]
+
+
+class NormalsStats(ctypes.Structure):
+    _fields_ = [("estimated", ctypes.c_uint64), ("knn_ms", ctypes.c_float), ("pca_ms", ctypes.c_float)]
 
 
 class ShardedOpts(ctypes.Structure):
@@ -211,6 +216,10 @@ def lib():
     L.pt_bake_compose_height_device.restype = i32
     L.pt_bake_compose_height_device.argtypes = [vp, vp, sz, vp, sz, vp, vp, vp, sz, vp, i32, vp, sz, i32, i32, vp, vp,
                                                 vp, vp, i32, vp]
+    L.pt_index_estimate_normals.restype = i32
+    L.pt_index_estimate_normals.argtypes = [vp, i32, dbl, vp, i32, vp, vp, ctypes.POINTER(NormalsStats)]
+    L.pt_estimate_normals_device.restype = i32
+    L.pt_estimate_normals_device.argtypes = [vp, i32, dbl, vp, i32, vp, vp, vp]
     L.pt_set_option.restype = i32
     L.pt_set_option.argtypes = [ctypes.c_char_p, i32]
     L.pt_get_option.restype = i32
@@ -311,6 +320,10 @@ def _as_points(a, what):
 
 def _radius(radius):
     return -1.0 if radius is None else float(radius)
+
+
+def _viewpoint(viewpoint):
+    return None if viewpoint is None else ctypes.cast((ctypes.c_double * 3)(*map(float, viewpoint)), ctypes.c_void_p)
 
 
 def _np_ptr(a):
@@ -459,6 +472,23 @@ class Tree:
         All outputs come from one k-NN pass."""
         return _bake(lib().pt_texture_bake_height, "pt_texture_bake_height", self._h, vertices, faces, k, resolution,
                      radius, pad, want, height_range)
+
+    def estimate_normals(self, k=16, radius=None, viewpoint=None, store=False):
+        """PCA normal estimation over each point's k nearest neighbours (DESIGN.md section 8, "Normal
+        estimation").  Returns a dict with ``normal`` float32 [n,3] ((0, 0, 0) without an estimate),
+        ``variation`` float32 [n] (surface variation, NaN without an estimate), both in the order of
+        the points the tree was built from, and ``stats`` (estimated, knn_ms, pca_ms).  Orientation:
+        the point's own normal where it is usable, else towards ``viewpoint`` (x, y, z) when given,
+        else the largest component positive.  ``store=True`` also replaces the tree's normals with
+        the estimates, so later ``transfer`` / ``bake`` calls blend them."""
+        n = self.size()
+        out = {"normal": np.empty((n, 3), dtype=np.float32), "variation": np.empty(n, dtype=np.float32)}
+        st = NormalsStats()
+        _check(lib().pt_index_estimate_normals(self._h, int(k), _radius(radius), _viewpoint(viewpoint),
+                                               1 if store else 0, _np_ptr(out["normal"]), _np_ptr(out["variation"]),
+                                               ctypes.byref(st)), "pt_index_estimate_normals")
+        out["stats"] = {"estimated": int(st.estimated), "knn_ms": st.knn_ms, "pca_ms": st.pca_ms}
+        return out
 
     def transfer_slab(self, queries_ptr, queries_are_xyz, m, k, radius, boxes6, rank, halo,
                       idx_ptr, rgba_ptr, normal_ptr, d2_ptr=None):
@@ -662,6 +692,22 @@ class DeviceTree(Tree):
                                          _tptr(radius2_per_query), _tptr(idx), _tptr(d2),
                                          _tptr(rgba), _tptr(normal), _tptr(cand),
                                          _stream_ptr(stream)), "pt_query_device")
+
+
+    def estimate_normals(self, k=16, radius=None, viewpoint=None, store=False, normal=None, variation=None,
+                         stream=None):
+        """``Tree.estimate_normals`` into pre-allocated CUDA tensors (``normal`` float32 [n,3],
+        ``variation`` float32 [n], either may be None; both None needs ``store``), asynchronous on
+        ``stream`` (default: torch's current stream)."""
+        import torch
+        n = self.size()
+        for t, cnt in ((normal, 3 * n), (variation, n)):
+            if t is not None:
+                assert t.is_cuda and t.is_contiguous() and t.dtype == torch.float32 and t.numel() == cnt
+        with torch.cuda.device(self.torch_device):
+            _check(lib().pt_estimate_normals_device(self._h, int(k), _radius(radius), _viewpoint(viewpoint),
+                                                    1 if store else 0, _tptr(normal), _tptr(variation),
+                                                    _stream_ptr(stream)), "pt_estimate_normals_device")
 
 
 def merge_device(lists, n_lists, m, k, idx=None, d2=None, rgba=None, normal=None, cand=None,

@@ -22,7 +22,7 @@ struct pt_index {
     pt::GridParams grid{};                // tables of this index (n_tables == 0: none)
     uint64_t     level_cells[22]{};       // occupied cells per lattice level (0: not counted)
     uint32_t    *fallback_word = nullptr; // device: samples the last launch handed to the warp kernel
-    uint32_t    *inv_perm = nullptr;      // original index -> position in pts (pt_texture.cu, built on demand)
+    uint32_t    *inv_perm = nullptr;      // original index -> position in pts (index_inverse_perm, built on demand)
     uint64_t     device_bytes = 0;
     cudaStream_t stream = nullptr;
     cudaEvent_t  ev[4]{};
@@ -82,6 +82,8 @@ int launch_query(pt_index *ix, const QueryParams &qp, cudaStream_t s);
 void fill_params(const pt_index *ix, QueryParams &qp);
 // squared radius bound: +inf for a negative, NaN or infinite radius
 double radius_to_r2(double radius);
+// ix->inv_perm (original index -> position in pts), built on ix->stream on first use (pt_texture.cu)
+int index_inverse_perm(pt_index *ix);
 // Stream-ordered allocation from the library's PRIVATE memory pool of the current device (the
 // application's default pool is never touched); release with pool_free.  dev_alloc / dev_free:
 // cudaMalloc / cudaFree for the long-lived buffers.  Both carry guard words under "pool_guard".

@@ -1,0 +1,389 @@
+// pt_normals.cu -- PCA normal estimation over each cloud point's k nearest neighbours (DESIGN.md
+// section 8, "Normal estimation"; CGAL's pca_estimate_normals, Open3D's and PCL's estimators).
+//
+// Per chunk of at most HEIGHT_CHUNK sorted records: the records' positions become the query rows
+// (row r = sorted record r, so the k-NN kernels see coherent samples), one launch_query writes the
+// neighbour lists, and normals_pca_kernel turns every list into a normal and a surface variation.
+// Everything is fp64 with every operation rounded on its own, in the order DESIGN.md states, so
+// that oracle/pt_normals_oracle.c equals it bit for bit.
+#include <algorithm>
+#include <cmath>
+#include <vector>
+
+#include "pt_bake.cuh"
+#include "pt_fp64.cuh"
+
+namespace pt {
+
+constexpr uint32_t NORMALS_NAN = 0x7fc00000u;   // the variation of a point without an estimate
+constexpr int JACOBI_MAX_SWEEPS = 50;
+
+static inline unsigned ncdiv(size_t a, size_t b) { return (unsigned)((a + b - 1) / b); }
+
+template <typename PT>
+__global__ void __launch_bounds__(256) normals_rows_kernel(const PT *pts, uint32_t r0, uint32_t count, double *xyz)
+{
+    const uint32_t i = blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= count) return;
+    const PT rec = pts[r0 + i];
+    xyz[3 * (size_t)i] = (double)rec.x;
+    xyz[3 * (size_t)i + 1] = (double)rec.y;
+    xyz[3 * (size_t)i + 2] = (double)rec.z;
+}
+
+// ROTATE of Numerical Recipes' jacobi: (g, h) <- (g - s (h + g tau), h + s (g - h tau))
+__device__ __forceinline__ void jacobi_rotate(double &gr, double &hr, double s, double tau)
+{
+    const double g = gr, h = hr;
+    gr = __dsub_rn(g, __dmul_rn(s, __dadd_rn(h, __dmul_rn(g, tau))));
+    hr = __dadd_rn(h, __dmul_rn(s, __dsub_rn(g, __dmul_rn(h, tau))));
+}
+
+// pivot (P, Q) of sweep `sweep` (1-based); a holds the upper triangle
+template <int P, int Q>
+__device__ __forceinline__ void jacobi_pivot(double a[3][3], double v[3][3], double d[3], double z[3], int sweep,
+                                             double tresh)
+{
+    const double apq = a[P][Q];
+    const double g = __dmul_rn(100.0, fabs(apq));
+    if (sweep > 4 && __dadd_rn(fabs(d[P]), g) == fabs(d[P]) && __dadd_rn(fabs(d[Q]), g) == fabs(d[Q])) {
+        a[P][Q] = 0.0;
+        return;
+    }
+    if (!(fabs(apq) > tresh)) return;
+    double h = __dsub_rn(d[Q], d[P]);
+    double t;
+    if (__dadd_rn(fabs(h), g) == fabs(h)) {
+        t = __ddiv_rn(apq, h);
+    } else {
+        const double theta = __ddiv_rn(__dmul_rn(0.5, h), apq);
+        t = __ddiv_rn(1.0, __dadd_rn(fabs(theta), __dsqrt_rn(__dadd_rn(1.0, __dmul_rn(theta, theta)))));
+        if (theta < 0.0) t = -t;
+    }
+    const double c = __ddiv_rn(1.0, __dsqrt_rn(__dadd_rn(1.0, __dmul_rn(t, t))));
+    const double s = __dmul_rn(t, c);
+    const double tau = __ddiv_rn(s, __dadd_rn(1.0, c));
+    h = __dmul_rn(t, apq);
+    z[P] = __dsub_rn(z[P], h);
+    z[Q] = __dadd_rn(z[Q], h);
+    d[P] = __dsub_rn(d[P], h);
+    d[Q] = __dadd_rn(d[Q], h);
+    a[P][Q] = 0.0;
+    if (P == 0 && Q == 1) jacobi_rotate(a[0][2], a[1][2], s, tau);
+    if (P == 0 && Q == 2) jacobi_rotate(a[0][1], a[1][2], s, tau);
+    if (P == 1 && Q == 2) jacobi_rotate(a[0][1], a[0][2], s, tau);
+#pragma unroll
+    for (int j = 0; j < 3; ++j) jacobi_rotate(v[j][P], v[j][Q], s, tau);
+}
+
+// Cyclic Jacobi on the symmetric scatter matrix: eigenvalues d, eigenvectors in the columns of v.
+__device__ __forceinline__ void jacobi3(const double c[6], double d[3], double v[3][3])
+{
+    double a[3][3] = {{c[0], c[1], c[2]}, {0.0, c[3], c[4]}, {0.0, 0.0, c[5]}};
+    double b[3] = {c[0], c[3], c[5]}, z[3] = {0.0, 0.0, 0.0};
+#pragma unroll
+    for (int i = 0; i < 3; ++i) {
+        d[i] = b[i];
+#pragma unroll
+        for (int j = 0; j < 3; ++j) v[i][j] = i == j ? 1.0 : 0.0;
+    }
+    for (int sweep = 1; sweep <= JACOBI_MAX_SWEEPS; ++sweep) {
+        const double sm = __dadd_rn(__dadd_rn(fabs(a[0][1]), fabs(a[0][2])), fabs(a[1][2]));
+        if (sm == 0.0) break;
+        const double tresh = sweep < 4 ? __ddiv_rn(__dmul_rn(0.2, sm), 9.0) : 0.0;
+        jacobi_pivot<0, 1>(a, v, d, z, sweep, tresh);
+        jacobi_pivot<0, 2>(a, v, d, z, sweep, tresh);
+        jacobi_pivot<1, 2>(a, v, d, z, sweep, tresh);
+#pragma unroll
+        for (int i = 0; i < 3; ++i) {
+            b[i] = __dadd_rn(b[i], z[i]);
+            d[i] = b[i];
+            z[i] = 0.0;
+        }
+    }
+}
+
+struct NormalsOut {
+    const pt_attr *attrs;     // input normals, original order (may be null: rule (a) never applies)
+    pt_attr *store;           // store: attrs (original order), else null
+    pt_attr *store_curve;     // store: attrs_curve (sorted order) where the index has it, else null
+    int has_view;
+    double vx, vy, vz;
+    float *normal;            // n x 3, original order (may be null)
+    float *variation;         // n, original order (may be null)
+    unsigned long long *estimated;   // += points with an estimate (may be null)
+};
+
+// A warp takes 32 consecutive rows (sorted records r0 + base ..).  It walks them in `width` rounds, a
+// group of `width` (the power of two >= k) lanes per row: lane j of a group gathers neighbour j
+// through the inverse permutation (independent random reads, in parallel), and the group forms the
+// centroid and then the six scatter sums in neighbour order through shuffles.  The sums go to the
+// row's own lane, and after the rounds every lane solves its row's 3 x 3 on its own, so the Jacobi
+// sweeps run 32 rows wide.  Every lane runs the same loops, so the shuffles see the full warp.
+template <typename PT>
+__global__ void __launch_bounds__(256)
+normals_pca_kernel(const PT *pts, const uint32_t *inv, uint32_t n_points, uint32_t r0, uint32_t count,
+                   const int32_t *idx, int k, int width, const NormalsOut o)
+{
+    const unsigned lane = threadIdx.x & 31u;
+    const uint32_t base = (uint32_t)(((size_t)blockIdx.x * blockDim.x + threadIdx.x) >> 5) * 32u;
+    if (base >= count) return;                                    // warp-uniform
+    const bool mine = base + lane < count;
+    const PosSorted<PT> pos{pts, inv};
+    double c[6] = {0.0, 0.0, 0.0, 0.0, 0.0, 0.0};
+    int my_cnt = 0;
+    const unsigned per_round = 32u / (unsigned)width;
+    const unsigned g = lane / (unsigned)width, j = lane % (unsigned)width, g0 = g * (unsigned)width;
+    const int from = (int)((lane % per_round) * (unsigned)width);  // a lane of the group that sums my row
+    for (unsigned r = 0; r < (unsigned)width; ++r) {
+        const uint32_t s = base + r * per_round + g;
+        bool has = false;
+        D3 p = {0.0, 0.0, 0.0};
+        if (s < count && (int)j < k) {
+            const int id = idx[(size_t)s * k + j];
+            if (id >= 0 && (uint32_t)id < n_points) {
+                double x[3];
+                pos.get(id, x);
+                p = D3{x[0], x[1], x[2]};
+                has = true;
+            }
+        }
+        // the list is its leading run of valid entries
+        const unsigned seg = (__ballot_sync(0xffffffffu, has) >> g0) & (width == 32 ? 0xffffffffu : ((1u << width) - 1u));
+        const int cnt = __ffsll(~(unsigned long long)seg) - 1;
+        D3 sum = {0.0, 0.0, 0.0};
+        for (int jj = 0; jj < k; ++jj) {
+            const D3 q = {shfl_d(p.x, (int)g0 + jj), shfl_d(p.y, (int)g0 + jj), shfl_d(p.z, (int)g0 + jj)};
+            if (jj < cnt) sum = d3_add(sum, q);
+        }
+        const double dc = (double)cnt;
+        const D3 e = d3_sub(p, D3{__ddiv_rn(sum.x, dc), __ddiv_rn(sum.y, dc), __ddiv_rn(sum.z, dc)});
+        const double t[6] = {__dmul_rn(e.x, e.x), __dmul_rn(e.x, e.y), __dmul_rn(e.x, e.z),
+                             __dmul_rn(e.y, e.y), __dmul_rn(e.y, e.z), __dmul_rn(e.z, e.z)};
+        double acc[6] = {0.0, 0.0, 0.0, 0.0, 0.0, 0.0};
+        for (int jj = 0; jj < k; ++jj) {
+#pragma unroll
+            for (int a = 0; a < 6; ++a) {
+                const double tj = shfl_d(t[a], (int)g0 + jj);
+                if (jj < cnt) acc[a] = __dadd_rn(acc[a], tj);
+            }
+        }
+        const bool take = lane / per_round == r;
+#pragma unroll
+        for (int a = 0; a < 6; ++a) {
+            const double v = shfl_d(acc[a], from);
+            if (take) c[a] = v;
+        }
+        const int tc = __shfl_sync(0xffffffffu, cnt, from);
+        if (take) my_cnt = tc;
+    }
+    if (!mine) return;
+
+    const uint32_t row = r0 + base + lane;
+    const PT rec = pts[row];
+    const uint32_t orig = (uint32_t)rec.idx;
+    const D3 pi = {(double)rec.x, (double)rec.y, (double)rec.z};
+    const double trace = __dadd_rn(__dadd_rn(c[0], c[3]), c[5]);
+    bool est = my_cnt >= 3 && trace > 0.0 && trace < INFINITY;
+    D3 n = {0.0, 0.0, 0.0};
+    double lam0 = 0.0;
+    if (est) {
+        double d[3], v[3][3];
+        jacobi3(c, d, v);
+        // the smallest eigenvalue, the lower column on ties (selects, not a dynamic index: no local memory)
+        lam0 = d[0];
+        D3 col = {v[0][0], v[1][0], v[2][0]};
+        if (d[1] < lam0) { lam0 = d[1]; col = D3{v[0][1], v[1][1], v[2][1]}; }
+        if (d[2] < lam0) { lam0 = d[2]; col = D3{v[0][2], v[1][2], v[2][2]}; }
+        n = d3_normalise(col);
+        est = d3_usable(n);
+    }
+    if (est) {
+        bool flip;
+        const pt_attr m = o.attrs ? o.attrs[orig] : pt_attr{};
+        const D3 md = {(double)m.nx, (double)m.ny, (double)m.nz};
+        if (o.attrs && d3_usable(md)) {
+            flip = d3_dot(n, md) < 0.0;                                             // (a) input normal
+        } else if (o.has_view) {
+            flip = d3_dot(n, d3_sub(D3{o.vx, o.vy, o.vz}, pi)) < 0.0;               // (b) viewpoint
+        } else {
+            const double ax = fabs(n.x), ay = fabs(n.y), az = fabs(n.z);      // (c) largest component
+            flip = (ax >= ay && ax >= az) ? n.x < 0.0 : (ay >= az ? n.y < 0.0 : n.z < 0.0);
+        }
+        if (flip) n = D3{-n.x, -n.y, -n.z};
+    }
+    const float fx = __double2float_rn(n.x), fy = __double2float_rn(n.y), fz = __double2float_rn(n.z);
+    if (o.normal) {
+        o.normal[3 * (size_t)orig] = fx;
+        o.normal[3 * (size_t)orig + 1] = fy;
+        o.normal[3 * (size_t)orig + 2] = fz;
+    }
+    if (o.variation)
+        o.variation[orig] = est ? __double2float_rn(__ddiv_rn(lam0 > 0.0 ? lam0 : 0.0, trace)) : __uint_as_float(NORMALS_NAN);
+    if (est && o.store) {
+        o.store[orig].nx = fx; o.store[orig].ny = fy; o.store[orig].nz = fz;
+        if (o.store_curve) { o.store_curve[row].nx = fx; o.store_curve[row].ny = fy; o.store_curve[row].nz = fz; }
+    }
+    if (o.estimated) {
+        const unsigned act = __activemask();
+        const unsigned got = __ballot_sync(act, est);
+        if (got && lane == (unsigned)(__ffs(act) - 1)) atomicAdd(o.estimated, (unsigned long long)__popc(got));
+    }
+}
+
+static int normals_width(int k)
+{
+    int w = 1;
+    while (w < k) w <<= 1;
+    return w;
+}
+
+// All points of ix in chunks, asynchronous on s.  marks (may be null): an event before the first
+// chunk and after each chunk's query and PCA kernel.
+template <typename PT>
+static int normals_run(pt_index *ix, int k, double radius, const NormalsOut &o, std::vector<cudaEvent_t> *marks,
+                       cudaStream_t s)
+{
+    const uint32_t n = ix->n;
+    const size_t chunk = std::min((size_t)HEIGHT_CHUNK, (size_t)n);
+    double *d_q = nullptr;
+    int32_t *d_idx = nullptr;
+    int rc = PT_OK;
+    auto fail = [&](cudaError_t e) { if (e != cudaSuccess && rc == PT_OK) rc = map_cuda_error(e); return e != cudaSuccess; };
+    auto mark = [&]() {
+        if (!marks) return false;
+        marks->emplace_back();
+        return fail(cudaEventCreate(&marks->back())) || fail(cudaEventRecord(marks->back(), s));
+    };
+    do {
+        if (mark()) break;
+        // built once per index on its own stream, which every later user of it is ordered after
+        const bool fresh = ix->inv_perm == nullptr;
+        if ((rc = index_inverse_perm(ix)) != PT_OK) break;
+        if (fresh && s != ix->stream && fail(cudaStreamSynchronize(ix->stream))) break;
+        if (pool_alloc((void **)&d_q, sizeof(double) * 3 * chunk, s) || pool_alloc((void **)&d_idx, sizeof(int32_t) * k * chunk, s)) {
+            rc = PT_ERR_OUT_OF_MEMORY;
+            break;
+        }
+        QueryParams qp{};
+        fill_params(ix, qp);
+        qp.ids = nullptr;          // the index's own ids: the PCA kernel reads its records by them
+        qp.k = k;
+        qp.r2 = radius_to_r2(radius);
+        qp.queries = d_q;
+        qp.idx_out = d_idx;
+        const PT *pts = (const PT *)ix->pts;
+        for (size_t c0 = 0; c0 < n; c0 += chunk) {
+            const uint32_t cm = (uint32_t)std::min(chunk, (size_t)n - c0);
+            normals_rows_kernel<PT><<<ncdiv(cm, 256), 256, 0, s>>>(pts, (uint32_t)c0, cm, d_q);
+            count_launch();
+            qp.m = cm;
+            if ((rc = launch_query(ix, qp, s)) != PT_OK) break;
+            if (mark()) break;
+            normals_pca_kernel<PT><<<ncdiv(cm, 256), 256, 0, s>>>(pts, ix->inv_perm, n, (uint32_t)c0, cm, d_idx, k,
+                                                                  normals_width(k), o);
+            count_launch();
+            if (fail(cudaGetLastError()) || mark()) break;
+        }
+    } while (0);
+    pool_free(d_q, s);
+    pool_free(d_idx, s);
+    return rc;
+}
+
+static int normals_check(const pt_index *ix, int k, const double *viewpoint, bool store, bool any_output)
+{
+    if (!ix || (!any_output && !store)) return PT_ERR_INVALID_ARG;
+    if (viewpoint && !(std::isfinite(viewpoint[0]) && std::isfinite(viewpoint[1]) && std::isfinite(viewpoint[2])))
+        return PT_ERR_INVALID_ARG;
+    if (k < 3) return PT_ERR_INVALID_ARG;             // a plane needs three points
+    if (k > PT_MAX_K) return PT_ERR_UNSUPPORTED;
+    if (store && !ix->attrs && ix->n) return PT_ERR_INVALID_ARG;
+    if (pt_device_count() == 0) return PT_ERR_NO_DEVICE;
+    return PT_OK;
+}
+
+static NormalsOut normals_out(pt_index *ix, const double *viewpoint, bool store, float *normal, float *variation,
+                              unsigned long long *estimated)
+{
+    NormalsOut o{};
+    o.attrs = ix->attrs;
+    o.store = store ? ix->attrs : nullptr;
+    o.store_curve = store ? ix->attrs_curve : nullptr;
+    o.has_view = viewpoint ? 1 : 0;
+    if (viewpoint) { o.vx = viewpoint[0]; o.vy = viewpoint[1]; o.vz = viewpoint[2]; }
+    o.normal = normal;
+    o.variation = variation;
+    o.estimated = estimated;
+    return o;
+}
+
+static int normals_device(pt_index *ix, int k, double radius, const NormalsOut &o, std::vector<cudaEvent_t> *marks,
+                          cudaStream_t s)
+{
+    return ix->coord_f64 ? normals_run<PointD>(ix, k, radius, o, marks, s) : normals_run<PointF>(ix, k, radius, o, marks, s);
+}
+
+}  // namespace pt
+
+using namespace pt;
+
+extern "C" int pt_estimate_normals_device(pt_index *ix, int k, double radius, const double *viewpoint, int store,
+                                          float *normal_out, float *variation_out, void *stream)
+{
+    const int rc = normals_check(ix, k, viewpoint, store != 0, normal_out || variation_out);
+    if (rc != PT_OK) return rc;
+    if (ix->n == 0) return PT_OK;
+    PT_CUDA(cudaSetDevice(ix->device));
+    return normals_device(ix, k, radius, normals_out(ix, viewpoint, store != 0, normal_out, variation_out, nullptr),
+                          nullptr, (cudaStream_t)stream);
+}
+
+extern "C" int pt_index_estimate_normals(pt_index *ix, int k, double radius, const double *viewpoint, int store,
+                                         float *normal_out, float *variation_out, pt_normals_stats *stats)
+{
+    int rc = normals_check(ix, k, viewpoint, store != 0, normal_out || variation_out);
+    if (rc != PT_OK) return rc;
+    if (stats) *stats = pt_normals_stats{0, 0.0f, 0.0f};
+    if (ix->n == 0) return PT_OK;
+    PT_CUDA(cudaSetDevice(ix->device));
+    cudaStream_t s = ix->stream;
+    const size_t n = ix->n;
+    float *d_normal = nullptr, *d_var = nullptr;
+    unsigned long long *d_est = nullptr, est = 0;
+    std::vector<cudaEvent_t> marks;
+    auto fail = [&](cudaError_t e) { if (e != cudaSuccess && rc == PT_OK) rc = map_cuda_error(e); return e != cudaSuccess; };
+    do {
+        if ((normal_out && pool_alloc((void **)&d_normal, sizeof(float) * 3 * n, s)) ||
+            (variation_out && pool_alloc((void **)&d_var, sizeof(float) * n, s)) ||
+            pool_alloc((void **)&d_est, sizeof(unsigned long long), s)) {
+            rc = PT_ERR_OUT_OF_MEMORY;
+            break;
+        }
+        if (fail(cudaMemsetAsync(d_est, 0, sizeof(unsigned long long), s))) break;
+        if ((rc = normals_device(ix, k, radius, normals_out(ix, viewpoint, store != 0, d_normal, d_var, d_est), &marks, s)) !=
+            PT_OK)
+            break;
+        if (normal_out && fail(cudaMemcpyAsync(normal_out, d_normal, sizeof(float) * 3 * n, cudaMemcpyDeviceToHost, s))) break;
+        if (variation_out && fail(cudaMemcpyAsync(variation_out, d_var, sizeof(float) * n, cudaMemcpyDeviceToHost, s))) break;
+        if (fail(cudaMemcpyAsync(&est, d_est, sizeof est, cudaMemcpyDeviceToHost, s))) break;
+        if (fail(cudaStreamSynchronize(s))) break;
+        if (stats) {
+            stats->estimated = est;
+            // marks: start, then per chunk (after the query, after the PCA kernel)
+            float t = 0.0f;
+            for (size_t c = 1; c + 1 < marks.size(); c += 2) {
+                if (cudaEventElapsedTime(&t, marks[c - 1], marks[c]) == cudaSuccess) stats->knn_ms += t;
+                if (cudaEventElapsedTime(&t, marks[c], marks[c + 1]) == cudaSuccess) stats->pca_ms += t;
+            }
+        }
+    } while (0);
+    cudaStreamSynchronize(s);
+    pool_free(d_normal, s);
+    pool_free(d_var, s);
+    pool_free(d_est, s);
+    for (auto &e : marks) if (e) cudaEventDestroy(e);
+    cudaStreamSynchronize(s);
+    cudaGetLastError();
+    return rc;
+}

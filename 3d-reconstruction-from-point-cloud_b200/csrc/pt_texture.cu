@@ -29,6 +29,7 @@
 #include <thrust/iterator/counting_iterator.h>
 
 #include "pt_bake.cuh"
+#include "pt_fp64.cuh"
 
 namespace pt {
 
@@ -64,13 +65,6 @@ tex_unpack_vertices_kernel(const Raw80t *raw, uint32_t n, MeshVertex *mv, double
     m.pad = 0;
     mv[i] = m;
     xyz[3 * (size_t)i] = r.ver[0]; xyz[3 * (size_t)i + 1] = r.ver[1]; xyz[3 * (size_t)i + 2] = r.ver[2];
-}
-
-template <typename PT>
-__global__ void __launch_bounds__(256) tex_inverse_perm_kernel(const PT *pts, uint32_t n, uint32_t *inv)
-{
-    const uint32_t i = blockIdx.x * blockDim.x + threadIdx.x;
-    if (i < n) inv[pts[i].idx] = i;
 }
 
 __device__ __forceinline__ double tx_area2(V2 p, V2 q, V2 r)
@@ -143,16 +137,6 @@ __device__ void tx_draw_triangle(const TexVertex &t0, const TexVertex &t1, const
     }
 }
 
-// where the position of cloud point `id` (original index) comes from
-template <typename PT> struct PosSorted {      // an index: sorted records + inverse permutation
-    const PT *pts;
-    const uint32_t *inv;
-    __device__ __forceinline__ void get(int id, double x[3]) const
-    {
-        const PT rec = pts[inv[id]];
-        x[0] = (double)rec.x; x[1] = (double)rec.y; x[2] = (double)rec.z;
-    }
-};
 struct PosPlain {                               // n x 3 doubles in original order
     const double *xyz;
     __device__ __forceinline__ void get(int id, double x[3]) const
@@ -438,13 +422,21 @@ static int texture_pipeline(pt_index *ix, POS pos, uint32_t n_points, const pt_a
     return rc;
 }
 
-// original index -> position in the sorted cloud, built once per index
 template <typename PT>
-static int index_inverse_perm(pt_index *ix)
+__global__ void __launch_bounds__(256) tex_inverse_perm_kernel(const PT *pts, uint32_t n, uint32_t *inv)
+{
+    const uint32_t i = blockIdx.x * blockDim.x + threadIdx.x;
+    if (i < n) inv[pts[i].idx] = i;
+}
+
+int index_inverse_perm(pt_index *ix)
 {
     if (!ix->inv_perm && ix->n) {
         PT_TRY(dev_alloc((void **)&ix->inv_perm, sizeof(uint32_t) * (size_t)ix->n));
-        tex_inverse_perm_kernel<PT><<<tcdiv(ix->n, 256), 256, 0, ix->stream>>>((const PT *)ix->pts, ix->n, ix->inv_perm);
+        if (ix->coord_f64)
+            tex_inverse_perm_kernel<PointD><<<tcdiv(ix->n, 256), 256, 0, ix->stream>>>((const PointD *)ix->pts, ix->n, ix->inv_perm);
+        else
+            tex_inverse_perm_kernel<PointF><<<tcdiv(ix->n, 256), 256, 0, ix->stream>>>((const PointF *)ix->pts, ix->n, ix->inv_perm);
         count_launch();
     }
     return PT_OK;
@@ -455,7 +447,7 @@ static int texture_render_index(pt_index *ix, const void *vertices, size_t n_ver
                                 size_t n_faces, int k, double radius, int res, int pad, uint8_t *bgra_out,
                                 pt_texture_stats *st)
 {
-    PT_TRY(index_inverse_perm<PT>(ix));
+    PT_TRY(index_inverse_perm(ix));
     PosSorted<PT> pos{(const PT *)ix->pts, ix->inv_perm};
     return texture_pipeline(ix, pos, ix->n, ix->attrs, true, nullptr, vertices, n_vertices, faces, n_faces, k, radius,
                             res, pad, bgra_out, st);
@@ -712,28 +704,6 @@ static int bake_compose(const uint32_t *texels, size_t count, const uint8_t *rgb
 // a.b = (a.x b.x + a.y b.y) + a.z b.z; "usable" = all components finite and a.a > 0; normalising
 // divides each component by sqrt(a.a).  Mesh rows are 8 doubles: x y z u v nx ny nz.  Frame rows
 // are 8 doubles: N xyz, T xyz, w, 0 -- all zero for a vertex without a frame.
-struct D3 { double x, y, z; };
-
-__device__ __forceinline__ D3 d3_add(D3 a, D3 b) { return {__dadd_rn(a.x, b.x), __dadd_rn(a.y, b.y), __dadd_rn(a.z, b.z)}; }
-__device__ __forceinline__ D3 d3_sub(D3 a, D3 b) { return {__dsub_rn(a.x, b.x), __dsub_rn(a.y, b.y), __dsub_rn(a.z, b.z)}; }
-__device__ __forceinline__ D3 d3_scale(double s, D3 a) { return {__dmul_rn(s, a.x), __dmul_rn(s, a.y), __dmul_rn(s, a.z)}; }
-__device__ __forceinline__ double d3_dot(D3 a, D3 b)
-{
-    return __dadd_rn(__dadd_rn(__dmul_rn(a.x, b.x), __dmul_rn(a.y, b.y)), __dmul_rn(a.z, b.z));
-}
-__device__ __forceinline__ D3 d3_cross(D3 a, D3 b)
-{
-    return {__dsub_rn(__dmul_rn(a.y, b.z), __dmul_rn(a.z, b.y)), __dsub_rn(__dmul_rn(a.z, b.x), __dmul_rn(a.x, b.z)),
-            __dsub_rn(__dmul_rn(a.x, b.y), __dmul_rn(a.y, b.x))};
-}
-__device__ __forceinline__ bool d3_finite(D3 a) { return isfinite(a.x) && isfinite(a.y) && isfinite(a.z); }
-__device__ __forceinline__ bool d3_usable(D3 a) { return d3_finite(a) && d3_dot(a, a) > 0.0; }
-__device__ __forceinline__ D3 d3_normalise(D3 a)
-{
-    const double l = __dsqrt_rn(d3_dot(a, a));
-    return {__ddiv_rn(a.x, l), __ddiv_rn(a.y, l), __ddiv_rn(a.z, l)};
-}
-__device__ __forceinline__ D3 d3_load(const double *p) { return {p[0], p[1], p[2]}; }
 // (b0 a + b1 b) + b2 c, per component
 __device__ __forceinline__ D3 d3_mix(const double bc[3], D3 a, D3 b, D3 c)
 {
@@ -972,8 +942,6 @@ __global__ void __launch_bounds__(256) bake_unpack_vertices_kernel(const Raw80t 
 // NaN (always the quiet NaN 0x7fc00000) is "no value".
 constexpr uint32_t HEIGHT_NAN = 0x7fc00000u;
 
-__device__ __forceinline__ double shfl_d(double v, int src) { return __shfl_sync(0xffffffffu, v, src); }
-
 // A warp takes 32 consecutive samples.  First each lane computes the normal of one of them; then
 // the warp walks them in `width` rounds, a group of `width` (the power of two >= k) lanes per
 // sample: lane j of a group gathers neighbour j through the position source (independent random
@@ -1200,7 +1168,7 @@ static int launch_height_index(pt_index *ix, const BakeMesh &M, const double *fr
                                const int32_t *sample_faces, const double *xyz, size_t count, const int32_t *idx, int k,
                                float *height, bool by_sample, cudaStream_t s)
 {
-    PT_TRY(index_inverse_perm<PT>(ix));
+    PT_TRY(index_inverse_perm(ix));
     const PosSorted<PT> pos{(const PT *)ix->pts, ix->inv_perm};
     return by_sample ? launch_height<true>(M, frames, texels, sample_faces, xyz, count, idx, k, pos, ix->n, height, s)
                      : launch_height<false>(M, frames, texels, sample_faces, xyz, count, idx, k, pos, ix->n, height, s);

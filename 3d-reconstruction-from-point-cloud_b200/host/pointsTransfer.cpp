@@ -19,7 +19,9 @@
 // same -R, -k, -r) and write them as PNG; -t FILE writes the tangent-space normal map as PNG and
 // -T FILE the input mesh as PLY with the per-vertex tangents (tx ty tz tw) that map is expressed
 // in, -H FILE the height map as a 16-bit greyscale PNG over the heights' own range (printed as
-// "Height range: lo hi").  All of them come from one bake.
+// "Height range: lo hi").  All of them come from one bake.  -e K first estimates the cloud's normals
+// by PCA over each point's K nearest neighbours (pt_index_estimate_normals) and stores them in the
+// index, so the transfer and the bake blend them: for scans whose nx ny nz columns are zero or noisy.
 #include <algorithm>
 #include <charconv>
 #include <chrono>
@@ -252,6 +254,8 @@ static int run(int argc, char **argv)
     std::string bake_name, normal_name;            // optional extras: the per-texel colour / normal maps
     std::string tangent_name, tangent_ply_name;    // ... the tangent-space normal map, the mesh with tangents
     std::string height_name;                       // ... the height map
+    bool estimate = false;                         // -e K: estimate the cloud's normals first
+    int estimate_k = 0;
     for (int i = 1; i < argc; ++i) {
         std::string a = argv[i];
         if (a == "-k" && i + 1 < argc) K = atoi(argv[++i]);
@@ -266,6 +270,7 @@ static int run(int argc, char **argv)
         else if (a == "-t" && i + 1 < argc) tangent_name = argv[++i];
         else if (a == "-T" && i + 1 < argc) tangent_ply_name = argv[++i];
         else if (a == "-H" && i + 1 < argc) height_name = argv[++i];
+        else if (a == "-e" && i + 1 < argc) { estimate = true; estimate_k = atoi(argv[++i]); }
         else pos_args.push_back(a);
     }
     if (pos_args.size() < 2) {
@@ -275,6 +280,10 @@ static int run(int argc, char **argv)
     if (K < 1 || K > PT_MAX_K || resolution < 1 || resolution > 32768 || n_gpus < 1 || n_gpus > 64) {
         // like every error path of the reference: a message, exit code 0
         std::cerr << "-k must be 1.." << PT_MAX_K << ", -R 1..32768 and -g 1..64" << std::endl;
+        return 0;
+    }
+    if (estimate && (estimate_k < 3 || estimate_k > PT_MAX_K || n_gpus > 1)) {
+        std::cerr << "-e must be 3.." << PT_MAX_K << " and estimates normals on one GPU (no -g)" << std::endl;
         return 0;
     }
     const bool bake = !bake_name.empty() || !normal_name.empty() || !tangent_name.empty() || !tangent_ply_name.empty() ||
@@ -326,6 +335,18 @@ static int run(int argc, char **argv)
     }
     std::cout << "Built Kd tree in: " << task_timer.time() << " seconds" << std::endl;
     task_timer.reset();
+    if (estimate) {
+        pt_normals_stats ns;
+        rc = pt_index_estimate_normals(index, estimate_k, radius, nullptr, 1, nullptr, nullptr, &ns);
+        if (rc != PT_OK) {
+            std::cerr << "pt_index_estimate_normals failed: " << pt_status_string(rc) << std::endl;
+            pt_index_free(index);
+            return 0;
+        }
+        std::cout << "Estimated normals: " << ns.estimated << " of " << points.size() << " points in "
+                  << task_timer.time() << " seconds" << std::endl;
+        task_timer.reset();
+    }
 
     Tokens mesh;
     if (!mesh.load(mesh_file_name)) {

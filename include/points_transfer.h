@@ -234,6 +234,36 @@ int pt_texture_bake_height(pt_index *index, const void *vertices, size_t n_verti
                            int resolution, int pad, const pt_bake_outputs *out /* may be NULL */,
                            pt_bake_height *height /* may be NULL, not both */, pt_bake_stats *stats);
 
+/* Normal estimation (DESIGN.md section 8, "Normal estimation"): the cloud's own normals by PCA over
+ * each point's k nearest neighbours, for clouds whose normals are missing (zero) or noisy.  Per
+ * point i: its k-NN list on this index (k, radius as pt_knn; the list normally holds i itself), no
+ * estimate with fewer than 3 entries; the centroid and the 3 x 3 scatter of the neighbours, no
+ * estimate when its trace is 0 (all neighbours at one position); cyclic Jacobi, and the unit
+ * eigenvector of the smallest eigenvalue is the normal.  Orientation, first rule that applies:
+ * (a) the point's input normal m is usable (finite, m.m > 0): n.m >= 0; (b) a viewpoint v is given:
+ * n.(v - p_i) >= 0; (c) the component of largest magnitude is >= 0 (lowest axis on ties).
+ * Everything is fp64 with every operation rounded on its own, so the results are deterministic.
+ *   normal_out     n x 3 floats, original point order, (0, 0, 0) without an estimate (may be NULL)
+ *   variation_out  n floats, surface variation lambda0 / (lambda0 + lambda1 + lambda2) (PCL's
+ *                  "curvature"), the quiet NaN 0x7fc00000 without an estimate (may be NULL)
+ *   store          != 0: every estimated normal replaces the point's normal in the index's
+ *                  attributes, so later pt_transfer / bake calls blend it; points without an
+ *                  estimate keep their input normal.  An index without attributes
+ *                  (pt_index_build_device with attrs = NULL) cannot store: PT_ERR_INVALID_ARG.
+ *   viewpoint      NULL or 3 finite doubles in host memory (rule (b)), else PT_ERR_INVALID_ARG
+ * Both outputs may be NULL only with store set.  k < 3: PT_ERR_INVALID_ARG; k > PT_MAX_K:
+ * PT_ERR_UNSUPPORTED.  The lists are kept, so the points are processed in chunks of at most 2^22
+ * (4 k bytes of lists each).  On a slab index (pt_build_opts.ids) the neighbours are that index's
+ * own points, ghost points included, and the outputs are in the index's own point order.  Host
+ * buffers, blocking; stats (may be NULL): points estimated and the device time of the k-NN and the
+ * PCA stages. */
+typedef struct pt_normals_stats {
+    uint64_t estimated;      /* points with an estimate */
+    float    knn_ms, pca_ms; /* device time of the k-NN self-queries and of the PCA kernel */
+} pt_normals_stats;
+int pt_index_estimate_normals(pt_index *index, int k, double radius, const double *viewpoint /* 3 or NULL */,
+                              int store, float *normal_out, float *variation_out, pt_normals_stats *stats);
+
 /* Device-buffer API: same operations with inputs/outputs already resident in
  * HBM on the index's device (bench `value`, multi-GPU slabs).  `stream` is a
  * cudaStream_t passed as void* (NULL = the CUDA default stream); these calls
@@ -270,6 +300,13 @@ int pt_query_device(pt_index *index, const double *queries_xyz, size_t m, int k,
                     double radius, const double *radius2_per_query,
                     int32_t *idx_out, double *d2_out, uint8_t *rgba_out,
                     float *normal_out, pt_cand *cand_out, void *stream);
+
+/* pt_index_estimate_normals on device buffers (normal_out n*3 floats, variation_out n floats, either
+ * may be NULL), asynchronous on `stream`; same arguments, rules and results.  viewpoint is in host
+ * memory.  With store the index's attributes change in `stream` order: synchronise `stream` before
+ * other calls on the index. */
+int pt_estimate_normals_device(pt_index *index, int k, double radius, const double *viewpoint, int store,
+                               float *normal_out, float *variation_out, void *stream);
 
 /* K5: merge n_lists candidate lists per query (lists[l*m*k + q*k + j], each
  * ascending, padded) into the global top-k and blend.  Runs on `device`. */
