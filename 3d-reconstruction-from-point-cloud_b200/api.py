@@ -53,7 +53,7 @@ ABI_SYMBOLS = (
     "pt_texture_bake", "pt_bake_texels_device", "pt_bake_compose_device",
     "pt_texture_bake_ex", "pt_bake_samples_device", "pt_bake_frames_device", "pt_bake_compose_tangent_device",
     "pt_texture_bake_height", "pt_bake_compose_height_device", "pt_sharded_bake",
-    "pt_index_estimate_normals", "pt_estimate_normals_device",
+    "pt_index_estimate_normals", "pt_estimate_normals_device", "pt_index_orient_normals",
 )
 # ... and include/pt_synth.h (bench / test scaffolding, its own library)
 SYNTH_SYMBOLS = ("pt_synth_cloud_device", "pt_synth_samples_device", "pt_synth_pack_points_device",
@@ -105,6 +105,11 @@ class BakeHeight(ctypes.Structure):
 
 class NormalsStats(ctypes.Structure):
     _fields_ = [("estimated", ctypes.c_uint64), ("knn_ms", ctypes.c_float), ("pca_ms", ctypes.c_float)]
+
+
+class OrientStats(ctypes.Structure):
+    _fields_ = [("oriented", ctypes.c_uint64), ("flipped", ctypes.c_uint64), ("components", ctypes.c_uint64),
+                ("edges", ctypes.c_uint64), ("knn_ms", ctypes.c_float), ("mst_ms", ctypes.c_float)]
 
 
 class ShardedOpts(ctypes.Structure):
@@ -220,6 +225,8 @@ def lib():
     L.pt_index_estimate_normals.argtypes = [vp, i32, dbl, vp, i32, vp, vp, ctypes.POINTER(NormalsStats)]
     L.pt_estimate_normals_device.restype = i32
     L.pt_estimate_normals_device.argtypes = [vp, i32, dbl, vp, i32, vp, vp, vp]
+    L.pt_index_orient_normals.restype = i32
+    L.pt_index_orient_normals.argtypes = [vp, i32, dbl, vp, i32, vp, vp, ctypes.POINTER(OrientStats)]
     L.pt_set_option.restype = i32
     L.pt_set_option.argtypes = [ctypes.c_char_p, i32]
     L.pt_get_option.restype = i32
@@ -488,6 +495,25 @@ class Tree:
                                                1 if store else 0, _np_ptr(out["normal"]), _np_ptr(out["variation"]),
                                                ctypes.byref(st)), "pt_index_estimate_normals")
         out["stats"] = {"estimated": int(st.estimated), "knn_ms": st.knn_ms, "pca_ms": st.pca_ms}
+        return out
+
+    def orient_normals(self, k=18, radius=None, viewpoint=None, store=False):
+        """Orients the tree's normals consistently by propagation along the minimum spanning forest of
+        the k-NN graph (DESIGN.md section 8, "Normal orientation").  Returns a dict with ``normal``
+        float32 [n,3] (the stored normal, negated where its sign flips; unchanged where it is not
+        usable), ``root`` int32 [n] (the id of the point's component root, -1 where it does not take
+        part), both in the order of the points the tree was built from, and ``stats`` (oriented,
+        flipped, components, edges, knn_ms, mst_ms).  Each component's root, its highest point, faces
+        ``viewpoint`` (x, y, z) when given, else +z.  ``store=True`` also replaces the tree's normals
+        with the oriented ones, so later ``transfer`` / ``bake`` calls blend them."""
+        n = self.size()
+        out = {"normal": np.empty((n, 3), dtype=np.float32), "root": np.empty(n, dtype=np.int32)}
+        st = OrientStats()
+        _check(lib().pt_index_orient_normals(self._h, int(k), _radius(radius), _viewpoint(viewpoint),
+                                             1 if store else 0, _np_ptr(out["normal"]), _np_ptr(out["root"]),
+                                             ctypes.byref(st)), "pt_index_orient_normals")
+        out["stats"] = {"oriented": int(st.oriented), "flipped": int(st.flipped), "components": int(st.components),
+                        "edges": int(st.edges), "knn_ms": st.knn_ms, "mst_ms": st.mst_ms}
         return out
 
     def transfer_slab(self, queries_ptr, queries_are_xyz, m, k, radius, boxes6, rank, halo,

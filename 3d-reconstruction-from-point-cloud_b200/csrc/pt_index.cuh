@@ -1,6 +1,9 @@
 // pt_index.cuh -- the opaque handle behind the C ABI and internal entry points.
 #pragma once
 
+#include <functional>
+#include <vector>
+
 #include "pt_common.cuh"
 
 struct pt_index {
@@ -84,6 +87,16 @@ void fill_params(const pt_index *ix, QueryParams &qp);
 double radius_to_r2(double radius);
 // ix->inv_perm (original index -> position in pts), built on ix->stream on first use (pt_texture.cu)
 int index_inverse_perm(pt_index *ix);
+// The k-NN self-query of every point of ix (pt_normals.cu), asynchronous on s, in chunks of at most
+// HEIGHT_CHUNK sorted records: row r (sorted record r) gets the list of the point it holds, in the
+// index's own ids.  keep: lists holds n x k and row r's list is at lists + r k; else lists holds one
+// chunk's rows and is reused.  then(c0, cm, lists of rows c0 .. c0 + cm) follows each chunk's query
+// and returns a status.  marks (may be null): an event before the first chunk and after each query.
+using ChunkThen = std::function<int(uint32_t c0, uint32_t cm, const int32_t *lists)>;
+int self_query_chunks(pt_index *ix, int k, double radius, int32_t *lists, bool keep, const ChunkThen &then,
+                      std::vector<cudaEvent_t> *marks, cudaStream_t s);
+// marks != null: appends an event recorded on s
+cudaError_t record_mark(std::vector<cudaEvent_t> *marks, cudaStream_t s);
 // Stream-ordered allocation from the library's PRIVATE memory pool of the current device (the
 // application's default pool is never touched); release with pool_free.  dev_alloc / dev_free:
 // cudaMalloc / cudaFree for the long-lived buffers.  Both carry guard words under "pool_guard".

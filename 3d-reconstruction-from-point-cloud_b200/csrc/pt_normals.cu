@@ -238,6 +238,62 @@ static int normals_width(int k)
     return w;
 }
 
+cudaError_t record_mark(std::vector<cudaEvent_t> *marks, cudaStream_t s)
+{
+    if (!marks) return cudaSuccess;
+    marks->emplace_back();
+    const cudaError_t e = cudaEventCreate(&marks->back());
+    return e != cudaSuccess ? e : cudaEventRecord(marks->back(), s);
+}
+
+template <typename PT>
+static int self_query_chunks_t(pt_index *ix, int k, double radius, int32_t *lists, bool keep, const ChunkThen &then,
+                               std::vector<cudaEvent_t> *marks, cudaStream_t s)
+{
+    const uint32_t n = ix->n;
+    const size_t chunk = std::min((size_t)HEIGHT_CHUNK, (size_t)n);
+    double *d_q = nullptr;
+    int rc = PT_OK;
+    auto fail = [&](cudaError_t e) { if (e != cudaSuccess && rc == PT_OK) rc = map_cuda_error(e); return e != cudaSuccess; };
+    do {
+        if (fail(record_mark(marks, s))) break;
+        // built once per index on its own stream, which every later user of it is ordered after
+        const bool fresh = ix->inv_perm == nullptr;
+        if ((rc = index_inverse_perm(ix)) != PT_OK) break;
+        if (fresh && s != ix->stream && fail(cudaStreamSynchronize(ix->stream))) break;
+        if (pool_alloc((void **)&d_q, sizeof(double) * 3 * chunk, s)) {
+            rc = PT_ERR_OUT_OF_MEMORY;
+            break;
+        }
+        QueryParams qp{};
+        fill_params(ix, qp);
+        qp.ids = nullptr;          // the index's own ids: the callers read its records by them
+        qp.k = k;
+        qp.r2 = radius_to_r2(radius);
+        qp.queries = d_q;
+        const PT *pts = (const PT *)ix->pts;
+        for (size_t c0 = 0; c0 < n; c0 += chunk) {
+            const uint32_t cm = (uint32_t)std::min(chunk, (size_t)n - c0);
+            normals_rows_kernel<PT><<<ncdiv(cm, 256), 256, 0, s>>>(pts, (uint32_t)c0, cm, d_q);
+            count_launch();
+            qp.m = cm;
+            qp.idx_out = keep ? lists + c0 * (size_t)k : lists;
+            if ((rc = launch_query(ix, qp, s)) != PT_OK) break;
+            if (fail(record_mark(marks, s))) break;
+            if ((rc = then((uint32_t)c0, cm, qp.idx_out)) != PT_OK) break;
+        }
+    } while (0);
+    pool_free(d_q, s);
+    return rc;
+}
+
+int self_query_chunks(pt_index *ix, int k, double radius, int32_t *lists, bool keep, const ChunkThen &then,
+                      std::vector<cudaEvent_t> *marks, cudaStream_t s)
+{
+    return ix->coord_f64 ? self_query_chunks_t<PointD>(ix, k, radius, lists, keep, then, marks, s)
+                         : self_query_chunks_t<PointF>(ix, k, radius, lists, keep, then, marks, s);
+}
+
 // All points of ix in chunks, asynchronous on s.  marks (may be null): an event before the first
 // chunk and after each chunk's query and PCA kernel.
 template <typename PT>
@@ -245,48 +301,20 @@ static int normals_run(pt_index *ix, int k, double radius, const NormalsOut &o, 
                        cudaStream_t s)
 {
     const uint32_t n = ix->n;
-    const size_t chunk = std::min((size_t)HEIGHT_CHUNK, (size_t)n);
-    double *d_q = nullptr;
     int32_t *d_idx = nullptr;
-    int rc = PT_OK;
-    auto fail = [&](cudaError_t e) { if (e != cudaSuccess && rc == PT_OK) rc = map_cuda_error(e); return e != cudaSuccess; };
-    auto mark = [&]() {
-        if (!marks) return false;
-        marks->emplace_back();
-        return fail(cudaEventCreate(&marks->back())) || fail(cudaEventRecord(marks->back(), s));
-    };
-    do {
-        if (mark()) break;
-        // built once per index on its own stream, which every later user of it is ordered after
-        const bool fresh = ix->inv_perm == nullptr;
-        if ((rc = index_inverse_perm(ix)) != PT_OK) break;
-        if (fresh && s != ix->stream && fail(cudaStreamSynchronize(ix->stream))) break;
-        if (pool_alloc((void **)&d_q, sizeof(double) * 3 * chunk, s) || pool_alloc((void **)&d_idx, sizeof(int32_t) * k * chunk, s)) {
-            rc = PT_ERR_OUT_OF_MEMORY;
-            break;
-        }
-        QueryParams qp{};
-        fill_params(ix, qp);
-        qp.ids = nullptr;          // the index's own ids: the PCA kernel reads its records by them
-        qp.k = k;
-        qp.r2 = radius_to_r2(radius);
-        qp.queries = d_q;
-        qp.idx_out = d_idx;
-        const PT *pts = (const PT *)ix->pts;
-        for (size_t c0 = 0; c0 < n; c0 += chunk) {
-            const uint32_t cm = (uint32_t)std::min(chunk, (size_t)n - c0);
-            normals_rows_kernel<PT><<<ncdiv(cm, 256), 256, 0, s>>>(pts, (uint32_t)c0, cm, d_q);
-            count_launch();
-            qp.m = cm;
-            if ((rc = launch_query(ix, qp, s)) != PT_OK) break;
-            if (mark()) break;
-            normals_pca_kernel<PT><<<ncdiv(cm, 256), 256, 0, s>>>(pts, ix->inv_perm, n, (uint32_t)c0, cm, d_idx, k,
+    if (pool_alloc((void **)&d_idx, sizeof(int32_t) * k * std::min((size_t)HEIGHT_CHUNK, (size_t)n), s))
+        return PT_ERR_OUT_OF_MEMORY;
+    const int rc = self_query_chunks(
+        ix, k, radius, d_idx, false,
+        [&](uint32_t c0, uint32_t cm, const int32_t *idx) {
+            normals_pca_kernel<PT><<<ncdiv(cm, 256), 256, 0, s>>>((const PT *)ix->pts, ix->inv_perm, n, c0, cm, idx, k,
                                                                   normals_width(k), o);
             count_launch();
-            if (fail(cudaGetLastError()) || mark()) break;
-        }
-    } while (0);
-    pool_free(d_q, s);
+            cudaError_t e = cudaGetLastError();
+            if (e == cudaSuccess) e = record_mark(marks, s);
+            return e == cudaSuccess ? PT_OK : map_cuda_error(e);
+        },
+        marks, s);
     pool_free(d_idx, s);
     return rc;
 }

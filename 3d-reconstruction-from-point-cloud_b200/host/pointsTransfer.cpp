@@ -22,6 +22,8 @@
 // "Height range: lo hi").  All of them come from one bake.  -e K first estimates the cloud's normals
 // by PCA over each point's K nearest neighbours (pt_index_estimate_normals) and stores them in the
 // index, so the transfer and the bake blend them: for scans whose nx ny nz columns are zero or noisy.
+// -O K then orients the index's normals consistently along the minimum spanning forest of the
+// K-NN graph (pt_index_orient_normals) and stores them: for normals whose signs are arbitrary.
 #include <algorithm>
 #include <charconv>
 #include <chrono>
@@ -256,6 +258,8 @@ static int run(int argc, char **argv)
     std::string height_name;                       // ... the height map
     bool estimate = false;                         // -e K: estimate the cloud's normals first
     int estimate_k = 0;
+    bool orient = false;                           // -O K: orient the cloud's normals (after -e)
+    int orient_k = 0;
     for (int i = 1; i < argc; ++i) {
         std::string a = argv[i];
         if (a == "-k" && i + 1 < argc) K = atoi(argv[++i]);
@@ -271,6 +275,7 @@ static int run(int argc, char **argv)
         else if (a == "-T" && i + 1 < argc) tangent_ply_name = argv[++i];
         else if (a == "-H" && i + 1 < argc) height_name = argv[++i];
         else if (a == "-e" && i + 1 < argc) { estimate = true; estimate_k = atoi(argv[++i]); }
+        else if (a == "-O" && i + 1 < argc) { orient = true; orient_k = atoi(argv[++i]); }
         else pos_args.push_back(a);
     }
     if (pos_args.size() < 2) {
@@ -284,6 +289,10 @@ static int run(int argc, char **argv)
     }
     if (estimate && (estimate_k < 3 || estimate_k > PT_MAX_K || n_gpus > 1)) {
         std::cerr << "-e must be 3.." << PT_MAX_K << " and estimates normals on one GPU (no -g)" << std::endl;
+        return 0;
+    }
+    if (orient && (orient_k < 2 || orient_k > PT_MAX_K || n_gpus > 1)) {
+        std::cerr << "-O must be 2.." << PT_MAX_K << " and orients normals on one GPU (no -g)" << std::endl;
         return 0;
     }
     const bool bake = !bake_name.empty() || !normal_name.empty() || !tangent_name.empty() || !tangent_ply_name.empty() ||
@@ -345,6 +354,18 @@ static int run(int argc, char **argv)
         }
         std::cout << "Estimated normals: " << ns.estimated << " of " << points.size() << " points in "
                   << task_timer.time() << " seconds" << std::endl;
+        task_timer.reset();
+    }
+    if (orient) {
+        pt_orient_stats os;
+        rc = pt_index_orient_normals(index, orient_k, radius, nullptr, 1, nullptr, nullptr, &os);
+        if (rc != PT_OK) {
+            std::cerr << "pt_index_orient_normals failed: " << pt_status_string(rc) << std::endl;
+            pt_index_free(index);
+            return 0;
+        }
+        std::cout << "Oriented normals: " << os.oriented << " of " << points.size() << " points, " << os.flipped
+                  << " flipped, " << os.components << " components in " << task_timer.time() << " seconds" << std::endl;
         task_timer.reset();
     }
 

@@ -264,6 +264,45 @@ typedef struct pt_normals_stats {
 int pt_index_estimate_normals(pt_index *index, int k, double radius, const double *viewpoint /* 3 or NULL */,
                               int store, float *normal_out, float *variation_out, pt_normals_stats *stats);
 
+/* Normal orientation (DESIGN.md section 8, "Normal orientation"): flips the signs of the normals
+ * the index holds so that they agree along the cloud's surface, by propagation along the minimum
+ * spanning forest of the k-NN graph (Hoppe et al.; CGAL's mst_orient_normals).  It orients, it does
+ * not estimate: run pt_index_estimate_normals with store first for a cloud without normals.  Point i
+ * takes part when its stored normal m_i is usable (finite, m.m > 0), with the unit normal n_i.  The
+ * edges join the points that take part and are in one another's k-NN list (k, radius as pt_knn, the
+ * union of both directions); edge {i, j} weighs w = 1 - |n_i.n_j| and edges are ordered by
+ * (w, min id, max id), so the forest is unique.  Each connected component is oriented from its own
+ * root, its point of largest z (lowest id on ties): with a viewpoint v the root's normal faces v
+ * (n.(v - p) >= 0), otherwise its z is made positive (its largest component where z is 0).  Along
+ * every forest edge the child keeps the parent's sign where n_p.n_c >= 0, else takes the opposite.
+ * Components are not oriented relative to one another: a radius that splits the graph, or a cloud of
+ * separate parts, gives several (stats components; root_out shows which root each point followed).
+ * Everything is fp64 with every operation rounded on its own, so the results are deterministic.
+ *   normal_out   n x 3 floats, original point order: the stored normal, each component negated
+ *                where its sign is flipped (exact); unchanged for points that do not take part
+ *                (may be NULL)
+ *   root_out     n int32: the id of the point's component root, -1 where it does not take part
+ *                (may be NULL)
+ *   store        != 0: the oriented normals replace the stored ones, so later pt_transfer / bake
+ *                calls blend them
+ *   viewpoint    NULL or 3 finite doubles in host memory, else PT_ERR_INVALID_ARG
+ * Both outputs may be NULL only with store set.  k < 2 or an index without attributes:
+ * PT_ERR_INVALID_ARG; k > PT_MAX_K: PT_ERR_UNSUPPORTED.  The edges are counted in 32 bits, so
+ * n * k must be <= INT32_MAX, otherwise PT_ERR_UNSUPPORTED before any work.  All lists are kept
+ * (4 n k bytes) and the graph takes about 24 bytes per edge.  On a slab index (pt_build_opts.ids)
+ * the graph is that index's own points.  Host buffers, blocking; stats (may be NULL). */
+typedef struct pt_orient_stats {
+    uint64_t oriented;    /* points that take part */
+    uint64_t flipped;     /* of those, points whose normal was negated */
+    uint64_t components;  /* connected components of the graph (trees of the forest) */
+    uint64_t edges;       /* undirected edges of the graph */
+    float    knn_ms, mst_ms;   /* device time of the k-NN self-queries and of the rest (edges,
+                                  spanning forest, signs) */
+} pt_orient_stats;
+int pt_index_orient_normals(pt_index *index, int k, double radius, const double *viewpoint /* 3 or NULL */,
+                            int store, float *normal_out /* n*3 */, int32_t *root_out /* n */,
+                            pt_orient_stats *stats);
+
 /* Device-buffer API: same operations with inputs/outputs already resident in
  * HBM on the index's device (bench `value`, multi-GPU slabs).  `stream` is a
  * cudaStream_t passed as void* (NULL = the CUDA default stream); these calls
