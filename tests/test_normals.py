@@ -167,6 +167,96 @@ def test_orientation_rules(pto):
     assert np.array_equal(b, a)
 
 
+# ---- degenerate spectra: tied and zero eigenvalues ------------------------------------------------
+DEGENERATE = {"cube": 9, "octahedron": 7, "collinear": 8, "plane": 8}     # kind -> k (the structure's size)
+TINY = -530          # 2^-530: the scatter products (~2^-1062) are subnormal
+
+
+def degenerate_cloud(kind, seed=0):
+    """(xyz float64 [n,3], k, aligned bool [n]): 216 structures 8 apart on a 6^3 lattice, whose k-NN
+    scatter has tied or zero eigenvalues -- cube corners or an octahedron around a centre point (three
+    equal), collinear runs (two equal smallest), plane patches (a zero smallest) -- and one background
+    point near every lattice cell's middle.  Every structure fits a ball of radius 0.9 and lies more
+    than 4 from the background, so the lists of its points hold exactly its own points.  Every other
+    structure is rotated (tilted: z = x for planes); ``aligned`` marks the points of the others, whose
+    scatter is exact.  Coordinates are fp32-representable; ids are shuffled."""
+    rng = np.random.default_rng(seed)
+    g = np.arange(6) * 8.0
+    centres = np.stack(np.meshgrid(g, g, g, indexing="ij"), -1).reshape(-1, 3)
+    parts, flags = [], []
+    for i, c in enumerate(centres):
+        a = (0.25, 0.5, 0.375)[i % 3]
+        aligned = i % 2 == 0
+        if kind == "cube":
+            local = a * np.r_[np.array(np.meshgrid([-1, 1], [-1, 1], [-1, 1])).reshape(3, -1).T, np.zeros((1, 3))]
+        elif kind == "octahedron":
+            local = a * np.r_[np.eye(3), -np.eye(3), np.zeros((1, 3))]
+        elif kind == "collinear":
+            local = np.outer((np.arange(12) - 5.5) * a / 4.0, [1.0, 0.0, 0.0])
+        else:
+            uv = rng.integers(-256, 257, (16, 2)) / 512.0
+            local = np.c_[uv, np.zeros(16)] if aligned else np.c_[uv[:, 0], uv[:, 1], uv[:, 0]]
+        if not aligned and kind != "plane":
+            q, _ = np.linalg.qr(rng.standard_normal((3, 3)))
+            local = local @ q
+        parts.append(c + local)
+        flags.append(np.full(len(local), aligned))
+    back = centres + 4.0 + rng.uniform(-1.0, 1.0, centres.shape)
+    xyz = np.r_[np.concatenate(parts), back].astype(np.float32).astype(np.float64)
+    aligned = np.r_[np.concatenate(flags), np.zeros(len(back), bool)]
+    p = rng.permutation(len(xyz))
+    return xyz[p], DEGENERATE[kind], aligned[p]
+
+
+def degenerate_normals(n, seed=1):
+    """Input normals for rule (a): random directions, every fifth one zero (rule (c) there)."""
+    m = np.random.default_rng(seed).standard_normal((n, 3)).astype(np.float32)
+    m[::5] = 0.0
+    return m
+
+
+@pytest.mark.parametrize("kind", sorted(DEGENERATE))
+def test_oracle_equals_numpy_on_degenerate_spectra(kind, pto):
+    xyz, k, aligned = degenerate_cloud(kind)
+    idx = pto_normals.neighbours(xyz, k)
+    nrm = degenerate_normals(len(xyz))
+    for normal, view in ((nrm, None), (None, (100.0, -30.0, 70.0)), (None, None)):
+        est = check_oracle_vs_numpy(xyz, normal, idx, view)
+        assert est.all()
+    check_exact_scatter(kind, aligned, *pto_normals.estimate(xyz, None, idx)[:2])
+
+
+def check_exact_scatter(kind, aligned, n, v):
+    """Known answers (rule (c)) where the scatter is exact: ties go to the lower Jacobi column."""
+    if kind in ("cube", "octahedron"):            # diag(s, s, s): no rotation at all
+        assert (n[aligned] == np.array([1, 0, 0], np.float32)).all()
+        assert (v[aligned] == np.float32(1.0 / 3.0)).all()
+    elif kind == "collinear":                     # diag(s, 0, 0)
+        assert (n[aligned] == np.array([0, 1, 0], np.float32)).all() and (v[aligned] == 0).all()
+    else:                                         # z = c: the third row and column are exact zeros
+        assert (n[aligned] == np.array([0, 0, 1], np.float32)).all() and (v[aligned] == 0).all()
+
+
+@pytest.mark.parametrize("kind", sorted(DEGENERATE))
+def test_oracle_on_subnormal_scatter(kind, pto):
+    """The degenerate clouds scaled by 2^-530: exact in fp64, but every scatter product is subnormal,
+    so the Jacobi sweeps round with a few significant bits and the numpy statement's eigenvectors
+    (eigh scales the matrix first) are no reference for the others.  What still holds: which points
+    get an estimate, the NaN bits, unit normals and the exact answers of the aligned structures, whose
+    products are exact multiples of 2^-1072.  The lists are those of the scaled cloud."""
+    xyz, k, aligned = degenerate_cloud(kind)
+    tiny = np.ldexp(xyz, TINY)
+    idx = pto_normals.neighbours(tiny, k)
+    for normal, view in ((degenerate_normals(len(xyz)), None), (None, (1.0, -2.0, 3.0)), (None, None)):
+        got_n, got_v, n_est = pto_normals.estimate(tiny, normal, idx, view)
+        est = numpy_normals(tiny, normal, idx, view)[3]
+        assert n_est == est.sum() == len(xyz)
+        assert np.array_equal(np.isnan(got_v), ~est)
+        assert np.abs(np.linalg.norm(got_n.astype(np.float64), axis=1) - 1.0).max() < 1e-6
+        assert ((got_v >= 0) & (got_v <= np.float32(1.0 / 3.0))).all()
+    check_exact_scatter(kind, aligned, *pto_normals.estimate(tiny, None, idx)[:2])
+
+
 # ---- accuracy against the analytic normals of a noisy scan ----------------------------------------
 ACCURACY = {8: (2.3, 7.5), 16: (1.0, 2.7), 32: (0.5, 1.3)}    # mean, p99 (degrees) bounds
 

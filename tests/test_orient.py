@@ -251,6 +251,102 @@ def test_moebius_strip(pto):
         assert got["components"] == 1
 
 
+# ---- ties: equal weights, equal top z, many components ---------------------------------------------
+def flat_lattice(g=100, permute=False, seed=6):
+    """(xyz, normal float32, radius): a g x g lattice on z = 0, every tenth point at z = -0.0, with
+    normals +-z of three lengths.  Every edge weight 1 - |d| is exactly 0, so the (lo, hi) keys alone
+    decide the forest, and every point shares the top z.  ``permute`` shuffles the ids, so that id
+    order differs from the lattice's (and the curve's) order."""
+    rng = np.random.default_rng(seed)
+    i, j = np.meshgrid(np.arange(g), np.arange(g), indexing="ij")
+    xyz = np.c_[i.ravel() * 0.5, j.ravel() * 0.5, np.zeros(g * g)]
+    xyz[::10, 2] = -0.0
+    m = np.zeros((g * g, 3), np.float32)
+    m[:, 2] = np.where(rng.random(g * g) < 0.5, -1.0, 1.0) * rng.choice([0.5, 1.0, 3.0], g * g)
+    if permute:
+        p = rng.permutation(g * g)
+        xyz, m = xyz[p], m[p]
+    return xyz, m, None
+
+
+def plateau(n=20_000, seed=7):
+    """A noisy patch cut flat at z = 0: about half the points share the top z, some of them -0.0."""
+    xyz, m = noisy_patch(n, seed)
+    xyz[:, 2] = np.minimum(xyz[:, 2], 0.0)
+    top = np.flatnonzero(xyz[:, 2] == 0.0)
+    xyz[top[::3], 2] = -0.0
+    return xyz.astype(np.float32).astype(np.float64), m.astype(np.float32), None
+
+
+FRUSTRATED = np.array([[1.0, 1.0, 0.0], [0.0, 1.0, 1.0], [1.0, 0.0, -1.0]])
+
+
+def clusters(count=3000, seed=8):
+    """(xyz, normal float32, radius): `count` clusters of 4 points, 10 apart, each inside a ball of
+    radius 0.3, and a radius of 1, so every list stays inside its cluster and every cluster is a
+    component of its own.  Three normals of each cluster are +-(1, 1, 0), +-(0, 1, 1), +-(1, 0, -1):
+    their unit vectors' pairwise |d| round to the same value, so the three edges tie, and the edge
+    signs around the triangle multiply to -1, so the sign a point gets depends on which two of the
+    three edges the (lo, hi) order puts in the forest.  The fourth normal is random; ids are shuffled."""
+    rng = np.random.default_rng(seed)
+    g = int(np.ceil(count ** 0.5))
+    c = np.c_[np.arange(count) % g * 10.0, np.arange(count) // g * 10.0, rng.uniform(-5.0, 5.0, count)]
+    xyz = (np.repeat(c, 4, axis=0) + rng.uniform(-0.17, 0.17, (4 * count, 3))).astype(np.float32).astype(np.float64)
+    m = np.empty((count, 4, 3))
+    m[:, :3] = FRUSTRATED[np.argsort(rng.random((count, 3)), axis=1)]
+    m[:, 3] = rng.standard_normal((count, 3))
+    m *= np.where(rng.random((count, 4)) < 0.5, -1.0, 1.0)[..., None]
+    p = rng.permutation(4 * count)
+    return xyz[p], m.reshape(-1, 3).astype(np.float32)[p], 1.0
+
+
+TIE_CLOUDS = {"lattice": flat_lattice, "lattice_permuted": lambda: flat_lattice(permute=True),
+              "plateau": plateau, "clusters": clusters}
+
+
+def list_edges(m, idx):
+    """(i, j, w) of every list entry j != i, with w = 1 - |d| as the definition computes it."""
+    m = m.astype(np.float64)
+    nh = m / np.sqrt(dot(m, m))[:, None]
+    i = np.repeat(np.arange(len(idx)), idx.shape[1]).reshape(idx.shape)
+    keep = (idx >= 0) & (idx != i)
+    i, j = i[keep], idx[keep]
+    return i, j, np.maximum(1.0 - np.abs(dot(nh[i], nh[j])), 0.0)
+
+
+def check_tie_cloud(name, xyz, m, idx, got):
+    """That each tie cloud reaches what it is built for."""
+    z = xyz[:, 2]
+    if name.startswith("lattice"):
+        assert (list_edges(m, idx)[2] == 0.0).all()                           # every weight is 0
+        assert (z == 0.0).all() and np.signbit(z).sum() == len(z) // 10
+        assert (got["normal"][:, 2] > 0).all()
+        if idx.shape[1] >= 8:                              # one component (k = 2 leaves pairs and chains)
+            assert got["components"] == 1
+            assert (got["root"] == 0).all()              # every z ties, -0.0 with +0.0: the lowest id
+    elif name == "plateau":
+        if idx.shape[1] >= 8:
+            r = np.bincount(got["root"][got["root"] >= 0]).argmax()            # the largest component
+            top = (got["root"] == r) & (z == 0.0)
+            assert z[r] == 0.0 and top.sum() > 1000 and np.signbit(z[top]).any() and not np.signbit(z[top]).all()
+    else:
+        i, j, w = list_edges(m, idx)
+        tri = (np.abs(m).sum(1) == 2.0) & (m == 0.0).any(1)                   # the +-FRUSTRATED normals
+        assert tri.sum() == 3 * len(z) // 4
+        if idx.shape[1] >= 4:                                                  # whole clusters in every list
+            assert got["components"] == len(z) // 4
+            assert len(np.unique(w[tri[i] & tri[j]])) == 1                     # one tied weight
+
+
+@pytest.mark.parametrize("name", sorted(TIE_CLOUDS))
+def test_oracle_equals_scipy_on_ties(name, pto):
+    xyz, m, radius = TIE_CLOUDS[name]()
+    for k in (2, 8, 32):
+        idx = pto_normals.neighbours(xyz, k, -1.0 if radius is None else radius)
+        got = check_oracle_vs_scipy(xyz, m, idx)
+        check_tie_cloud(name, xyz, m, idx, got)
+
+
 # ---- CLI ---------------------------------------------------------------------------------------------
 def _cli():
     from test_cli import CLI
