@@ -3,10 +3,10 @@
  * "Tangent-space bake", "Height bake").  TEST INFRASTRUCTURE ONLY, like the rest of oracle/.  The
  * reference has no per-texel path; this file states the project's own frozen definitions, which
  * csrc/pt_texture.cu must equal bit for bit (tests/test_bake.py, tests/test_bake_tangent.py,
- * tests/test_bake_height.py).  Built on its own into libpt_bake_oracle.so by oracle/pto_bake.py,
- * which takes the neighbour lists, the blend and the 8-bit padding from libpt_oracle.so (pto.KdTree,
- * pto.blend, pto.texture_pad).  Fp64 throughout, no FMA (-ffp-contract=off, the flags of
- * oracle/Makefile), every operation in the order the definition states.
+ * tests/test_bake_height.py).  Built into libpt_oracle.so with the rest of oracle/; its binding
+ * oracle/pto_bake.py takes the neighbour lists, the blend and the 8-bit padding from pto.KdTree,
+ * pto.blend and pto.texture_pad.  Fp64 throughout, no FMA (-ffp-contract=off, oracle/Makefile),
+ * every operation in the order the definition states.
  *
  *   texels      Texel (col, row) of a res x res image, row 0 on top, samples p = (col + 0.5,
  *               res - row - 0.5) in UV * res units.  Face f covers it iff the barycentrics of p in

@@ -1,19 +1,21 @@
-"""ctypes binding of the CPU oracle (oracle/libpt_oracle.so).
+"""ctypes binding of the CPU oracle (oracle/libpt_oracle.so, every C statement under oracle/).
 
 TEST INFRASTRUCTURE ONLY -- see oracle/pt_oracle.h.  Imported by tests/,
 ``__graft_entry__.smoke()`` and bench.py's cpu_baseline / ``--impl reference``
 legs; never by the product package.  The neighbour SEARCH is parity-unpinned (no reference
 goldens, CGAL absent); the metric, the box bound and the record layout are pinned on the
 reference's own headers through ``ref_metric()`` (oracle/ref_shim.cpp -> oracle/_ref/).
+This module loads the one library; pto_bake, pto_normals and pto_orient declare their own entry
+points on it through ``bind()``.
 """
 import ctypes
 import os
 import subprocess
+import tempfile
 
 import numpy as np
 
 _HERE = os.path.dirname(os.path.abspath(__file__))
-_LIB_PATH = os.path.join(_HERE, "libpt_oracle.so")
 
 # Byte-for-byte mirror of the reference ``struct Point`` (src/Point.h:1-6).
 POINT_DTYPE = np.dtype(
@@ -24,14 +26,18 @@ assert POINT_DTYPE.itemsize == 80
 
 
 def build(force=False):
-    """Compile the C restatement (gcc, oracle/Makefile)."""
-    if force or not os.path.exists(_LIB_PATH) or (
-        os.path.getmtime(_LIB_PATH) < max(os.path.getmtime(os.path.join(_HERE, f))
-                                          for f in ("pt_oracle.c", "pt_synth_host.c", "pt_texture_oracle.c", "pt_oracle.h"))
-    ):
-        subprocess.run(["make", "-C", _HERE, "-B" if force else "-s"], check=True,
-                       stdout=subprocess.DEVNULL)
-    return _LIB_PATH
+    """Compile the C oracle (gcc, oracle/Makefile) unless the library is up to date; returns its
+    path.  Where make cannot update oracle/ (a read-only tree), the library is built in a per-user
+    temporary directory instead."""
+    make = ["make", "-C", _HERE, "-s"] + (["-B"] if force else [])
+    try:
+        subprocess.run(make, check=True, stdout=subprocess.DEVNULL, stderr=subprocess.DEVNULL)
+        return os.path.join(_HERE, "libpt_oracle.so")
+    except subprocess.CalledProcessError:
+        out = os.path.join(tempfile.gettempdir(), f"pt_oracle_{os.getuid()}")
+    os.makedirs(out, exist_ok=True)
+    subprocess.run(make + ["OUT=" + out], check=True, stdout=subprocess.DEVNULL)
+    return os.path.join(out, "libpt_oracle.so")
 
 
 _REF_PATH = os.path.join(_HERE, "_ref", "libref_metric.so")
@@ -73,48 +79,50 @@ def ref_metric():
     return _ref
 
 
+_vp, _i64, _i32, _dbl, _u64 = ctypes.c_void_p, ctypes.c_int64, ctypes.c_int, ctypes.c_double, ctypes.c_uint64
+# (name, restype, argtypes) of this module's entry points; bind() adds the other modules' tables
+_PROTOS = [
+    ("pto_transformed_distance", _dbl, [_vp, _vp]),
+    ("pto_min_distance_to_rectangle", _dbl, [_vp, _vp, _vp, _vp]),
+    ("pto_new_distance", _dbl, [_dbl, _dbl, _dbl]),
+    ("pto_transformed_radius", _dbl, [_dbl]),
+    ("pto_knn_bruteforce", _i32, [_vp, _i64, _vp, _i64, _i32, _dbl, _vp, _vp, _i32]),
+    ("pto_blend", _i32, [_vp, _i64, _i64, _i32, _vp, _vp, _vp, _vp]),
+    ("pto_kdtree_build", _vp, [_vp, _i64, _i32]),
+    ("pto_kdtree_free", None, [_vp]),
+    ("pto_kdtree_node_count", _i64, [_vp]),
+    ("pto_kdtree_knn", _i32, [_vp, _vp, _i64, _i32, _dbl, _i32, _vp, _vp, _i32]),
+    ("pto_reference_face_loop", _i64, [_vp, _vp, _vp, _i64, _i32, _i32]),
+    ("pto_max_threads", _i32, []),
+    ("pto_synth_cloud", _i32, [_vp, _i64, _i32, _u64, _u64, _dbl, _dbl, _dbl, _dbl, _dbl, _i32]),
+    ("pto_synth_samples", _i32, [_vp, _i64, _i64, _dbl, _dbl, _dbl, _dbl, _i32]),
+    ("pto_texture_faces", _i32, [_vp, _vp, _vp, _i32, _vp, _i64, _i32, _vp, _vp]),
+    ("pto_texture_pad", _i32, [_vp, _i32, _vp]),
+]
 _lib = None
 
 
+def _declare(L, protos):
+    for name, res, args in protos:
+        fn = getattr(L, name)
+        fn.restype, fn.argtypes = res, args
+
+
+def bind(protos):
+    """Declare more entry points of lib() from (name, restype, argtypes) rows, now if the library
+    is loaded, else when it is."""
+    protos = list(protos)
+    _PROTOS.extend(protos)
+    if _lib is not None:
+        _declare(_lib, protos)
+
+
 def lib():
+    """The oracle library, built by build() if needed, with every bound prototype declared."""
     global _lib
     if _lib is None:
-        if not os.path.exists(_LIB_PATH):
-            build()
-        L = ctypes.CDLL(_LIB_PATH)
-        vp, i64, i32, dbl = ctypes.c_void_p, ctypes.c_int64, ctypes.c_int, ctypes.c_double
-        L.pto_transformed_distance.restype = dbl
-        L.pto_transformed_distance.argtypes = [vp, vp]
-        L.pto_min_distance_to_rectangle.restype = dbl
-        L.pto_min_distance_to_rectangle.argtypes = [vp, vp, vp, vp]
-        L.pto_new_distance.restype = dbl
-        L.pto_new_distance.argtypes = [dbl, dbl, dbl]
-        L.pto_transformed_radius.restype = dbl
-        L.pto_transformed_radius.argtypes = [dbl]
-        L.pto_knn_bruteforce.restype = i32
-        L.pto_knn_bruteforce.argtypes = [vp, i64, vp, i64, i32, dbl, vp, vp, i32]
-        L.pto_blend.restype = i32
-        L.pto_blend.argtypes = [vp, i64, i64, i32, vp, vp, vp, vp]
-        L.pto_kdtree_build.restype = vp
-        L.pto_kdtree_build.argtypes = [vp, i64, i32]
-        L.pto_kdtree_free.restype = None
-        L.pto_kdtree_free.argtypes = [vp]
-        L.pto_kdtree_node_count.restype = i64
-        L.pto_kdtree_node_count.argtypes = [vp]
-        L.pto_kdtree_knn.restype = i32
-        L.pto_kdtree_knn.argtypes = [vp, vp, i64, i32, dbl, i32, vp, vp, i32]
-        L.pto_reference_face_loop.restype = i64
-        L.pto_reference_face_loop.argtypes = [vp, vp, vp, i64, i32, i32]
-        L.pto_max_threads.restype = i32
-        u64 = ctypes.c_uint64
-        L.pto_synth_cloud.restype = i32
-        L.pto_synth_cloud.argtypes = [vp, i64, i32, u64, u64, dbl, dbl, dbl, dbl, dbl, i32]
-        L.pto_synth_samples.restype = i32
-        L.pto_synth_samples.argtypes = [vp, i64, i64, dbl, dbl, dbl, dbl, i32]
-        L.pto_texture_faces.restype = i32
-        L.pto_texture_faces.argtypes = [vp, vp, vp, i32, vp, i64, i32, vp, vp]
-        L.pto_texture_pad.restype = i32
-        L.pto_texture_pad.argtypes = [vp, i32, vp]
+        L = ctypes.CDLL(build())
+        _declare(L, _PROTOS)
         _lib = L
     return _lib
 

@@ -1,67 +1,26 @@
 """ctypes binding of the per-texel bake oracle (oracle/pt_bake_oracle.c): the object-space,
 tangent-space and height bakes.
 
-TEST INFRASTRUCTURE ONLY, like oracle/pto.py, whose k-NN, blend and padding it uses.  The C file
-is compiled on first use with the flags of oracle/Makefile (-ffp-contract=off: no FMA) into
-oracle/libpt_bake_oracle.so, or into a per-user temporary directory where oracle/ is read-only.
+TEST INFRASTRUCTURE ONLY, like oracle/pto.py, whose library holds it and whose k-NN, blend and
+padding it uses.
 """
 import ctypes
-import os
-import subprocess
-import tempfile
 
 import numpy as np
 
 from . import pto
 
-_HERE = os.path.dirname(os.path.abspath(__file__))
-_SRC = os.path.join(_HERE, "pt_bake_oracle.c")
-_DEPS = (_SRC, os.path.join(_HERE, "pt_oracle.h"))
-_CFLAGS = ["-O3", "-std=c11", "-fPIC", "-ffp-contract=off", "-Wall", "-Wextra"]
-_lib_handle = None
-
-
-def build(force=False):
-    """Compile pt_bake_oracle.c (gcc) unless an up-to-date library exists; returns its path."""
-    newest = max(os.path.getmtime(f) for f in _DEPS)
-    for d in (_HERE, os.path.join(tempfile.gettempdir(), f"pto_bake_{os.getuid()}")):
-        path = os.path.join(d, "libpt_bake_oracle.so")
-        if not force and os.path.exists(path) and os.path.getmtime(path) >= newest:
-            return path
-        tmp = f"{path}.{os.getpid()}.tmp"
-        try:
-            os.makedirs(d, exist_ok=True)
-            subprocess.run(["/usr/bin/gcc", *_CFLAGS, "-I" + _HERE, "-shared", "-o", tmp, _SRC, "-lm"],
-                           check=True, stdout=subprocess.DEVNULL,
-                           stderr=subprocess.DEVNULL if d == _HERE else None)
-            os.replace(tmp, path)
-            return path
-        except (OSError, subprocess.CalledProcessError):
-            if os.path.exists(tmp):
-                os.remove(tmp)
-            if d != _HERE:
-                raise
-    raise RuntimeError("unreachable")
-
-
-def _lib():
-    global _lib_handle
-    if _lib_handle is None:
-        L = ctypes.CDLL(build())
-        vp, i64, i32 = ctypes.c_void_p, ctypes.c_int64, ctypes.c_int
-        for name, res, args in (
-                ("pto_bake_texels", i64, [vp, i64, vp, i64, i32, vp, vp, vp]),
-                ("pto_bake_encode", i32, [ctypes.c_float]),
-                ("pto_bake_compose", i32, [vp, i64, vp, vp, i32, vp, vp, vp]),
-                ("pto_bake_frames", i32, [vp, i64, vp, i64, vp, vp]),
-                ("pto_bake_compose_tangent", i32, [vp, i64, vp, vp, i64, vp, vp, i64, vp, vp, i32, vp, vp]),
-                ("pto_bake_height", i32, [vp, i64, vp, vp, i64, vp, vp, vp, i64, vp, i64, vp, vp, i32, i32, vp]),
-                ("pto_bake_height_encode", i64, [vp, i64, vp, vp, vp]),
-                ("pto_bake_height_pad", i32, [vp, vp, i32, vp])):
-            fn = getattr(L, name)
-            fn.restype, fn.argtypes = res, args
-        _lib_handle = L
-    return _lib_handle
+_vp, _i64, _i32 = ctypes.c_void_p, ctypes.c_int64, ctypes.c_int
+pto.bind([
+    ("pto_bake_texels", _i64, [_vp, _i64, _vp, _i64, _i32, _vp, _vp, _vp]),
+    ("pto_bake_encode", _i32, [ctypes.c_float]),
+    ("pto_bake_compose", _i32, [_vp, _i64, _vp, _vp, _i32, _vp, _vp, _vp]),
+    ("pto_bake_frames", _i32, [_vp, _i64, _vp, _i64, _vp, _vp]),
+    ("pto_bake_compose_tangent", _i32, [_vp, _i64, _vp, _vp, _i64, _vp, _vp, _i64, _vp, _vp, _i32, _vp, _vp]),
+    ("pto_bake_height", _i32, [_vp, _i64, _vp, _vp, _i64, _vp, _vp, _vp, _i64, _vp, _i64, _vp, _vp, _i32, _i32, _vp]),
+    ("pto_bake_height_encode", _i64, [_vp, _i64, _vp, _vp, _vp]),
+    ("pto_bake_height_pad", _i32, [_vp, _vp, _i32, _vp]),
+])
 
 
 # ---- texels and the object-space maps ------------------------------------------------------------
@@ -72,8 +31,8 @@ def bake_samples(vertices, faces, resolution):
     faces = np.ascontiguousarray(faces, dtype=np.int32).reshape(-1, 3)
     n = resolution * resolution
     texels, xyz, owner = np.empty(n, np.uint32), np.empty((n, 3), np.float64), np.empty(n, np.int32)
-    m = _lib().pto_bake_texels(pto._ptr(vertices), vertices.shape[0], pto._ptr(faces), faces.shape[0],
-                               resolution, pto._ptr(texels), pto._ptr(xyz), pto._ptr(owner))
+    m = pto.lib().pto_bake_texels(pto._ptr(vertices), vertices.shape[0], pto._ptr(faces), faces.shape[0],
+                                  resolution, pto._ptr(texels), pto._ptr(xyz), pto._ptr(owner))
     assert m >= 0, m
     return texels[:m].copy(), xyz[:m].copy(), owner[:m].copy()
 
@@ -86,7 +45,7 @@ def bake_texels(vertices, faces, resolution):
 
 def bake_encode(n):
     """The normal-map byte of one fp32 normal component."""
-    return _lib().pto_bake_encode(float(n))
+    return pto.lib().pto_bake_encode(float(n))
 
 
 def bake_compose(texels, rgba, normal, resolution, pad=True):
@@ -99,8 +58,8 @@ def bake_compose(texels, rgba, normal, resolution, pad=True):
     bgra = np.empty((resolution, resolution, 4), dtype=np.uint8)
     nbgra = np.empty((resolution, resolution, 4), dtype=np.uint8)
     nf = np.empty((resolution, resolution, 3), dtype=np.float32)
-    rc = _lib().pto_bake_compose(pto._ptr(texels), texels.shape[0], pto._ptr(rgba), pto._ptr(normal),
-                                 resolution, pto._ptr(bgra), pto._ptr(nbgra), pto._ptr(nf))
+    rc = pto.lib().pto_bake_compose(pto._ptr(texels), texels.shape[0], pto._ptr(rgba), pto._ptr(normal),
+                                    resolution, pto._ptr(bgra), pto._ptr(nbgra), pto._ptr(nf))
     assert rc == 0, rc
     if pad:
         bgra, nbgra = pto.texture_pad(bgra), pto.texture_pad(nbgra)
@@ -134,8 +93,8 @@ def bake_frames(vertices, faces):
     faces = np.ascontiguousarray(faces, dtype=np.int32).reshape(-1, 3)
     n = vertices.shape[0]
     frames, tangents = np.empty((n, 8), np.float64), np.empty((n, 4), np.float32)
-    rc = _lib().pto_bake_frames(pto._ptr(vertices), n, pto._ptr(faces), faces.shape[0], pto._ptr(frames),
-                                pto._ptr(tangents))
+    rc = pto.lib().pto_bake_frames(pto._ptr(vertices), n, pto._ptr(faces), faces.shape[0], pto._ptr(frames),
+                                   pto._ptr(tangents))
     assert rc == 0, rc
     return frames, tangents
 
@@ -154,9 +113,9 @@ def bake_compose_tangent(vertices, frames, faces, texels, sample_faces, rgba, no
     assert texels.shape[0] == sample_faces.shape[0] == rgba.shape[0] == normal.shape[0]
     tb = np.empty((resolution, resolution, 4), np.uint8)
     tn = np.empty((resolution, resolution, 3), np.float32)
-    rc = _lib().pto_bake_compose_tangent(pto._ptr(vertices), vertices.shape[0], pto._ptr(frames), pto._ptr(faces),
-                                         faces.shape[0], pto._ptr(texels), pto._ptr(sample_faces), texels.shape[0],
-                                         pto._ptr(rgba), pto._ptr(normal), resolution, pto._ptr(tb), pto._ptr(tn))
+    rc = pto.lib().pto_bake_compose_tangent(pto._ptr(vertices), vertices.shape[0], pto._ptr(frames), pto._ptr(faces),
+                                            faces.shape[0], pto._ptr(texels), pto._ptr(sample_faces), texels.shape[0],
+                                            pto._ptr(rgba), pto._ptr(normal), resolution, pto._ptr(tb), pto._ptr(tn))
     assert rc == 0, rc
     if pad:
         tb = pto.texture_pad(tb)
@@ -192,10 +151,10 @@ def bake_height(vertices, frames, faces, texels, sample_faces, xyz, points, idx,
     m, k = idx.shape
     assert texels.shape[0] == sample_faces.shape[0] == xyz.shape[0] == m == d2.shape[0]
     h = np.empty((resolution, resolution), np.float32)
-    rc = _lib().pto_bake_height(pto._ptr(vertices), vertices.shape[0], pto._ptr(frames), pto._ptr(faces),
-                                faces.shape[0], pto._ptr(texels), pto._ptr(sample_faces), pto._ptr(xyz), m,
-                                pto._ptr(points), points.shape[0], pto._ptr(idx), pto._ptr(d2), k, resolution,
-                                pto._ptr(h))
+    rc = pto.lib().pto_bake_height(pto._ptr(vertices), vertices.shape[0], pto._ptr(frames), pto._ptr(faces),
+                                   faces.shape[0], pto._ptr(texels), pto._ptr(sample_faces), pto._ptr(xyz), m,
+                                   pto._ptr(points), points.shape[0], pto._ptr(idx), pto._ptr(d2), k, resolution,
+                                   pto._ptr(h))
     assert rc == 0, rc
     return h
 
@@ -206,8 +165,8 @@ def bake_height_encode(height, height_range=None):
     codes = np.empty(height.shape, np.uint16)
     used = np.empty(2, np.float64)
     rin = None if height_range is None else np.ascontiguousarray(height_range, dtype=np.float64)
-    valued = _lib().pto_bake_height_encode(pto._ptr(height), height.size, None if rin is None else pto._ptr(rin),
-                                           pto._ptr(codes), pto._ptr(used))
+    valued = pto.lib().pto_bake_height_encode(pto._ptr(height), height.size, None if rin is None else pto._ptr(rin),
+                                              pto._ptr(codes), pto._ptr(used))
     return codes, (float(used[0]), float(used[1])), int(valued)
 
 
@@ -217,7 +176,7 @@ def bake_height_pad(height, codes):
     codes = np.ascontiguousarray(codes, dtype=np.uint16)
     res = height.shape[0]
     out = np.empty_like(codes)
-    assert _lib().pto_bake_height_pad(pto._ptr(height), pto._ptr(codes), res, pto._ptr(out)) == 0
+    assert pto.lib().pto_bake_height_pad(pto._ptr(height), pto._ptr(codes), res, pto._ptr(out)) == 0
     return out
 
 

@@ -1,55 +1,16 @@
 """ctypes binding of the normal-estimation oracle (oracle/pt_normals_oracle.c).
 
-TEST INFRASTRUCTURE ONLY, like oracle/pto.py, whose exact k-NN it uses for the neighbour lists.  The
-C file is compiled on first use with -ffp-contract=off (no FMA) and OpenMP into
-oracle/libpt_normals_oracle.so, or into a per-user temporary directory where oracle/ is read-only.
+TEST INFRASTRUCTURE ONLY, like oracle/pto.py, whose library holds it and whose exact k-NN it uses
+for the neighbour lists.
 """
 import ctypes
-import os
-import subprocess
-import tempfile
 
 import numpy as np
 
 from . import pto
 
-_HERE = os.path.dirname(os.path.abspath(__file__))
-_SRC = os.path.join(_HERE, "pt_normals_oracle.c")
-_CFLAGS = ["-O3", "-std=c11", "-fPIC", "-ffp-contract=off", "-fopenmp", "-Wall", "-Wextra"]
-_lib_handle = None
-
-
-def build(force=False):
-    """Compile pt_normals_oracle.c (gcc) unless an up-to-date library exists; returns its path."""
-    newest = os.path.getmtime(_SRC)
-    for d in (_HERE, os.path.join(tempfile.gettempdir(), f"pto_normals_{os.getuid()}")):
-        path = os.path.join(d, "libpt_normals_oracle.so")
-        if not force and os.path.exists(path) and os.path.getmtime(path) >= newest:
-            return path
-        tmp = f"{path}.{os.getpid()}.tmp"
-        try:
-            os.makedirs(d, exist_ok=True)
-            subprocess.run(["/usr/bin/gcc", *_CFLAGS, "-shared", "-o", tmp, _SRC, "-lm"], check=True,
-                           stdout=subprocess.DEVNULL, stderr=subprocess.DEVNULL if d == _HERE else None)
-            os.replace(tmp, path)
-            return path
-        except (OSError, subprocess.CalledProcessError):
-            if os.path.exists(tmp):
-                os.remove(tmp)
-            if d != _HERE:
-                raise
-    raise RuntimeError("unreachable")
-
-
-def _lib():
-    global _lib_handle
-    if _lib_handle is None:
-        L = ctypes.CDLL(build())
-        vp, i64 = ctypes.c_void_p, ctypes.c_int64
-        L.pto_estimate_normals.restype = i64
-        L.pto_estimate_normals.argtypes = [vp, vp, i64, vp, i64, vp, ctypes.c_int, vp, vp, vp, vp]
-        _lib_handle = L
-    return _lib_handle
+_vp, _i64 = ctypes.c_void_p, ctypes.c_int64
+pto.bind([("pto_estimate_normals", _i64, [_vp, _vp, _i64, _vp, _i64, _vp, ctypes.c_int, _vp, _vp, _vp, _vp])])
 
 
 def estimate(xyz, normal, idx, viewpoint=None, rows=None, fp64=False):
@@ -68,10 +29,10 @@ def estimate(xyz, normal, idx, viewpoint=None, rows=None, fp64=False):
     view = None if viewpoint is None else np.ascontiguousarray(viewpoint, dtype=np.float64).reshape(3)
     out_n, out_v = np.empty((m, 3), np.float32), np.empty(m, np.float32)
     out64 = np.empty((m, 4), np.float64) if fp64 else None
-    est = _lib().pto_estimate_normals(pto._ptr(xyz), None if nrm is None else pto._ptr(nrm), xyz.shape[0],
-                                      None if rws is None else pto._ptr(rws), m, pto._ptr(idx), k,
-                                      None if view is None else pto._ptr(view), pto._ptr(out_n), pto._ptr(out_v),
-                                      None if out64 is None else pto._ptr(out64))
+    est = pto.lib().pto_estimate_normals(pto._ptr(xyz), None if nrm is None else pto._ptr(nrm), xyz.shape[0],
+                                         None if rws is None else pto._ptr(rws), m, pto._ptr(idx), k,
+                                         None if view is None else pto._ptr(view), pto._ptr(out_n), pto._ptr(out_v),
+                                         None if out64 is None else pto._ptr(out64))
     assert est >= 0, est
     return (out_n, out_v, int(est)) + ((out64,) if fp64 else ())
 

@@ -23,9 +23,8 @@ e. Consumers in one UTM frame: the bake (colour, tangent, height), normal estima
 import numpy as np
 import pytest
 
-import orient_oracle
 import test_frames as tf
-from oracle import pto_normals
+from oracle import pto_normals, pto_orient
 from test_bake import grid_mesh
 from test_bake_height import check_height
 from test_bake_tangent import check_bake_ex, tilted_normals
@@ -312,7 +311,7 @@ def test_normals_in_utm_frame(pkg, pto, utm_case, torch_cuda):
             what = ("utm", k, radius)
             check_normals(pto, tree, P, tree.estimate_normals(k, radius=radius), pto_normals.estimate(xyz, m, idx),
                           idx, radius, what)
-            ref_o = orient_oracle.orient(xyz, m, idx)
+            ref_o = pto_orient.orient(xyz, m, idx)
             assert ref_o["flipped"] > 0
             check_orient(pto, tree, P, tree.orient_normals(k, radius=radius), ref_o, idx, radius, what)
 

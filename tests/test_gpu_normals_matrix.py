@@ -13,10 +13,9 @@ differing points equals pto.knn_bruteforce, which tells a k-NN fault from a PCA 
 import numpy as np
 import pytest
 
-import orient_oracle
 import test_normals as tn
 import test_orient as to
-from oracle import pto_normals
+from oracle import pto_normals, pto_orient
 from test_gpu_parity import MODES
 
 pytestmark = pytest.mark.gpu
@@ -139,7 +138,7 @@ def matrix_refs(pkg, pto, torch_cuda):
         refs = {}
         for k, radius in RUNS:
             idx = pto_normals.neighbours(xyz, k, -1.0 if radius is None else radius)
-            refs[k, radius] = (idx, pto_normals.estimate(xyz, m, idx), orient_oracle.orient(xyz, m, idx))
+            refs[k, radius] = (idx, pto_normals.estimate(xyz, m, idx), pto_orient.orient(xyz, m, idx))
         out[name] = (P, refs)
     return out
 
@@ -270,7 +269,7 @@ def test_chunk_edges(n, pkg, pto, torch_cuda):
             check_normals(pto, tree, P, got, pto_normals.estimate(xyz, m, idx), idx, None, (n, k))
         if n == CHUNK + 1:
             idx = pto_normals.neighbours(xyz, 18)
-            ref = orient_oracle.orient(xyz, m, idx)
+            ref = pto_orient.orient(xyz, m, idx)
             assert ref["flipped"] > n // 4
             check_orient(pto, tree, P, tree.orient_normals(18), ref, idx, None, n)
     finally:
@@ -311,7 +310,7 @@ def test_orientation_ties(name, pkg, pto, torch_cuda):
     top z (-0.0 with +0.0), and 3 000 components whose tied weights close frustrated triangles."""
     xyz, m, radius = to.TIE_CLOUDS[name]()
     lists = {k: pto_normals.neighbours(xyz, k, -1.0 if radius is None else radius) for k in (2, 8, 32)}
-    refs = {k: orient_oracle.orient(xyz, m, idx) for k, idx in lists.items()}
+    refs = {k: pto_orient.orient(xyz, m, idx) for k, idx in lists.items()}
     for k, idx in lists.items():
         to.check_tie_cloud(name, xyz, m, idx, refs[k])
     P = pkg.make_points(xyz, normal=m)

@@ -1,7 +1,7 @@
 """Normal orientation (DESIGN.md section 8, "Normal orientation"): signs propagated along the minimum
 spanning forest of the k-NN graph under (w = 1 - |n_i.n_j|, lo, hi), from each component's top point.
 
-CPU part: the oracle (tests/orient_oracle.c via tests/orient_oracle.py) against an independent
+CPU part: the oracle (oracle/pt_orient_oracle.c via oracle/pto_orient.py) against an independent
 statement (scipy's minimum_spanning_tree on the edge ranks, breadth_first_order), known answers on
 closed surfaces, and the CLI's refusals.  GPU part: pt_index_orient_normals and the CLI must equal the
 oracle bit for bit; `store` must feed transfers and bakes."""
@@ -15,8 +15,7 @@ import pytest
 from scipy.sparse import coo_matrix
 from scipy.sparse.csgraph import breadth_first_order, connected_components, minimum_spanning_tree
 
-import orient_oracle
-from oracle import pto_normals
+from oracle import pto_normals, pto_orient
 
 GOLDEN = sorted(glob.glob(os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden", "*.npz")))
 VIEW = (0.3, -2.0, 5.0)
@@ -88,7 +87,7 @@ def scipy_orient(xyz, normal, idx, viewpoint=None):
 
 
 def check_oracle_vs_scipy(xyz, normal, idx, viewpoint=None):
-    got = orient_oracle.orient(xyz, normal, idx, viewpoint)
+    got = pto_orient.orient(xyz, normal, idx, viewpoint)
     ref_n, ref_root, ref_parent, counts = scipy_orient(xyz, normal, idx, viewpoint)
     assert np.array_equal(got["normal"].view(np.uint32), ref_n.view(np.uint32))
     assert np.array_equal(got["root"], ref_root)
@@ -172,7 +171,7 @@ def test_closed_surfaces_come_out_outward(shape, pto):
         xyz, d = np.r_[a, b], np.r_[da, db]
         comp_of, n_comp = np.r_[np.zeros(20_000, int), np.ones(20_000, int)], 2
     m = scramble(d, rng)
-    got = orient_oracle.orient_normals(xyz, m, 18)
+    got = pto_orient.orient_normals(xyz, m, 18)
     assert got["components"] == n_comp and got["oriented"] == len(xyz)
     assert (dot(got["normal"].astype(np.float64), d) > 0).all()
     assert np.array_equal(got["root"], expected_roots(xyz, comp_of))
@@ -186,7 +185,7 @@ def test_pca_normals_of_a_sphere_come_out_outward(pto):
     assert e == len(xyz)
     inward = (dot(est.astype(np.float64), d) < 0).mean()
     assert 0.3 < inward < 0.7, inward
-    got = orient_oracle.orient_normals(xyz, est, 18)
+    got = pto_orient.orient_normals(xyz, est, 18)
     assert got["components"] == 1 and (dot(got["normal"].astype(np.float64), d) > 0).all()
 
 
@@ -393,7 +392,7 @@ def test_gpu_equals_oracle_on_golden_clouds(path, pkg, pto):
                 for radius in (None, float(g["radius"])):
                     idx = pto_normals.neighbours(g["xyz"], k, -1.0 if radius is None else radius)
                     for view in (None, VIEW):
-                        ref = orient_oracle.orient(g["xyz"], nrm, idx, view)
+                        ref = pto_orient.orient(g["xyz"], nrm, idx, view)
                         assert_same(tree.orient_normals(k, radius=radius, viewpoint=view), ref, (k, radius, view))
 
 
@@ -411,7 +410,7 @@ def test_gpu_equals_oracle_on_shapes(pkg, pto):
         xyz = xyz.astype(np.float32).astype(np.float64)                  # the positions an F32 index stores
         with pkg.Tree(pkg.make_points(xyz, normal=m)) as tree:
             for k, view in ((8, None), (18, None), (18, (0.0, 0.0, 10.0))):
-                ref = orient_oracle.orient(xyz, m, pto_normals.neighbours(xyz, k), view)
+                ref = pto_orient.orient(xyz, m, pto_normals.neighbours(xyz, k), view)
                 assert_same(tree.orient_normals(k, viewpoint=view), ref, k)
 
 
@@ -427,7 +426,7 @@ def test_gpu_more_than_one_chunk(pkg, pto):
     xyz = P["ver"].astype(np.float32).astype(np.float64)
     with pkg.Tree(P) as tree:
         got = tree.orient_normals(18)
-    ref = orient_oracle.orient(xyz, m, pto_normals.neighbours(xyz, 18))
+    ref = pto_orient.orient(xyz, m, pto_normals.neighbours(xyz, 18))
     assert_same(got, ref)
 
 

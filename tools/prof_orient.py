@@ -12,7 +12,7 @@ call to after the first call at each k: the pool keeps what it maps and k ascend
 that k's peak, an upper bound (fragmentation, the outputs' device buffers included).
 Same-run checks (exit 1 on a failure): two calls give identical outputs, and a --check-points cloud
 of cfg2's density equals the CPU oracle bit for bit; the oracle path (exact k-NN on a kd-tree + the C
-statement of tests/orient_oracle.c) is timed on it.  The card's name and power limit are read in the
+statement of oracle/pt_orient_oracle.c) is timed on it.  The card's name and power limit are read in the
 same run.
 
     python tools/prof_orient.py [--reps 5] [--check-points 4000000] [--out report.json]
@@ -28,7 +28,6 @@ import numpy as np
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 sys.path.insert(0, ROOT)
-sys.path.insert(0, os.path.join(ROOT, "tests"))
 
 EDGE_KERNELS = ("orient_unit_kernel", "orient_mask_kernel", "orient_edges_kernel", "DeviceScan")
 
@@ -78,8 +77,7 @@ def main():
 
     import torch
     import __graft_entry__ as ge
-    import orient_oracle
-    from oracle import pto, pto_normals
+    from oracle import pto, pto_normals, pto_orient
 
     pkg = ge.package()
     assert torch.cuda.is_available(), "prof_orient.py needs a CUDA device"
@@ -134,7 +132,7 @@ def main():
         t0 = time.perf_counter()
         idx = pto_normals.neighbours(xyz, k)
         t1 = time.perf_counter()
-        ref = orient_oracle.orient(xyz, nrm, idx)
+        ref = pto_orient.orient(xyz, nrm, idx)
         t2 = time.perf_counter()
         ok = bool(np.array_equal(got["normal"].view(np.uint32), ref["normal"].view(np.uint32)) and
                   np.array_equal(got["root"], ref["root"]) and
