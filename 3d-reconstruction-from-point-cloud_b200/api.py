@@ -54,6 +54,7 @@ ABI_SYMBOLS = (
     "pt_texture_bake_ex", "pt_bake_samples_device", "pt_bake_frames_device", "pt_bake_compose_tangent_device",
     "pt_texture_bake_height", "pt_bake_compose_height_device", "pt_sharded_bake",
     "pt_index_estimate_normals", "pt_estimate_normals_device", "pt_index_orient_normals",
+    "pt_sharded_estimate_normals",
 )
 # ... and include/pt_synth.h (bench / test scaffolding, its own library)
 SYNTH_SYMBOLS = ("pt_synth_cloud_device", "pt_synth_samples_device", "pt_synth_pack_points_device",
@@ -225,6 +226,8 @@ def lib():
     L.pt_index_estimate_normals.argtypes = [vp, i32, dbl, vp, i32, vp, vp, ctypes.POINTER(NormalsStats)]
     L.pt_estimate_normals_device.restype = i32
     L.pt_estimate_normals_device.argtypes = [vp, i32, dbl, vp, i32, vp, vp, vp]
+    L.pt_sharded_estimate_normals.restype = i32
+    L.pt_sharded_estimate_normals.argtypes = [vp, i32, dbl, vp, i32, vp, vp, ctypes.POINTER(NormalsStats)]
     L.pt_index_orient_normals.restype = i32
     L.pt_index_orient_normals.argtypes = [vp, i32, dbl, vp, i32, vp, vp, ctypes.POINTER(OrientStats)]
     L.pt_set_option.restype = i32
@@ -488,14 +491,8 @@ class Tree:
         the point's own normal where it is usable, else towards ``viewpoint`` (x, y, z) when given,
         else the largest component positive.  ``store=True`` also replaces the tree's normals with
         the estimates, so later ``transfer`` / ``bake`` calls blend them."""
-        n = self.size()
-        out = {"normal": np.empty((n, 3), dtype=np.float32), "variation": np.empty(n, dtype=np.float32)}
-        st = NormalsStats()
-        _check(lib().pt_index_estimate_normals(self._h, int(k), _radius(radius), _viewpoint(viewpoint),
-                                               1 if store else 0, _np_ptr(out["normal"]), _np_ptr(out["variation"]),
-                                               ctypes.byref(st)), "pt_index_estimate_normals")
-        out["stats"] = {"estimated": int(st.estimated), "knn_ms": st.knn_ms, "pca_ms": st.pca_ms}
-        return out
+        return _estimate_normals(lib().pt_index_estimate_normals, "pt_index_estimate_normals", self._h, self.size(),
+                                 k, radius, viewpoint, store)
 
     def orient_normals(self, k=18, radius=None, viewpoint=None, store=False):
         """Orients the tree's normals consistently by propagation along the minimum spanning forest of
@@ -566,6 +563,18 @@ def _bake(fn, name, handle, vertices, faces, k, resolution, radius, pad, want, h
     return out
 
 
+def _estimate_normals(fn, name, handle, n, k, radius, viewpoint, store):
+    """Output arrays and result dict of ``Tree.estimate_normals`` and ``ShardedTree.estimate_normals``:
+    ``fn`` is ``pt_index_estimate_normals`` or ``pt_sharded_estimate_normals``, which take the same
+    arguments after the handle."""
+    out = {"normal": np.empty((n, 3), dtype=np.float32), "variation": np.empty(n, dtype=np.float32)}
+    st = NormalsStats()
+    _check(fn(handle, int(k), _radius(radius), _viewpoint(viewpoint), 1 if store else 0, _np_ptr(out["normal"]),
+              _np_ptr(out["variation"]), ctypes.byref(st)), name)
+    out["stats"] = {"estimated": int(st.estimated), "knn_ms": st.knn_ms, "pca_ms": st.pca_ms}
+    return out
+
+
 class ShardedTree:
     """The cloud sharded over several GPUs of one box by the C++ host (``pt_sharded_*``,
     csrc/pt_sharded.cu): same calls as ``Tree``, ids index the caller's ``points``."""
@@ -616,6 +625,17 @@ class ShardedTree:
         own device; ``stats["knn_ms"]`` is the host wall time of that part."""
         return _bake(lib().pt_sharded_bake, "pt_sharded_bake", self._h, vertices, faces, k, resolution, radius, pad,
                      want, height_range)
+
+    def estimate_normals(self, k=16, radius=None, viewpoint=None, store=False):
+        """``Tree.estimate_normals`` on the sharded cloud (``pt_sharded_estimate_normals``): same
+        arguments and result, ``normal``, ``variation`` and ``stats["estimated"]`` byte-identical to
+        ``Tree.estimate_normals`` on one index of the same cloud.  Each slab estimates the points it
+        owns on its own device; ``stats["knn_ms"]`` is the host wall time of that stage and
+        ``stats["pca_ms"]`` the PCA kernels' device time summed over the slabs.  ``store=True`` also
+        replaces the normals in every slab that holds the point, so later ``transfer`` / ``bake``
+        calls blend them, and keeps them across rebuilds of the slabs."""
+        return _estimate_normals(lib().pt_sharded_estimate_normals, "pt_sharded_estimate_normals", self._h,
+                                 self._points.shape[0], k, radius, viewpoint, store)
 
     def close(self):
         if getattr(self, "_h", None) and self._h.value:

@@ -92,9 +92,37 @@ int index_inverse_perm(pt_index *ix);
 // index's own ids.  keep: lists holds n x k and row r's list is at lists + r k; else lists holds one
 // chunk's rows and is reused.  then(c0, cm, lists of rows c0 .. c0 + cm) follows each chunk's query
 // and returns a status.  marks (may be null): an event before the first chunk and after each query.
+// rows (device, may be null): only the n_rows sorted records rows[0 .. n_rows - 1] are queried, and
+// row r is sorted record rows[r].  ghost (may be null): launch_ghost_check on each chunk's rows.
+struct BakeGhost;
 using ChunkThen = std::function<int(uint32_t c0, uint32_t cm, const int32_t *lists)>;
 int self_query_chunks(pt_index *ix, int k, double radius, int32_t *lists, bool keep, const ChunkThen &then,
-                      std::vector<cudaEvent_t> *marks, cudaStream_t s);
+                      std::vector<cudaEvent_t> *marks, cudaStream_t s, const uint32_t *rows = nullptr,
+                      uint32_t n_rows = 0, const BakeGhost *ghost = nullptr);
+// The argument rules of pt_index_estimate_normals that do not concern the index: PT_OK or its error.
+int normals_check_args(int k, const double *viewpoint, bool store, bool any_output);
+// One slab of pt_sharded_estimate_normals (pt_normals.cu), on ix's device and stream: the normals of
+// the records the slab owns -- those whose x the host's cut rule (the number of the n_slabs - 1
+// ascending interior `cuts` c with !(x < c)) gives to slab `self`, n_own of them as build_slabs
+// counted (PT_ERR_UNSUPPORTED otherwise) -- into normal_out (n_own x 3) / variation_out (n_own),
+// host buffers, in ascending local id.  check: the ghost-zone check runs on the own rows against
+// the slabs' own boxes (host, n_slabs x 6) and `halo`, and *needs = 1 when it flags the step.  Adds
+// the points estimated to *estimated and sets *pca_ms to the PCA kernels' device time.
+// Synchronises.
+struct NormalsSlab {
+    const double *cuts;
+    int n_slabs, self;
+    size_t n_own;
+    const double *boxes;
+    double halo;
+    bool check;
+};
+int normals_slab(pt_index *ix, int k, double radius, const double *viewpoint, const NormalsSlab &sl,
+                 float *normal_out, float *variation_out, unsigned long long *estimated, float *pca_ms,
+                 int *needs);
+// Writes values (host, n x 3 floats in ix's local order, x NaN: leave that point as it is) into the
+// normals of ix's attrs and attrs_curve, on ix's stream; synchronises.
+int normals_store(pt_index *ix, const float *values);
 // marks != null: appends an event recorded on s
 cudaError_t record_mark(std::vector<cudaEvent_t> *marks, cudaStream_t s);
 // Stream-ordered allocation from the library's PRIVATE memory pool of the current device (the

@@ -5,10 +5,15 @@
 // (row r = sorted record r, so the k-NN kernels see coherent samples), one launch_query writes the
 // neighbour lists, and normals_pca_kernel turns every list into a normal and a surface variation.
 // Everything is fp64 with every operation rounded on its own, in the order DESIGN.md states, so
-// that oracle/pt_normals_oracle.c equals it bit for bit.
+// that oracle/pt_normals_oracle.c equals it bit for bit.  A sharded cloud (pt_sharded.cu) runs the
+// same kernels per slab over the rows of the records the slab owns (normals_slab, DESIGN.md
+// section 8, "Sharded normal estimation").
 #include <algorithm>
 #include <cmath>
 #include <vector>
+
+#include <cub/device/device_select.cuh>
+#include <thrust/iterator/counting_iterator.h>
 
 #include "pt_bake.cuh"
 #include "pt_fp64.cuh"
@@ -20,15 +25,29 @@ constexpr int JACOBI_MAX_SWEEPS = 50;
 
 static inline unsigned ncdiv(size_t a, size_t b) { return (unsigned)((a + b - 1) / b); }
 
-template <typename PT>
-__global__ void __launch_bounds__(256) normals_rows_kernel(const PT *pts, uint32_t r0, uint32_t count, double *xyz)
+// Query row i of a chunk is sorted record r0 + i, or with LIST sorted record rows[r0 + i].
+template <typename PT, bool LIST>
+__device__ __forceinline__ void normals_rows(const PT *pts, const uint32_t *rows, uint32_t r0, uint32_t count, double *xyz)
 {
     const uint32_t i = blockIdx.x * blockDim.x + threadIdx.x;
     if (i >= count) return;
-    const PT rec = pts[r0 + i];
+    const PT rec = pts[LIST ? rows[r0 + i] : r0 + i];
     xyz[3 * (size_t)i] = (double)rec.x;
     xyz[3 * (size_t)i + 1] = (double)rec.y;
     xyz[3 * (size_t)i + 2] = (double)rec.z;
+}
+
+template <typename PT>
+__global__ void __launch_bounds__(256) normals_rows_kernel(const PT *pts, uint32_t r0, uint32_t count, double *xyz)
+{
+    normals_rows<PT, false>(pts, nullptr, r0, count, xyz);
+}
+
+template <typename PT>
+__global__ void __launch_bounds__(256)
+normals_rows_list_kernel(const PT *pts, const uint32_t *rows, uint32_t r0, uint32_t count, double *xyz)
+{
+    normals_rows<PT, true>(pts, rows, r0, count, xyz);
 }
 
 // ROTATE of Numerical Recipes' jacobi: (g, h) <- (g - s (h + g tau), h + s (g - h tau))
@@ -120,10 +139,11 @@ struct NormalsOut {
 // centroid and then the six scatter sums in neighbour order through shuffles.  The sums go to the
 // row's own lane, and after the rounds every lane solves its row's 3 x 3 on its own, so the Jacobi
 // sweeps run 32 rows wide.  Every lane runs the same loops, so the shuffles see the full warp.
-template <typename PT>
-__global__ void __launch_bounds__(256)
-normals_pca_kernel(const PT *pts, const uint32_t *inv, uint32_t n_points, uint32_t r0, uint32_t count,
-                   const int32_t *idx, int k, int width, const NormalsOut o)
+// With LIST, row r0 + i of the chunk is sorted record rows[r0 + i] instead of r0 + i.
+template <typename PT, bool LIST>
+__device__ __forceinline__ void normals_pca(const PT *pts, const uint32_t *inv, uint32_t n_points, const uint32_t *rows,
+                                            uint32_t r0, uint32_t count, const int32_t *idx, int k, int width,
+                                            const NormalsOut &o)
 {
     const unsigned lane = threadIdx.x & 31u;
     const uint32_t base = (uint32_t)(((size_t)blockIdx.x * blockDim.x + threadIdx.x) >> 5) * 32u;
@@ -179,7 +199,7 @@ normals_pca_kernel(const PT *pts, const uint32_t *inv, uint32_t n_points, uint32
     }
     if (!mine) return;
 
-    const uint32_t row = r0 + base + lane;
+    const uint32_t row = LIST ? rows[r0 + base + lane] : r0 + base + lane;
     const PT rec = pts[row];
     const uint32_t orig = (uint32_t)rec.idx;
     const D3 pi = {(double)rec.x, (double)rec.y, (double)rec.z};
@@ -231,6 +251,22 @@ normals_pca_kernel(const PT *pts, const uint32_t *inv, uint32_t n_points, uint32
     }
 }
 
+template <typename PT>
+__global__ void __launch_bounds__(256)
+normals_pca_kernel(const PT *pts, const uint32_t *inv, uint32_t n_points, uint32_t r0, uint32_t count,
+                   const int32_t *idx, int k, int width, const NormalsOut o)
+{
+    normals_pca<PT, false>(pts, inv, n_points, nullptr, r0, count, idx, k, width, o);
+}
+
+template <typename PT>
+__global__ void __launch_bounds__(256)
+normals_pca_list_kernel(const PT *pts, const uint32_t *inv, uint32_t n_points, const uint32_t *rows, uint32_t r0,
+                        uint32_t count, const int32_t *idx, int k, int width, const NormalsOut o)
+{
+    normals_pca<PT, true>(pts, inv, n_points, rows, r0, count, idx, k, width, o);
+}
+
 static int normals_width(int k)
 {
     int w = 1;
@@ -248,11 +284,12 @@ cudaError_t record_mark(std::vector<cudaEvent_t> *marks, cudaStream_t s)
 
 template <typename PT>
 static int self_query_chunks_t(pt_index *ix, int k, double radius, int32_t *lists, bool keep, const ChunkThen &then,
-                               std::vector<cudaEvent_t> *marks, cudaStream_t s)
+                               std::vector<cudaEvent_t> *marks, cudaStream_t s, const uint32_t *rows, uint32_t n_rows,
+                               const BakeGhost *ghost)
 {
-    const uint32_t n = ix->n;
+    const uint32_t n = rows ? n_rows : ix->n;
     const size_t chunk = std::min((size_t)HEIGHT_CHUNK, (size_t)n);
-    double *d_q = nullptr;
+    double *d_q = nullptr, *d_d2 = nullptr;
     int rc = PT_OK;
     auto fail = [&](cudaError_t e) { if (e != cudaSuccess && rc == PT_OK) rc = map_cuda_error(e); return e != cudaSuccess; };
     do {
@@ -261,7 +298,8 @@ static int self_query_chunks_t(pt_index *ix, int k, double radius, int32_t *list
         const bool fresh = ix->inv_perm == nullptr;
         if ((rc = index_inverse_perm(ix)) != PT_OK) break;
         if (fresh && s != ix->stream && fail(cudaStreamSynchronize(ix->stream))) break;
-        if (pool_alloc((void **)&d_q, sizeof(double) * 3 * chunk, s)) {
+        if (pool_alloc((void **)&d_q, sizeof(double) * 3 * chunk, s) ||
+            (ghost && pool_alloc((void **)&d_d2, sizeof(double) * k * chunk, s))) {
             rc = PT_ERR_OUT_OF_MEMORY;
             break;
         }
@@ -271,27 +309,36 @@ static int self_query_chunks_t(pt_index *ix, int k, double radius, int32_t *list
         qp.k = k;
         qp.r2 = radius_to_r2(radius);
         qp.queries = d_q;
+        qp.d2_out = d_d2;
         const PT *pts = (const PT *)ix->pts;
         for (size_t c0 = 0; c0 < n; c0 += chunk) {
             const uint32_t cm = (uint32_t)std::min(chunk, (size_t)n - c0);
-            normals_rows_kernel<PT><<<ncdiv(cm, 256), 256, 0, s>>>(pts, (uint32_t)c0, cm, d_q);
+            if (rows)
+                normals_rows_list_kernel<PT><<<ncdiv(cm, 256), 256, 0, s>>>(pts, rows, (uint32_t)c0, cm, d_q);
+            else
+                normals_rows_kernel<PT><<<ncdiv(cm, 256), 256, 0, s>>>(pts, (uint32_t)c0, cm, d_q);
             count_launch();
             qp.m = cm;
             qp.idx_out = keep ? lists + c0 * (size_t)k : lists;
             if ((rc = launch_query(ix, qp, s)) != PT_OK) break;
+            if (ghost && (rc = launch_ghost_check(d_q, d_d2, cm, k, qp.r2, ghost->boxes, ghost->n_ranks, ghost->self,
+                                                  ghost->halo, ghost->flag, s)) != PT_OK)
+                break;
             if (fail(record_mark(marks, s))) break;
             if ((rc = then((uint32_t)c0, cm, qp.idx_out)) != PT_OK) break;
         }
     } while (0);
     pool_free(d_q, s);
+    pool_free(d_d2, s);
     return rc;
 }
 
 int self_query_chunks(pt_index *ix, int k, double radius, int32_t *lists, bool keep, const ChunkThen &then,
-                      std::vector<cudaEvent_t> *marks, cudaStream_t s)
+                      std::vector<cudaEvent_t> *marks, cudaStream_t s, const uint32_t *rows, uint32_t n_rows,
+                      const BakeGhost *ghost)
 {
-    return ix->coord_f64 ? self_query_chunks_t<PointD>(ix, k, radius, lists, keep, then, marks, s)
-                         : self_query_chunks_t<PointF>(ix, k, radius, lists, keep, then, marks, s);
+    return ix->coord_f64 ? self_query_chunks_t<PointD>(ix, k, radius, lists, keep, then, marks, s, rows, n_rows, ghost)
+                         : self_query_chunks_t<PointF>(ix, k, radius, lists, keep, then, marks, s, rows, n_rows, ghost);
 }
 
 // All points of ix in chunks, asynchronous on s.  marks (may be null): an event before the first
@@ -319,13 +366,21 @@ static int normals_run(pt_index *ix, int k, double radius, const NormalsOut &o, 
     return rc;
 }
 
-static int normals_check(const pt_index *ix, int k, const double *viewpoint, bool store, bool any_output)
+int normals_check_args(int k, const double *viewpoint, bool store, bool any_output)
 {
-    if (!ix || (!any_output && !store)) return PT_ERR_INVALID_ARG;
+    if (!any_output && !store) return PT_ERR_INVALID_ARG;
     if (viewpoint && !(std::isfinite(viewpoint[0]) && std::isfinite(viewpoint[1]) && std::isfinite(viewpoint[2])))
         return PT_ERR_INVALID_ARG;
     if (k < 3) return PT_ERR_INVALID_ARG;             // a plane needs three points
     if (k > PT_MAX_K) return PT_ERR_UNSUPPORTED;
+    return PT_OK;
+}
+
+static int normals_check(const pt_index *ix, int k, const double *viewpoint, bool store, bool any_output)
+{
+    if (!ix) return PT_ERR_INVALID_ARG;
+    const int rc = normals_check_args(k, viewpoint, store, any_output);
+    if (rc != PT_OK) return rc;
     if (store && !ix->attrs && ix->n) return PT_ERR_INVALID_ARG;
     if (pt_device_count() == 0) return PT_ERR_NO_DEVICE;
     return PT_OK;
@@ -350,6 +405,213 @@ static int normals_device(pt_index *ix, int k, double radius, const NormalsOut &
                           cudaStream_t s)
 {
     return ix->coord_f64 ? normals_run<PointD>(ix, k, radius, o, marks, s) : normals_run<PointF>(ix, k, radius, o, marks, s);
+}
+
+// ---- sharded clouds (DESIGN.md section 8, "Sharded normal estimation") ------------------------------
+// A slab's own records: the host's cut rule on the stored x, which widens to the caller's x exactly
+// in both storage modes, so this is the owner build_slabs gave the point.
+template <typename PT>
+struct SlabOwnRow {
+    const PT *pts;
+    const double *cuts;       // device, n_cuts ascending
+    int n_cuts, self;
+    __device__ __forceinline__ bool operator()(uint32_t r) const
+    {
+        const double x = (double)pts[r].x;
+        int slab = 0;
+        for (int j = 0; j < n_cuts; ++j) slab += !(x < cuts[j]) ? 1 : 0;
+        return slab == self;
+    }
+};
+
+// ... and the same rule by local id i (the record at sorted position inv[i])
+template <typename PT>
+struct SlabOwnLocal {
+    SlabOwnRow<PT> own;
+    const uint32_t *inv;
+    __device__ __forceinline__ bool operator()(uint32_t i) const { return own(inv[i]); }
+};
+
+// row j of the compact outputs takes the results of local id own[j]
+__global__ void __launch_bounds__(256)
+normals_compact_kernel(const uint32_t *own, uint32_t m, const float *normal, const float *variation, float *c_normal,
+                       float *c_variation)
+{
+    const uint32_t j = blockIdx.x * blockDim.x + threadIdx.x;
+    if (j >= m) return;
+    const uint32_t i = own[j];
+    c_normal[3 * (size_t)j] = normal[3 * (size_t)i];
+    c_normal[3 * (size_t)j + 1] = normal[3 * (size_t)i + 1];
+    c_normal[3 * (size_t)j + 2] = normal[3 * (size_t)i + 2];
+    c_variation[j] = variation[i];
+}
+
+// attrs[i] and attrs_curve[inv[i]] take the normal values[i] where its x is not NaN
+__global__ void __launch_bounds__(256)
+normals_store_kernel(const float *values, uint32_t n, const uint32_t *inv, pt_attr *attrs, pt_attr *attrs_curve)
+{
+    const uint32_t i = blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= n) return;
+    const float x = values[3 * (size_t)i];
+    if (x != x) return;
+    const float y = values[3 * (size_t)i + 1], z = values[3 * (size_t)i + 2];
+    attrs[i].nx = x; attrs[i].ny = y; attrs[i].nz = z;
+    if (attrs_curve) {
+        const uint32_t r = inv[i];
+        attrs_curve[r].nx = x; attrs_curve[r].ny = y; attrs_curve[r].nz = z;
+    }
+}
+
+template <typename PT>
+static int normals_slab_t(pt_index *ix, int k, double radius, const double *viewpoint, const NormalsSlab &sl,
+                          float *normal_out, float *variation_out, unsigned long long *estimated, float *pca_ms,
+                          int *needs)
+{
+    cudaStream_t s = ix->stream;
+    const uint32_t n = ix->n;
+    uint32_t *d_rows = nullptr, *d_count = nullptr, *d_flag = nullptr;
+    int32_t *d_idx = nullptr;
+    float *d_normal = nullptr, *d_var = nullptr, *d_cnormal = nullptr, *d_cvar = nullptr;
+    double *d_boxes = nullptr;          // n_slabs x 6 boxes, then the n_slabs - 1 cuts
+    unsigned long long *d_est = nullptr, est = 0;
+    void *d_tmp = nullptr;
+    uint32_t n_rows = 0, flag = 0;
+    std::vector<cudaEvent_t> marks;
+    int rc = PT_OK;
+    auto fail = [&](cudaError_t e) { if (e != cudaSuccess && rc == PT_OK) rc = map_cuda_error(e); return e != cudaSuccess; };
+    do {
+        if (sl.n_slabs < 1 || sl.n_slabs > BAKE_MAX_SLABS || sl.self < 0 || sl.self >= sl.n_slabs) {
+            rc = PT_ERR_INVALID_ARG;
+            break;
+        }
+        const int R = sl.n_slabs;
+        if (pool_alloc((void **)&d_boxes, sizeof(double) * (7 * R - 1), s) ||
+            pool_alloc((void **)&d_rows, sizeof(uint32_t) * n, s) || pool_alloc((void **)&d_count, sizeof(uint32_t), s) ||
+            pool_alloc((void **)&d_flag, sizeof(uint32_t), s)) {
+            rc = PT_ERR_OUT_OF_MEMORY;
+            break;
+        }
+        if (fail(cudaMemcpyAsync(d_boxes, sl.boxes, sizeof(double) * 6 * R, cudaMemcpyHostToDevice, s)) ||
+            (R > 1 && fail(cudaMemcpyAsync(d_boxes + 6 * R, sl.cuts, sizeof(double) * (R - 1), cudaMemcpyHostToDevice, s))) ||
+            fail(cudaMemsetAsync(d_flag, 0, sizeof(uint32_t), s)))
+            break;
+        // the own records in ascending sorted position, so the self-queries stay curve-coherent
+        const SlabOwnRow<PT> own{(const PT *)ix->pts, d_boxes + 6 * R, R - 1, sl.self};
+        thrust::counting_iterator<uint32_t> ids(0);
+        size_t row_bytes = 0, local_bytes = 0;
+        if (fail(cub::DeviceSelect::If(nullptr, row_bytes, ids, d_rows, d_count, (int)n, own, s)) ||
+            fail(cub::DeviceSelect::If(nullptr, local_bytes, ids, d_rows, d_count, (int)n, SlabOwnLocal<PT>{own, nullptr}, s)))
+            break;
+        if (pool_alloc(&d_tmp, std::max(std::max(row_bytes, local_bytes), (size_t)1), s)) {
+            rc = PT_ERR_OUT_OF_MEMORY;
+            break;
+        }
+        if (fail(cub::DeviceSelect::If(d_tmp, row_bytes, ids, d_rows, d_count, (int)n, own, s))) break;
+        count_launch();
+        if (fail(cudaMemcpyAsync(&n_rows, d_count, sizeof n_rows, cudaMemcpyDeviceToHost, s)) ||
+            fail(cudaStreamSynchronize(s)))
+            break;
+        // the records this rule selects are the ones build_slabs counted as the slab's own
+        if (n_rows != sl.n_own) {
+            rc = PT_ERR_UNSUPPORTED;
+            break;
+        }
+        if (n_rows == 0) break;
+        const size_t chunk = std::min((size_t)HEIGHT_CHUNK, (size_t)n_rows);
+        if (pool_alloc((void **)&d_idx, sizeof(int32_t) * k * chunk, s) ||
+            pool_alloc((void **)&d_normal, sizeof(float) * 3 * n, s) || pool_alloc((void **)&d_var, sizeof(float) * n, s) ||
+            pool_alloc((void **)&d_cnormal, sizeof(float) * 3 * n_rows, s) ||
+            pool_alloc((void **)&d_cvar, sizeof(float) * n_rows, s) || pool_alloc((void **)&d_est, sizeof(unsigned long long), s)) {
+            rc = PT_ERR_OUT_OF_MEMORY;
+            break;
+        }
+        if (fail(cudaMemsetAsync(d_est, 0, sizeof(unsigned long long), s))) break;
+        const BakeGhost ghost{d_boxes, R, sl.self, sl.halo, d_flag};
+        // no store here: the caller stores once every slab has passed its check
+        const NormalsOut o = normals_out(ix, viewpoint, false, d_normal, d_var, d_est);
+        rc = self_query_chunks(
+            ix, k, radius, d_idx, false,
+            [&](uint32_t c0, uint32_t cm, const int32_t *idx) {
+                normals_pca_list_kernel<PT><<<ncdiv(cm, 256), 256, 0, s>>>((const PT *)ix->pts, ix->inv_perm, n, d_rows, c0,
+                                                                           cm, idx, k, normals_width(k), o);
+                count_launch();
+                cudaError_t e = cudaGetLastError();
+                if (e == cudaSuccess) e = record_mark(&marks, s);
+                return e == cudaSuccess ? PT_OK : map_cuda_error(e);
+            },
+            &marks, s, d_rows, n_rows, sl.check ? &ghost : nullptr);
+        if (rc != PT_OK) break;
+        // only the own records' results travel to the host, in ascending local id (the order of their
+        // global ids); the row list is free again in stream order and takes their local ids
+        if (fail(cub::DeviceSelect::If(d_tmp, local_bytes, ids, d_rows, d_count, (int)n,
+                                       SlabOwnLocal<PT>{own, ix->inv_perm}, s)))
+            break;
+        count_launch();
+        normals_compact_kernel<<<ncdiv(n_rows, 256), 256, 0, s>>>(d_rows, n_rows, d_normal, d_var, d_cnormal, d_cvar);
+        count_launch();
+        if (fail(cudaGetLastError())) break;
+        if (fail(cudaMemcpyAsync(normal_out, d_cnormal, sizeof(float) * 3 * n_rows, cudaMemcpyDeviceToHost, s)) ||
+            fail(cudaMemcpyAsync(variation_out, d_cvar, sizeof(float) * n_rows, cudaMemcpyDeviceToHost, s)) ||
+            fail(cudaMemcpyAsync(&est, d_est, sizeof est, cudaMemcpyDeviceToHost, s)) ||
+            fail(cudaMemcpyAsync(&flag, d_flag, sizeof flag, cudaMemcpyDeviceToHost, s)) || fail(cudaStreamSynchronize(s)))
+            break;
+        *estimated += est;
+        *needs = sl.check && flag ? 1 : 0;
+        // marks: start, then per chunk (after the query and check, after the PCA kernel)
+        float t = 0.0f;
+        for (size_t c = 1; c + 1 < marks.size(); c += 2)
+            if (cudaEventElapsedTime(&t, marks[c], marks[c + 1]) == cudaSuccess) *pca_ms += t;
+    } while (0);
+    cudaStreamSynchronize(s);
+    void *frees[] = {d_rows, d_count, d_flag, d_idx, d_normal, d_var, d_cnormal, d_cvar, d_boxes, d_est, d_tmp};
+    for (void *p : frees) pool_free(p, s);
+    for (auto &e : marks) if (e) cudaEventDestroy(e);
+    cudaStreamSynchronize(s);
+    cudaGetLastError();
+    return rc;
+}
+
+int normals_slab(pt_index *ix, int k, double radius, const double *viewpoint, const NormalsSlab &sl,
+                 float *normal_out, float *variation_out, unsigned long long *estimated, float *pca_ms, int *needs)
+{
+    *pca_ms = 0.0f;
+    *needs = 0;
+    if (!ix) return PT_ERR_INVALID_ARG;
+    if (ix->n == 0) return PT_OK;
+    PT_CUDA(cudaSetDevice(ix->device));
+    return ix->coord_f64
+               ? normals_slab_t<PointD>(ix, k, radius, viewpoint, sl, normal_out, variation_out, estimated, pca_ms, needs)
+               : normals_slab_t<PointF>(ix, k, radius, viewpoint, sl, normal_out, variation_out, estimated, pca_ms, needs);
+}
+
+int normals_store(pt_index *ix, const float *values)
+{
+    if (!ix) return PT_ERR_INVALID_ARG;
+    if (ix->n == 0) return PT_OK;             // an empty index (a slab that owns nothing) has no attrs
+    if (!ix->attrs) return PT_ERR_INVALID_ARG;
+    PT_CUDA(cudaSetDevice(ix->device));
+    cudaStream_t s = ix->stream;
+    const uint32_t n = ix->n;
+    float *d_values = nullptr;
+    int rc = index_inverse_perm(ix);
+    auto fail = [&](cudaError_t e) { if (e != cudaSuccess && rc == PT_OK) rc = map_cuda_error(e); return e != cudaSuccess; };
+    do {
+        if (rc != PT_OK) break;
+        if (pool_alloc((void **)&d_values, sizeof(float) * 3 * n, s)) {
+            rc = PT_ERR_OUT_OF_MEMORY;
+            break;
+        }
+        if (fail(cudaMemcpyAsync(d_values, values, sizeof(float) * 3 * n, cudaMemcpyHostToDevice, s))) break;
+        normals_store_kernel<<<ncdiv(n, 256), 256, 0, s>>>(d_values, n, ix->inv_perm, ix->attrs, ix->attrs_curve);
+        count_launch();
+        if (fail(cudaGetLastError())) break;
+        fail(cudaStreamSynchronize(s));
+    } while (0);
+    cudaStreamSynchronize(s);
+    pool_free(d_values, s);
+    cudaStreamSynchronize(s);
+    cudaGetLastError();
+    return rc;
 }
 
 }  // namespace pt

@@ -18,6 +18,11 @@
 //             home device, pt_bake.cuh pieces); the samples are partitioned by slab there, each
 //             slab answers its rows on its own device (k-NN + blend + ghost check + heights from
 //             its own records) and the results are scattered back into sample order.
+//   normals : pt_index_estimate_normals on the sharded cloud (DESIGN.md section 8, "Sharded normal
+//             estimation"): every slab estimates the points it owns on its own device, from its
+//             own records with the ghost-zone check on those rows, and the host scatters the
+//             results into the caller's point order.  A store reaches every copy of a point (the
+//             live slab indexes, and the records of every later rebuild).
 //
 // The reference has no multi-GPU path (its query loop is src/pointsTransfer.cpp:465-479); the
 // torch.distributed / NCCL form of the same sharding (one process per GPU, unsorted samples
@@ -27,6 +32,7 @@
 #include <chrono>
 #include <cmath>
 #include <cstring>
+#include <functional>
 #include <new>
 #include <thread>
 #include <vector>
@@ -50,6 +56,8 @@ struct Slab {
     int device = 0;
     size_t n_own = 0, n_ghost = 0;
     double box[6] = {INFINITY, INFINITY, INFINITY, -INFINITY, -INFINITY, -INFINITY};   // own points
+    std::vector<int32_t> ids;         // the global id of every record, in the index's local order
+    std::vector<uint8_t> own;         // 1 where that record is one of the slab's own points
 };
 
 }  // namespace
@@ -64,6 +72,9 @@ struct pt_sharded {
     double halo_auto = 0.0;           // the bounding-box estimate (4x the expected k-th neighbour distance)
     int coord_mode = PT_COORD_AUTO;
     int rebuilds = 0;
+    // the normals pt_sharded_estimate_normals stored, n x 3 in point order (x NaN: none, the point
+    // keeps its input normal); empty until the first store.  build_slabs puts them in the records.
+    std::vector<float> stored;
 };
 
 namespace {
@@ -73,6 +84,8 @@ void free_slabs(pt_sharded *S)
     for (auto &s : S->slabs) {
         if (s.index) pt_index_free(s.index);
         s.index = nullptr;
+        std::vector<int32_t>().swap(s.ids);
+        std::vector<uint8_t>().swap(s.own);
     }
 }
 
@@ -110,8 +123,10 @@ int build_slabs(pt_sharded *S)
             Slab &s = S->slabs[r];
             std::vector<Rec80> rec;
             std::vector<int32_t> ids;
+            std::vector<uint8_t> own;
             rec.reserve(s.n_own + s.n_own / 16 + 1024);
             ids.reserve(s.n_own + s.n_own / 16 + 1024);
+            own.reserve(s.n_own + s.n_own / 16 + 1024);
             const double *b = s.box;
             for (size_t i = 0; i < n; ++i) {          // index order: global ids ascending
                 bool take = owner[i] == r;
@@ -121,7 +136,15 @@ int build_slabs(pt_sharded *S)
                     const double ez = std::max(std::max(b[2] - P[i].ver[2], P[i].ver[2] - b[5]), 0.0);
                     take = ex * ex + ey * ey + ez * ez <= h2;
                 }
-                if (take) { rec.push_back(P[i]); ids.push_back((int32_t)i); }
+                if (take) {
+                    rec.push_back(P[i]);
+                    ids.push_back((int32_t)i);
+                    own.push_back(owner[i] == r ? 1 : 0);
+                    // a stored normal, widened: the build narrows it back to the same float
+                    const float *m = S->stored.empty() ? nullptr : &S->stored[3 * i];
+                    if (m && m[0] == m[0])
+                        for (int a = 0; a < 3; ++a) rec.back().normal[a] = (double)m[a];
+                }
             }
             s.n_ghost = rec.size() - s.n_own;
             pt_build_opts o;
@@ -130,6 +153,8 @@ int build_slabs(pt_sharded *S)
             o.coord_mode = S->coord_mode;
             o.ids = ids.data();
             status[r] = pt_index_build(rec.data(), rec.size(), &o, &s.index);
+            s.ids = std::move(ids);
+            s.own = std::move(own);
           } catch (...) { status[r] = PT_ERR_OUT_OF_MEMORY; }     // nothing is thrown across the ABI
     };
     for (int r = 0; r < R; ++r) {
@@ -434,6 +459,116 @@ int sharded_bake(pt_sharded *S, const void *vertices, size_t n_vertices, const i
     return rc;
 }
 
+// pt_index_estimate_normals on the sharded cloud; arguments checked, S->n > 0.
+int sharded_normals(pt_sharded *S, int k, double radius, const double *viewpoint, bool store, float *normal_out,
+                    float *variation_out, pt_normals_stats *stats)
+{
+    const int R = (int)S->slabs.size();
+    const auto t0 = std::chrono::steady_clock::now();
+    std::vector<std::vector<float>> nrm(R), var(R);
+    std::vector<unsigned long long> est(R, 0);
+    std::vector<float> pca(R, 0.0f);
+    auto each_slab = [&](const std::function<int(int)> &f) {
+        std::vector<int> status(R, PT_OK);
+        std::vector<std::thread> th;
+        auto work = [&](int r) {
+            try {
+                status[r] = f(r);
+            } catch (...) { status[r] = PT_ERR_OUT_OF_MEMORY; }
+        };
+        for (int r = 0; r < R; ++r) {
+            try { th.emplace_back(work, r); } catch (...) { work(r); }
+        }
+        for (auto &t : th) t.join();
+        for (int r = 0; r < R; ++r)
+            if (status[r] != PT_OK) return status[r];
+        return (int)PT_OK;
+    };
+    // every slab estimates its own points; nothing reaches the caller or the slabs before all pass
+    int rc = PT_OK;
+    bool done = false;
+    for (int attempt = 0; attempt < 8 && !done; ++attempt) {
+        std::vector<int> needs(R, 0);
+        rc = each_slab([&](int r) {
+            const Slab &sl = S->slabs[r];
+            est[r] = 0;
+            pca[r] = 0.0f;
+            if (!sl.index) return (int)PT_ERR_INVALID_ARG;
+            if (sl.n_own == 0) return (int)PT_OK;
+            nrm[r].resize(3 * sl.n_own);
+            var[r].resize(sl.n_own);
+            // a slab whose index holds the whole cloud answers every point exactly: no check
+            const bool whole = sl.n_own + sl.n_ghost == S->n;
+            const pt::NormalsSlab job{S->cuts.data() + 1, R, r, sl.n_own, S->boxes.data(), S->halo, !whole};
+            return pt::normals_slab(sl.index, k, radius, viewpoint, job, nrm[r].data(), var[r].data(), &est[r], &pca[r],
+                                    &needs[r]);
+        });
+        if (rc != PT_OK) return rc;
+        done = std::none_of(needs.begin(), needs.end(), [](int v) { return v != 0; });
+        if (done) break;
+        // some k-th-neighbour ball may leave a ghost zone: widen it and estimate again
+        S->halo = std::max(4.0 * S->halo, S->halo_auto);
+        ++S->rebuilds;
+        if ((rc = build_slabs(S)) != PT_OK) return rc;
+    }
+    if (!done) return PT_ERR_UNSUPPORTED;
+    // the own entries into the caller's point order (slabs own disjoint points)
+    if (store && S->stored.empty()) S->stored.assign(3 * S->n, NAN);
+    // each slab's own results come in ascending local id: the i-th goes to the global id of the
+    // slab's i-th own record.  Ranges of records over a share of the host's cores.
+    const size_t share = std::max(1u, std::thread::hardware_concurrency() / (unsigned)R);
+    rc = each_slab([&](int r) {
+        const Slab &sl = S->slabs[r];
+        if (sl.n_own == 0) return (int)PT_OK;
+        const float *nr = nrm[r].data(), *vr = var[r].data();
+        const size_t nl = sl.ids.size(), parts = std::min(share, nl / 65536 + 1), step = (nl + parts - 1) / parts;
+        std::vector<size_t> first(parts + 1, 0);           // own records before each range
+        for (size_t p = 0; p < parts; ++p)
+            first[p + 1] = first[p] + (size_t)std::count(sl.own.begin() + std::min(nl, p * step),
+                                                         sl.own.begin() + std::min(nl, (p + 1) * step), (uint8_t)1);
+        if (first[parts] != sl.n_own) return (int)PT_ERR_UNSUPPORTED;
+        auto scatter = [&](size_t p) {
+            size_t j = first[p];
+            for (size_t l = p * step; l < std::min(nl, (p + 1) * step); ++l) {
+                if (!sl.own[l]) continue;                                  // a ghost: its owner writes it
+                const size_t g = (size_t)sl.ids[l];
+                if (normal_out) memcpy(normal_out + 3 * g, nr + 3 * j, sizeof(float) * 3);
+                if (variation_out) variation_out[g] = vr[j];
+                if (store && vr[j] == vr[j]) memcpy(&S->stored[3 * g], nr + 3 * j, sizeof(float) * 3);   // estimated
+                ++j;
+            }
+        };
+        std::vector<std::thread> th;
+        for (size_t p = 1; p < parts; ++p) {
+            try { th.emplace_back(scatter, p); } catch (...) { scatter(p); }
+        }
+        scatter(0);
+        for (auto &t : th) t.join();
+        return (int)PT_OK;
+    });
+    // every copy of every point, own and ghost, takes the stored normals
+    if (rc == PT_OK && store)
+        rc = each_slab([&](int r) {
+            const Slab &sl = S->slabs[r];
+            if (sl.ids.empty()) return (int)PT_OK;                         // a slab without records
+            std::vector<float> values(3 * sl.ids.size());
+            for (size_t l = 0; l < sl.ids.size(); ++l)
+                memcpy(&values[3 * l], &S->stored[3 * (size_t)sl.ids[l]], sizeof(float) * 3);
+            return pt::normals_store(sl.index, values.data());
+        });
+    if (rc != PT_OK) return rc;
+    if (stats) {
+        stats->knn_ms = std::chrono::duration<float, std::milli>(std::chrono::steady_clock::now() - t0).count();
+        stats->pca_ms = 0.0f;
+        stats->estimated = 0;
+        for (int r = 0; r < R; ++r) {
+            stats->estimated += est[r];
+            stats->pca_ms += pca[r];
+        }
+    }
+    return PT_OK;
+}
+
 }  // namespace
 
 extern "C" {
@@ -540,6 +675,20 @@ int pt_sharded_bake(pt_sharded *S, const void *vertices, size_t n_vertices, cons
     if (pt_device_count() == 0) return PT_ERR_NO_DEVICE;
     try {
         return sharded_bake(S, vertices, n_vertices, faces, n_faces, k, radius, resolution, pad, o, height, stats);
+    } catch (...) { return PT_ERR_OUT_OF_MEMORY; }
+}
+
+int pt_sharded_estimate_normals(pt_sharded *S, int k, double radius, const double *viewpoint, int store,
+                                float *normal_out, float *variation_out, pt_normals_stats *stats)
+{
+    if (!S) return PT_ERR_INVALID_ARG;
+    const int rc = pt::normals_check_args(k, viewpoint, store != 0, normal_out || variation_out);
+    if (rc != PT_OK) return rc;
+    if (pt_device_count() == 0) return PT_ERR_NO_DEVICE;
+    if (stats) *stats = pt_normals_stats{0, 0.0f, 0.0f};
+    if (S->n == 0) return PT_OK;
+    try {
+        return sharded_normals(S, k, radius, viewpoint, store != 0, normal_out, variation_out, stats);
     } catch (...) { return PT_ERR_OUT_OF_MEMORY; }
 }
 

@@ -514,6 +514,27 @@ int pt_sharded_bake(pt_sharded *sharded, const void *vertices, size_t n_vertices
                     const int32_t *faces, size_t n_faces, int k, double radius,
                     int resolution, int pad, const pt_bake_outputs *out /* may be NULL */,
                     pt_bake_height *height /* may be NULL, not both */, pt_bake_stats *stats);
+/* pt_index_estimate_normals on the sharded cloud (DESIGN.md section 8, "Sharded normal estimation"):
+ * same arguments, argument rules and error codes (a NULL handle: PT_ERR_INVALID_ARG), and
+ * normal_out (n x 3) and variation_out (n), in the order of the caller's `points`, are
+ * byte-identical to pt_index_estimate_normals on one pt_index built from the same cloud (NaN bits
+ * included), as is stats->estimated, for any slab count, device list, halo and coordinate mode.
+ * Every slab estimates the points it owns on its own device, from its own records, with the
+ * ghost-zone check on those rows; a ghost zone found too narrow widens the halo and rebuilds the
+ * slabs as pt_sharded_transfer does (counted in `rebuilds`).  store != 0: every estimated normal
+ * replaces the point's normal in every slab that holds the point (its owner and the ghost zones),
+ * so later pt_sharded_transfer / pt_sharded_bake calls blend it, and the handle keeps the stored
+ * normals (12 bytes per point, from the first store on) so that rebuilt slabs hold them too; points
+ * without an estimate keep their input normal.  Nothing is written or stored before every slab has
+ * passed its check.  Stats:
+ *   estimated  points with an estimate
+ *   knn_ms     host wall time of the slab stage: the slabs' self-queries, ghost checks and PCA
+ *              kernels, rebuilds included, the copies to the host, the scatter into point order
+ *              and the store, ending in a synchronise
+ *   pca_ms     device time of the PCA kernels, summed over the slabs, in the final attempt */
+int pt_sharded_estimate_normals(pt_sharded *sharded, int k, double radius,
+                                const double *viewpoint /* 3 or NULL */, int store, float *normal_out,
+                                float *variation_out, pt_normals_stats *stats);
 
 /* pt_texture_render for neighbour lists that were computed elsewhere (e.g. pt_sharded_knn): the
  * cloud's positions and colours are uploaded to `device` in original order, idx[n_vertices * k]
