@@ -11,8 +11,8 @@
 //             pipeline chunk -- and the results land in the caller's arrays in sample order.
 //             A step is final iff no sample's k-th-neighbour ball can leave its slab's ghost
 //             zone towards another slab (exactness argument: DESIGN.md section 6).  If some
-//             slab reports needs_exchange the halo is widened (x4, at least the bounding-box estimate), the slabs are rebuilt and the
-//             call is repeated, so the result is always exact; `rebuilds` counts that.
+//             slab reports needs_exchange the halo is widened (widen_and_rebuild), the slabs are
+//             rebuilt and the call is repeated, so the result is always exact; `rebuilds` counts that.
 //   bake    : the per-texel bake of pt_texture_bake_height on the sharded cloud (DESIGN.md section
 //             8, "Sharded bake"): raster, frames, composition and padding on slab 0's device (the
 //             home device, pt_bake.cuh pieces); the samples are partitioned by slab there, each
@@ -113,6 +113,14 @@ int build_slabs(pt_sharded *S)
             s.box[3 + a] = std::max(s.box[3 + a], P[i].ver[a]);
         }
     }
+    // A slab below the last that owns no point gets an empty x-range, so every path (the host
+    // routing of sharded_query, bake_partition, the own rows of the normals) sends what falls in
+    // its range to the next slab that owns points.  Its index has no records, and the ghost check
+    // of an empty box would flag every attempt.  No point changes owner (no point lies in that
+    // range), and once applied the rule changes nothing on later builds.  Every cut is some point's
+    // x, so the last slab owns a point unless the cloud is empty.
+    for (int r = 0; r + 1 < R; ++r)
+        if (S->slabs[r].n_own == 0) S->cuts[r + 1] = S->cuts[r];
     S->boxes.assign((size_t)R * 6, 0.0);
     for (int r = 0; r < R; ++r) memcpy(&S->boxes[(size_t)r * 6], S->slabs[r].box, sizeof(double) * 6);
     std::vector<int> status(R, PT_OK);
@@ -166,6 +174,32 @@ int build_slabs(pt_sharded *S)
     return PT_OK;
 }
 
+constexpr int ATTEMPTS = 8;           // answers per call: the first, then one per widening
+
+// A slab whose index holds the whole cloud answers every sample exactly: its ghost check is moot.
+bool holds_cloud(const pt_sharded *S, const Slab &s) { return s.n_own + s.n_ghost == S->n; }
+
+// After attempt `attempt` found some ghost zone too narrow: widen the halo and rebuild the slabs.
+// x4, at least the bounding-box estimate, at most the diagonal of the cloud's bounding box (the
+// union of the own boxes), and that diagonal for the last attempt.  At the diagonal every slab that
+// owns a point holds the whole cloud (holds_cloud) and the others receive nothing (build_slabs), so
+// the last attempt is final whatever the cloud's units and however far the samples lie.
+int widen_and_rebuild(pt_sharded *S, int attempt)
+{
+    double lo[3] = {INFINITY, INFINITY, INFINITY}, hi[3] = {-INFINITY, -INFINITY, -INFINITY};
+    for (const Slab &s : S->slabs)
+        for (int a = 0; a < 3; ++a) { lo[a] = std::min(lo[a], s.box[a]); hi[a] = std::max(hi[a], s.box[3 + a]); }
+    double diag2 = 0.0;
+    for (int a = 0; a < 3; ++a) {
+        const double e = std::max(hi[a] - lo[a], 0.0);
+        diag2 += e * e;
+    }
+    const double diag = std::sqrt(diag2);
+    S->halo = attempt + 2 >= ATTEMPTS ? diag : std::min(std::max(4.0 * S->halo, S->halo_auto), diag);
+    ++S->rebuilds;
+    return build_slabs(S);
+}
+
 int sharded_query(pt_sharded *S, const void *queries, size_t m, int k, double radius, int32_t *idx_out,
                   double *d2_out, uint8_t *rgba_out, float *normal_out)
 {
@@ -181,7 +215,7 @@ int sharded_query(pt_sharded *S, const void *queries, size_t m, int k, double ra
         const int r = (int)(std::upper_bound(S->cuts.begin() + 1, S->cuts.end() - 1, x) - (S->cuts.begin() + 1));
         mine[r].push_back((uint32_t)i);
     }
-    for (int attempt = 0; attempt < 8; ++attempt) {
+    for (int attempt = 0; attempt < ATTEMPTS; ++attempt) {
         std::vector<int> status(R, PT_OK), needs(R, 0);
         std::vector<std::thread> th;
         auto work = [&](int r) {
@@ -209,8 +243,8 @@ int sharded_query(pt_sharded *S, const void *queries, size_t m, int k, double ra
                                           nullptr, &need);
                 }
                 status[r] = rc;
-                needs[r] = need;
-                if (rc != PT_OK || need) return;
+                needs[r] = holds_cloud(S, S->slabs[r]) ? 0 : need;
+                if (rc != PT_OK || needs[r]) return;
                 for (size_t j = 0; j < mr; ++j) {          // results back into sample order
                     const size_t d = sel[j];
                     if (idx_out) memcpy(idx_out + d * k, idx.data() + j * k, sizeof(int32_t) * k);
@@ -230,13 +264,12 @@ int sharded_query(pt_sharded *S, const void *queries, size_t m, int k, double ra
             again |= needs[r] != 0;
         }
         if (!again) return PT_OK;
+        if (attempt + 1 == ATTEMPTS) break;
         // some k-th-neighbour ball may leave a ghost zone: widen it and answer the call again
-        S->halo = std::max(4.0 * S->halo, S->halo_auto);
-        ++S->rebuilds;
-        const int rc = build_slabs(S);
+        const int rc = widen_and_rebuild(S, attempt);
         if (rc != PT_OK) return rc;
     }
-    return PT_ERR_UNSUPPORTED;
+    return PT_ERR_UNSUPPORTED;        // a guard: the last attempt is final for finite input
 }
 
 // Sample rows in slab order on the home device (struct of arrays, so a slab's rows are one range
@@ -326,8 +359,7 @@ int slab_bake(pt_sharded *S, int r, int home, const pt::BakeJob &J, const BakeRo
         if (fail(cudaMemcpyAsync(boxes, S->boxes.data(), sizeof(double) * 6 * R, cudaMemcpyHostToDevice, s)) ||
             fail(cudaMemsetAsync(flag, 0, sizeof(uint32_t), s)))
             break;
-        // a slab whose index holds the whole cloud answers every sample exactly: no check
-        const bool whole = sl.n_own + sl.n_ghost == S->n;
+        const bool whole = holds_cloud(S, sl);
         const BakeGhost ghost{boxes, (int)R, r, S->halo, flag};
         const BakeMesh M = copy ? BakeMesh{d.mesh, BAKE_ROW, (uint32_t)nv, d.faces, (uint32_t)nf, J.res} : J.M;
         const double *frames = copy ? d.mesh + BAKE_ROW * nv : J.d_frames;
@@ -390,7 +422,7 @@ int sharded_answer(pt_sharded *S, int home, pt::BakeJob &J, int k, double radius
                                  rows.xyz, rows.texel, rows.face, starts.data(), s)) != PT_OK)
             break;
         bool done = false;
-        for (int attempt = 0; attempt < 8 && !done; ++attempt) {
+        for (int attempt = 0; attempt < ATTEMPTS && !done; ++attempt) {
             std::vector<int> status(R, PT_OK), needs(R, 0);
             std::vector<std::thread> th;
             auto work = [&](int r) {
@@ -411,13 +443,12 @@ int sharded_answer(pt_sharded *S, int home, pt::BakeJob &J, int k, double radius
             }
             if (rc != PT_OK) break;
             if (!again) { done = true; break; }
+            if (attempt + 1 == ATTEMPTS) break;
             // some k-th-neighbour ball may leave a ghost zone: widen it and answer the rows again
-            S->halo = std::max(4.0 * S->halo, S->halo_auto);
-            ++S->rebuilds;
-            if ((rc = build_slabs(S)) != PT_OK) break;
+            if ((rc = widen_and_rebuild(S, attempt)) != PT_OK) break;
         }
         if (rc != PT_OK) break;
-        if (!done) { rc = PT_ERR_UNSUPPORTED; break; }
+        if (!done) { rc = PT_ERR_UNSUPPORTED; break; }          // a guard, as in sharded_query
         if (fail(cudaSetDevice(home))) break;
         const uint32_t routed = (uint32_t)starts[R];
         if ((rc = launch_scatter_rows(rows.rgba, sel, routed, 4, J.d_rgba, s)) != PT_OK ||
@@ -487,7 +518,7 @@ int sharded_normals(pt_sharded *S, int k, double radius, const double *viewpoint
     // every slab estimates its own points; nothing reaches the caller or the slabs before all pass
     int rc = PT_OK;
     bool done = false;
-    for (int attempt = 0; attempt < 8 && !done; ++attempt) {
+    for (int attempt = 0; attempt < ATTEMPTS && !done; ++attempt) {
         std::vector<int> needs(R, 0);
         rc = each_slab([&](int r) {
             const Slab &sl = S->slabs[r];
@@ -497,21 +528,17 @@ int sharded_normals(pt_sharded *S, int k, double radius, const double *viewpoint
             if (sl.n_own == 0) return (int)PT_OK;
             nrm[r].resize(3 * sl.n_own);
             var[r].resize(sl.n_own);
-            // a slab whose index holds the whole cloud answers every point exactly: no check
-            const bool whole = sl.n_own + sl.n_ghost == S->n;
-            const pt::NormalsSlab job{S->cuts.data() + 1, R, r, sl.n_own, S->boxes.data(), S->halo, !whole};
+            const pt::NormalsSlab job{S->cuts.data() + 1, R, r, sl.n_own, S->boxes.data(), S->halo, !holds_cloud(S, sl)};
             return pt::normals_slab(sl.index, k, radius, viewpoint, job, nrm[r].data(), var[r].data(), &est[r], &pca[r],
                                     &needs[r]);
         });
         if (rc != PT_OK) return rc;
         done = std::none_of(needs.begin(), needs.end(), [](int v) { return v != 0; });
-        if (done) break;
+        if (done || attempt + 1 == ATTEMPTS) break;
         // some k-th-neighbour ball may leave a ghost zone: widen it and estimate again
-        S->halo = std::max(4.0 * S->halo, S->halo_auto);
-        ++S->rebuilds;
-        if ((rc = build_slabs(S)) != PT_OK) return rc;
+        if ((rc = widen_and_rebuild(S, attempt)) != PT_OK) return rc;
     }
-    if (!done) return PT_ERR_UNSUPPORTED;
+    if (!done) return PT_ERR_UNSUPPORTED;                     // a guard, as in sharded_query
     // the own entries into the caller's point order (slabs own disjoint points)
     if (store && S->stored.empty()) S->stored.assign(3 * S->n, NAN);
     // each slab's own results come in ascending local id: the i-th goes to the global id of the
@@ -609,21 +636,24 @@ int pt_sharded_build(const void *points, size_t n, const pt_sharded_opts *opts, 
         std::sort(S->cuts.begin() + 1, S->cuts.end() - 1);
     }
     // ghost-zone width: given, or a multiple of the expected k-th-neighbour distance estimated
-    // from the bounding box (surface and volume estimate, the larger one); a call that finds it
-    // too small widens it (sharded_query)
+    // from the bounding box (line, surface and volume estimate, the largest one); a call that finds
+    // it too small widens it (widen_and_rebuild)
     S->halo = opts->halo;
     {
         double lo[3] = {INFINITY, INFINITY, INFINITY}, hi[3] = {-INFINITY, -INFINITY, -INFINITY};
         for (size_t i = 0; i < n; i += (n > 1000000 ? n / 1000000 : 1))
             for (int a = 0; a < 3; ++a) { lo[a] = std::min(lo[a], S->points[i].ver[a]); hi[a] = std::max(hi[a], S->points[i].ver[a]); }
-        double e[3] = {hi[0] - lo[0], hi[1] - lo[1], hi[2] - lo[2]};
+        double e[3] = {std::max(hi[0] - lo[0], 0.0), std::max(hi[1] - lo[1], 0.0), std::max(hi[2] - lo[2], 0.0)};
         std::sort(e, e + 3);
         const double kk = opts->k_hint > 0 ? opts->k_hint : 20;
         const double nn = n ? (double)n : 1.0;
-        const double r_surface = std::sqrt(kk * std::max(e[1] * e[2], 0.0) / (M_PI * nn));
-        const double r_volume = std::cbrt(3.0 * kk * std::max(e[0] * e[1] * e[2], 0.0) / (4.0 * M_PI * nn));
-        S->halo_auto = 4.0 * std::max(r_surface, r_volume);
-        if (!(S->halo_auto > 0.0) || !std::isfinite(S->halo_auto)) S->halo_auto = 1e-3;
+        const double r_surface = std::sqrt(kk * e[1] * e[2] / (M_PI * nn));
+        const double r_volume = std::cbrt(3.0 * kk * e[0] * e[1] * e[2] / (4.0 * M_PI * nn));
+        const double r_line = kk * e[2] / nn;
+        // no wider than the box's diagonal, beyond which a ghost zone takes no more points
+        const double diag = std::sqrt(e[0] * e[0] + e[1] * e[1] + e[2] * e[2]);
+        S->halo_auto = std::min(4.0 * std::max(std::max(r_surface, r_volume), r_line), diag);
+        if (!std::isfinite(S->halo_auto)) S->halo_auto = 0.0;
         if (!(S->halo > 0.0)) S->halo = S->halo_auto;
     }
     const int rc = build_slabs(S);

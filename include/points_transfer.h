@@ -471,13 +471,15 @@ int pt_transfer_slab(pt_index *index, const void *queries, int queries_are_xyz, 
  * `halo`, samples routed to the slab whose x-range holds them, one host thread per slab.  Same
  * contract as pt_knn / pt_transfer (blocking, query order, ascending (d2, index), ids are indices
  * into the caller's `points`); results are exact for any geometry: a call that finds a ghost
- * zone too narrow widens `halo`, rebuilds the slabs and answers again (counted in `rebuilds`).
+ * zone too narrow widens `halo`, rebuilds the slabs and answers again (counted in `rebuilds`),
+ * at most 7 times per call and never past the diagonal of the cloud's bounding box.
  * `points` must stay valid until pt_sharded_free.  n < 2^31 points in total. */
 typedef struct pt_sharded pt_sharded;
 typedef struct pt_sharded_opts {
     int        n_devices;  /* number of slabs, 1..64 */
     const int *devices;    /* CUDA ordinal of every slab (may repeat); NULL => slab r on r mod device count */
-    double     halo;       /* ghost-zone width; <= 0: 4x the expected k_hint-th neighbour distance */
+    double     halo;       /* ghost-zone width; <= 0: 4x the expected k_hint-th neighbour distance,
+                              at most the bounding-box diagonal */
     int        k_hint;     /* k the halo estimate is made for (default 20) */
     int        coord_mode; /* PT_COORD_* */
     int        reserved[8];
