@@ -56,6 +56,8 @@ static std::atomic<int> g_chain_pdl{1};   // hand-over kernels launched as progr
 int opt_chain_pdl() { return g_chain_pdl.load(); }
 static std::atomic<int> g_grid_claim{1};   // span kernel: warps claim their next pair with an atomic when each has > 2 pairs (0: static stride)
 int opt_grid_claim() { return g_grid_claim.load(); }
+static std::atomic<int> g_grid_block{1};   // span kernel: stage the block run of the sample's cell where the index has them (0: never)
+int opt_grid_block() { return g_grid_block.load(); }
 static std::atomic<int> g_grid_min_occ10{40};    // finest table: finest level with >= this / 10 points per occupied cell
 static std::atomic<int> g_grid_lookup_cost{8};   // grid_plan: cost of one bucket look-up, in candidates
 static std::atomic<int> g_grid_admit100{100};    // grid_plan: a block is tried first when rc cells >= this / 100 expected k-th distances
@@ -66,6 +68,8 @@ static std::atomic<int> g_grid_pair_used{0};   // introspection: did the last gr
 void note_grid_pair_used(int used) { g_grid_pair_used.store(used); }
 static std::atomic<int> g_grid_span_used{0};   // introspection: did the last grid launch run knn_grid_span_kernel
 void note_grid_span_used(int used) { g_grid_span_used.store(used); }
+static std::atomic<int> g_grid_block_used{0};   // introspection: did the last grid launch run knn_grid_block_kernel
+void note_grid_block_used(int used) { g_grid_block_used.store(used); }
 int opt_sort_bits() { return g_sort_bits.load(); }
 size_t opt_pool_keep_bytes()
 {
@@ -114,6 +118,7 @@ int set_option(const char *name, int value)
     if (!strcmp(name, "grid_span")) { g_grid_span.store(value ? 1 : 0); return PT_OK; }
     if (!strcmp(name, "chain_pdl")) { g_chain_pdl.store(value ? 1 : 0); return PT_OK; }
     if (!strcmp(name, "grid_claim")) { g_grid_claim.store(value ? 1 : 0); return PT_OK; }
+    if (!strcmp(name, "grid_block")) { g_grid_block.store(value ? 1 : 0); return PT_OK; }
     if (!strcmp(name, "sort_bits")) { g_sort_bits.store(value); return PT_OK; }
     if (!strcmp(name, "pool_keep_mb")) { g_pool_keep_mb.store(value < 0 ? -1 : value); return PT_OK; }
     if (!strcmp(name, "pool_guard")) { g_pool_guard.store(value ? 1 : 0); return PT_OK; }
@@ -141,6 +146,8 @@ int get_option(const char *name, int *value)
     if (!strcmp(name, "grid_span_used")) { *value = g_grid_span_used.load(); return PT_OK; }
     if (!strcmp(name, "chain_pdl")) { *value = g_chain_pdl.load(); return PT_OK; }
     if (!strcmp(name, "grid_claim")) { *value = g_grid_claim.load(); return PT_OK; }
+    if (!strcmp(name, "grid_block")) { *value = g_grid_block.load(); return PT_OK; }
+    if (!strcmp(name, "grid_block_used")) { *value = g_grid_block_used.load(); return PT_OK; }
     if (!strcmp(name, "sort_bits")) { *value = g_sort_bits.load(); return PT_OK; }
     if (!strcmp(name, "pool_keep_mb")) { *value = g_pool_keep_mb.load(); return PT_OK; }
     if (!strcmp(name, "pool_guard")) { *value = g_pool_guard.load(); return PT_OK; }
@@ -205,6 +212,7 @@ static void destroy_index(pt_index *ix)
     pool_free(ix->pts, ix->stream);
     pool_free(ix->boxes, ix->stream);
     pool_free(ix->grid_mem, ix->stream);
+    pool_free(ix->blk_mem, ix->stream);
     pool_free(ix->attrs_curve, ix->stream);
     pool_free(ix->attrs, ix->stream);         // (attributes and ids too: cudaMalloc / cudaFree of 0.8 GB cost milliseconds)
     pool_free(ix->ids, ix->stream);

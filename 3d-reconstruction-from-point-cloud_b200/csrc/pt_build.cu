@@ -682,6 +682,8 @@ static int build_impl(pt_index *ix, In in, uint32_t n)
     // cell tables over the curve order (the kd refinement reorders inside blocks: no cell runs)
     if (kp.order != 2) PT_TRY(build_grid(ix, keys, first_bit, kp.lo, kp.inv_cell, ext));
     lap("grid tables");
+    if (sizeof(Out) == 16) PT_TRY(build_blocks(ix));
+    lap("block runs");
 
     // box pyramid
     uint64_t total = 0;
@@ -725,7 +727,7 @@ static int build_impl(pt_index *ix, In in, uint32_t n)
     arena_guard.p = nullptr;
     cudaStreamSynchronize(s);
     pool_trim(ix->device, opt_pool_keep_bytes());   // "pool_keep_mb" of it stays mapped for the next build
-    ix->device_bytes = sizeof(Out) * n_pad + sizeof(Box) * total + ix->grid_bytes +
+    ix->device_bytes = sizeof(Out) * n_pad + sizeof(Box) * total + ix->grid_bytes + ix->blk_bytes +
                        (ix->attrs ? sizeof(pt_attr) * (size_t)n : 0) +
                        (ix->attrs_curve ? sizeof(pt_attr) * (size_t)n : 0) +
                        (ix->ids ? sizeof(int32_t) * (size_t)n : 0);

@@ -79,6 +79,17 @@ struct __align__(16) GridBucket {
 };
 static_assert(sizeof(GridBucket) == 32, "one sector per bucket");
 
+// Slot of the block-run table (pt_knn_span.cuh, build_blocks): one per occupied cell of the level
+// the runs are built for, found by hashing the cell's lattice coordinates; four slots = one
+// aligned 64-byte group.
+struct __align__(16) BlockSlot {
+    unsigned long long key;    // cell coordinates x | y << 21 | z << 42; ~0 = empty slot
+    uint32_t           off;    // first 16-byte unit of the run
+    uint32_t           meta;   // records | heads << 16; BLOCK_MISS: the block cannot be staged
+};
+static_assert(sizeof(BlockSlot) == 16, "four slots per 64-byte group");
+constexpr uint32_t BLOCK_MISS = 0x80000000u;
+
 constexpr int GRID_MAX_TABLES = 4;
 constexpr int GRID_MAX_ATTEMPTS = 4;
 struct GridTable {
@@ -99,6 +110,11 @@ struct GridParams {
     int       n_attempts;
     unsigned char att_tab[GRID_MAX_ATTEMPTS], att_rc[GRID_MAX_ATTEMPTS];
     float     expect_cand;     // candidates the first attempt is expected to stage per sample (host estimate)
+    // block runs of the cells of level blk_level (null: none)
+    const BlockSlot *blk;
+    const uint4     *blk_runs;
+    uint32_t         blk_cap;  // slots (a multiple of 4; linear probing in 4-slot groups, load <= 1/3)
+    int              blk_level;
 };
 
 struct QueryParams {

@@ -22,6 +22,8 @@ struct pt_index {
     double       bb_lo[3]{}, bb_hi[3]{};
     pt::GridBucket *grid_mem = nullptr;   // all cell tables (pt_grid.cu), pooled allocation
     size_t       grid_bytes = 0;
+    void        *blk_mem = nullptr;       // block-run table and runs (build_blocks), pooled allocation
+    size_t       blk_bytes = 0;
     pt::GridParams grid{};                // tables of this index (n_tables == 0: none)
     uint64_t     level_cells[22]{};       // occupied cells per lattice level (0: not counted)
     uint32_t    *fallback_word = nullptr; // device: samples the last launch handed to the warp kernel
@@ -137,6 +139,8 @@ void pool_trim(int device, size_t keep_bytes);
 int build_grid(pt_index *ix, const unsigned long long *keys, int low_shift, const double lo[3],
                double inv_cell21, double extent);
 int grid_plan(const pt_index *ix, int k, double r2, GridParams &gp);
+// The block runs of ix's cell tables (pt_knn.cu), when they fit the memory budget; synchronises.
+int build_blocks(pt_index *ix);
 int launch_merge(const pt_cand *lists, int n_lists, uint32_t m, int k, int32_t *idx_out,
                  double *d2_out, uint8_t *rgba_out, float *normal_out, pt_cand *cand_out,
                  cudaStream_t s);
@@ -178,11 +182,13 @@ int  opt_grid_span();
 int  opt_chain_pdl();
 int  opt_sharded_copy();
 int  opt_grid_claim();
+int  opt_grid_block();
 int  opt_grid_min_occ10();
 int  opt_grid_admit100();
 int  opt_grid_lookup_cost();
 void note_grid_pair_used(int used);
 void note_grid_span_used(int used);
+void note_grid_block_used(int used);
 int  opt_sort_bits();
 size_t opt_pool_keep_bytes();
 int  opt_pool_guard();

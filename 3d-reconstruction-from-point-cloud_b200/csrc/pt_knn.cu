@@ -14,6 +14,7 @@
 //     sample but the shortest latency and no per-sample state limits: it answers small launches
 //     and re-runs the samples the other two hand over (exact fallback).
 #include <type_traits>
+#include <cub/device/device_scan.cuh>
 #include "pt_index.cuh"
 
 namespace pt {
@@ -393,6 +394,76 @@ __global__ void __launch_bounds__(256) empty_result_kernel(const QueryParams P)
 #include "pt_knn_span.cuh"
 namespace pt {
 
+// Block runs (pt_knn_span.cuh) for the level a k = 16 search plans its first attempt on, when that
+// attempt is one the span kernel runs (a 3^3 block expected to fit a half-warp).  Count pass,
+// exclusive scan, fill pass.  The runs store each point once per block that holds it (about nine
+// times the cloud's records on a scanned surface), so they are built only when table and runs fit
+// a quarter of the device memory free at this point -- the rest stays for the queries'
+// workspaces, the normals' lists and a second index -- and their offsets fit 32 bits of 16-byte
+// units.  Otherwise the index has none and every query stages spans as before.
+constexpr size_t BLOCK_FREE_SHARE = 4;    // the runs may take 1 / this of the free device memory
+
+int build_blocks(pt_index *ix)
+{
+    ix->blk_mem = nullptr;
+    ix->blk_bytes = 0;
+    GridParams gp;
+    if (ix->coord_f64 || grid_plan(ix, 16, INFINITY, gp) == 0 || gp.att_rc[0] != 1 ||
+        gp.expect_cand > 0.74f * (float)PAIR_CAP)
+        return PT_OK;
+    cudaStream_t s = ix->stream;
+    const GridTable T = gp.tab[gp.att_tab[0]];
+    const uint64_t cells = ix->level_cells[T.level];
+    const uint64_t tab_cap = (3 * cells + 8) & ~3ull;           // load <= 1/3, whole 4-slot groups
+    if (tab_cap > 0xfffffff0ull) return PT_OK;
+    const PointF *pts = reinterpret_cast<const PointF *>(ix->pts);
+    const unsigned blocks = (unsigned)(((uint64_t)T.cap * 16 + 255) / 256);
+    // units[b]: 16-byte units of bucket b's runs; off = their exclusive sum, off[cap] = all units
+    unsigned long long *units = nullptr;
+    PT_TRY(pool_alloc((void **)&units, sizeof(unsigned long long) * 2 * ((size_t)T.cap + 1), s));
+    unsigned long long *off = units + T.cap + 1;
+    struct Free {
+        void *p; cudaStream_t s;
+        ~Free() { pool_free(p, s); }
+    } units_guard{units, s};
+    PT_CUDA(cudaMemsetAsync(units + T.cap, 0, sizeof(unsigned long long), s));
+    block_run_kernel<true><<<blocks, 256, 0, s>>>(T, units, nullptr, pts, nullptr, nullptr, 0);
+    count_launch();
+    PT_CUDA(cudaGetLastError());
+    size_t tmp_bytes = 0;
+    PT_CUDA(cub::DeviceScan::ExclusiveSum(nullptr, tmp_bytes, units, off, (int)T.cap + 1, s));
+    void *tmp = nullptr;
+    PT_TRY(pool_alloc(&tmp, tmp_bytes, s));
+    const cudaError_t e = cub::DeviceScan::ExclusiveSum(tmp, tmp_bytes, units, off, (int)T.cap + 1, s);
+    pool_free(tmp, s);
+    PT_CUDA(e);
+    unsigned long long total_units = 0;
+    PT_CUDA(cudaMemcpyAsync(&total_units, off + T.cap, sizeof total_units, cudaMemcpyDeviceToHost, s));
+    PT_CUDA(cudaStreamSynchronize(s));
+    const size_t tab_bytes = sizeof(BlockSlot) * tab_cap, bytes = tab_bytes + sizeof(uint4) * total_units;
+    size_t free_b = 0, total_b = 0;
+    PT_CUDA(cudaMemGetInfo(&free_b, &total_b));
+    if (verbose())
+        fprintf(stderr, "[points_transfer] block runs level %d: %llu cells, %llu units, %.3f GB (free %.3f GB)\n",
+                T.level, (unsigned long long)cells, total_units, (double)bytes * 1e-9, (double)free_b * 1e-9);
+    if (total_units > 0xffffffffull || bytes > free_b / BLOCK_FREE_SHARE) return PT_OK;
+    void *mem = nullptr;
+    PT_TRY(pool_alloc(&mem, bytes, s));
+    ix->blk_mem = mem;
+    ix->blk_bytes = bytes;
+    BlockSlot *tab = reinterpret_cast<BlockSlot *>(mem);
+    uint4 *runs = reinterpret_cast<uint4 *>(reinterpret_cast<char *>(mem) + tab_bytes);
+    PT_CUDA(cudaMemsetAsync(tab, 0xff, tab_bytes, s));
+    block_run_kernel<false><<<blocks, 256, 0, s>>>(T, nullptr, off, pts, runs, tab, (uint32_t)tab_cap);
+    count_launch();
+    PT_CUDA(cudaGetLastError());
+    ix->grid.blk = tab;
+    ix->grid.blk_runs = runs;
+    ix->grid.blk_cap = (uint32_t)tab_cap;
+    ix->grid.blk_level = T.level;
+    return PT_OK;
+}
+
 // Launch plan.  Every launch gets its OWN hand-over workspace (two sample lists with their
 // counters) from the library's stream-ordered pool, so launches of one index that are in flight
 // on different streams never share state:
@@ -421,10 +492,12 @@ static int launch_chain(pt_index *ix, const QueryParams &qp, int variant, cudaSt
         // two samples per warp with one look-up per parent cell and one copy per span where the
         // pair kernel would run (pt_knn_span.cuh); otherwise launch_grid picks
         const bool span = grid_span_applies<PT>(qp);
+        const bool block = span && grid_block_applies(qp);
         note_grid_span_used(span ? 1 : 0);
+        note_grid_block_used(block ? 1 : 0);
         if (span) {
             note_grid_pair_used(0);
-            rc = launch_grid_span(qp, ix->sm_count, count1, list1, ws + 1, s);
+            rc = launch_grid_span(qp, block, ix->sm_count, count1, list1, ws + 1, s);
         } else {
             rc = launch_grid<PT>(qp, ix->sm_count, count1, list1, s);
         }

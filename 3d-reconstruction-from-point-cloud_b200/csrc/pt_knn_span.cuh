@@ -75,6 +75,190 @@ __device__ __forceinline__ void for_each_span(uint32_t inr, uint32_t brk, const 
     }
 }
 
+// Look-ups of the 3^3 block around cell c: sub-lane j < 8 of each half takes parent j of the
+// block's 2 x 2 x 2 parents.  Along an axis the block's cells c - 1 .. c + 1 lie in parents
+// ((c + 1) >> 1) - 1 and (c + 1) >> 1; child bit b of parent q is cell 2q + b, inside the block iff
+// it is one of c - 1 .. c + 1 and below ncell (the unsigned compare also rejects "negative"
+// cells).  Gives the lane's parent start, the curve ranks of its children inside the block (inr)
+// and of its occupied children outside it (brk), its cum[] fields, and dense when the parent has
+// too many points for them.
+__device__ __forceinline__ void span_parent(const GridTable &T, const uint32_t c[3], uint32_t ncell, unsigned sl,
+                                            bool look, uint32_t &pstart, uint32_t &inr, uint32_t &brk, uint4 &cum,
+                                            bool &dense)
+{
+    pstart = 0;
+    inr = 0;
+    brk = 0;
+    cum = make_uint4(0u, 0u, 0u, 0u);
+    dense = false;
+    if (look && sl < 8u) {
+        uint32_t pq[3], oct = 0xffu;
+#pragma unroll
+        for (int ax = 0; ax < 3; ++ax) {
+            pq[ax] = ((c[ax] + 1u) >> 1) - 1u + ((sl >> ax) & 1u);
+            const uint32_t x0 = 2u * pq[ax], x1 = x0 + 1u;
+            const bool b0 = x0 - c[ax] + 1u < 3u && x0 < ncell, b1 = x1 - c[ax] + 1u < 3u && x1 < ncell;
+            // octants o with bit `ax` of o = 0 (b0) or 1 (b1)
+            const uint32_t m1 = ax == 0 ? 0xaau : (ax == 1 ? 0xccu : 0xf0u);
+            oct &= (b0 ? (~m1 & 0xffu) : 0u) | (b1 ? m1 : 0u);
+        }
+        uint32_t perm = 0;
+#ifdef PT_STATS
+        if (oct) atomicAdd(&g_stats[16], 1ull);
+#endif
+        if (oct && grid_parent_lookup(T.buckets, T.cap, pq[0], pq[1], pq[2], pstart, perm, cum)) {
+            const uint32_t occ = perm >> 24, om = oct & occ;
+            if (om && (cum.x & 0xffffu) == 0xffffu) dense = true;
+            else if (om) {
+#pragma unroll
+                for (int o = 0; o < 8; ++o) {
+                    const uint32_t rb = 1u << ((perm >> (3 * o)) & 7u);
+                    if ((om >> o) & 1u) inr |= rb;
+                    else if ((occ >> o) & 1u) brk |= rb;
+                }
+            }
+        }
+    }
+}
+
+// Spans << 24 | points of this lane's parent (mine_v), its inclusive sum over the half's parents
+// (incl); returns the half's sum.  Every lane of the warp calls it.
+__device__ __forceinline__ uint32_t span_scan(uint32_t inr, uint32_t brk, const uint4 &cum, unsigned sl,
+                                              unsigned hbase, uint32_t &mine_v, uint32_t &incl)
+{
+    mine_v = 0;
+    for_each_span(inr, brk, cum, [&](uint32_t, uint32_t n) { mine_v += (1u << 24) + n; });
+    incl = mine_v;
+#pragma unroll
+    for (int o = 1; o < 8; o <<= 1) {
+        const uint32_t y = __shfl_up_sync(0xffffffffu, incl, o);
+        if (sl >= (unsigned)o) incl += y;
+    }
+    return __shfl_sync(0xffffffffu, incl, (int)(hbase | 7u));
+}
+
+// ---- block runs (pt_index::blk_mem, built by build_blocks) ---------------------------------------
+// For every occupied cell c of one table level, one run holds the records the span kernel stages
+// for a sample in c, in its slot order, followed by its span heads (padded to an even count).
+// The table slot gives the run's place and size, so one probe and two bulk copies stage a sample.
+__device__ __forceinline__ unsigned long long block_key(const uint32_t c[3])
+{
+    return (unsigned long long)c[0] | ((unsigned long long)c[1] << 21) | ((unsigned long long)c[2] << 42);
+}
+__device__ __forceinline__ uint32_t block_heads_pad(uint32_t nspan) { return (nspan + 1u) & ~1u; }
+
+// The slot of cell `key`: its meta (BLOCK_MISS when the cell is empty) and, for a stageable
+// run, the run's offset in 16-byte units.  Four slots are probed at a time (one aligned 64-byte
+// group = one DRAM fetch); a group is filled in slot order, so an empty slot ends the search.
+__device__ __forceinline__ uint32_t block_lookup(const BlockSlot *tab, uint32_t cap, unsigned long long key,
+                                                 uint32_t &off)
+{
+    const uint32_t ngroups = cap >> 2;
+    uint32_t g = __umulhi(grid_hash_q(key), ngroups);
+    for (;;) {
+        const uint4 *p = reinterpret_cast<const uint4 *>(tab + 4 * (size_t)g);
+        uint4 v[4];
+#pragma unroll
+        for (int i = 0; i < 4; ++i) v[i] = __ldg(p + i);
+        bool open = false, found = false;
+        uint32_t hit_off = 0, hit_meta = BLOCK_MISS;
+#pragma unroll
+        for (int i = 0; i < 4; ++i) {              // selects, not an indexed (local-memory) array
+            const unsigned long long ki = (unsigned long long)v[i].x | ((unsigned long long)v[i].y << 32);
+            const bool m = ki == key;
+            hit_off = m ? v[i].z : hit_off;
+            hit_meta = m ? v[i].w : hit_meta;
+            found |= m;
+            open |= ki == ~0ull;
+        }
+        if (found) { off = hit_off; return hit_meta; }
+        if (open) return BLOCK_MISS;
+        if (++g == ngroups) g = 0;
+    }
+}
+
+// One pass of build_blocks over the buckets of table T: a half-warp per bucket, its children in
+// octant order, each through the span kernel's own look-ups and span order.  COUNT: the run
+// units (16 bytes) of the bucket's children into units[bucket].  Otherwise: each child's run at
+// runs + off[bucket] + (units of the bucket's earlier children), and its slot in tab.
+template <bool COUNT>
+__global__ void __launch_bounds__(256)
+block_run_kernel(const GridTable T, unsigned long long *units, const unsigned long long *off, const PointF *pts,
+                 uint4 *runs, BlockSlot *tab, uint32_t tab_cap)
+{
+    __shared__ uint2 s_heads[256 / 16][SPAN_MAX];
+    const unsigned lane = threadIdx.x & 31u, sl = lane & 15u, hbase = lane & 16u;
+    uint2 *heads = s_heads[threadIdx.x >> 4];
+    const uint32_t b = (blockIdx.x * blockDim.x + threadIdx.x) >> 4;
+    unsigned long long key = ~0ull;
+    uint32_t perm = 0;
+    if (b < T.cap) {
+        key = T.buckets[b].key;
+        perm = T.buckets[b].perm;
+    }
+    const uint32_t occ = key != ~0ull ? perm >> 24 : 0u;
+    const uint32_t ncell = 1u << T.level;
+    const uint32_t par[3] = {(uint32_t)(key & 0x1fffffu), (uint32_t)((key >> 21) & 0x1fffffu),
+                             (uint32_t)((key >> 42) & 0x1fffffu)};
+    unsigned long long u_sum = 0;
+    for (int o = 0; o < 8; ++o) {                // all lanes: the look-ups end in warp shuffles
+        const bool look = (occ >> o) & 1u;
+        const uint32_t c[3] = {2u * par[0] + (o & 1u), 2u * par[1] + ((o >> 1) & 1u), 2u * par[2] + ((o >> 2) & 1u)};
+        uint32_t pstart, inr, brk, mine_v, incl;
+        uint4 cum;
+        bool dense;
+        span_parent(T, c, ncell, sl, look, pstart, inr, brk, cum, dense);
+        const uint32_t hsum = span_scan(inr, brk, cum, sl, hbase, mine_v, incl);
+        const uint32_t total = hsum & 0xffffffu, nspan = hsum >> 24;
+        const bool dense_h = ((__ballot_sync(0xffffffffu, dense) >> hbase) & 0xffffu) != 0u;
+        // the span kernel stages such a block only when it holds <= PAIR_CAP records and no dense parent
+        const bool ok = look && !dense_h && total <= (uint32_t)PAIR_CAP;
+        const uint32_t u = ok ? total + block_heads_pad(nspan) / 2u : 0u;
+        if (!COUNT && look) {
+            uint4 *run = runs + off[b] + u_sum;
+            if (ok) {
+                uint32_t slot = (incl - mine_v) & 0xffffffu, e = (incl - mine_v) >> 24;
+                for_each_span(inr, brk, cum, [&](uint32_t first, uint32_t n) {
+                    heads[e] = make_uint2(slot, pstart + first);
+                    slot += n;
+                    ++e;
+                });
+            }
+            __syncwarp(0xffffu << hbase);
+            if (ok) {
+                for (uint32_t j = sl; j < total; j += 16u) {     // last head with first slot <= j
+                    uint32_t lo = 0, n = nspan;
+                    while (n > 1u) {
+                        const uint32_t h = n >> 1;
+                        if (heads[lo + h].x <= j) lo += h;
+                        n -= h;
+                    }
+                    run[j] = __ldg(reinterpret_cast<const uint4 *>(pts + heads[lo].y + (j - heads[lo].x)));
+                }
+                uint2 *hout = reinterpret_cast<uint2 *>(run + total);
+                for (uint32_t e = sl; e < block_heads_pad(nspan); e += 16u)
+                    hout[e] = e < nspan ? heads[e] : make_uint2(0u, 0u);
+            }
+            if (sl == 0u) {
+                const unsigned long long ck = block_key(c);
+                uint32_t s = 4u * __umulhi(grid_hash_q(ck), tab_cap >> 2);
+                for (;;) {                           // the order block_lookup probes in
+                    BlockSlot *S = tab + s;
+                    if (atomicCAS(&S->key, ~0ull, ck) == ~0ull) {
+                        S->off = ok ? (uint32_t)(off[b] + u_sum) : 0u;
+                        S->meta = ok ? total | (nspan << 16) : BLOCK_MISS;
+                        break;
+                    }
+                    if (++s == tab_cap) s = 0;
+                }
+            }
+            __syncwarp(0xffffu << hbase);            // the heads are free for the next child
+        }
+        u_sum += u;
+    }
+    if (COUNT && sl == 0u && b < T.cap) units[b] = u_sum;
+}
+
 // Outputs of both halves: pair_emit (pt_knn_grid.cuh) with the winner's attribute record passed
 // in.  Same arithmetic, in the same order (frozen blend, DESIGN.md section 5).
 __device__ __forceinline__ void span_emit(const QueryParams &P, uint32_t s, bool em, uint32_t mine, double d,
@@ -153,8 +337,11 @@ __device__ __forceinline__ void span_emit(const QueryParams &P, uint32_t s, bool
 // n_warps.. in claiming order) instead of taking every n_warps-th pair, so that the persistent
 // launch ends with the last pair rather than with the warp whose pairs happened to be slowest.
 // Which warp answers a pair never changes the pair's answer.
-__global__ void __launch_bounds__(GRID_WARPS * 32, PT_SPAN_MIN_BLOCKS)
-knn_grid_span_kernel(const QueryParams P, uint32_t *ovf_count, uint32_t *ovf_list, uint32_t *claim)
+// BLOCK: a sample stages the block run of its cell (P.grid.blk) instead of the eight parents' spans;
+// the staged records and heads are the same, so is everything from the selection on.
+template <bool BLOCK>
+__device__ __forceinline__ void span_body(const QueryParams &P, uint32_t *ovf_count, uint32_t *ovf_list,
+                                          uint32_t *claim)
 {
     extern __shared__ __align__(128) unsigned char g_smem[];
     const unsigned lane = threadIdx.x & 31, wib = threadIdx.x >> 5;
@@ -220,53 +407,29 @@ knn_grid_span_kernel(const QueryParams P, uint32_t *ovf_count, uint32_t *ovf_lis
         const double slack = G.slack + 1.8e-15 * (fabs(qx) + fabs(qy) + fabs(qz));
         const double g = (double)gl * G.cell21 - slack;
         const double g2 = g > 0.0 ? __dmul_rd(g, g) : 0.0;
-        // ---- look-ups: sub-lane j < 8 takes parent j of the block's 2 x 2 x 2 parents ---------------
-        // Along an axis the block's cells c - 1 .. c + 1 lie in parents ((c + 1) >> 1) - 1 and
-        // (c + 1) >> 1; child bit b of parent q is cell 2q + b, inside the block iff it is one of
-        // c - 1 .. c + 1 and below ncell (the unsigned compare also rejects "negative" cells).
-        uint32_t pstart = 0, inr = 0, brk = 0;
-        uint4 cum = make_uint4(0u, 0u, 0u, 0u);
-        bool dense = false;
-        if (look && sl < 8u) {
-            uint32_t pq[3], oct = 0xffu;
-#pragma unroll
-            for (int ax = 0; ax < 3; ++ax) {
-                pq[ax] = ((c[ax] + 1u) >> 1) - 1u + ((sl >> ax) & 1u);
-                const uint32_t x0 = 2u * pq[ax], x1 = x0 + 1u;
-                const bool b0 = x0 - c[ax] + 1u < 3u && x0 < ncell, b1 = x1 - c[ax] + 1u < 3u && x1 < ncell;
-                // octants o with bit `ax` of o = 0 (b0) or 1 (b1)
-                const uint32_t m1 = ax == 0 ? 0xaau : (ax == 1 ? 0xccu : 0xf0u);
-                oct &= (b0 ? (~m1 & 0xffu) : 0u) | (b1 ? m1 : 0u);
-            }
-            uint32_t perm = 0;
-#ifdef PT_STATS
-            if (oct) atomicAdd(&g_stats[16], 1ull);
-#endif
-            if (oct && grid_parent_lookup(T.buckets, T.cap, pq[0], pq[1], pq[2], pstart, perm, cum)) {
-                const uint32_t occ = perm >> 24, om = oct & occ;
-                if (om && (cum.x & 0xffffu) == 0xffffu) dense = true;
-                else if (om) {
-#pragma unroll
-                    for (int o = 0; o < 8; ++o) {
-                        const uint32_t rb = 1u << ((perm >> (3 * o)) & 7u);
-                        if ((om >> o) & 1u) inr |= rb;
-                        else if ((occ >> o) & 1u) brk |= rb;
-                    }
-                }
-            }
+        uint32_t total, nspan;
+        bool dense_h;
+        // block runs: the slot of the sample's cell (sub-lane 0); an empty cell is a miss like a
+        // block that cannot be staged, and goes to the whole-warp redo
+        uint32_t boff = 0, bmeta = BLOCK_MISS;
+        // span staging: sub-lane j < 8 takes parent j of the block's 2 x 2 x 2 parents
+        uint32_t pstart, inr, brk, mine_v, incl;
+        uint4 cum;
+        if constexpr (BLOCK) {
+            if (look && sl == 0u) bmeta = block_lookup(G.blk, G.blk_cap, block_key(c), boff);
+            bmeta = __shfl_sync(0xffffffffu, bmeta, (int)hbase);
+            boff = __shfl_sync(0xffffffffu, boff, (int)hbase);
+            total = bmeta & 0xffffu;
+            nspan = (bmeta >> 16) & 0xffu;
+            dense_h = (bmeta & BLOCK_MISS) != 0u;
+        } else {
+            bool dense;
+            span_parent(T, c, ncell, sl, look, pstart, inr, brk, cum, dense);
+            const uint32_t hsum = span_scan(inr, brk, cum, sl, hbase, mine_v, incl);
+            total = hsum & 0xffffffu;
+            nspan = hsum >> 24;
+            dense_h = ((__ballot_sync(0xffffffffu, dense) >> hbase) & 0xffffu) != 0u;
         }
-        // spans << 24 | points of this lane's parent
-        uint32_t mine_v = 0;
-        for_each_span(inr, brk, cum, [&](uint32_t, uint32_t n) { mine_v += (1u << 24) + n; });
-        uint32_t incl = mine_v;
-#pragma unroll
-        for (int o = 1; o < 8; o <<= 1) {
-            const uint32_t y = __shfl_up_sync(0xffffffffu, incl, o);
-            if (sl >= (unsigned)o) incl += y;
-        }
-        const uint32_t hsum = __shfl_sync(0xffffffffu, incl, (int)(hbase | 7u));
-        const uint32_t total = hsum & 0xffffffu, nspan = hsum >> 24;
-        const bool dense_h = ((__ballot_sync(0xffffffffu, dense) >> hbase) & 0xffffu) != 0u;
         const bool go = look && !dense_h && total <= (uint32_t)PAIR_CAP && (total >= (uint32_t)k || r2 <= g2);
         const uint32_t tot = go ? total : 0u;
         const uint32_t tA = __shfl_sync(0xffffffffu, tot, 0), tB = __shfl_sync(0xffffffffu, tot, 16);
@@ -277,20 +440,33 @@ knn_grid_span_kernel(const QueryParams P, uint32_t *ovf_count, uint32_t *ovf_lis
         if (tA + tB > 0u) {
             fence_proxy_async();
             __syncwarp();
-            if (lane == 0) mbar_arrive_expect(bar, (tA + tB) * (uint32_t)sizeof(PointF));
-            __syncwarp();
-            if (go) {
-                uint32_t slot = (incl - mine_v) & 0xffffffu, e = (incl - mine_v) >> 24;
-                for_each_span(inr, brk, cum, [&](uint32_t first, uint32_t n) {
-                    bulk_g2s(smem_u32(cand + slot), pts + pstart + first, n * (uint32_t)sizeof(PointF), bar);
-                    heads[e] = make_uint2(slot, pstart + first);
-                    slot += n;
-                    ++e;
-                });
+            if constexpr (BLOCK) {
+                // records and heads of the run: 16 bytes per record, 8 per (padded) head
+                const uint32_t hb = go ? block_heads_pad(nspan) * (uint32_t)sizeof(uint2) : 0u;
+                const uint32_t hbA = __shfl_sync(0xffffffffu, hb, 0), hbB = __shfl_sync(0xffffffffu, hb, 16);
+                if (lane == 0) mbar_arrive_expect(bar, (tA + tB) * (uint32_t)sizeof(PointF) + hbA + hbB);
+                __syncwarp();
+                if (go && sl == 0u) {
+                    const uint4 *run = G.blk_runs + boff;
+                    bulk_g2s(smem_u32(cand), run, total * (uint32_t)sizeof(PointF), bar);
+                    bulk_g2s(smem_u32(heads), run + total, hb, bar);
+                }
+            } else {
+                if (lane == 0) mbar_arrive_expect(bar, (tA + tB) * (uint32_t)sizeof(PointF));
+                __syncwarp();
+                if (go) {
+                    uint32_t slot = (incl - mine_v) & 0xffffffu, e = (incl - mine_v) >> 24;
+                    for_each_span(inr, brk, cum, [&](uint32_t first, uint32_t n) {
+                        bulk_g2s(smem_u32(cand + slot), pts + pstart + first, n * (uint32_t)sizeof(PointF), bar);
+                        heads[e] = make_uint2(slot, pstart + first);
+                        slot += n;
+                        ++e;
+                    });
+                }
             }
             __syncwarp();                           // the span heads are visible to the whole half
 #ifdef PT_STATS
-            if (go) {   // spans whose sorted start is the sorted end of another span of the half
+            if (!BLOCK && go) {   // spans whose sorted start is the sorted end of another span of the half
                 uint32_t hits = 0;
                 for (uint32_t a = sl; a < nspan; a += 16u)
                     for (uint32_t b = 0; b < nspan; ++b) {
@@ -380,6 +556,18 @@ knn_grid_span_kernel(const QueryParams P, uint32_t *ovf_count, uint32_t *ovf_lis
 #endif
 }
 
+__global__ void __launch_bounds__(GRID_WARPS * 32, PT_SPAN_MIN_BLOCKS)
+knn_grid_span_kernel(const QueryParams P, uint32_t *ovf_count, uint32_t *ovf_list, uint32_t *claim)
+{
+    span_body<false>(P, ovf_count, ovf_list, claim);
+}
+
+__global__ void __launch_bounds__(GRID_WARPS * 32, PT_SPAN_MIN_BLOCKS)
+knn_grid_block_kernel(const QueryParams P, uint32_t *ovf_count, uint32_t *ovf_list, uint32_t *claim)
+{
+    span_body<true>(P, ovf_count, ovf_list, claim);
+}
+
 // The pair kernel's conditions (launch_grid) plus the curve-ordered attributes wherever the
 // launch reads attributes.
 template <typename PT>
@@ -392,14 +580,22 @@ static bool grid_span_applies(const QueryParams &qp)
            (qp.attrs_curve != nullptr || qp.attrs == nullptr || !want_attr);
 }
 
-static int launch_grid_span(const QueryParams &qp, int sm_count, uint32_t *count, uint32_t *list, uint32_t *claim,
-                            cudaStream_t s)
+// Under grid_span_applies: whether the launch stages block runs -- the index has them for the level
+// of the launch's first attempt.
+static bool grid_block_applies(const QueryParams &qp)
 {
+    return opt_grid_block() != 0 && qp.grid.blk != nullptr && qp.grid.tab[qp.grid.att_tab[0]].level == qp.grid.blk_level;
+}
+
+static int launch_grid_span(const QueryParams &qp, bool block, int sm_count, uint32_t *count, uint32_t *list,
+                            uint32_t *claim, cudaStream_t s)
+{
+    const auto kernel = block ? knn_grid_block_kernel : knn_grid_span_kernel;
     const size_t smem = (sizeof(PointF) * 2 * PAIR_CAP + sizeof(uint2) * 2 * SPAN_MAX + 8) * GRID_WARPS;
     if (smem > 48 * 1024)
-        PT_CUDA(cudaFuncSetAttribute(knn_grid_span_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+        PT_CUDA(cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
     int per_sm = 0;
-    PT_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, knn_grid_span_kernel, GRID_WARPS * 32, smem));
+    PT_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, kernel, GRID_WARPS * 32, smem));
     if (per_sm < 1) per_sm = 1;
     const unsigned want = ((qp.m + 1u) / 2u + GRID_WARPS - 1) / GRID_WARPS;
     const unsigned resident = (unsigned)(sm_count * per_sm);
@@ -408,7 +604,7 @@ static int launch_grid_span(const QueryParams &qp, int sm_count, uint32_t *count
     // 0.342 -> 0.311 ms, cfg5 7.00 -> 6.49 ms); at cfg1 (1.2 pairs per warp) the static stride is
     // 1 us faster (DESIGN.md section 4)
     const bool use_claim = opt_grid_claim() != 0 && (qp.m + 1u) / 2u > 2u * blocks * GRID_WARPS;
-    knn_grid_span_kernel<<<blocks, GRID_WARPS * 32, smem, s>>>(qp, count, list, use_claim ? claim : nullptr);
+    kernel<<<blocks, GRID_WARPS * 32, smem, s>>>(qp, count, list, use_claim ? claim : nullptr);
     count_launch();
     PT_CUDA(cudaGetLastError());
     return PT_OK;
