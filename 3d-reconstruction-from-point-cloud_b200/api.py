@@ -54,7 +54,7 @@ ABI_SYMBOLS = (
     "pt_texture_bake_ex", "pt_bake_samples_device", "pt_bake_frames_device", "pt_bake_compose_tangent_device",
     "pt_texture_bake_height", "pt_bake_compose_height_device", "pt_sharded_bake",
     "pt_index_estimate_normals", "pt_estimate_normals_device", "pt_index_orient_normals",
-    "pt_sharded_estimate_normals",
+    "pt_sharded_estimate_normals", "pt_sharded_orient_normals",
 )
 # ... and include/pt_synth.h (bench / test scaffolding, its own library)
 SYNTH_SYMBOLS = ("pt_synth_cloud_device", "pt_synth_samples_device", "pt_synth_pack_points_device",
@@ -230,6 +230,8 @@ def lib():
     L.pt_sharded_estimate_normals.argtypes = [vp, i32, dbl, vp, i32, vp, vp, ctypes.POINTER(NormalsStats)]
     L.pt_index_orient_normals.restype = i32
     L.pt_index_orient_normals.argtypes = [vp, i32, dbl, vp, i32, vp, vp, ctypes.POINTER(OrientStats)]
+    L.pt_sharded_orient_normals.restype = i32
+    L.pt_sharded_orient_normals.argtypes = [vp, i32, dbl, vp, i32, vp, vp, ctypes.POINTER(OrientStats)]
     L.pt_set_option.restype = i32
     L.pt_set_option.argtypes = [ctypes.c_char_p, i32]
     L.pt_get_option.restype = i32
@@ -503,15 +505,8 @@ class Tree:
         flipped, components, edges, knn_ms, mst_ms).  Each component's root, its highest point, faces
         ``viewpoint`` (x, y, z) when given, else +z.  ``store=True`` also replaces the tree's normals
         with the oriented ones, so later ``transfer`` / ``bake`` calls blend them."""
-        n = self.size()
-        out = {"normal": np.empty((n, 3), dtype=np.float32), "root": np.empty(n, dtype=np.int32)}
-        st = OrientStats()
-        _check(lib().pt_index_orient_normals(self._h, int(k), _radius(radius), _viewpoint(viewpoint),
-                                             1 if store else 0, _np_ptr(out["normal"]), _np_ptr(out["root"]),
-                                             ctypes.byref(st)), "pt_index_orient_normals")
-        out["stats"] = {"oriented": int(st.oriented), "flipped": int(st.flipped), "components": int(st.components),
-                        "edges": int(st.edges), "knn_ms": st.knn_ms, "mst_ms": st.mst_ms}
-        return out
+        return _orient_normals(lib().pt_index_orient_normals, "pt_index_orient_normals", self._h, self.size(), k,
+                               radius, viewpoint, store)
 
     def transfer_slab(self, queries_ptr, queries_are_xyz, m, k, radius, boxes6, rank, halo,
                       idx_ptr, rgba_ptr, normal_ptr, d2_ptr=None):
@@ -572,6 +567,19 @@ def _estimate_normals(fn, name, handle, n, k, radius, viewpoint, store):
     _check(fn(handle, int(k), _radius(radius), _viewpoint(viewpoint), 1 if store else 0, _np_ptr(out["normal"]),
               _np_ptr(out["variation"]), ctypes.byref(st)), name)
     out["stats"] = {"estimated": int(st.estimated), "knn_ms": st.knn_ms, "pca_ms": st.pca_ms}
+    return out
+
+
+def _orient_normals(fn, name, handle, n, k, radius, viewpoint, store):
+    """Output arrays and result dict of ``Tree.orient_normals`` and ``ShardedTree.orient_normals``:
+    ``fn`` is ``pt_index_orient_normals`` or ``pt_sharded_orient_normals``, which take the same
+    arguments after the handle."""
+    out = {"normal": np.empty((n, 3), dtype=np.float32), "root": np.empty(n, dtype=np.int32)}
+    st = OrientStats()
+    _check(fn(handle, int(k), _radius(radius), _viewpoint(viewpoint), 1 if store else 0, _np_ptr(out["normal"]),
+              _np_ptr(out["root"]), ctypes.byref(st)), name)
+    out["stats"] = {"oriented": int(st.oriented), "flipped": int(st.flipped), "components": int(st.components),
+                    "edges": int(st.edges), "knn_ms": st.knn_ms, "mst_ms": st.mst_ms}
     return out
 
 
@@ -636,6 +644,18 @@ class ShardedTree:
         calls blend them, and keeps them across rebuilds of the slabs."""
         return _estimate_normals(lib().pt_sharded_estimate_normals, "pt_sharded_estimate_normals", self._h,
                                  self._points.shape[0], k, radius, viewpoint, store)
+
+    def orient_normals(self, k=18, radius=None, viewpoint=None, store=False):
+        """``Tree.orient_normals`` on the sharded cloud (``pt_sharded_orient_normals``): same arguments
+        and result, ``normal``, ``root`` and the four counts of ``stats`` byte-identical to
+        ``Tree.orient_normals`` on one index of the same cloud.  Each slab builds the edges of the points
+        it owns and the spanning forest of the edges between them on its own device; slab 0's device
+        joins them into the cloud's forest.  ``stats["knn_ms"]`` is the host wall time of the slab
+        stage and ``stats["mst_ms"]`` that of the rest.  ``store=True`` also replaces the normals in
+        every slab that holds the point, so later ``transfer`` / ``bake`` calls blend them, and keeps
+        them across rebuilds of the slabs."""
+        return _orient_normals(lib().pt_sharded_orient_normals, "pt_sharded_orient_normals", self._h,
+                               self._points.shape[0], k, radius, viewpoint, store)
 
     def close(self):
         if getattr(self, "_h", None) and self._h.value:

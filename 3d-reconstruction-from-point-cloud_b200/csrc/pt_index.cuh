@@ -122,6 +122,56 @@ struct NormalsSlab {
 int normals_slab(pt_index *ix, int k, double radius, const double *viewpoint, const NormalsSlab &sl,
                  float *normal_out, float *variation_out, unsigned long long *estimated, float *pca_ms,
                  int *needs);
+// The rows a slab owns and their self-query, shared by normals_slab and orient_slab (pt_normals.cu).
+// slab_rows_select, on ix's device and stream: boxes, cuts and a zeroed flag to the device, and
+// rows[0 .. n_rows - 1] = the sorted positions of the records the cut rule gives to slab `self`, in
+// ascending order; n_rows != sl.n_own is PT_ERR_UNSUPPORTED.  Synchronises.  tmp holds tmp_bytes,
+// enough for a cub select over ix->n records.  slab_rows_query: self_query_chunks over those rows,
+// with the ghost-zone check when sl.check; *flag turns non-zero when it flags the step.
+struct SlabRows {
+    double *boxes = nullptr;          // device: n_slabs x 6 own boxes, then the n_slabs - 1 cuts
+    uint32_t *rows = nullptr, *count = nullptr, *flag = nullptr;
+    void *tmp = nullptr;
+    size_t tmp_bytes = 0;
+    uint32_t n_rows = 0;
+};
+int slab_rows_select(pt_index *ix, const NormalsSlab &sl, SlabRows &w);
+int slab_rows_query(pt_index *ix, int k, double radius, const NormalsSlab &sl, const SlabRows &w, int32_t *lists,
+                    bool keep, const ChunkThen &then, std::vector<cudaEvent_t> *marks);
+void slab_rows_free(SlabRows &w, cudaStream_t s);
+// The argument rules of pt_index_orient_normals that do not concern the index: PT_OK or its error.
+int orient_check_args(int k, const double *viewpoint, bool store, bool any_output);
+// An edge of the orientation graph (pt_orient.cu)
+struct OrientEdge {
+    unsigned long long w;     // bits of w = 1 - |d| >= +0
+    unsigned long long key;   // lo << 32 | hi (point ids)
+    uint32_t u, v;            // rows; v's LAB_BIT: d < 0
+};
+// One slab of pt_sharded_orient_normals (pt_orient.cu), on ix's device and stream: the self-query of
+// the own rows as normals_slab runs it (*needs = 1 when the ghost check flags the step), the edges of
+// the own points' lists, and the minimum spanning forest of the intra-slab edges.  Replaces `forest`
+// and `cross` with that forest's edges and the slab's cross edges (one end owned elsewhere), their
+// u, v and key in global ids (ix->ids), and sets *intra to the intra-slab edge count.  Synchronises.
+int orient_slab(pt_index *ix, int k, double radius, const NormalsSlab &sl, std::vector<OrientEdge> &forest,
+                std::vector<OrientEdge> &cross, uint64_t *intra, int *needs);
+// The rest of pt_sharded_orient_normals, on the current device and stream s: the minimum spanning
+// forest of the slabs' forests and cross edges (sorted by key and deduplicated first; *unique_cross
+// counts what is left) over the cloud's n points, then roots, signs and outputs in point order.
+// Host arrays: normal (n x 3, the doubles the slabs' records were built from: the stored normal
+// widened, else the input normal), pos (with a viewpoint the n x 3 positions, else the n z values,
+// as the caller gave them), normal_out (n x 3) and root_out (n).
+// counts: oriented, flipped, components.  Synchronises.
+struct OrientHome {
+    size_t n;
+    const double *normal;
+    const double *pos;
+    const double *viewpoint;
+    float *normal_out;
+    int32_t *root_out;
+};
+int orient_home(const OrientHome &h, const std::vector<std::vector<OrientEdge>> &forest,
+                const std::vector<std::vector<OrientEdge>> &cross, uint64_t *unique_cross,
+                unsigned long long counts[3], cudaStream_t s);
 // Writes values (host, n x 3 floats in ix's local order, x NaN: leave that point as it is) into the
 // normals of ix's attrs and attrs_curve, on ix's stream; synchronises.
 int normals_store(pt_index *ix, const float *values);

@@ -463,20 +463,10 @@ normals_store_kernel(const float *values, uint32_t n, const uint32_t *inv, pt_at
 }
 
 template <typename PT>
-static int normals_slab_t(pt_index *ix, int k, double radius, const double *viewpoint, const NormalsSlab &sl,
-                          float *normal_out, float *variation_out, unsigned long long *estimated, float *pca_ms,
-                          int *needs)
+static int slab_rows_select_t(pt_index *ix, const NormalsSlab &sl, SlabRows &w)
 {
     cudaStream_t s = ix->stream;
     const uint32_t n = ix->n;
-    uint32_t *d_rows = nullptr, *d_count = nullptr, *d_flag = nullptr;
-    int32_t *d_idx = nullptr;
-    float *d_normal = nullptr, *d_var = nullptr, *d_cnormal = nullptr, *d_cvar = nullptr;
-    double *d_boxes = nullptr;          // n_slabs x 6 boxes, then the n_slabs - 1 cuts
-    unsigned long long *d_est = nullptr, est = 0;
-    void *d_tmp = nullptr;
-    uint32_t n_rows = 0, flag = 0;
-    std::vector<cudaEvent_t> marks;
     int rc = PT_OK;
     auto fail = [&](cudaError_t e) { if (e != cudaSuccess && rc == PT_OK) rc = map_cuda_error(e); return e != cudaSuccess; };
     do {
@@ -485,37 +475,77 @@ static int normals_slab_t(pt_index *ix, int k, double radius, const double *view
             break;
         }
         const int R = sl.n_slabs;
-        if (pool_alloc((void **)&d_boxes, sizeof(double) * (7 * R - 1), s) ||
-            pool_alloc((void **)&d_rows, sizeof(uint32_t) * n, s) || pool_alloc((void **)&d_count, sizeof(uint32_t), s) ||
-            pool_alloc((void **)&d_flag, sizeof(uint32_t), s)) {
+        if (pool_alloc((void **)&w.boxes, sizeof(double) * (7 * R - 1), s) ||
+            pool_alloc((void **)&w.rows, sizeof(uint32_t) * n, s) || pool_alloc((void **)&w.count, sizeof(uint32_t), s) ||
+            pool_alloc((void **)&w.flag, sizeof(uint32_t), s)) {
             rc = PT_ERR_OUT_OF_MEMORY;
             break;
         }
-        if (fail(cudaMemcpyAsync(d_boxes, sl.boxes, sizeof(double) * 6 * R, cudaMemcpyHostToDevice, s)) ||
-            (R > 1 && fail(cudaMemcpyAsync(d_boxes + 6 * R, sl.cuts, sizeof(double) * (R - 1), cudaMemcpyHostToDevice, s))) ||
-            fail(cudaMemsetAsync(d_flag, 0, sizeof(uint32_t), s)))
+        if (fail(cudaMemcpyAsync(w.boxes, sl.boxes, sizeof(double) * 6 * R, cudaMemcpyHostToDevice, s)) ||
+            (R > 1 && fail(cudaMemcpyAsync(w.boxes + 6 * R, sl.cuts, sizeof(double) * (R - 1), cudaMemcpyHostToDevice, s))) ||
+            fail(cudaMemsetAsync(w.flag, 0, sizeof(uint32_t), s)))
             break;
         // the own records in ascending sorted position, so the self-queries stay curve-coherent
-        const SlabOwnRow<PT> own{(const PT *)ix->pts, d_boxes + 6 * R, R - 1, sl.self};
+        const SlabOwnRow<PT> own{(const PT *)ix->pts, w.boxes + 6 * R, R - 1, sl.self};
         thrust::counting_iterator<uint32_t> ids(0);
         size_t row_bytes = 0, local_bytes = 0;
-        if (fail(cub::DeviceSelect::If(nullptr, row_bytes, ids, d_rows, d_count, (int)n, own, s)) ||
-            fail(cub::DeviceSelect::If(nullptr, local_bytes, ids, d_rows, d_count, (int)n, SlabOwnLocal<PT>{own, nullptr}, s)))
+        if (fail(cub::DeviceSelect::If(nullptr, row_bytes, ids, w.rows, w.count, (int)n, own, s)) ||
+            fail(cub::DeviceSelect::If(nullptr, local_bytes, ids, w.rows, w.count, (int)n, SlabOwnLocal<PT>{own, nullptr}, s)))
             break;
-        if (pool_alloc(&d_tmp, std::max(std::max(row_bytes, local_bytes), (size_t)1), s)) {
+        w.tmp_bytes = std::max(std::max(row_bytes, local_bytes), (size_t)1);
+        if (pool_alloc(&w.tmp, w.tmp_bytes, s)) {
             rc = PT_ERR_OUT_OF_MEMORY;
             break;
         }
-        if (fail(cub::DeviceSelect::If(d_tmp, row_bytes, ids, d_rows, d_count, (int)n, own, s))) break;
+        if (fail(cub::DeviceSelect::If(w.tmp, row_bytes, ids, w.rows, w.count, (int)n, own, s))) break;
         count_launch();
-        if (fail(cudaMemcpyAsync(&n_rows, d_count, sizeof n_rows, cudaMemcpyDeviceToHost, s)) ||
+        if (fail(cudaMemcpyAsync(&w.n_rows, w.count, sizeof w.n_rows, cudaMemcpyDeviceToHost, s)) ||
             fail(cudaStreamSynchronize(s)))
             break;
         // the records this rule selects are the ones build_slabs counted as the slab's own
-        if (n_rows != sl.n_own) {
-            rc = PT_ERR_UNSUPPORTED;
-            break;
-        }
+        if (w.n_rows != sl.n_own) rc = PT_ERR_UNSUPPORTED;
+    } while (0);
+    return rc;
+}
+
+int slab_rows_select(pt_index *ix, const NormalsSlab &sl, SlabRows &w)
+{
+    return ix->coord_f64 ? slab_rows_select_t<PointD>(ix, sl, w) : slab_rows_select_t<PointF>(ix, sl, w);
+}
+
+int slab_rows_query(pt_index *ix, int k, double radius, const NormalsSlab &sl, const SlabRows &w, int32_t *lists,
+                    bool keep, const ChunkThen &then, std::vector<cudaEvent_t> *marks)
+{
+    const BakeGhost ghost{w.boxes, sl.n_slabs, sl.self, sl.halo, w.flag};
+    return self_query_chunks(ix, k, radius, lists, keep, then, marks, ix->stream, w.rows, w.n_rows,
+                             sl.check ? &ghost : nullptr);
+}
+
+void slab_rows_free(SlabRows &w, cudaStream_t s)
+{
+    void *frees[] = {w.boxes, w.rows, w.count, w.flag, w.tmp};
+    for (void *p : frees) pool_free(p, s);
+    w = SlabRows{};
+}
+
+template <typename PT>
+static int normals_slab_t(pt_index *ix, int k, double radius, const double *viewpoint, const NormalsSlab &sl,
+                          float *normal_out, float *variation_out, unsigned long long *estimated, float *pca_ms,
+                          int *needs)
+{
+    cudaStream_t s = ix->stream;
+    const uint32_t n = ix->n;
+    SlabRows w;
+    int32_t *d_idx = nullptr;
+    float *d_normal = nullptr, *d_var = nullptr, *d_cnormal = nullptr, *d_cvar = nullptr;
+    unsigned long long *d_est = nullptr, est = 0;
+    uint32_t flag = 0;
+    std::vector<cudaEvent_t> marks;
+    int rc = PT_OK;
+    auto fail = [&](cudaError_t e) { if (e != cudaSuccess && rc == PT_OK) rc = map_cuda_error(e); return e != cudaSuccess; };
+    do {
+        if ((rc = slab_rows_select_t<PT>(ix, sl, w)) != PT_OK) break;
+        const uint32_t n_rows = w.n_rows;
         if (n_rows == 0) break;
         const size_t chunk = std::min((size_t)HEIGHT_CHUNK, (size_t)n_rows);
         if (pool_alloc((void **)&d_idx, sizeof(int32_t) * k * chunk, s) ||
@@ -526,34 +556,34 @@ static int normals_slab_t(pt_index *ix, int k, double radius, const double *view
             break;
         }
         if (fail(cudaMemsetAsync(d_est, 0, sizeof(unsigned long long), s))) break;
-        const BakeGhost ghost{d_boxes, R, sl.self, sl.halo, d_flag};
         // no store here: the caller stores once every slab has passed its check
         const NormalsOut o = normals_out(ix, viewpoint, false, d_normal, d_var, d_est);
-        rc = self_query_chunks(
-            ix, k, radius, d_idx, false,
+        rc = slab_rows_query(
+            ix, k, radius, sl, w, d_idx, false,
             [&](uint32_t c0, uint32_t cm, const int32_t *idx) {
-                normals_pca_list_kernel<PT><<<ncdiv(cm, 256), 256, 0, s>>>((const PT *)ix->pts, ix->inv_perm, n, d_rows, c0,
+                normals_pca_list_kernel<PT><<<ncdiv(cm, 256), 256, 0, s>>>((const PT *)ix->pts, ix->inv_perm, n, w.rows, c0,
                                                                            cm, idx, k, normals_width(k), o);
                 count_launch();
                 cudaError_t e = cudaGetLastError();
                 if (e == cudaSuccess) e = record_mark(&marks, s);
                 return e == cudaSuccess ? PT_OK : map_cuda_error(e);
             },
-            &marks, s, d_rows, n_rows, sl.check ? &ghost : nullptr);
+            &marks);
         if (rc != PT_OK) break;
         // only the own records' results travel to the host, in ascending local id (the order of their
         // global ids); the row list is free again in stream order and takes their local ids
-        if (fail(cub::DeviceSelect::If(d_tmp, local_bytes, ids, d_rows, d_count, (int)n,
+        const SlabOwnRow<PT> own{(const PT *)ix->pts, w.boxes + 6 * sl.n_slabs, sl.n_slabs - 1, sl.self};
+        if (fail(cub::DeviceSelect::If(w.tmp, w.tmp_bytes, thrust::counting_iterator<uint32_t>(0), w.rows, w.count, (int)n,
                                        SlabOwnLocal<PT>{own, ix->inv_perm}, s)))
             break;
         count_launch();
-        normals_compact_kernel<<<ncdiv(n_rows, 256), 256, 0, s>>>(d_rows, n_rows, d_normal, d_var, d_cnormal, d_cvar);
+        normals_compact_kernel<<<ncdiv(n_rows, 256), 256, 0, s>>>(w.rows, n_rows, d_normal, d_var, d_cnormal, d_cvar);
         count_launch();
         if (fail(cudaGetLastError())) break;
         if (fail(cudaMemcpyAsync(normal_out, d_cnormal, sizeof(float) * 3 * n_rows, cudaMemcpyDeviceToHost, s)) ||
             fail(cudaMemcpyAsync(variation_out, d_cvar, sizeof(float) * n_rows, cudaMemcpyDeviceToHost, s)) ||
             fail(cudaMemcpyAsync(&est, d_est, sizeof est, cudaMemcpyDeviceToHost, s)) ||
-            fail(cudaMemcpyAsync(&flag, d_flag, sizeof flag, cudaMemcpyDeviceToHost, s)) || fail(cudaStreamSynchronize(s)))
+            fail(cudaMemcpyAsync(&flag, w.flag, sizeof flag, cudaMemcpyDeviceToHost, s)) || fail(cudaStreamSynchronize(s)))
             break;
         *estimated += est;
         *needs = sl.check && flag ? 1 : 0;
@@ -563,7 +593,8 @@ static int normals_slab_t(pt_index *ix, int k, double radius, const double *view
             if (cudaEventElapsedTime(&t, marks[c], marks[c + 1]) == cudaSuccess) *pca_ms += t;
     } while (0);
     cudaStreamSynchronize(s);
-    void *frees[] = {d_rows, d_count, d_flag, d_idx, d_normal, d_var, d_cnormal, d_cvar, d_boxes, d_est, d_tmp};
+    slab_rows_free(w, s);
+    void *frees[] = {d_idx, d_normal, d_var, d_cnormal, d_cvar, d_est};
     for (void *p : frees) pool_free(p, s);
     for (auto &e : marks) if (e) cudaEventDestroy(e);
     cudaStreamSynchronize(s);

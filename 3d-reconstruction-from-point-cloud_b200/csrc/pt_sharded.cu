@@ -23,6 +23,10 @@
 //             own records with the ghost-zone check on those rows, and the host scatters the
 //             results into the caller's point order.  A store reaches every copy of a point (the
 //             live slab indexes, and the records of every later rebuild).
+//   orient  : pt_index_orient_normals on the sharded cloud (DESIGN.md section 8, "Sharded normal
+//             orientation"): every slab builds the edges of the points it owns and the minimum
+//             spanning forest of its intra-slab edges on its own device; the home device joins
+//             those forests and the cross-slab edges into the global forest and orients from it.
 //
 // The reference has no multi-GPU path (its query loop is src/pointsTransfer.cpp:465-479); the
 // torch.distributed / NCCL form of the same sharding (one process per GPU, unsorted samples
@@ -72,8 +76,9 @@ struct pt_sharded {
     double halo_auto = 0.0;           // the bounding-box estimate (4x the expected k-th neighbour distance)
     int coord_mode = PT_COORD_AUTO;
     int rebuilds = 0;
-    // the normals pt_sharded_estimate_normals stored, n x 3 in point order (x NaN: none, the point
-    // keeps its input normal); empty until the first store.  build_slabs puts them in the records.
+    // the normals pt_sharded_estimate_normals / pt_sharded_orient_normals stored, n x 3 in point
+    // order (x NaN: none, the point keeps its input normal); empty until the first store.
+    // build_slabs puts them in the records.
     std::vector<float> stored;
 };
 
@@ -87,6 +92,13 @@ void free_slabs(pt_sharded *S)
         std::vector<int32_t>().swap(s.ids);
         std::vector<uint8_t>().swap(s.own);
     }
+}
+
+// The normal point i's records hold where it is stored, else null: its input normal
+const float *stored_normal(const pt_sharded *S, size_t i)
+{
+    const float *m = S->stored.empty() ? nullptr : &S->stored[3 * i];
+    return m && m[0] == m[0] ? m : nullptr;
 }
 
 // (re)builds every slab index for the current halo
@@ -149,8 +161,8 @@ int build_slabs(pt_sharded *S)
                     ids.push_back((int32_t)i);
                     own.push_back(owner[i] == r ? 1 : 0);
                     // a stored normal, widened: the build narrows it back to the same float
-                    const float *m = S->stored.empty() ? nullptr : &S->stored[3 * i];
-                    if (m && m[0] == m[0])
+                    const float *m = stored_normal(S, i);
+                    if (m)
                         for (int a = 0; a < 3; ++a) rec.back().normal[a] = (double)m[a];
                 }
             }
@@ -490,6 +502,38 @@ int sharded_bake(pt_sharded *S, const void *vertices, size_t n_vertices, const i
     return rc;
 }
 
+// f(r) for r = 0 .. R - 1, one host thread each (one per slab): the first error, else PT_OK
+int on_threads(int R, const std::function<int(int)> &f)
+{
+    std::vector<int> status(R, PT_OK);
+    std::vector<std::thread> th;
+    auto work = [&](int r) {
+        try {
+            status[r] = f(r);
+        } catch (...) { status[r] = PT_ERR_OUT_OF_MEMORY; }
+    };
+    for (int r = 0; r < R; ++r) {
+        try { th.emplace_back(work, r); } catch (...) { work(r); }
+    }
+    for (auto &t : th) t.join();
+    for (int r = 0; r < R; ++r)
+        if (status[r] != PT_OK) return status[r];
+    return (int)PT_OK;
+}
+
+// every copy of every point, own and ghost, takes the stored normals
+int store_slabs(pt_sharded *S)
+{
+    return on_threads((int)S->slabs.size(), [&](int r) {
+        const Slab &sl = S->slabs[r];
+        if (sl.ids.empty()) return (int)PT_OK;                         // a slab without records
+        std::vector<float> values(3 * sl.ids.size());
+        for (size_t l = 0; l < sl.ids.size(); ++l)
+            memcpy(&values[3 * l], &S->stored[3 * (size_t)sl.ids[l]], sizeof(float) * 3);
+        return pt::normals_store(sl.index, values.data());
+    });
+}
+
 // pt_index_estimate_normals on the sharded cloud; arguments checked, S->n > 0.
 int sharded_normals(pt_sharded *S, int k, double radius, const double *viewpoint, bool store, float *normal_out,
                     float *variation_out, pt_normals_stats *stats)
@@ -499,28 +543,12 @@ int sharded_normals(pt_sharded *S, int k, double radius, const double *viewpoint
     std::vector<std::vector<float>> nrm(R), var(R);
     std::vector<unsigned long long> est(R, 0);
     std::vector<float> pca(R, 0.0f);
-    auto each_slab = [&](const std::function<int(int)> &f) {
-        std::vector<int> status(R, PT_OK);
-        std::vector<std::thread> th;
-        auto work = [&](int r) {
-            try {
-                status[r] = f(r);
-            } catch (...) { status[r] = PT_ERR_OUT_OF_MEMORY; }
-        };
-        for (int r = 0; r < R; ++r) {
-            try { th.emplace_back(work, r); } catch (...) { work(r); }
-        }
-        for (auto &t : th) t.join();
-        for (int r = 0; r < R; ++r)
-            if (status[r] != PT_OK) return status[r];
-        return (int)PT_OK;
-    };
     // every slab estimates its own points; nothing reaches the caller or the slabs before all pass
     int rc = PT_OK;
     bool done = false;
     for (int attempt = 0; attempt < ATTEMPTS && !done; ++attempt) {
         std::vector<int> needs(R, 0);
-        rc = each_slab([&](int r) {
+        rc = on_threads(R, [&](int r) {
             const Slab &sl = S->slabs[r];
             est[r] = 0;
             pca[r] = 0.0f;
@@ -544,7 +572,7 @@ int sharded_normals(pt_sharded *S, int k, double radius, const double *viewpoint
     // each slab's own results come in ascending local id: the i-th goes to the global id of the
     // slab's i-th own record.  Ranges of records over a share of the host's cores.
     const size_t share = std::max(1u, std::thread::hardware_concurrency() / (unsigned)R);
-    rc = each_slab([&](int r) {
+    rc = on_threads(R, [&](int r) {
         const Slab &sl = S->slabs[r];
         if (sl.n_own == 0) return (int)PT_OK;
         const float *nr = nrm[r].data(), *vr = var[r].data();
@@ -573,16 +601,7 @@ int sharded_normals(pt_sharded *S, int k, double radius, const double *viewpoint
         for (auto &t : th) t.join();
         return (int)PT_OK;
     });
-    // every copy of every point, own and ghost, takes the stored normals
-    if (rc == PT_OK && store)
-        rc = each_slab([&](int r) {
-            const Slab &sl = S->slabs[r];
-            if (sl.ids.empty()) return (int)PT_OK;                         // a slab without records
-            std::vector<float> values(3 * sl.ids.size());
-            for (size_t l = 0; l < sl.ids.size(); ++l)
-                memcpy(&values[3 * l], &S->stored[3 * (size_t)sl.ids[l]], sizeof(float) * 3);
-            return pt::normals_store(sl.index, values.data());
-        });
+    if (rc == PT_OK && store) rc = store_slabs(S);
     if (rc != PT_OK) return rc;
     if (stats) {
         stats->knn_ms = std::chrono::duration<float, std::milli>(std::chrono::steady_clock::now() - t0).count();
@@ -592,6 +611,90 @@ int sharded_normals(pt_sharded *S, int k, double radius, const double *viewpoint
             stats->estimated += est[r];
             stats->pca_ms += pca[r];
         }
+    }
+    return PT_OK;
+}
+
+// pt_index_orient_normals on the sharded cloud (DESIGN.md section 8, "Sharded normal orientation");
+// arguments checked, S->n > 0.
+int sharded_orient(pt_sharded *S, int k, double radius, const double *viewpoint, bool store, float *normal_out,
+                   int32_t *root_out, pt_orient_stats *stats)
+{
+    const int R = (int)S->slabs.size();
+    const size_t n = S->n;
+    const auto t0 = std::chrono::steady_clock::now();
+    std::vector<std::vector<pt::OrientEdge>> forest(R), cross(R);
+    std::vector<uint64_t> intra(R, 0);
+    // every slab: its own rows' lists, edges and intra-slab forest; nothing reaches the caller or the
+    // slabs before all pass their ghost checks
+    int rc = PT_OK;
+    bool done = false;
+    for (int attempt = 0; attempt < ATTEMPTS && !done; ++attempt) {
+        std::vector<int> needs(R, 0);
+        rc = on_threads(R, [&](int r) {
+            const Slab &sl = S->slabs[r];
+            forest[r].clear();
+            cross[r].clear();
+            intra[r] = 0;
+            if (!sl.index) return (int)PT_ERR_INVALID_ARG;
+            if (sl.n_own == 0) return (int)PT_OK;
+            const pt::NormalsSlab job{S->cuts.data() + 1, R, r, sl.n_own, S->boxes.data(), S->halo, !holds_cloud(S, sl)};
+            return pt::orient_slab(sl.index, k, radius, job, forest[r], cross[r], &intra[r], &needs[r]);
+        });
+        if (rc != PT_OK) return rc;
+        done = std::none_of(needs.begin(), needs.end(), [](int v) { return v != 0; });
+        if (done || attempt + 1 == ATTEMPTS) break;
+        // some k-th-neighbour ball may leave a ghost zone: widen it and run the stage again
+        if ((rc = widen_and_rebuild(S, attempt)) != PT_OK) return rc;
+    }
+    if (!done) return PT_ERR_UNSUPPORTED;                     // a guard, as in sharded_query
+    const auto t1 = std::chrono::steady_clock::now();
+    // the home device's inputs in point order: the normals the records were built from (the device
+    // narrows them as the build does), and the caller's z (with a viewpoint, the whole position)
+    const int home = S->slabs[0].device;
+    const size_t dims = viewpoint ? 3 : 1;
+    std::vector<double> normal(3 * n);
+    std::vector<float> nrm_tmp(normal_out ? 0 : 3 * n);
+    std::vector<double> pos(dims * n);
+    std::vector<int32_t> root_tmp(root_out ? 0 : n);
+    float *nrm = normal_out ? normal_out : nrm_tmp.data();
+    int32_t *root = root_out ? root_out : root_tmp.data();
+    const Rec80 *P = S->points;
+    const size_t parts = std::max(1u, std::thread::hardware_concurrency()), step = (n + parts - 1) / parts;
+    on_threads((int)parts, [&](int p) {
+        for (size_t i = p * step; i < std::min(n, (p + 1) * step); ++i) {
+            const float *m = stored_normal(S, i);
+            for (int a = 0; a < 3; ++a) normal[3 * i + a] = m ? (double)m[a] : P[i].normal[a];
+            for (size_t a = 0; a < dims; ++a) pos[dims * i + a] = P[i].ver[3 - dims + a];
+        }
+        return (int)PT_OK;
+    });
+    unsigned long long counts[3] = {0, 0, 0};
+    uint64_t unique_cross = 0;
+    {
+        PT_CUDA(cudaSetDevice(home));
+        cudaStream_t s = nullptr;
+        PT_CUDA(cudaStreamCreateWithFlags(&s, cudaStreamNonBlocking));
+        const pt::OrientHome h{n, normal.data(), pos.data(), viewpoint, nrm, root};
+        rc = pt::orient_home(h, forest, cross, &unique_cross, counts, s);
+        cudaStreamDestroy(s);
+        if (rc != PT_OK) return rc;
+    }
+    // the oriented normals of the points that take part (root >= 0) into every copy of them
+    if (store) {
+        if (S->stored.empty()) S->stored.assign(3 * n, NAN);
+        for (size_t i = 0; i < n; ++i)
+            if (root[i] >= 0) memcpy(&S->stored[3 * i], nrm + 3 * i, sizeof(float) * 3);
+        if ((rc = store_slabs(S)) != PT_OK) return rc;
+    }
+    if (stats) {
+        stats->oriented = counts[0];
+        stats->flipped = counts[1];
+        stats->components = counts[2];
+        stats->edges = unique_cross;
+        for (int r = 0; r < R; ++r) stats->edges += intra[r];
+        stats->knn_ms = std::chrono::duration<float, std::milli>(t1 - t0).count();
+        stats->mst_ms = std::chrono::duration<float, std::milli>(std::chrono::steady_clock::now() - t1).count();
     }
     return PT_OK;
 }
@@ -719,6 +822,20 @@ int pt_sharded_estimate_normals(pt_sharded *S, int k, double radius, const doubl
     if (S->n == 0) return PT_OK;
     try {
         return sharded_normals(S, k, radius, viewpoint, store != 0, normal_out, variation_out, stats);
+    } catch (...) { return PT_ERR_OUT_OF_MEMORY; }
+}
+
+int pt_sharded_orient_normals(pt_sharded *S, int k, double radius, const double *viewpoint, int store,
+                              float *normal_out, int32_t *root_out, pt_orient_stats *stats)
+{
+    if (!S) return PT_ERR_INVALID_ARG;
+    const int rc = pt::orient_check_args(k, viewpoint, store != 0, normal_out || root_out);
+    if (rc != PT_OK) return rc;
+    if (pt_device_count() == 0) return PT_ERR_NO_DEVICE;
+    if (stats) *stats = pt_orient_stats{0, 0, 0, 0, 0.0f, 0.0f};
+    if (S->n == 0) return PT_OK;
+    try {
+        return sharded_orient(S, k, radius, viewpoint, store != 0, normal_out, root_out, stats);
     } catch (...) { return PT_ERR_OUT_OF_MEMORY; }
 }
 

@@ -537,6 +537,32 @@ int pt_sharded_bake(pt_sharded *sharded, const void *vertices, size_t n_vertices
 int pt_sharded_estimate_normals(pt_sharded *sharded, int k, double radius,
                                 const double *viewpoint /* 3 or NULL */, int store, float *normal_out,
                                 float *variation_out, pt_normals_stats *stats);
+/* pt_index_orient_normals on the sharded cloud (DESIGN.md section 8, "Sharded normal orientation"):
+ * same arguments, argument rules and error codes (a NULL handle: PT_ERR_INVALID_ARG), and
+ * normal_out (n x 3) and root_out (n, global ids), in the order of the caller's `points`, are
+ * byte-identical to pt_index_orient_normals on one pt_index built from the same cloud, as are
+ * stats->oriented, flipped, components and edges, for any slab count, device list, halo and
+ * coordinate mode.  A point takes part when the normal its records hold (the stored one, else its
+ * input normal) is usable.  Every slab builds the edges of the points it owns and the minimum
+ * spanning forest of the edges between them on its own device, with the ghost-zone check on its
+ * own rows; a ghost zone found too narrow widens the halo and rebuilds the slabs as
+ * pt_sharded_transfer does (counted in `rebuilds`).  Slab 0's device (the home device) joins those
+ * forests and the edges between slabs into the cloud's forest and orients every component from
+ * its root.  One difference from the single index: the n * k <= INT32_MAX limit applies to each
+ * slab's records (own and ghost) times k, not to the whole cloud, so a cloud too large for one
+ * index can be oriented; a slab over it is PT_ERR_UNSUPPORTED.  A cloud within the single index's
+ * limit is within every slab's.  store != 0 as in pt_sharded_estimate_normals: the oriented normal
+ * of every point that takes part replaces its normal in every slab that holds it, and the handle
+ * keeps it for rebuilt slabs.  Nothing is written or stored before every slab has passed its check.
+ * Stats:
+ *   knn_ms     host wall time of the slab stage: self-queries, ghost checks, edges and the slabs'
+ *              forests, rebuilds included, ending in a synchronise
+ *   mst_ms     host wall time of the rest: the copies to the home device, the cloud's forest,
+ *              roots, signs, the outputs and the store */
+int pt_sharded_orient_normals(pt_sharded *sharded, int k, double radius,
+                              const double *viewpoint /* 3 or NULL */, int store,
+                              float *normal_out /* n*3 */, int32_t *root_out /* n */,
+                              pt_orient_stats *stats);
 
 /* pt_texture_render for neighbour lists that were computed elsewhere (e.g. pt_sharded_knn): the
  * cloud's positions and colours are uploaded to `device` in original order, idx[n_vertices * k]
